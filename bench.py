@@ -2,7 +2,7 @@
 """bench.py — events/s of the EventCalib hot path (detection: ingest -> windows -> DBSCAN -> circle fit; residual
 evaluation: association -> J^T J / J^T r -> cost) on the BASELINE.json configurations.
 
-    python bench.py [--config C2|C3|C4|C5] --gpus N --steps K --warmup W [--impl reference] [--events E]
+    python bench.py [--config C2|C3|C4|C5] --gpus N --steps K --warmup W [--impl reference] [--events E] [--dump-outputs DIR]
 
   C2 (default; the configuration BASELINE.json's metric is quoted on): per GPU a synthetic 20 M-event DAVIS346 (346x260)
      circle-grid stream, 2 Mev/s, tiling windows of 1.5 ms (= 3 x MotionTimeStep), DBSCAN eps 4 / minPts 2, cluster filter,
@@ -14,9 +14,9 @@ evaluation: association -> J^T J / J^T r -> cost) on the BASELINE.json configura
   C4 the full dynamic calibration: a FIXED residual set (the C2 stream cut to --events, default 7 M), knots every 25 ms,
      exactly 50 LM iterations (normal equations + inter-GPU sum + solve + cost of the candidate), residuals sharded over
      the N GPUs (strong scaling).
-One "step" = one pass of the hot path over the per-GPU stream (C4: one LM iteration).  N > 1: windows are independent, so
-rank r holds the r-th slice of a longer stream (weak scaling, no data-path collective); value = all events of all ranks /
-max-over-ranks device time.
+One "step" = one pass of the hot path over the per-GPU stream (C4: one run of the LM loop, --lm-iters iterations).
+N > 1: windows are independent, so rank r holds the r-th slice of a longer stream (weak scaling, no data-path collective);
+value = all events of all ranks / max-over-ranks device time.
 
   value    device-resident: the packed 25-byte records are already in HBM when the timed region starts
   e2e      through the C ABI with HOST buffers: pinned-host records -> H2D -> front end -> D2H of the per-window
@@ -26,6 +26,13 @@ max-over-ranks device time.
            candidate pairs exact, circle centres and radii 1e-9 relative, residual count exact and cost 1e-9 relative.
            Any mismatch makes the run fail (exit code 1) after the line is printed.
   roofline / cpu_baseline / clocks: see DESIGN.md §Measurement.
+
+--dump-outputs DIR writes, after the timed steps, what the last timed step computed (rank 0) as DIR/<name>.npy in float64:
+per-window summaries, candidate circles, the clustered points with their labels and, with the residual evaluation, the
+packed normal equations, the cost and the residual count (C4: the LM result).  A sweep leaves the outputs of its last
+point.  The files stay under 64 MB: a larger array is cut to a fixed seeded sample of its rows, whose indices go to
+DIR/<name>_rows.npy.  The inputs are generated from fixed seeds, so two builds run with the same arguments can be compared
+file by file.
 """
 import argparse
 import json
@@ -71,6 +78,37 @@ def peaks():
         except Exception:
             pass
     return 6650.0, "fallback (B200_PROFILING.md)"
+
+
+DUMP_BYTES = 60 << 20   # array bytes of --dump-outputs: under 64 MB with the .npy headers
+
+
+def dump_outputs(dirname, arrays, large=()):
+    """Writes every array as dirname/<name>.npy in float64.  The arrays named in `large` share what DUMP_BYTES leaves
+    after the others; one that exceeds its share keeps a seeded sample of its rows (first axis), indices in <name>_rows.npy."""
+    out = {k: np.asarray(v, np.float64) for k, v in arrays.items()}
+    share = (DUMP_BYTES - sum(v.nbytes for k, v in out.items() if k not in large)) // max(1, len(large))
+    for k in large:
+        a = out[k]
+        if a.nbytes > share:
+            m = int(share // (a.nbytes // len(a) + 8))
+            rows = np.sort(np.random.default_rng(0).choice(len(a), m, replace=False))
+            out[k], out[k + "_rows"] = a[rows], rows.astype(np.float64)
+    assert sum(v.nbytes for v in out.values()) <= DUMP_BYTES
+    os.makedirs(dirname, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(dirname, k + ".npy"), v)
+
+
+def frontend_outputs(ctx):
+    """What a caller reads back after ecb_frontend_run: per-window summaries, candidate circles, points + labels."""
+    s = ctx.summary()
+    out = {"window_" + f: s[f] for f in s.dtype.names}
+    out["candidates"] = ctx.candidates(max(1, int(s["n_candidates"].max())) if len(s) else 1)
+    for pol in (0, 1):
+        xy, lab = ctx.points(pol)
+        out["points_xy_label_pol%d" % pol] = np.concatenate([xy, lab[:, None]], axis=1)
+    return out
 
 
 def make_workload(cfg, n_events, rank):
@@ -403,11 +441,13 @@ def run_c4(args, cfg, rank, world, local):
         run_once()
     sampler = ClockSampler(local) if rank == 0 else None
     l0 = ctx.launches
-    runs = [run_once() for _ in range(max(1, min(args.steps, 3)))]
+    runs = [run_once() for _ in range(args.steps)]
     launches = (ctx.launches - l0) // len(runs)
     clocks = sampler.stop() if sampler else None
     ms = float(np.mean([r[0] for r in runs]))
     summ = runs[-1][1]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {k: v for k, v in summ.items() if k != "reserved"})
     tot_res = n_res
     if world > 1:
         t = torch.tensor([float(n_res)], device="cuda", dtype=torch.float64)
@@ -435,8 +475,8 @@ def run_c4(args, cfg, rank, world, local):
         it = summ["iterations"]
         unit = "residuals x LM iterations / s"
         value = tot_res * it / (ms * 1e-3)
-        line = {"metric": METRIC, "value": value, "unit": unit, "n_gpus": world, "steps": it, "warmup": args.warmup,
-                "ms_per_step": ms / max(it, 1), "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "dtype": "f64",
+        line = {"metric": METRIC, "value": value, "unit": unit, "n_gpus": world, "steps": args.steps, "warmup": args.warmup,
+                "ms_per_step": ms, "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "dtype": "f64",
                 "data": "synthetic",
                 "config": {"workload": "C4: full dynamic calibration on a fixed problem — %d residual blocks from a %d-event DAVIS346 "
                                        "stream, %d control points (knots every 25 ms, D = %d), intrinsics +2 %%, exactly %d LM iterations "
@@ -514,7 +554,12 @@ def main():
     ap.add_argument("--median-mode", type=int, default=1, help="cluster centre: 0 canonical, 1 std::nth_element over BFS order (the reference's)")
     ap.add_argument("--slice-plan", default="", help="relative sizes of the e2e time slices, e.g. 1,2,3,3,2,1 (overrides --slices)")
     ap.add_argument("--lm-iters", type=int, default=0, help="LM iterations of C4 (default 50)")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR", help="write the outputs of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs records the GPU path (--impl ours)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     cfg = CONFIGS[args.config]
     if args.events <= 0:
@@ -600,6 +645,7 @@ def main():
     # outside the hot path); rank r owns segment r (EventCalibSpline splits the map into segments at gaps,
     # EventCalibSpline.cpp:319-348); every rank knows all segments, holds only its own residuals
     do_res = cfg["residual"]
+    last = {}   # scalars the last device-resident step returned (--dump-outputs)
     n_res, segs, mine, xch, xch_check = 0, None, None, None, None
     rot = np.zeros((0, 4))
     if do_res:
@@ -648,10 +694,10 @@ def main():
             the fused exchange) + the cost-only evaluation of this rank's residuals"""
             # device-resident step: the key-frame tables are inputs like the records and lie in HBM (ecb_cost_associate_device);
             # the end-to-end step below uploads them from host arrays inside the timed region
-            ctx.cost_associate_device(d_kf_t.data_ptr(), d_kf_c.data_ptr(), len(mine["kf_t"]), mine["circles"].shape[1],
-                                      d_lm.data_ptr(), mine["step"])
+            last["n_residuals"] = ctx.cost_associate_device(d_kf_t.data_ptr(), d_kf_c.data_ptr(), len(mine["kf_t"]),
+                                                            mine["circles"].shape[1], d_lm.data_ptr(), mine["step"])
             normal_eq_all_ranks(intr, rot, trans)
-            ctx.cost_eval(intr, rot, trans)
+            last["cost"] = ctx.cost_eval(intr, rot, trans)
 
     def step_device():
         ctx.load_events_device(d_raw.data_ptr(), n)
@@ -769,6 +815,11 @@ def main():
     ms = timed(step_device, args.steps)
     launches = ctx.launches - l0
     value = world * n_pass * args.steps / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        outs = frontend_outputs(ctx)
+        if do_res:
+            outs.update(last, normal_eq=d_ne.cpu().numpy())
+        dump_outputs(args.dump_outputs, outs, large=("candidates", "points_xy_label_pol0", "points_xy_label_pol1"))
 
     # per-kernel durations, measured live with CUDA events on the launching stream (separate pass; the front-end stages
     # of a sweep are those of its last point)

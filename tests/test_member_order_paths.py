@@ -12,6 +12,7 @@ against the UNMODIFIED reference DBSCAN (oracle/_ref: dbscan.h + kdtree.cpp comp
 This is pure Python over the same integer decisions the kernel takes (floor(eps^2), ceil(eps)); the CUDA kernel itself is
 compared with the reference in tests/test_gpu_frontend.py and tests/test_gpu_golden.py."""
 import math
+import os
 
 import numpy as np
 import pytest
@@ -117,4 +118,23 @@ def test_member_order_from_root_paths(oracle_mod, kind, eps):
                 continue
             assert _member_order(P, members, eps) == [int(m) for m in members]
             checked += 1
+    assert checked >= 6
+
+
+def test_member_order_of_the_stored_reference_clusters():
+    """The same restatement against the member lists the unmodified reference DBSCAN returned, as stored in
+    tests/golden/dbscan_reference.npz (tests/golden/make_golden.py): runs where the reference itself is absent."""
+    g =np.load(os.path.join(os.path.dirname(__file__), "golden", "dbscan_reference.npz"))
+    checked = 0
+    for k in range(int(g["n_cases"])):
+        eps, mp = (float(v) for v in g["par_%d" % k])
+        if mp != 2:
+            continue
+        P = [tuple(p) for p in g["pts_%d" % k].astype(float).tolist()]
+        off = np.concatenate([[0], np.cumsum(g["sizes_%d" % k])])
+        for c in range(len(off) - 1):
+            members = [int(m) for m in g["members_%d" % k][off[c]:off[c + 1]]]
+            if len(members) >= 3:
+                assert _member_order(P, members, eps) == members, "case %d cluster %d" % (k, c)
+                checked += 1
     assert checked >= 6
