@@ -49,6 +49,11 @@ class WindowSummary(C.Structure):
                 ("point_offset", C.c_int64 * 2)]
 
 
+class CovarianceSummary(C.Structure):
+    _fields_ = [("cost", C.c_double), ("sigma2", C.c_double), ("min_relative_pivot", C.c_double), ("n_residuals", C.c_int64),
+                ("dimension", C.c_int32), ("deficient_index", C.c_int32)]
+
+
 SUMMARY_DTYPE = np.dtype([("ev_lo", "<i8"), ("ev_hi", "<i8"), ("n_points", "<i4", 2), ("n_clusters", "<i4", 2),
                           ("n_kept", "<i4", 2), ("n_candidates", "<i4"), ("status", "<u4"), ("point_offset", "<i8", 2)])
 assert SUMMARY_DTYPE.itemsize == C.sizeof(WindowSummary)
@@ -66,7 +71,7 @@ SYMBOLS = ["ecb_ctx_create", "ecb_ctx_destroy", "ecb_last_error", "ecb_launch_co
            "ecb_lm_destroy", "ecb_lm_dimension", "ecb_lm_begin", "ecb_lm_propose", "ecb_lm_feedback", "ecb_lm_update",
            "ecb_lm_state", "ecb_lm_trace", "ecb_calibrate", "ecb_lm_device_create", "ecb_lm_device_destroy",
            "ecb_lm_device_set_exchange", "ecb_lm_device_begin", "ecb_lm_device_iterate", "ecb_lm_device_running",
-           "ecb_lm_device_result", "ecb_calibrate_device"]
+           "ecb_lm_device_result", "ecb_calibrate_device", "ecb_covariance"]
 
 _lib = None
 
@@ -153,6 +158,7 @@ def load_library():
     lib.ecb_lm_device_running.argtypes = [vp]
     lib.ecb_lm_device_result.argtypes = [vp, vp, vp, vp, C.POINTER(LmSummary), vp, i32]
     lib.ecb_calibrate_device.argtypes = [vp, vp, vp, vp, C.POINTER(LmSummary), vp, i32]
+    lib.ecb_covariance.argtypes = [vp, i32, vp, vp, vp, vp, vp, i64, vp, vp, vp, C.POINTER(CovarianceSummary)]
     _lib = lib
     return lib
 
@@ -500,6 +506,40 @@ class Context:
                                          C.byref(summ), _ptr(tr), trace_rows))
         rows = int(np.count_nonzero(tr[:, 2]))
         return intr, rot, trans, {f[0]: getattr(summ, f[0]) for f in LmSummary._fields_}, tr[:rows]
+
+    def covariance(self, n_cp, intr, rot, trans, d_packed=None, n_residuals_total=0):
+        """Covariance Z = H^-1 of the parameters at x (ecb_covariance): the selected inverse on the band / arrow pattern.
+        Returns a dict: ok, cov_intrinsics [9,9], cov_band [6C,24] (Z(j+r, j) at [j, r]), cov_cross [9,6C], cost, sigma2,
+        min_relative_pivot, n_residuals, dimension, deficient_index and std_intrinsics = sqrt(sigma2 diag Z_cc).  A rank-deficient
+        system gives ok=False, the index of the failing pivot and no arrays.  d_packed: device pointer of an already-summed packed
+        buffer (several GPUs); n_residuals_total: residual count over all ranks (0: this context's).  control_point_covariance()
+        takes the 6 x 6 block of one control point out of the result."""
+        n_cp = np.ascontiguousarray(np.atleast_1d(n_cp), np.int32)
+        a = [np.ascontiguousarray(v, np.float64) for v in (intr, rot, trans)]
+        n = 6 * int(n_cp.sum())
+        zc, zb, zx = np.zeros((9, 9)), np.zeros((n, 24)), np.zeros((9, n))
+        s = CovarianceSummary()
+        rc = self.lib.ecb_covariance(self.h, len(n_cp), _ptr(n_cp), _ptr(a[0]), _ptr(a[1]), _ptr(a[2]),
+                                     C.c_void_p(d_packed) if d_packed else None, int(n_residuals_total), _ptr(zc), _ptr(zb),
+                                     _ptr(zx), C.byref(s))
+        if rc != FAILED:
+            self._chk(rc)
+        out = {f[0]: getattr(s, f[0]) for f in CovarianceSummary._fields_}
+        out["ok"] = rc == OK
+        if rc == OK:
+            out.update(cov_intrinsics=zc, cov_band=zb, cov_cross=zx, std_intrinsics=np.sqrt(s.sigma2 * np.diag(zc)))
+        return out
+
+
+def control_point_covariance(cov, c):
+    """6 x 6 block Z of control point c (rotation tangent 3, translation 3) from the band of Context.covariance()"""
+    band = cov["cov_band"]
+    out = np.empty((6, 6))
+    for a in range(6):
+        for b in range(6):
+            lo, hi = min(a, b), max(a, b)
+            out[a, b] = band[6 * c + lo, hi - lo]
+    return out
 
 
 def lm_options(**kw):

@@ -170,11 +170,13 @@ int ecb_ctx_create(int device, void *stream, ecb_ctx **out) {
 }
 
 void ecb_cost_free(ecb_ctx *ctx);
+void ecb_covariance_free(ecb_ctx *ctx);
 
 void ecb_ctx_destroy(ecb_ctx *c) {
     if (!c) return;
     cudaSetDevice(c->device);
     cudaStreamSynchronize(c->stream);
+    ecb_covariance_free(c);
     ecb_cost_free(c);
     DevBuf *bufs[] = {&c->ev_raw, &c->ev_t, &c->ev_xyp, &c->ev_flag, &c->win_t, &c->win_lohi, &c->win_ptoff, &c->summary,
                       &c->arrive, &c->pts[0], &c->pts[1], &c->labels[0], &c->labels[1], &c->scratch, &c->ktab, &c->kmem,

@@ -71,6 +71,8 @@ struct ecb_ctx {
     size_t up_cap = 0, up_off = 0;
     // cost evaluation (ecb_cost.cu)
     void *cost = nullptr;
+    // covariance workspace (ecb_lmdev.cu), kept for repeated calls with the same spline layout
+    void *cov = nullptr;
 };
 
 int ecb_fail(ecb_ctx *ctx, int code, const char *fmt, ...);

@@ -27,6 +27,7 @@
 #include <string.h>
 
 #include <algorithm>
+#include <climits>
 #include <vector>
 
 #include "ecb_common.cuh"
@@ -71,6 +72,7 @@ struct LmBufs {
     double *Lb, *La, *Cc0, *dC, *Lc, *xi, *ysol;  // factorisation workspace (Lc: 1 / L(j, j) of the band)
     double *trace;
     LmScalars *s;
+    double *Lcc;                      // k_lm_corner stores its 9 x 9 factor here when set (the covariance; NULL in the LM)
 };
 
 __device__ __forceinline__ void record(LmScalars *s, double *trace, double accepted) {
@@ -462,6 +464,9 @@ __global__ void k_lm_corner(LmDims d, LmBufs b) {
                 Cw[r][c] = v / Cw[c][c];
             }
         }
+    if (b.Lcc)  // a failed row keeps its non-positive pivot, later rows their partial Schur complement
+        for (int r = 0; r < NI; ++r)
+            for (int c = 0; c <= r; ++c) b.Lcc[r * NI + c] = Cw[r][c];
     if (!ok) {
         s->factor_fail = 1;
         return;
@@ -705,6 +710,197 @@ __global__ void k_lm_epoch(const int *go, unsigned long long *epoch) {
 }
 
 __global__ void k_lm_set_cost(LmBufs b, const double *v) { b.s->candidate_cost = *v; }
+
+// ---- covariance of the parameters: Z = H^-1 on the band / arrow pattern (selected inversion) -----------------------------------
+// ecb_covariance runs k_lm_assemble, k_lm_build, k_lm_factor and k_lm_corner unchanged on M = S H S with S = diag(H)^-1/2 (1 where
+// the diagonal is 0) and no damping (radius = +inf: the damping term dg / radius adds exactly 0), then the kernels below.
+constexpr double COV_MIN_PIVOT = 1e-12;  // relative pivot L(j, j)^2 / M(j, j) at or below which the system counts as rank deficient
+constexpr int COV_THREADS = 256;
+constexpr int CW = NB - 1 + NI;          // selected-inversion window: 23 band rows + 9 intrinsics = 32
+
+struct CovBufs {
+    double *Zb, *Zx, *Zc;  // outputs, unscaled: band (column major like Hb), cross 9 x n, corner 9 x 9
+    double *Zcs, *Lcc;     // scaled corner of Z, corner factor of k_lm_corner
+    double *res;           // cost, min relative pivot, first deficient index (-1: none)
+};
+
+// Jacobi equilibration to a unit diagonal and the state the LM kernels read
+__global__ void k_cov_begin(LmDims d, LmBufs b) {
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < d.D; i += gridDim.x * blockDim.x) {
+        const double h = h_diag(d, b, i);
+        b.scale[i] = h > 0.0 ? 1.0 / sqrt(h) : 1.0;
+        if (i < d.n) b.Lc[i] = 0.0;  // a pivot the factorisation does not reach (it stops a segment at a failed pivot) stays 0
+    }
+    if (blockIdx.x == 0 && threadIdx.x == 0) {
+        LmScalars *s = b.s;
+        s->running = 1;
+        s->radius = INFINITY;
+        s->reuse_diagonal = 0;
+        s->factor_fail = 0;
+    }
+}
+
+// relative pivots of the factorisation: their minimum and the first index j with L(j, j)^2 / M(j, j) <= COV_MIN_PIVOT (or a
+// failed pivot); the band comes first in the factorisation, so a band failure is reported before the intrinsics
+__global__ void __launch_bounds__(1024) k_cov_pivots(LmDims d, LmBufs b, CovBufs c) {
+    __shared__ double smin[1024];
+    __shared__ int sbad[1024];
+    const int tid = threadIdx.x;
+    double mn = INFINITY;
+    int bad = INT_MAX;
+    for (int i = tid; i < d.D; i += blockDim.x) {
+        double rel;
+        if (i < d.n) {
+            const double rc = b.Lc[i], m = b.Hb[(size_t) i * NB] * b.scale[i] * b.scale[i];
+            if (rc == 0.0) continue;  // behind a failed pivot of the same segment
+            rel = (isfinite(rc) && m > 0.0) ? 1.0 / (rc * rc * m) : 0.0;
+        } else {
+            const int r = i - d.n;
+            const double l = c.Lcc[r * NI + r], m = b.Cc0[r * NA + r];
+            rel = (l > 0.0 && m > 0.0) ? l * l / m : 0.0;
+        }
+        mn = fmin(mn, rel);
+        if (!(rel > COV_MIN_PIVOT)) bad = min(bad, i);
+    }
+    smin[tid] = mn;
+    sbad[tid] = bad;
+    __syncthreads();
+    for (int st = 512; st > 0; st >>= 1) {
+        if (tid < st) {
+            smin[tid] = fmin(smin[tid], smin[tid + st]);
+            sbad[tid] = min(sbad[tid], sbad[tid + st]);
+        }
+        __syncthreads();
+    }
+    if (tid == 0) {
+        c.res[0] = b.s->cost;
+        c.res[1] = smin[0];
+        c.res[2] = sbad[0] == INT_MAX ? -1.0 : (double) sbad[0];
+    }
+}
+
+// Z_cc = (L_cc L_cc^T)^-1 of the 9 x 9 Schur factor: W = L_cc^-1 column by column (one thread each), Z_cc = W^T W
+__global__ void k_cov_corner(LmDims d, LmBufs b, CovBufs c) {
+    __shared__ double W[NI][NI];
+    if (c.res[2] >= 0.0) return;
+    const int t = threadIdx.x;
+    if (t < NI) {
+        for (int r = 0; r < NI; ++r) {
+            double v = r == t ? 1.0 : 0.0;
+            for (int k = t; k < r; ++k) v -= c.Lcc[r * NI + k] * W[k][t];
+            W[r][t] = r < t ? 0.0 : v / c.Lcc[r * NI + r];
+        }
+    }
+    __syncthreads();
+    if (t < NI * NI) {
+        const int r = t / NI, q = t % NI, lo = max(r, q);
+        double v = 0.0;
+        for (int k = lo; k < NI; ++k) v += W[k][r] * W[k][q];
+        c.Zcs[t] = v;
+        c.Zc[t] = v * (b.scale[d.n + min(r, q)] * b.scale[d.n + lo]);  // the same rounding for (r, q) and (q, r): symmetric
+    }
+}
+
+// Selected inversion (Takahashi) of one segment, blocked by control point like k_lm_factor.  With B the 6 columns of the block
+// and K the rows L couples to them (the next 18 band rows of the segment and the 9 intrinsics), Z L = L^-T gives
+//   Z_{R,B} = -Z_{R,K} T,   Z_BB = L_BB^-T L_BB^-1 - Z_{K,B}^T T,   T = L_KB L_BB^-1,
+// for R = the next 23 band rows + the intrinsics (the band reach of the block's last column).  Every Z_{R,K} lies in the
+// 32 x 32 window of Z the previous block left in shared memory; the window then slides up by one block.  The result equals the
+// scalar recurrence Z_ij = -(1 / L_jj) sum_{k in N(j)} Z_ik L_kj run column by column.  Outputs are unscaled by S on the way out.
+__global__ void __launch_bounds__(COV_THREADS) k_cov_selinv(LmDims d, LmBufs b, CovBufs c) {
+    __shared__ double Zw[2][CW * CW];  // window: index w < 23 -> band row j0 + 6 + w of the segment, w >= 23 -> intrinsic w - 23
+    __shared__ double LB[FB][FB], LK[NB - FB + NI][FB], T[NB - FB + NI][FB], Wb[FB][FB], Y[CW][FB], ZB[FB][FB], rdg[FB];
+    if (c.res[2] >= 0.0) return;
+    const int sg = blockIdx.x, tid = threadIdx.x, n = d.n;
+    const int js = 6 * d.seg_cp_off[sg], ns = 6 * d.seg_ncp[sg];
+    constexpr int NK = NB - FB + NI;   // 27 coupled rows: window indices 0..17 and 23..31
+    auto kwin = [](int q) { return q < NB - FB ? q : q + (NB - 1) - (NB - FB); };
+    for (int e = tid; e < CW * CW; e += COV_THREADS) {  // the last block's window: rows past the segment are 0, the corner is Z_cc
+        const int r = e / CW, q = e % CW;
+        Zw[0][e] = (r >= NB - 1 && q >= NB - 1) ? c.Zcs[(r - (NB - 1)) * NI + (q - (NB - 1))] : 0.0;
+    }
+    int cur = 0;
+    for (int j0 = ns - FB; j0 >= 0; j0 -= FB) {
+        const double *Zp = Zw[cur];
+        double *Zn = Zw[cur ^ 1];
+        const int g0 = js + j0;  // global index of the block's first column
+        // L of the block: L_BB (6 x 6 lower), L_KB (27 x 6), 1 / L(j, j)
+        if (tid < FB * FB) {
+            const int r = tid / FB, k = tid % FB;
+            LB[r][k] = r >= k ? b.Lb[(size_t) (g0 + k) * NB + (r - k)] : 0.0;
+            if (r == 0) rdg[k] = b.Lc[g0 + k];
+        } else if (tid < FB * FB + NK * FB) {
+            const int q = (tid - FB * FB) / FB, k = (tid - FB * FB) % FB;
+            LK[q][k] = q < NB - FB ? (j0 + FB + q < ns ? b.Lb[(size_t) (g0 + k) * NB + (FB + q - k)] : 0.0)
+                                   : b.La[(size_t) (q - (NB - FB)) * n + g0 + k];
+        }
+        __syncthreads();
+        if (tid < NK) {  // T row q: T_q L_BB = L_Kq, columns right to left
+            double t[FB];
+#pragma unroll
+            for (int k = FB - 1; k >= 0; --k) {
+                double v = LK[tid][k];
+#pragma unroll
+                for (int m = k + 1; m < FB; ++m) v -= t[m] * LB[m][k];
+                t[k] = v * rdg[k];
+            }
+#pragma unroll
+            for (int k = 0; k < FB; ++k) T[tid][k] = t[k];
+        } else if (tid >= 32 && tid < 32 + FB) {  // column k of W = L_BB^-1
+            const int k = tid - 32;
+#pragma unroll
+            for (int r = 0; r < FB; ++r) {
+                double v = r == k ? 1.0 : 0.0;
+                for (int m = k; m < r; ++m) v -= LB[r][m] * Wb[m][k];
+                Wb[r][k] = r < k ? 0.0 : v * rdg[r];
+            }
+        }
+        __syncthreads();
+        if (tid < CW * FB) {  // Z_{R,B} = -Z_{R,K} T
+            const int w = tid / FB, k = tid % FB;
+            double v = 0.0;
+#pragma unroll 9
+            for (int q = 0; q < NK; ++q) v += Zp[w * CW + kwin(q)] * T[q][k];
+            Y[w][k] = -v;
+        }
+        __syncthreads();
+        if (tid < FB * FB) {  // Z_BB (lower triangle, mirrored)
+            const int r = tid / FB, k = tid % FB;
+            if (r >= k) {
+                double v = 0.0;
+                for (int m = r; m < FB; ++m) v += Wb[m][r] * Wb[m][k];
+                for (int q = 0; q < NK; ++q) v -= Y[kwin(q)][r] * T[q][k];
+                ZB[r][k] = v;
+                ZB[k][r] = v;
+            }
+        }
+        __syncthreads();
+        // outputs of the block's 6 columns, and the window of the next block (band rows j0 - 6 + 6 .. , i.e. B first)
+        for (int e = tid; e < FB * NB + NI * FB; e += COV_THREADS) {
+            if (e < FB * NB) {
+                const int k = e / NB, r = e % NB, i = j0 + k + r;  // row inside the segment
+                double v = 0.0;
+                if (i < ns) v = (i < j0 + FB ? ZB[i - j0][k] : Y[i - j0 - FB][k]) * b.scale[js + i] * b.scale[g0 + k];
+                c.Zb[(size_t) (g0 + k) * NB + r] = v;
+            } else {
+                const int a = (e - FB * NB) / FB, k = (e - FB * NB) % FB;
+                c.Zx[(size_t) a * n + g0 + k] = Y[NB - 1 + a][k] * b.scale[n + a] * b.scale[g0 + k];
+            }
+        }
+        for (int e = tid; e < CW * CW; e += COV_THREADS) {
+            const int r = e / CW, q = e % CW;
+            const int orr = r < FB ? -1 : (r < NB - 1 ? r - FB : r), oq = q < FB ? -1 : (q < NB - 1 ? q - FB : q);
+            double v;
+            if (orr < 0 && oq < 0) v = ZB[r][q];
+            else if (orr < 0) v = Y[oq][r];
+            else if (oq < 0) v = Y[orr][q];
+            else v = Zp[orr * CW + oq];
+            Zn[e] = v;
+        }
+        __syncthreads();
+        cur ^= 1;
+    }
+}
 
 }  // namespace
 
@@ -998,3 +1194,99 @@ int ecb_calibrate_device(ecb_lm_device *lm, double *intrinsics, double *rot_cp, 
 }
 
 }  // extern "C"
+
+// ---- ecb_covariance ------------------------------------------------------------------------------------------------------------
+// The workspace (the LM's factorisation buffers for this spline layout + the outputs) stays on the context between calls.
+struct CovWork {
+    std::vector<int32_t> n_cp;
+    ecb_lm_device *lm = nullptr;
+    DevBuf out;
+    CovBufs c;
+};
+
+extern "C" void ecb_covariance_free(ecb_ctx *ctx) {
+    if (!ctx || !ctx->cov) return;
+    CovWork *w = (CovWork *) ctx->cov;
+    ecb_lm_device_destroy(w->lm);
+    if (w->out.p) cudaFree(w->out.p);
+    delete w;
+    ctx->cov = nullptr;
+}
+
+extern "C" int ecb_covariance(ecb_ctx *ctx, int n_splines, const int32_t *n_cp, const double *intrinsics, const double *rot_cp,
+                              const double *trans_cp, const void *d_packed, int64_t n_residuals_total, double *cov_intrinsics,
+                              double *cov_band, double *cov_cross, ecb_covariance_summary *summary) {
+    if (!ctx || n_splines < 1 || !n_cp || !intrinsics || !rot_cp || !trans_cp || n_residuals_total < 0) return ECB_ERR_ARG;
+    if (!ctx->cost) return ecb_fail(ctx, ECB_ERR_STATE, "ecb_cost_setup first");
+    cudaSetDevice(ctx->device);
+    int rc;
+    std::vector<int32_t> key(n_cp, n_cp + n_splines);
+    CovWork *w = (CovWork *) ctx->cov;
+    if (!w || w->n_cp != key) {
+        ecb_covariance_free(ctx);
+        w = new CovWork();
+        w->n_cp = key;
+        if ((rc = ecb_lm_device_create(ctx, n_splines, n_cp, nullptr, &w->lm))) {
+            delete w;
+            return rc;
+        }
+        const size_t n = (size_t) w->lm->dims.n;
+        const size_t cnt[6] = {n * NB, NI * n, NI * NI, NI * NI, NI * NI, 4};
+        size_t total = 0;
+        for (size_t k : cnt) total += k;
+        if ((rc = ecb_reserve(ctx, w->out, total * 8))) {
+            ecb_lm_device_destroy(w->lm);
+            delete w;
+            return rc;
+        }
+        double *p = (double *) w->out.p;
+        double **dst[6] = {&w->c.Zb, &w->c.Zx, &w->c.Zc, &w->c.Zcs, &w->c.Lcc, &w->c.res};
+        for (int k = 0; k < 6; ++k) *dst[k] = p, p += cnt[k];
+        ctx->cov = w;
+    }
+    ecb_lm_device *lm = w->lm;
+    const LmDims &d = lm->dims;
+    const size_t C = (size_t) d.C;
+    LmBufs b = lm->bufs;
+    b.Lcc = w->c.Lcc;
+    if ((rc = ecb_h2d(ctx, b.x, intrinsics, 72))) return rc;
+    if ((rc = ecb_h2d(ctx, b.x + 9, rot_cp, 32 * C))) return rc;
+    if ((rc = ecb_h2d(ctx, b.x + 9 + 4 * C, trans_cp, 24 * C))) return rc;
+    if (d_packed) {
+        b.ne = (double *) d_packed;  // already summed over the ranks: every rank factorises the same system
+    } else {
+        ECB_CUDA(ctx, cudaMemsetAsync(b.ne, 0, (lm->ne_doubles + 2) * 8, ctx->stream));
+        if ((rc = ecb_cost_dev_normal_eq(ctx, b.x, nullptr, b.ne))) return rc;
+    }
+    const int blocks = ctx->sm_count * 2;
+    k_lm_assemble<<<blocks, 256, 0, ctx->stream>>>(d, b, nullptr);
+    k_cov_begin<<<std::min(blocks, (d.D + 255) / 256), 256, 0, ctx->stream>>>(d, b);
+    k_lm_build<<<blocks, 256, 0, ctx->stream>>>(d, b, lm->opt);
+    k_lm_factor<<<d.n_seg, FACTOR_THREADS, 0, ctx->stream>>>(d, b);
+    k_lm_corner<<<1, 32, 0, ctx->stream>>>(d, b);
+    k_cov_pivots<<<1, 1024, 0, ctx->stream>>>(d, b, w->c);
+    k_cov_corner<<<1, 96, 0, ctx->stream>>>(d, b, w->c);
+    k_cov_selinv<<<d.n_seg, COV_THREADS, 0, ctx->stream>>>(d, b, w->c);
+    ctx->launches += 8;
+    if ((rc = ecb_check(ctx, cudaGetLastError(), "covariance kernels"))) return rc;
+    double res[3];
+    if ((rc = ecb_d2h(ctx, res, w->c.res, sizeof res))) return rc;
+    int64_t m = n_residuals_total;
+    if (m == 0 && (rc = ecb_cost_layout(ctx, nullptr, nullptr, &m, nullptr))) return rc;
+    const int deficient = (int) res[2];
+    if (summary) {
+        summary->cost = res[0];
+        summary->n_residuals = m;
+        summary->dimension = d.D;
+        summary->sigma2 = m > d.D ? 2.0 * res[0] / (double) (m - d.D) : NAN;
+        summary->min_relative_pivot = res[1];
+        summary->deficient_index = deficient;
+    }
+    if (deficient >= 0)
+        return ecb_fail(ctx, ECB_FAILED, "covariance: normal equations rank deficient at parameter %d (relative pivot <= %g)", deficient,
+                        COV_MIN_PIVOT);
+    if (cov_intrinsics && (rc = ecb_d2h(ctx, cov_intrinsics, w->c.Zc, NI * NI * 8))) return rc;
+    if (cov_band && (rc = ecb_d2h(ctx, cov_band, w->c.Zb, (size_t) d.n * NB * 8))) return rc;
+    if (cov_cross && (rc = ecb_d2h(ctx, cov_cross, w->c.Zx, (size_t) NI * d.n * 8))) return rc;
+    return ECB_OK;
+}

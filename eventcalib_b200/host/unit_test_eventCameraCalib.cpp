@@ -380,6 +380,29 @@ int main(int argc, char **argv) {
         std::cout << "Intrinsics after optimization:";
         printEigenLike(std::cout, spline.intrinsics().data(), 1, 9);
         std::cout << std::endl;
+        if (getenv("ECB_COVARIANCE") && atoi(getenv("ECB_COVARIANCE")) != 0) {  // uncertainty of the result (no reference output)
+            EventCalibSpline::Covariance cov;
+            const int rc = spline.covariance(cov);
+            if (rc == ECB_OK) {
+                const std::array<double, 9> sd = cov.stdIntrinsics();
+                std::cout << "Intrinsics standard deviation:";
+                printEigenLike(std::cout, sd.data(), 1, 9);
+                std::cout << std::endl;
+                std::ofstream f(std::string(argv[3]) + "/IntrinsicsCovariance.txt");
+                f.precision(17);
+                f << "# sigma2 = 2 cost / (residuals - parameters), " << cov.summary.n_residuals << " residuals, " << cov.summary.dimension
+                  << " parameters\n" << cov.summary.sigma2 << "\n# Z = (J^T J)^-1 of fx fy cx cy k1 k2 k3 k4 k5 (covariance = sigma2 Z)\n";
+                for (int r = 0; r < 9; ++r)
+                    for (int c = 0; c < 9; ++c) f << cov.intrinsics[(size_t) (9 * r + c)] << (c == 8 ? "\n" : " ");
+                f << "# standard deviation sqrt(sigma2 Z_ii)\n";
+                for (int i = 0; i < 9; ++i) f << sd[(size_t) i] << (i == 8 ? "\n" : " ");
+            } else if (rc == ECB_FAILED) {
+                std::cerr << "ecb: no covariance: " << spline.lastError() << std::endl;
+            } else {
+                std::cerr << "ecb: " << spline.lastError() << std::endl;
+                return 1;
+            }
+        }
         spline.saveKeyFrameTrajectoryTUM(std::string(argv[3]) + "/TrajectoryByEvent.txt", stamps);  // eventCameraCalib.cpp:212
         if (!getenv("ECB_NO_IMAGES")) {  // :214-227: SavePath/image/<timestamp>.png = cf->image() of every key frame
             const std::string dir = std::string(argv[3]) + "/image/";

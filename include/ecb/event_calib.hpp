@@ -984,6 +984,35 @@ public:
         if (summary) *summary = sum;
         return true;
     }
+    // Uncertainty of the calibration (ecb_covariance): Z = H^-1 at the current point (where optimize() left it) on the band /
+    // arrow pattern, sigma^2 = 2 cost / (residuals - parameters), standard deviation of parameter i = sqrt(sigma^2 Z_ii).
+    struct Covariance {
+        std::array<double, 81> intrinsics{};  // Z of fx fy cx cy k1 .. k5, row major
+        std::vector<double> band;             // 6C x 24: Z(j + r, j) at [j * 24 + r], control point c owns rows 6c .. 6c+5
+        std::vector<double> cross;            // 9 x 6C: Z(intrinsic i, j) at [i * 6C + j]
+        ecb_covariance_summary summary{};
+        std::array<double, 9> stdIntrinsics() const {
+            std::array<double, 9> s{};
+            for (int i = 0; i < 9; ++i) s[(size_t) i] = std::sqrt(summary.sigma2 * intrinsics[(size_t) (10 * i)]);
+            return s;
+        }
+    };
+    // ECB_OK, ECB_FAILED for rank-deficient normal equations (out.summary.deficient_index names the parameter), < 0 on errors
+    int covariance(Covariance &out) const { return covarianceAt(ev_->ctx, n_cp_, intr_, seg_, nullptr, 0, out); }
+    // the same at a given point; d_packed / n_residuals_total as ecb_covariance (an already-summed buffer of several GPUs)
+    static int covarianceAt(ecb_ctx *ctx, const std::vector<int32_t> &n_cp, const std::array<double, 9> &intr,
+                            const std::vector<Segment> &seg, const void *d_packed, int64_t n_residuals_total, Covariance &out) {
+        std::vector<double> rot, trans;
+        for (auto &s : seg) {
+            rot.insert(rot.end(), s.rot_cp.begin(), s.rot_cp.end());
+            trans.insert(trans.end(), s.trans_cp.begin(), s.trans_cp.end());
+        }
+        const size_t n = trans.size() * 2;  // 6 C
+        out.band.assign(n * 24, 0.0);
+        out.cross.assign(9 * n, 0.0);
+        return ecb_covariance(ctx, (int) n_cp.size(), n_cp.data(), intr.data(), rot.data(), trans.data(), d_packed, n_residuals_total,
+                              out.intrinsics.data(), out.band.data(), out.cross.data(), &out.summary);
+    }
     const std::array<double, 9> &intrinsics() const { return intr_; }
     const std::vector<Segment> &segments() const { return seg_; }
     // EventCalibSpline.hpp:286-303: index of the segment whose knot range holds t, else -1

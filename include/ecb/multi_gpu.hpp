@@ -262,6 +262,61 @@ public:
         solved_ = true;
         return ok;
     }
+    // Covariance at the current point (EventCalibSpline::covariance).  Several GPUs: the normal equations are summed over the
+    // shards by the exchange into a device buffer on every shard, and every shard factorises and inverts the same sum; the ranks'
+    // results are bit-identical (checked), rank 0's is returned.
+    int covariance(EventCalibSpline::Covariance &out) {
+        const int G = (int) sp_.size();
+        if (G == 1) return EventCalibSpline::covarianceAt(ev_->shard[0]->ctx, n_cp_, intrinsics(), segments(), nullptr, 0, out);
+        auto ctx = [&](int g) { return ev_->shard[(size_t) g]->ctx; };
+        std::vector<double> rot, trans;
+        for (auto &s : segments()) {
+            rot.insert(rot.end(), s.rot_cp.begin(), s.rot_cp.end());
+            trans.insert(trans.end(), s.trans_cp.begin(), s.trans_cp.end());
+        }
+        const std::array<double, 9> intr = intrinsics();
+        std::vector<void *> buf((size_t) G, nullptr), packed((size_t) G, nullptr);
+        std::vector<EventCalibSpline::Covariance> cov((size_t) G);
+        std::vector<int> rc((size_t) G, ECB_OK);
+        int64_t n_total = 0;
+        auto release = [&]() {
+            for (int g = 0; g < G; ++g) {
+                ecb_synchronize(ctx(g));
+                if (buf[(size_t) g]) ecb_device_free(ctx(g), buf[(size_t) g]);
+                if (packed[(size_t) g]) ecb_device_free(ctx(g), packed[(size_t) g]);
+            }
+        };
+        try {
+            for (int g = 0; g < G; ++g) {
+                int64_t nr = 0, nd = 0;
+                if (ecb_cost_layout(ctx(g), nullptr, nullptr, &nr, &nd) != ECB_OK) throw std::runtime_error(ecb_last_error(ctx(g)));
+                n_total += nr;
+                for (int h = 0; h < G; ++h)
+                    if (h != g && ecb_enable_peer_access(ctx(g), ev_->device[(size_t) h]) != ECB_OK) throw std::runtime_error(ecb_last_error(ctx(g)));
+                if (ecb_device_alloc(ctx(g), ecb_exchange_buffer_bytes(ctx(g), G), &buf[(size_t) g]) != ECB_OK ||
+                    ecb_device_alloc(ctx(g), (size_t) nd * 8, &packed[(size_t) g]) != ECB_OK)
+                    throw std::runtime_error(ecb_last_error(ctx(g)));
+            }
+            forEachShard(G, [&](int g) {  // the receive side waits for the peers: one host thread per shard
+                if (ecb_cost_normal_eq_exchange(ctx(g), intr.data(), rot.data(), trans.data(), g, G, buf.data(), 1, ECB_EXCHANGE_BOTH,
+                                                packed[(size_t) g], nullptr) != ECB_OK ||
+                    ecb_synchronize(ctx(g)) != ECB_OK)
+                    throw std::runtime_error(ecb_last_error(ctx(g)));
+                rc[(size_t) g] = EventCalibSpline::covarianceAt(ctx(g), n_cp_, intr, segments(), packed[(size_t) g], n_total, cov[(size_t) g]);
+                if (rc[(size_t) g] < 0) throw std::runtime_error(ecb_last_error(ctx(g)));
+            });
+        } catch (...) {
+            release();
+            throw;
+        }
+        release();
+        for (int g = 1; g < G; ++g)
+            if (rc[(size_t) g] != rc[0] || cov[(size_t) g].intrinsics != cov[0].intrinsics || cov[(size_t) g].band != cov[0].band ||
+                cov[(size_t) g].cross != cov[0].cross)
+                throw std::runtime_error("multi-GPU covariance: the ranks' results differ");
+        out = cov[0];
+        return rc[0];
+    }
     const std::array<double, 9> &intrinsics() const { return solved_ ? result_intr_ : sp_[0]->intrinsics(); }
     const std::vector<Segment> &segments() const { return solved_ ? seg_ : sp_[0]->segments(); }
     int saveKeyFrameTrajectoryTUM(const std::string &filename, const std::vector<double> &keyframeStamps) const {

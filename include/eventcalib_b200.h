@@ -323,6 +323,32 @@ int ecb_lm_device_result(ecb_lm_device *lm, double *intrinsics, double *rot_cp, 
 int ecb_calibrate_device(ecb_lm_device *lm, double *intrinsics, double *rot_cp, double *trans_cp, ecb_lm_summary *summary,
                          double *trace, int trace_rows);
 
+/* ---- uncertainty of the calibration: covariance of the intrinsics and the spline control points ----------------------------
+ * x is the parameter point in the tangent space of the selected rotation model: control point c owns rows 6c .. 6c+5 (rotation
+ * tangent 3, translation 3) of the flat order over all segments, the 9 intrinsics come last (D = 6 C + 9).  H = J^T J at x
+ * (Huber corrector applied, as ecb_cost_normal_eq).  Z = H^-1 as ceres::Covariance returns it with default options (no sigma^2
+ * scaling); the standard deviation of parameter i is sqrt(sigma2 Z_ii) with sigma2 = 2 cost / (n_residuals - D) (OpenCV's
+ * calibrateCameraExtended convention).  Z is computed on the device: Cholesky factor of S H S (S = diag(H)^-1/2, 1 where the
+ * diagonal is 0) with the LM's band-arrow factorisation, undamped, then the selected inverse of that factor, i.e. the entries of
+ * Z on the band / arrow pattern: every control point's 6 x 6 block, any 4 consecutive control points (a pose on the spline), the
+ * intrinsics.  FP64, deterministic.
+ *   d_packed: NULL = evaluate the normal equations at x on this context; else an already-summed packed buffer on this context's
+ *             device (layout of ecb_cost_normal_eq, e.g. the d_out of ecb_cost_normal_eq_exchange): every rank then computes the
+ *             same result bit for bit
+ *   n_residuals_total: residual count of sigma2; 0 = this context's count
+ *   cov_intrinsics[9 x 9]; cov_band[6C x 24] = Z(j + r, j) at [j * 24 + r] (0 past the end of a segment); cov_cross[9 x 6C] =
+ *   Z(intrinsic i, j) at [i * 6C + j].  Output pointers may be NULL.
+ * A relative pivot L(j,j)^2 / M(j,j) <= 1e-12 or a zero diagonal (a control point without residuals, an intrinsic nothing
+ * constrains) returns ECB_FAILED with summary->deficient_index = j and writes no covariance; deficient_index is -1 otherwise. */
+typedef struct {
+    double cost, sigma2, min_relative_pivot;  /* sigma2 is NaN when n_residuals <= dimension */
+    int64_t n_residuals;
+    int32_t dimension, deficient_index;
+} ecb_covariance_summary;
+int ecb_covariance(ecb_ctx *ctx, int n_splines, const int32_t *n_cp, const double *intrinsics, const double *rot_cp,
+                   const double *trans_cp, const void *d_packed, int64_t n_residuals_total, double *cov_intrinsics, double *cov_band,
+                   double *cov_cross, ecb_covariance_summary *summary);
+
 #ifdef __cplusplus
 }
 #endif
