@@ -71,7 +71,8 @@ SYMBOLS = ["ecb_ctx_create", "ecb_ctx_destroy", "ecb_last_error", "ecb_launch_co
            "ecb_lm_destroy", "ecb_lm_dimension", "ecb_lm_begin", "ecb_lm_propose", "ecb_lm_feedback", "ecb_lm_update",
            "ecb_lm_state", "ecb_lm_trace", "ecb_calibrate", "ecb_lm_device_create", "ecb_lm_device_destroy",
            "ecb_lm_device_set_exchange", "ecb_lm_device_begin", "ecb_lm_device_iterate", "ecb_lm_device_running",
-           "ecb_lm_device_result", "ecb_calibrate_device", "ecb_covariance"]
+           "ecb_lm_device_result", "ecb_calibrate_device", "ecb_covariance", "ecb_pose_covariance",
+           "ecb_pose_covariance_device"]
 
 _lib = None
 
@@ -159,6 +160,8 @@ def load_library():
     lib.ecb_lm_device_result.argtypes = [vp, vp, vp, vp, C.POINTER(LmSummary), vp, i32]
     lib.ecb_calibrate_device.argtypes = [vp, vp, vp, vp, C.POINTER(LmSummary), vp, i32]
     lib.ecb_covariance.argtypes = [vp, i32, vp, vp, vp, vp, vp, i64, vp, vp, vp, C.POINTER(CovarianceSummary)]
+    lib.ecb_pose_covariance.argtypes = [vp, vp, i64, vp, vp, C.POINTER(C.c_int64)]
+    lib.ecb_pose_covariance_device.argtypes = [vp, vp, i64, vp, vp, C.POINTER(C.c_int64)]
     _lib = lib
     return lib
 
@@ -529,6 +532,27 @@ class Context:
         if rc == OK:
             out.update(cov_intrinsics=zc, cov_band=zb, cov_cross=zx, std_intrinsics=np.sqrt(s.sigma2 * np.diag(zc)))
         return out
+
+    def pose_covariance(self, times):
+        """6 x 6 covariance Sigma(t) of the trajectory's pose at the given times (ecb_pose_covariance), from the last successful
+        covariance() on this context.  Returns a dict: pose (n, 7) = tx ty tz qx qy qz qw, cov (n, 6, 6) over (dtheta body
+        frame, dp world frame), n_valid.  Times outside every segment, and NaN, give NaN rows.  Not scaled by sigma2."""
+        t = np.ascontiguousarray(np.atleast_1d(times), np.float64)
+        n = len(t)
+        pose, cov = np.empty((n, 7)), np.empty((n, 6, 6))
+        nv = C.c_int64()
+        self._chk(self.lib.ecb_pose_covariance(self.h, _ptr(t), n, _ptr(pose), _ptr(cov), C.byref(nv)))
+        return {"pose": pose, "cov": cov, "n_valid": nv.value}
+
+    def pose_covariance_device(self, d_times, n, d_pose, d_cov, count=True):
+        """ecb_pose_covariance_device on raw device pointers (e.g. torch CUDA tensors' data_ptr()): n float64 times in, n x 7
+        poses and n x 36 covariances out (either pointer may be 0).  Enqueued on the context's stream; with count=True it waits
+        and returns the number of valid queries, else returns None at once."""
+        nv = C.c_int64()
+        self._chk(self.lib.ecb_pose_covariance_device(self.h, C.c_void_p(d_times) if d_times else None, int(n),
+                                                      C.c_void_p(d_pose) if d_pose else None,
+                                                      C.c_void_p(d_cov) if d_cov else None, C.byref(nv) if count else None))
+        return nv.value if count else None
 
 
 def control_point_covariance(cov, c):

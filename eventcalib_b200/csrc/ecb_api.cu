@@ -182,7 +182,7 @@ void ecb_ctx_destroy(ecb_ctx *c) {
                       &c->arrive, &c->pts[0], &c->pts[1], &c->labels[0], &c->labels[1], &c->scratch, &c->ktab, &c->kmem,
                       &c->cand, &c->status, &c->db_pix, &c->db_off, &c->db_labels, &c->db_hdr, &c->db_scratch, &c->db_dims,
                       &c->fit_in, &c->fit_off, &c->fit_out, &c->db_hdr_b, &c->db_ktab, &c->db_counter, &c->kd_tree, &c->bfs_key,
-                      &c->bfs_items, &c->bfs_front, &c->bfs_tab, &c->ord_htab, &c->pair_tab};
+                      &c->bfs_items, &c->bfs_front, &c->bfs_tab, &c->ord_htab, &c->pair_tab, &c->pose_io};
     for (DevBuf *b : bufs)
         if (b->p) cudaFree(b->p);
     for (DevBuf &b : c->gh)

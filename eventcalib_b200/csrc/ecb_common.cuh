@@ -73,7 +73,28 @@ struct ecb_ctx {
     void *cost = nullptr;
     // covariance workspace (ecb_lmdev.cu), kept for repeated calls with the same spline layout
     void *cov = nullptr;
+    // incremented by ecb_cost_setup and ecb_cost_set_rotation_model: a covariance computed before refers to other knots or
+    // another rotation tangent
+    uint64_t spline_gen = 0;
+    // staging of the host variant of ecb_pose_covariance (ecb_pose_cov.cu)
+    DevBuf pose_io;
 };
+
+// the splines of ecb_cost_setup on the device (ecb_cost.cu); ECB_ERR_STATE before the setup
+struct EcbSplineView {
+    const double *knots;
+    const int *knot_off, *ncp, *cp_off;
+    int n_splines, total_cp, so3;
+};
+extern "C" int ecb_cost_spline_view(ecb_ctx *ctx, EcbSplineView *v);
+// the result of the last successful ecb_covariance (ecb_lmdev.cu): the band of Z (layout of cov_band), the point x
+// (intrinsics 9 | rotation 4C | translation 3C), the rotation model and ctx->spline_gen at that call; ECB_ERR_STATE without one
+struct EcbCovView {
+    const double *Zb, *x;
+    int total_cp, so3;
+    uint64_t spline_gen;
+};
+extern "C" int ecb_covariance_view(ecb_ctx *ctx, EcbCovView *v);
 
 int ecb_fail(ecb_ctx *ctx, int code, const char *fmt, ...);
 int ecb_reserve(ecb_ctx *ctx, DevBuf &b, size_t bytes);

@@ -19,6 +19,7 @@
 #include <algorithm>
 #include <vector>
 
+#include "ecb_bspline.cuh"
 #include "ecb_common.cuh"
 #include "ecb_residual_so3.h"
 
@@ -57,54 +58,6 @@ CostState *state(ecb_ctx *ctx) {
 }
 
 // ------------------------------------------------------------------------------------ prepare ----
-__device__ __forceinline__ int find_span_dev(const double *knots, int nk, double u) {  // BsplineReal.hpp:208-231
-    const int degree = 3;
-    const int n = nk - 2 - degree;
-    if (u == knots[n + 1]) return n;
-    int low = degree, high = n + 1, mid = (low + high) / 2;
-    while (u < knots[mid] || u >= knots[mid + 1]) {
-        if (u < knots[mid]) high = mid; else low = mid;
-        mid = (low + high) / 2;
-    }
-    return mid;
-}
-
-// same span (the one with knots[mid] <= u < knots[mid+1] is unique) from a proportional guess and a short walk: the
-// reference's interior knots are nearly uniform (NURBS-book eq. 9.68), so the dependent-load chain of the bisection goes away
-__device__ __forceinline__ int find_span_guess(const double *knots, int nk, double u) {
-    const int degree = 3;
-    const int n = nk - 2 - degree;
-    if (u == knots[n + 1]) return n;
-    const double k0 = knots[degree], k1 = knots[n + 1];
-    int mid = degree + (int) ((u - k0) / (k1 - k0) * (double) (n + 1 - degree));
-    mid = max(degree, min(n, mid));
-    for (int s = 0; s < 8 && mid > degree && u < knots[mid]; ++s) --mid;
-    for (int s = 0; s < 8 && mid < n && u >= knots[mid + 1]; ++s) ++mid;
-    if (u < knots[mid] || u >= knots[mid + 1]) return find_span_dev(knots, nk, u);
-    return mid;
-}
-
-__device__ __forceinline__ void basis_dev(const double *knots, int span, double u, double *N) {  // BsplineReal.hpp:107-145
-    double ndu[4][4], left[4], right[4];
-    ndu[0][0] = 1;
-#pragma unroll
-    for (int j = 1; j <= 3; j++) {
-        left[j] = u - knots[span + 1 - j];
-        right[j] = knots[span + j] - u;
-        double saved = 0.0;
-#pragma unroll
-        for (int r = 0; r < j; ++r) {
-            ndu[j][r] = right[r + 1] + left[j - r];
-            double temp = __ddiv_rn(ndu[r][j - 1], ndu[j][r]);
-            ndu[r][j] = __dadd_rn(saved, __dmul_rn(right[r + 1], temp));
-            saved = __dmul_rn(left[j - r], temp);
-        }
-        ndu[j][j] = saved;
-    }
-#pragma unroll
-    for (int j = 0; j <= 3; j++) N[j] = ndu[j][3];
-}
-
 __global__ void k_prepare(const double *__restrict__ t, const int *__restrict__ spl, int64_t n, const double *__restrict__ knots,
                           const int *__restrict__ knot_off, const int *__restrict__ ncp, const int *__restrict__ cp_off,
                           const int *__restrict__ span_off, double *__restrict__ basis, int *__restrict__ cp0,
@@ -825,6 +778,7 @@ int ecb_cost_setup(ecb_ctx *ctx, int n_splines, const int32_t *n_cp, const doubl
     st->total_cp = co;
     st->total_spans = so;
     st->knots.assign(knots, knots + ko);
+    ++ctx->spline_gen;
     st->radius = circle_radius;
     st->huber = huber_delta;
     st->n_res = 0;
@@ -847,6 +801,20 @@ int ecb_cost_set_rotation_model(ecb_ctx *ctx, int use_so3) {
     if (!ctx || !ctx->cost) return ecb_fail(ctx, ECB_ERR_STATE, "ecb_cost_setup first");
     if (use_so3 != 0 && use_so3 != 1) return ECB_ERR_ARG;
     ((CostState *) ctx->cost)->so3 = use_so3;
+    ++ctx->spline_gen;
+    return ECB_OK;
+}
+
+int ecb_cost_spline_view(ecb_ctx *ctx, EcbSplineView *v) {
+    if (!ctx || !ctx->cost) return ECB_ERR_STATE;
+    const CostState *st = (const CostState *) ctx->cost;
+    v->knots = (const double *) st->d_knots.p;
+    v->knot_off = (const int *) st->d_knot_off.p;
+    v->ncp = (const int *) st->d_ncp.p;
+    v->cp_off = (const int *) st->d_cp_off.p;
+    v->n_splines = st->n_splines;
+    v->total_cp = st->total_cp;
+    v->so3 = st->so3;
     return ECB_OK;
 }
 

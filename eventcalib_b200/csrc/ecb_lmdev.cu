@@ -1202,6 +1202,10 @@ struct CovWork {
     ecb_lm_device *lm = nullptr;
     DevBuf out;
     CovBufs c;
+    // set when a call succeeds: the rotation model it differentiated in and ctx->spline_gen (ecb_pose_covariance reads Z and x)
+    bool valid = false;
+    int so3 = 0;
+    uint64_t spline_gen = 0;
 };
 
 extern "C" void ecb_covariance_free(ecb_ctx *ctx) {
@@ -1244,6 +1248,7 @@ extern "C" int ecb_covariance(ecb_ctx *ctx, int n_splines, const int32_t *n_cp, 
         for (int k = 0; k < 6; ++k) *dst[k] = p, p += cnt[k];
         ctx->cov = w;
     }
+    w->valid = false;
     ecb_lm_device *lm = w->lm;
     const LmDims &d = lm->dims;
     const size_t C = (size_t) d.C;
@@ -1288,5 +1293,21 @@ extern "C" int ecb_covariance(ecb_ctx *ctx, int n_splines, const int32_t *n_cp, 
     if (cov_intrinsics && (rc = ecb_d2h(ctx, cov_intrinsics, w->c.Zc, NI * NI * 8))) return rc;
     if (cov_band && (rc = ecb_d2h(ctx, cov_band, w->c.Zb, (size_t) d.n * NB * 8))) return rc;
     if (cov_cross && (rc = ecb_d2h(ctx, cov_cross, w->c.Zx, (size_t) NI * d.n * 8))) return rc;
+    EcbSplineView sv;
+    if ((rc = ecb_cost_spline_view(ctx, &sv))) return rc;
+    w->valid = true;
+    w->so3 = sv.so3;
+    w->spline_gen = ctx->spline_gen;
+    return ECB_OK;
+}
+
+extern "C" int ecb_covariance_view(ecb_ctx *ctx, EcbCovView *v) {
+    const CovWork *w = (const CovWork *) ctx->cov;
+    if (!w || !w->valid) return ECB_ERR_STATE;
+    v->Zb = w->c.Zb;
+    v->x = w->lm->bufs.x;
+    v->total_cp = w->lm->dims.C;
+    v->so3 = w->so3;
+    v->spline_gen = w->spline_gen;
     return ECB_OK;
 }

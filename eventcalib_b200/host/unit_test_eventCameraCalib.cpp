@@ -380,10 +380,12 @@ int main(int argc, char **argv) {
         std::cout << "Intrinsics after optimization:";
         printEigenLike(std::cout, spline.intrinsics().data(), 1, 9);
         std::cout << std::endl;
-        if (getenv("ECB_COVARIANCE") && atoi(getenv("ECB_COVARIANCE")) != 0) {  // uncertainty of the result (no reference output)
+        const bool want_cov = getenv("ECB_COVARIANCE") && atoi(getenv("ECB_COVARIANCE")) != 0;
+        const bool want_traj_cov = getenv("ECB_TRAJECTORY_COVARIANCE") && atoi(getenv("ECB_TRAJECTORY_COVARIANCE")) != 0;
+        if (want_cov || want_traj_cov) {  // uncertainty of the result (no reference output)
             EventCalibSpline::Covariance cov;
             const int rc = spline.covariance(cov);
-            if (rc == ECB_OK) {
+            if (rc == ECB_OK && want_cov) {
                 const std::array<double, 9> sd = cov.stdIntrinsics();
                 std::cout << "Intrinsics standard deviation:";
                 printEigenLike(std::cout, sd.data(), 1, 9);
@@ -398,9 +400,27 @@ int main(int argc, char **argv) {
                 for (int i = 0; i < 9; ++i) f << sd[(size_t) i] << (i == 8 ? "\n" : " ");
             } else if (rc == ECB_FAILED) {
                 std::cerr << "ecb: no covariance: " << spline.lastError() << std::endl;
-            } else {
+            } else if (rc != ECB_OK) {
                 std::cerr << "ecb: " << spline.lastError() << std::endl;
                 return 1;
+            }
+            if (rc == ECB_OK && want_traj_cov) {  // one line per line of TrajectoryByEvent.txt: its stamp, then sigma2 Sigma row major
+                std::vector<double> pose, pc;
+                if (spline.poseCovariance(stamps, pose, pc) != ECB_OK) {
+                    std::cerr << "ecb: " << spline.lastError() << std::endl;
+                    return 1;
+                }
+                std::ofstream f(std::string(argv[3]) + "/TrajectoryCovariance.txt");
+                f << "# covariance sigma2 Sigma of the pose at each stamp of TrajectoryByEvent.txt: stamp, then 36 entries row major\n"
+                  << "# tangent: dtheta_x dtheta_y dtheta_z (body frame, R = R^ Exp(dtheta), radians), dp_x dp_y dp_z (t - t^, world "
+                     "frame, units of the trajectory)\n"
+                  << "# sigma2 = 2 cost / (residuals - parameters) = " << std::setprecision(17) << cov.summary.sigma2 << "\n";
+                for (size_t k = 0; k < stamps.size(); ++k) {
+                    if (std::isnan(pose[7 * k])) continue;  // outside every segment: TrajectoryByEvent.txt skips the stamp too
+                    f << std::fixed << std::setprecision(10) << stamps[k] << std::defaultfloat << std::setprecision(17);
+                    for (int e = 0; e < 36; ++e) f << " " << cov.summary.sigma2 * pc[36 * k + (size_t) e];
+                    f << "\n";
+                }
             }
         }
         spline.saveKeyFrameTrajectoryTUM(std::string(argv[3]) + "/TrajectoryByEvent.txt", stamps);  // eventCameraCalib.cpp:212

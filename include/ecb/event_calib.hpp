@@ -1013,6 +1013,19 @@ public:
         return ecb_covariance(ctx, (int) n_cp.size(), n_cp.data(), intr.data(), rot.data(), trans.data(), d_packed, n_residuals_total,
                               out.intrinsics.data(), out.band.data(), out.cross.data(), &out.summary);
     }
+    // Uncertainty of the trajectory (ecb_pose_covariance), after covariance(): pose[7 n] = tx ty tz qx qy qz qw and cov[36 n] =
+    // Sigma(t) row major over (dtheta body frame, dp world frame) at each time; NaN rows for times outside every segment.
+    // The covariance is cov.summary.sigma2 Sigma.  ECB_OK, or < 0 (ECB_ERR_STATE without a successful covariance()).
+    int poseCovariance(const std::vector<double> &times, std::vector<double> &pose, std::vector<double> &cov,
+                       int64_t *n_valid = nullptr) const {
+        return poseCovarianceAt(ev_->ctx, times, pose, cov, n_valid);
+    }
+    static int poseCovarianceAt(ecb_ctx *ctx, const std::vector<double> &times, std::vector<double> &pose, std::vector<double> &cov,
+                                int64_t *n_valid) {
+        pose.assign(7 * times.size(), 0.0);
+        cov.assign(36 * times.size(), 0.0);
+        return ecb_pose_covariance(ctx, times.data(), (int64_t) times.size(), pose.data(), cov.data(), n_valid);
+    }
     const std::array<double, 9> &intrinsics() const { return intr_; }
     const std::vector<Segment> &segments() const { return seg_; }
     // EventCalibSpline.hpp:286-303: index of the segment whose knot range holds t, else -1

@@ -317,6 +317,12 @@ public:
         out = cov[0];
         return rc[0];
     }
+    // Pose covariance (EventCalibSpline::poseCovariance) after covariance(): every rank holds the same Z bit for bit, rank 0's
+    // context answers.
+    int poseCovariance(const std::vector<double> &times, std::vector<double> &pose, std::vector<double> &cov,
+                       int64_t *n_valid = nullptr) const {
+        return EventCalibSpline::poseCovarianceAt(ev_->shard[0]->ctx, times, pose, cov, n_valid);
+    }
     const std::array<double, 9> &intrinsics() const { return solved_ ? result_intr_ : sp_[0]->intrinsics(); }
     const std::vector<Segment> &segments() const { return solved_ ? seg_ : sp_[0]->segments(); }
     int saveKeyFrameTrajectoryTUM(const std::string &filename, const std::vector<double> &keyframeStamps) const {

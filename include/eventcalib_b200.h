@@ -349,6 +349,23 @@ int ecb_covariance(ecb_ctx *ctx, int n_splines, const int32_t *n_cp, const doubl
                    const double *trans_cp, const void *d_packed, int64_t n_residuals_total, double *cov_intrinsics, double *cov_band,
                    double *cov_cross, ecb_covariance_summary *summary);
 
+/* ---- uncertainty of the trajectory: 6 x 6 covariance of the pose at any time on the spline ------------------------------
+ * For a time t, let s be the first segment whose knot range holds t (EventCalibSpline::time2splineIdx) and i its span.  The
+ * pose (R^, t^) at t is what EventCalibSpline::evaluate returns for the rotation model in use.  The tangent of the output is
+ * dtheta (body frame, R = R^ Exp(dtheta), radians) then dp = t - t^ (world frame, units of the translation control points).
+ * cov = Sigma(t) = J Z_blk J^T with J (6 x 24) the derivative of (dtheta, dp) with respect to the tangent parameters of control
+ * points i-3 .. i in the order and rotation model of ecb_covariance, and Z_blk their 24 x 24 block of Z.  No sigma^2 scaling:
+ * the covariance is sigma2 Sigma (sigma2 of ecb_covariance_summary).
+ * Uses the Z and x of the last successful ecb_covariance on ctx (with several GPUs every rank holds the same Z bit for bit);
+ * ECB_ERR_STATE without one, or when ecb_cost_setup or ecb_cost_set_rotation_model ran after it.
+ *   pose[n][7] = tx ty tz qx qy qz qw (the order of TrajectoryByEvent.txt); cov[n][36] = Sigma row major, exactly symmetric.
+ *   pose and cov may each be NULL.  A time outside every segment, or NaN, gives a NaN row and is not counted in *n_valid.
+ *   n == 0 is valid, n < 0 returns ECB_ERR_ARG.  A query's output does not depend on the batch it is in.  FP64.
+ * ecb_pose_covariance takes host arrays (staged through device buffers); ecb_pose_covariance_device takes device arrays and is
+ * asynchronous on the context's stream unless n_valid (a host pointer, may be NULL) is asked for. */
+int ecb_pose_covariance(ecb_ctx *ctx, const double *times, int64_t n, double *pose, double *cov, int64_t *n_valid);
+int ecb_pose_covariance_device(ecb_ctx *ctx, const double *d_times, int64_t n, double *d_pose, double *d_cov, int64_t *n_valid);
+
 #ifdef __cplusplus
 }
 #endif
