@@ -54,6 +54,24 @@ class CovarianceSummary(C.Structure):
                 ("dimension", C.c_int32), ("deficient_index", C.c_int32)]
 
 
+# the order of every intrinsics array (ecb_residual.h): bit i of a constant-intrinsics mask is INTRINSIC_NAMES[i].  In the spline
+# stage k1 .. k5 are the coefficients of the inverse radial polynomial, not OpenCV's distortion coefficients.
+INTRINSIC_NAMES = ("fx", "fy", "cx", "cy", "k1", "k2", "k3", "k4", "k5")
+
+
+def constant_intrinsics_mask(names):
+    """Bit mask of ecb_cost_set_constant_intrinsics from an iterable of INTRINSIC_NAMES (a string: comma- or space-separated
+    names); empty means none.  An unknown name raises ValueError."""
+    if isinstance(names, str):
+        names = names.replace(",", " ").split()
+    mask = 0
+    for nm in names:
+        if nm not in INTRINSIC_NAMES:
+            raise ValueError("unknown intrinsic %r (names: %s)" % (nm, " ".join(INTRINSIC_NAMES)))
+        mask |= 1 << INTRINSIC_NAMES.index(nm)
+    return mask
+
+
 SUMMARY_DTYPE = np.dtype([("ev_lo", "<i8"), ("ev_hi", "<i8"), ("n_points", "<i4", 2), ("n_clusters", "<i4", 2),
                           ("n_kept", "<i4", 2), ("n_candidates", "<i4"), ("status", "<u4"), ("point_offset", "<i8", 2)])
 assert SUMMARY_DTYPE.itemsize == C.sizeof(WindowSummary)
@@ -64,11 +82,12 @@ SYMBOLS = ["ecb_ctx_create", "ecb_ctx_destroy", "ecb_last_error", "ecb_launch_co
            "ecb_frontend_summary", "ecb_frontend_total_points", "ecb_frontend_points", "ecb_frontend_candidates",
            "ecb_frontend_clusters", "ecb_frontend_rectify", "ecb_frontend_device_ptrs", "ecb_dbscan_run", "ecb_dbscan_run_batch",
            "ecb_dbscan_run_ordered", "ecb_dbscan_run_batch_ordered", "ecb_dbscan_run_nd",
-           "ecb_fit_circles", "ecb_set_profiling", "ecb_stage_ms", "ecb_cost_setup", "ecb_cost_set_rotation_model", "ecb_cost_layout",
+           "ecb_fit_circles", "ecb_set_profiling", "ecb_stage_ms", "ecb_cost_setup", "ecb_cost_set_rotation_model",
+           "ecb_cost_set_constant_intrinsics", "ecb_cost_layout",
            "ecb_cost_associate", "ecb_cost_associate_device", "ecb_cost_get_association", "ecb_cost_set_residuals", "ecb_cost_eval", "ecb_cost_normal_eq",
            "ecb_exchange_buffer_bytes", "ecb_cost_normal_eq_exchange", "ecb_device_alloc", "ecb_device_free", "ecb_ipc_export",
            "ecb_ipc_open", "ecb_ipc_close", "ecb_enable_peer_access", "ecb_lm_default_options", "ecb_lm_create",
-           "ecb_lm_destroy", "ecb_lm_dimension", "ecb_lm_begin", "ecb_lm_propose", "ecb_lm_feedback", "ecb_lm_update",
+           "ecb_lm_destroy", "ecb_lm_dimension", "ecb_lm_set_constant_intrinsics", "ecb_lm_begin", "ecb_lm_propose", "ecb_lm_feedback", "ecb_lm_update",
            "ecb_lm_state", "ecb_lm_trace", "ecb_calibrate", "ecb_lm_device_create", "ecb_lm_device_destroy",
            "ecb_lm_device_set_exchange", "ecb_lm_device_begin", "ecb_lm_device_iterate", "ecb_lm_device_running",
            "ecb_lm_device_result", "ecb_calibrate_device", "ecb_covariance", "ecb_pose_covariance",
@@ -111,6 +130,7 @@ def load_library():
     lib.ecb_frontend_device_ptrs.argtypes = [vp, C.POINTER(vp), C.POINTER(vp), C.POINTER(i32)]
     lib.ecb_frontend_rectify.argtypes = [vp, vp, i32, i32, vp, dbl, i32, i32, i32, vp, vp]
     lib.ecb_cost_set_rotation_model.argtypes = [vp, i32]
+    lib.ecb_cost_set_constant_intrinsics.argtypes = [vp, u32]
     lib.ecb_exchange_buffer_bytes.argtypes = [vp, i32]
     lib.ecb_exchange_buffer_bytes.restype = C.c_size_t
     lib.ecb_cost_normal_eq_exchange.argtypes = [vp, vp, vp, vp, i32, i32, vp, C.c_uint64, i32, vp, vp]
@@ -143,6 +163,7 @@ def load_library():
     lib.ecb_lm_destroy.argtypes = [vp]
     lib.ecb_lm_destroy.restype = None
     lib.ecb_lm_dimension.argtypes = [vp]
+    lib.ecb_lm_set_constant_intrinsics.argtypes = [vp, u32]
     lib.ecb_lm_begin.argtypes = [vp, vp, vp, vp, vp]
     lib.ecb_lm_propose.argtypes = [vp, vp, vp, vp]
     lib.ecb_lm_feedback.argtypes = [vp, dbl]
@@ -394,6 +415,12 @@ class Context:
     def cost_set_rotation_model(self, use_so3):
         """0: normalised quaternion spline (useSO3: 0); 1: cumulative SO(3) spline + LocalParameterizationSO3 (useSO3: 1)"""
         self._chk(self.lib.ecb_cost_set_rotation_model(self.h, int(use_so3)))
+
+    def set_constant_intrinsics(self, names):
+        """Holds the named intrinsics (INTRINSIC_NAMES; empty: none) at their start values in calibrate() and DeviceLm (captured
+        when a DeviceLm is created), and conditions covariance() on them: their rows and columns of Z are zeros and
+        dimension counts the free parameters.  Kept by the context across cost_setup."""
+        self._chk(self.lib.ecb_cost_set_constant_intrinsics(self.h, constant_intrinsics_mask(names)))
 
     # ---- fused reduce + inter-GPU exchange of the normal equations ----
     def exchange_buffer_bytes(self, n_ranks):
@@ -659,6 +686,12 @@ class LmState:
             self.lib.ecb_lm_destroy(self.h)
         except Exception:
             pass
+
+    def set_constant_intrinsics(self, names):
+        """intrinsics held at their start values (INTRINSIC_NAMES; empty: none); before begin(), EcbError(ERR_STATE) after"""
+        rc = self.lib.ecb_lm_set_constant_intrinsics(self.h, constant_intrinsics_mask(names))
+        if rc != OK:
+            raise EcbError(rc, "ecb_lm_set_constant_intrinsics: %s" % ("call it before begin()" if rc == ERR_STATE else "bad mask"))
 
     def begin(self, intr, rot, trans, packed):
         a = [np.ascontiguousarray(v, np.float64) for v in (intr, rot, trans, packed)]

@@ -73,9 +73,11 @@ struct ecb_ctx {
     void *cost = nullptr;
     // covariance workspace (ecb_lmdev.cu), kept for repeated calls with the same spline layout
     void *cov = nullptr;
-    // incremented by ecb_cost_setup and ecb_cost_set_rotation_model: a covariance computed before refers to other knots or
-    // another rotation tangent
+    // incremented by ecb_cost_setup, ecb_cost_set_rotation_model and a change of const_intrinsics: a covariance computed before
+    // refers to other knots, another rotation tangent or other free parameters
     uint64_t spline_gen = 0;
+    // intrinsics held constant in the spline stage (ecb_cost_set_constant_intrinsics): bit i = intrinsic i (fx fy cx cy k1 .. k5)
+    uint32_t const_intrinsics = 0;
     // staging of the host variant of ecb_pose_covariance (ecb_pose_cov.cu)
     DevBuf pose_io;
 };
@@ -95,6 +97,21 @@ struct EcbCovView {
     uint64_t spline_gen;
 };
 extern "C" int ecb_covariance_view(ecb_ctx *ctx, EcbCovView *v);
+
+// Constant intrinsics: the reduced problem of a Ceres SubsetManifold on the intrinsics block.  Once the packed normal equations
+// are assembled, the row and column of J^T J and the entry of J^T r of every constant intrinsic are zeroed; the Jacobi scale, the
+// clamped LM diagonal, the zero step component and the zero projected gradient follow from the unchanged LM code.  Entry (ri, ci)
+// of the assembled system or of the covariance: ri / ci = intrinsic index of its row / column, -1 for a control-point row or
+// column (and for the column of J^T r).  Mask 0 passes every entry unchanged.
+#define ECB_ALL_INTRINSICS 0x1FFu
+#ifdef __CUDACC__
+__host__ __device__ __forceinline__
+#else
+inline
+#endif
+double ecb_zero_constant(uint32_t mask, int ri, int ci, double v) {
+    return ((ri >= 0 && ((mask >> ri) & 1u)) || (ci >= 0 && ((mask >> ci) & 1u))) ? 0.0 : v;
+}
 
 int ecb_fail(ecb_ctx *ctx, int code, const char *fmt, ...);
 int ecb_reserve(ecb_ctx *ctx, DevBuf &b, size_t bytes);

@@ -805,6 +805,16 @@ int ecb_cost_set_rotation_model(ecb_ctx *ctx, int use_so3) {
     return ECB_OK;
 }
 
+int ecb_cost_set_constant_intrinsics(ecb_ctx *ctx, uint32_t mask) {
+    if (!ctx) return ECB_ERR_ARG;
+    if (mask > ECB_ALL_INTRINSICS) return ecb_fail(ctx, ECB_ERR_ARG, "constant intrinsics mask 0x%x has bits above the 9 intrinsics", mask);
+    if (mask != ctx->const_intrinsics) {
+        ctx->const_intrinsics = mask;
+        ++ctx->spline_gen;  // Z depends on the free parameters: a covariance computed before no longer answers ecb_pose_covariance
+    }
+    return ECB_OK;
+}
+
 int ecb_cost_spline_view(ecb_ctx *ctx, EcbSplineView *v) {
     if (!ctx || !ctx->cost) return ECB_ERR_STATE;
     const CostState *st = (const CostState *) ctx->cost;

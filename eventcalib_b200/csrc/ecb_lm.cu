@@ -177,7 +177,8 @@ struct ecb_lm {
     std::vector<double> g;          // J^T r at x (unscaled), internal order
     std::vector<double> scale, diag, step, delta;
     double cost = 0, radius = 0, decrease_factor = 2, model_cost_change = 0, candidate_cost = 0;
-    bool have_scale = false, reuse_diagonal = false;
+    bool have_scale = false, reuse_diagonal = false, begun = false;
+    uint32_t const_mask = 0;        // constant intrinsics (ecb_lm_set_constant_intrinsics)
     int iteration = 0, successful = 0, termination = ECB_LM_RUNNING, invalid_steps = 0;
     double gradient_max_norm = 0, step_norm = 0, x_norm = 0;
     std::vector<double> trace;
@@ -214,6 +215,14 @@ struct ecb_lm {
                     const int i = map[a], j = map[b];
                     if (i >= j) H.add(i, j, B[a * 33 + b]);
                 }
+            }
+        }
+        if (const_mask) {  // constant intrinsics: their rows / columns of J^T J and entries of J^T r become exact zeros
+            const int n = H.n;
+            for (int r = 0; r < NI; ++r) {
+                for (int j = 0; j < n; ++j) H.A[(size_t) r * n + j] = ecb_zero_constant(const_mask, r, -1, H.A[(size_t) r * n + j]);
+                for (int c = 0; c < NI; ++c) H.C[r * NI + c] = ecb_zero_constant(const_mask, r, c, H.C[r * NI + c]);
+                g[n + r] = ecb_zero_constant(const_mask, r, -1, g[n + r]);
             }
         }
         cost = packed[(size_t) n_spans * OUT_STRIDE];
@@ -283,12 +292,21 @@ void ecb_lm_destroy(ecb_lm *lm) { delete lm; }
 
 int ecb_lm_dimension(const ecb_lm *lm) { return lm ? lm->D : 0; }
 
+// intrinsics held at their start values (bit i = intrinsic i); before ecb_lm_begin only
+int ecb_lm_set_constant_intrinsics(ecb_lm *lm, uint32_t mask) {
+    if (!lm || mask > ECB_ALL_INTRINSICS) return ECB_ERR_ARG;
+    if (lm->begun) return ECB_ERR_STATE;
+    lm->const_mask = mask;
+    return ECB_OK;
+}
+
 // first evaluation at x (iteration 0)
 int ecb_lm_begin(ecb_lm *lm, const double *intr, const double *rot, const double *trans, const double *packed) {
     if (!lm || !intr || !rot || !trans || !packed) return ECB_ERR_ARG;
     lm->intr.assign(intr, intr + 9);
     lm->rot.assign(rot, rot + 4 * (size_t) lm->C);
     lm->trans.assign(trans, trans + 3 * (size_t) lm->C);
+    lm->begun = true;
     lm->assemble(packed);
     lm->iteration = 0;
     lm->successful = 0;
@@ -470,6 +488,7 @@ int ecb_calibrate(ecb_ctx *ctx, int n_splines, const int32_t *n_cp, double *intr
         ecb_lm_destroy(lm);
         return ecb_fail(ctx, ECB_ERR_ARG, "spline layout differs from ecb_cost_setup");
     }
+    ecb_lm_set_constant_intrinsics(lm, ctx->const_intrinsics);
     std::vector<double> packed((size_t) nd), ci(9), cr(4 * (size_t) tcp), ct(3 * (size_t) tcp);
     rc = ecb_cost_normal_eq(ctx, intrinsics, rot_cp, trans_cp, nullptr, packed.data(), nullptr);
     int st = rc ? rc : ecb_lm_begin(lm, intrinsics, rot_cp, trans_cp, packed.data());

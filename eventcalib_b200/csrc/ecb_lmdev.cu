@@ -106,8 +106,8 @@ __device__ __forceinline__ void quat_plus_dev(const double *x, const double *d, 
 __device__ __forceinline__ int local_idx(int o, int k) { return k < 3 ? 9 + 3 * o + k : 21 + 3 * o + (k - 3); }
 
 // ---- packed per-span normal equations -> band / arrow / corner / gradient, spans added in ascending order (the host
-// state machine's order, ecb_lm.cu assemble) --------------------------------------------------------------------------------
-__global__ void k_lm_assemble(LmDims d, LmBufs b, const int *go) {
+// state machine's order, ecb_lm.cu assemble); the rows / columns of constant intrinsics (cmask) come out as exact zeros ---------
+__global__ void k_lm_assemble(LmDims d, LmBufs b, const int *go, uint32_t cmask) {
     if (go && *go == 0) return;
     const int n = d.n;
     const long long total = (long long) n * NB + (long long) NI * n + NI * NI + d.D;
@@ -134,12 +134,12 @@ __global__ void k_lm_assemble(LmDims d, LmBufs b, const int *go) {
             const int s0 = max(0, lj - 3), s1 = min(lj, d.seg_ncp[sg] - 4);
             double v = 0.0;
             for (int ls = s0; ls <= s1; ++ls) v += b.ne[(size_t) (d.seg_span_off[sg] + ls) * OUT_STRIDE + r * 33 + local_idx(lj - ls, kj)];
-            b.Ha[q] = v;
+            b.Ha[q] = ecb_zero_constant(cmask, r, -1, v);
         } else if (e < (long long) n * NB + (long long) NI * n + NI * NI) {  // corner
             const int q = (int) (e - (long long) n * NB - (long long) NI * n), r = q / NI, c = q % NI;
             double v = 0.0;
             for (int s = 0; s < d.n_spans; ++s) v += b.ne[(size_t) s * OUT_STRIDE + max(r, c) * 33 + min(r, c)];
-            b.Hc[q] = v;
+            b.Hc[q] = ecb_zero_constant(cmask, r, c, v);
         } else {  // gradient
             const int i = (int) (e - (long long) n * NB - (long long) NI * n - NI * NI);
             double v = 0.0;
@@ -149,6 +149,7 @@ __global__ void k_lm_assemble(LmDims d, LmBufs b, const int *go) {
                 for (int ls = s0; ls <= s1; ++ls) v += b.ne[(size_t) (d.seg_span_off[sg] + ls) * OUT_STRIDE + 1089 + local_idx(li - ls, ki)];
             } else {
                 for (int s = 0; s < d.n_spans; ++s) v += b.ne[(size_t) s * OUT_STRIDE + 1089 + (i - n)];
+                v = ecb_zero_constant(cmask, i - n, -1, v);
             }
             b.g[i] = v;
         }
@@ -714,6 +715,9 @@ __global__ void k_lm_set_cost(LmBufs b, const double *v) { b.s->candidate_cost =
 // ---- covariance of the parameters: Z = H^-1 on the band / arrow pattern (selected inversion) -----------------------------------
 // ecb_covariance runs k_lm_assemble, k_lm_build, k_lm_factor and k_lm_corner unchanged on M = S H S with S = diag(H)^-1/2 (1 where
 // the diagonal is 0) and no damping (radius = +inf: the damping term dg / radius adds exactly 0), then the kernels below.
+// Constant intrinsics (cmask): their rows / columns of H are zero after k_lm_assemble; k_cov_begin gives them a unit diagonal, so
+// M is the free block and an identity block that the factorisation keeps apart exactly, and Z of the free block is the inverse of
+// H restricted to the free parameters.  k_cov_corner and k_cov_selinv write exact zeros into their rows / columns of Z.
 constexpr double COV_MIN_PIVOT = 1e-12;  // relative pivot L(j, j)^2 / M(j, j) at or below which the system counts as rank deficient
 constexpr int COV_THREADS = 256;
 constexpr int CW = NB - 1 + NI;          // selected-inversion window: 23 band rows + 9 intrinsics = 32
@@ -725,8 +729,9 @@ struct CovBufs {
 };
 
 // Jacobi equilibration to a unit diagonal and the state the LM kernels read
-__global__ void k_cov_begin(LmDims d, LmBufs b) {
+__global__ void k_cov_begin(LmDims d, LmBufs b, uint32_t cmask) {
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < d.D; i += gridDim.x * blockDim.x) {
+        if (i >= d.n && ((cmask >> (i - d.n)) & 1u)) b.Hc[(i - d.n) * (NI + 1)] = 1.0;  // constant intrinsic: unit diagonal
         const double h = h_diag(d, b, i);
         b.scale[i] = h > 0.0 ? 1.0 / sqrt(h) : 1.0;
         if (i < d.n) b.Lc[i] = 0.0;  // a pivot the factorisation does not reach (it stops a segment at a failed pivot) stays 0
@@ -780,7 +785,7 @@ __global__ void __launch_bounds__(1024) k_cov_pivots(LmDims d, LmBufs b, CovBufs
 }
 
 // Z_cc = (L_cc L_cc^T)^-1 of the 9 x 9 Schur factor: W = L_cc^-1 column by column (one thread each), Z_cc = W^T W
-__global__ void k_cov_corner(LmDims d, LmBufs b, CovBufs c) {
+__global__ void k_cov_corner(LmDims d, LmBufs b, CovBufs c, uint32_t cmask) {
     __shared__ double W[NI][NI];
     if (c.res[2] >= 0.0) return;
     const int t = threadIdx.x;
@@ -797,7 +802,7 @@ __global__ void k_cov_corner(LmDims d, LmBufs b, CovBufs c) {
         double v = 0.0;
         for (int k = lo; k < NI; ++k) v += W[k][r] * W[k][q];
         c.Zcs[t] = v;
-        c.Zc[t] = v * (b.scale[d.n + min(r, q)] * b.scale[d.n + lo]);  // the same rounding for (r, q) and (q, r): symmetric
+        c.Zc[t] = ecb_zero_constant(cmask, r, q, v * (b.scale[d.n + min(r, q)] * b.scale[d.n + lo]));  // the same rounding for (r, q) and (q, r): symmetric
     }
 }
 
@@ -807,7 +812,7 @@ __global__ void k_cov_corner(LmDims d, LmBufs b, CovBufs c) {
 // for R = the next 23 band rows + the intrinsics (the band reach of the block's last column).  Every Z_{R,K} lies in the
 // 32 x 32 window of Z the previous block left in shared memory; the window then slides up by one block.  The result equals the
 // scalar recurrence Z_ij = -(1 / L_jj) sum_{k in N(j)} Z_ik L_kj run column by column.  Outputs are unscaled by S on the way out.
-__global__ void __launch_bounds__(COV_THREADS) k_cov_selinv(LmDims d, LmBufs b, CovBufs c) {
+__global__ void __launch_bounds__(COV_THREADS) k_cov_selinv(LmDims d, LmBufs b, CovBufs c, uint32_t cmask) {
     __shared__ double Zw[2][CW * CW];  // window: index w < 23 -> band row j0 + 6 + w of the segment, w >= 23 -> intrinsic w - 23
     __shared__ double LB[FB][FB], LK[NB - FB + NI][FB], T[NB - FB + NI][FB], Wb[FB][FB], Y[CW][FB], ZB[FB][FB], rdg[FB];
     if (c.res[2] >= 0.0) return;
@@ -884,7 +889,7 @@ __global__ void __launch_bounds__(COV_THREADS) k_cov_selinv(LmDims d, LmBufs b, 
                 c.Zb[(size_t) (g0 + k) * NB + r] = v;
             } else {
                 const int a = (e - FB * NB) / FB, k = (e - FB * NB) % FB;
-                c.Zx[(size_t) a * n + g0 + k] = Y[NB - 1 + a][k] * b.scale[n + a] * b.scale[g0 + k];
+                c.Zx[(size_t) a * n + g0 + k] = ecb_zero_constant(cmask, a, -1, Y[NB - 1 + a][k] * b.scale[n + a] * b.scale[g0 + k]);
             }
         }
         for (int e = tid; e < CW * CW; e += COV_THREADS) {
@@ -915,6 +920,7 @@ struct ecb_lm_device {
     void *recv[ECB_MAX_PEERS] = {};
     double *d_cand_cost = nullptr;
     uint32_t generation = 0;
+    uint32_t const_intrinsics = 0;  // the context's constant intrinsics at creation
     bool begun = false;
     // ECB_LM_TIMING=1: CUDA events around the phases of every enqueued iteration (solve | candidate cost | scalar exchange |
     // decide + commit | normal equations (+ exchange) | assemble), averaged and printed to stderr by ecb_lm_device_result
@@ -939,6 +945,7 @@ int ecb_lm_device_create(ecb_ctx *ctx, int n_splines, const int32_t *n_cp, const
     cudaSetDevice(ctx->device);
     ecb_lm_device *lm = new ecb_lm_device();
     lm->ctx = ctx;
+    lm->const_intrinsics = ctx->const_intrinsics;
     if (opt) lm->opt = *opt; else ecb_lm_default_options(&lm->opt);
     const int n = 6 * C, D = n + NI;
     // integer tables
@@ -1050,7 +1057,7 @@ int ecb_lm_device_begin(ecb_lm_device *lm, const double *intrinsics, const doubl
     if ((rc = ecb_h2d(ctx, lm->bufs.s, &h, sizeof h))) return rc;
     if ((rc = lmdev_normal_eq(lm))) return rc;
     const int blocks = ctx->sm_count * 2;
-    k_lm_assemble<<<blocks, 256, 0, ctx->stream>>>(lm->dims, lm->bufs, nullptr);
+    k_lm_assemble<<<blocks, 256, 0, ctx->stream>>>(lm->dims, lm->bufs, nullptr, lm->const_intrinsics);
     ECB_LAUNCHED(ctx);
     k_lm_init<<<std::min(blocks, (lm->dims.D + 255) / 256), 256, 0, ctx->stream>>>(lm->dims, lm->bufs, lm->opt);
     ECB_LAUNCHED(ctx);
@@ -1103,7 +1110,7 @@ int ecb_lm_device_iterate(ecb_lm_device *lm, int n_iterations) {
         mark(4);
         if ((rc = lmdev_normal_eq(lm))) return rc;
         mark(5);
-        k_lm_assemble<<<blocks, 256, 0, ctx->stream>>>(lm->dims, lm->bufs, &s->accepted);
+        k_lm_assemble<<<blocks, 256, 0, ctx->stream>>>(lm->dims, lm->bufs, &s->accepted, lm->const_intrinsics);
         k_lm_gradnorm<<<1, 1024, 0, ctx->stream>>>(lm->dims, lm->bufs, lm->opt, &s->accepted);
         ctx->launches += 2;
         mark(6);
@@ -1264,14 +1271,15 @@ extern "C" int ecb_covariance(ecb_ctx *ctx, int n_splines, const int32_t *n_cp, 
         if ((rc = ecb_cost_dev_normal_eq(ctx, b.x, nullptr, b.ne))) return rc;
     }
     const int blocks = ctx->sm_count * 2;
-    k_lm_assemble<<<blocks, 256, 0, ctx->stream>>>(d, b, nullptr);
-    k_cov_begin<<<std::min(blocks, (d.D + 255) / 256), 256, 0, ctx->stream>>>(d, b);
+    const uint32_t cmask = ctx->const_intrinsics;
+    k_lm_assemble<<<blocks, 256, 0, ctx->stream>>>(d, b, nullptr, cmask);
+    k_cov_begin<<<std::min(blocks, (d.D + 255) / 256), 256, 0, ctx->stream>>>(d, b, cmask);
     k_lm_build<<<blocks, 256, 0, ctx->stream>>>(d, b, lm->opt);
     k_lm_factor<<<d.n_seg, FACTOR_THREADS, 0, ctx->stream>>>(d, b);
     k_lm_corner<<<1, 32, 0, ctx->stream>>>(d, b);
     k_cov_pivots<<<1, 1024, 0, ctx->stream>>>(d, b, w->c);
-    k_cov_corner<<<1, 96, 0, ctx->stream>>>(d, b, w->c);
-    k_cov_selinv<<<d.n_seg, COV_THREADS, 0, ctx->stream>>>(d, b, w->c);
+    k_cov_corner<<<1, 96, 0, ctx->stream>>>(d, b, w->c, cmask);
+    k_cov_selinv<<<d.n_seg, COV_THREADS, 0, ctx->stream>>>(d, b, w->c, cmask);
     ctx->launches += 8;
     if ((rc = ecb_check(ctx, cudaGetLastError(), "covariance kernels"))) return rc;
     double res[3];
@@ -1279,11 +1287,12 @@ extern "C" int ecb_covariance(ecb_ctx *ctx, int n_splines, const int32_t *n_cp, 
     int64_t m = n_residuals_total;
     if (m == 0 && (rc = ecb_cost_layout(ctx, nullptr, nullptr, &m, nullptr))) return rc;
     const int deficient = (int) res[2];
+    const int dim = d.D - __builtin_popcount(cmask);  // free parameters
     if (summary) {
         summary->cost = res[0];
         summary->n_residuals = m;
-        summary->dimension = d.D;
-        summary->sigma2 = m > d.D ? 2.0 * res[0] / (double) (m - d.D) : NAN;
+        summary->dimension = dim;
+        summary->sigma2 = m > dim ? 2.0 * res[0] / (double) (m - dim) : NAN;
         summary->min_relative_pivot = res[1];
         summary->deficient_index = deficient;
     }

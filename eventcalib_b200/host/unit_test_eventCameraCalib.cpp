@@ -21,6 +21,12 @@
 // every GPU holds the records of its block, one host thread + context per GPU (include/ecb/multi_gpu.hpp); the spline
 // optimisation shards the residuals the same way and sums the normal equations over NVLink inside the kernels.  The frames,
 // candidates and key-frame map do not depend on the number of GPUs.
+//
+// ECB_CONSTANT_INTRINSICS=k3,k4,k5 (comma- or space-separated names of fx fy cx cy k1 .. k5; k1 .. k5 are the spline stage's
+// inverse radial polynomial, not the YAML's Fix_K* OpenCV coefficients) holds those intrinsics at their initial values in the
+// spline optimisation, which the reference does not offer: it prints a "Constant intrinsics:" line before the optimisation, and
+// the covariance files (ECB_COVARIANCE, ECB_TRAJECTORY_COVARIANCE) are conditional on them.  An unknown name, or the variable
+// together with ECB_REFERENCE_SIGNATURES (the reference's constructor frees all nine), ends the program with exit code 1.
 #include <algorithm>
 #include <cstdio>
 #include <cstdlib>
@@ -71,6 +77,22 @@ int main(int argc, char **argv) {
         return 1;
     }
     std::cout.precision(8);
+    uint32_t constIntrinsics = 0;  // checked before any file or GPU work
+    if (const char *ci = getenv("ECB_CONSTANT_INTRINSICS")) {
+        if (getenv("ECB_REFERENCE_SIGNATURES")) {
+            std::cerr << "ecb: ECB_CONSTANT_INTRINSICS cannot be combined with ECB_REFERENCE_SIGNATURES (the reference's "
+                         "EventCalibSpline frees all 9 intrinsics)" << std::endl;
+            return 1;
+        }
+        std::string unknown;
+        const int m = ecb::constantIntrinsicsMask(ci, &unknown);
+        if (m < 0) {
+            std::cerr << "ecb: ECB_CONSTANT_INTRINSICS: unknown intrinsic '" << unknown << "' (names: fx fy cx cy k1 k2 k3 k4 k5)"
+                      << std::endl;
+            return 1;
+        }
+        constIntrinsics = (uint32_t) m;
+    }
     Settings fs;
     if (!fs.open(argv[1])) {
         std::cerr << "Failed to open settings file at: " << argv[1] << std::endl;
@@ -363,6 +385,19 @@ int main(int argc, char **argv) {
             return 0;
         }
         ShardedCalibSpline spline(opt_events, segments, intrinsics, motionTimeStep, pattern->circleRadius, useSO3);
+        if (constIntrinsics) {
+            static const char *const names[9] = {"fx", "fy", "cx", "cy", "k1", "k2", "k3", "k4", "k5"};
+            std::ostringstream line;
+            line.precision(17);
+            line << "Constant intrinsics:";
+            for (int i = 0; i < 9; ++i)
+                if ((constIntrinsics >> i) & 1u) line << " " << names[i] << " = " << intrinsics[(size_t) i];
+            std::cout << line.str() << std::endl;
+            if (spline.setConstantIntrinsics(constIntrinsics) != ECB_OK) {
+                std::cerr << "ecb: " << spline.lastError() << std::endl;
+                return 1;
+            }
+        }
         std::vector<std::array<double, 3>> landmarks;
         const std::vector<double> board = ini.boardPoints();
         for (size_t k = 0; k + 2 < board.size(); k += 3) landmarks.push_back({board[k], board[k + 1], board[k + 2]});

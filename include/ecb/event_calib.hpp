@@ -43,6 +43,30 @@
 #include "dbscan.h"
 #include "image_lite.hpp"
 
+namespace ecb {
+// Constant intrinsics of the spline stage (ecb_cost_set_constant_intrinsics) from comma- or space-separated names of
+// fx fy cx cy k1 k2 k3 k4 k5 (k1 .. k5: the inverse radial polynomial, not OpenCV's coefficients).  Returns the mask (0 for no
+// names), or -1 with the first unknown token in *unknown.
+inline int constantIntrinsicsMask(const std::string &names, std::string *unknown = nullptr) {
+    static const char *const kNames[9] = {"fx", "fy", "cx", "cy", "k1", "k2", "k3", "k4", "k5"};
+    std::string list = names;
+    std::replace(list.begin(), list.end(), ',', ' ');
+    std::istringstream is(list);
+    std::string tok;
+    int mask = 0;
+    while (is >> tok) {
+        int i = 0;
+        while (i < 9 && tok != kNames[i]) ++i;
+        if (i == 9) {
+            if (unknown) *unknown = tok;
+            return -1;
+        }
+        mask |= 1 << i;
+    }
+    return mask;
+}
+}  // namespace ecb
+
 namespace opengv2 {
 
 struct Vec2 {
@@ -790,6 +814,9 @@ public:
             throw std::logic_error(ecb_last_error(ev_->ctx));  // HuberLoss(0.2 r), EventCalibSpline.cpp:197
         ecb_cost_set_rotation_model(ev_->ctx, useSO3_ ? 1 : 0);
     }
+    // Intrinsics held at their current values by optimize() (bit i = intrinsic i in the OFFSET_* order, see
+    // ecb::constantIntrinsicsMask); covariance() is then conditional on them.  0 (default): all 9 free, as in the reference.
+    int setConstantIntrinsics(uint32_t mask) { return ecb_cost_set_constant_intrinsics(ev_->ctx, mask); }
     // ---- the reference constructor's own set-up (EventCalibSpline.cpp:14-113) from the key frames of the map ----
     struct KeyPose {
         double timeStamp;
@@ -985,7 +1012,8 @@ public:
         return true;
     }
     // Uncertainty of the calibration (ecb_covariance): Z = H^-1 at the current point (where optimize() left it) on the band /
-    // arrow pattern, sigma^2 = 2 cost / (residuals - parameters), standard deviation of parameter i = sqrt(sigma^2 Z_ii).
+    // arrow pattern, sigma^2 = 2 cost / (residuals - parameters), standard deviation of parameter i = sqrt(sigma^2 Z_ii).  With
+    // constant intrinsics (setConstantIntrinsics) Z is conditional on them: their rows / columns are 0, and so their deviation.
     struct Covariance {
         std::array<double, 81> intrinsics{};  // Z of fx fy cx cy k1 .. k5, row major
         std::vector<double> band;             // 6C x 24: Z(j + r, j) at [j * 24 + r], control point c owns rows 6c .. 6c+5

@@ -187,6 +187,15 @@ public:
         for (auto &s : events->shard) sp_.emplace_back(new EventCalibSpline(s, segments, intrinsics, motionTimeStep, circleRadius, useSO3));
         for (auto &s : segments) n_cp_.push_back((int32_t) (s.rot_cp.size() / 4));
     }
+    // constant intrinsics (EventCalibSpline::setConstantIntrinsics) on every shard's context: every rank zeroes the same rows of
+    // the same summed normal equations, so the replicated state machine and the covariance stay bit-identical across ranks
+    int setConstantIntrinsics(uint32_t mask) {
+        for (auto &s : sp_) {
+            const int rc = s->setConstantIntrinsics(mask);
+            if (rc != ECB_OK) return rc;
+        }
+        return ECB_OK;
+    }
     int64_t associate(const std::vector<KeyFrame> &kf, const std::vector<std::array<double, 3>> &landmarks) {
         std::vector<int64_t> n(sp_.size(), 0);
         forEachShard((int) sp_.size(), [&](int g) { n[(size_t) g] = sp_[(size_t) g]->associate(kf, landmarks); });

@@ -196,6 +196,18 @@ int ecb_cost_setup(ecb_ctx *ctx, int n_splines, const int32_t *n_cp, const doubl
  *               LocalParameterizationSO3 (hpp:65-156, BsplineSO3.hpp:190-221); rot_cp are then Sophus::SO3d coefficients (x,y,z,w)
  * Also selects the Plus operation of the host LM step (ecb_lm_options.rotation_model must match). */
 int ecb_cost_set_rotation_model(ecb_ctx *ctx, int use_so3);
+/* Intrinsics held constant in the spline optimisation.  Bit i of mask = intrinsic i in the order fx fy cx cy k1 k2 k3 k4 k5 (the
+ * order of every intrinsics array here).  k1 .. k5 are the coefficients of the INVERSE radial polynomial of the spline stage, not
+ * OpenCV's distortion coefficients (the YAML's Fix_K* keys name those).  0 (default): all 9 are free, as in the reference.
+ * The optimisation is the reduced problem, what Ceres does with a SubsetManifold on the intrinsics block: the rows and columns of
+ * the constant intrinsics in J^T J and their entries of J^T r are zeroed once the normal equations are assembled, so their step is
+ * exactly 0 and they keep their start values exactly (==).  The parameter-tolerance test still uses |x| of the full vector.
+ * ecb_covariance then returns the covariance conditional on the constant intrinsics: Z = the inverse of H restricted to the free
+ * parameters, exact zeros in the rows and columns of the constant ones, dimension = D - popcount(mask).
+ * A property of the context: it survives ecb_cost_setup.  ecb_calibrate and ecb_covariance read it at each call,
+ * ecb_lm_device_create captures it.  Changing it makes ecb_pose_covariance return ECB_ERR_STATE until the next ecb_covariance.
+ * mask > 0x1FF returns ECB_ERR_ARG. */
+int ecb_cost_set_constant_intrinsics(ecb_ctx *ctx, uint32_t mask);
 /* total control points, total span blocks (sum of n_cp-3), residual count, doubles in the packed result */
 int ecb_cost_layout(ecb_ctx *ctx, int32_t *total_cp, int32_t *total_spans, int64_t *n_residuals, int64_t *out_doubles);
 /* Residual blocks from the loaded events (association loop of optimize(), :157-192, with findCenter,
@@ -284,6 +296,8 @@ void ecb_lm_default_options(ecb_lm_options *o);
 ecb_lm *ecb_lm_create(int n_splines, const int32_t *n_cp, const ecb_lm_options *opt);
 void ecb_lm_destroy(ecb_lm *lm);
 int ecb_lm_dimension(const ecb_lm *lm);
+/* constant intrinsics of this state machine (mask as ecb_cost_set_constant_intrinsics); before ecb_lm_begin, ECB_ERR_STATE after */
+int ecb_lm_set_constant_intrinsics(ecb_lm *lm, uint32_t mask);
 int ecb_lm_begin(ecb_lm *lm, const double *intrinsics, const double *rot_cp, const double *trans_cp, const double *packed);
 int ecb_lm_propose(ecb_lm *lm, double *cand_intrinsics, double *cand_rot_cp, double *cand_trans_cp);
 int ecb_lm_feedback(ecb_lm *lm, double candidate_cost);
@@ -339,7 +353,9 @@ int ecb_calibrate_device(ecb_lm_device *lm, double *intrinsics, double *rot_cp, 
  *   cov_intrinsics[9 x 9]; cov_band[6C x 24] = Z(j + r, j) at [j * 24 + r] (0 past the end of a segment); cov_cross[9 x 6C] =
  *   Z(intrinsic i, j) at [i * 6C + j].  Output pointers may be NULL.
  * A relative pivot L(j,j)^2 / M(j,j) <= 1e-12 or a zero diagonal (a control point without residuals, an intrinsic nothing
- * constrains) returns ECB_FAILED with summary->deficient_index = j and writes no covariance; deficient_index is -1 otherwise. */
+ * constrains) returns ECB_FAILED with summary->deficient_index = j and writes no covariance; deficient_index is -1 otherwise.
+ * With constant intrinsics (ecb_cost_set_constant_intrinsics) Z is conditional on them: their rows and columns of cov_intrinsics and
+ * cov_cross are exact zeros, they are never deficient, and dimension (the D of sigma2) counts the free parameters only. */
 typedef struct {
     double cost, sigma2, min_relative_pivot;  /* sigma2 is NaN when n_residuals <= dimension */
     int64_t n_residuals;
