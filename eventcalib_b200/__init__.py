@@ -54,6 +54,18 @@ class CovarianceSummary(C.Structure):
                 ("dimension", C.c_int32), ("deficient_index", C.c_int32)]
 
 
+class ResidualGroup(C.Structure):
+    """ecb_residual_group: statistics of a group of raw residuals r (board units, not pixels)"""
+    _fields_ = [("count", C.c_int64), ("n_downweighted", C.c_int64), ("sum", C.c_double), ("sum_sq", C.c_double),
+                ("max_abs", C.c_double), ("cost", C.c_double)]
+
+
+RESIDUAL_GROUP_DTYPE = np.dtype([("count", "<i8"), ("n_downweighted", "<i8"), ("sum", "<f8"), ("sum_sq", "<f8"),
+                                 ("max_abs", "<f8"), ("cost", "<f8")])
+assert RESIDUAL_GROUP_DTYPE.itemsize == C.sizeof(ResidualGroup)
+RESIDUALS_BY = {"keyframe": 0, "circle": 1, "sensor_cell": 2}
+
+
 # the order of every intrinsics array (ecb_residual.h): bit i of a constant-intrinsics mask is INTRINSIC_NAMES[i].  In the spline
 # stage k1 .. k5 are the coefficients of the inverse radial polynomial, not OpenCV's distortion coefficients.
 INTRINSIC_NAMES = ("fx", "fy", "cx", "cy", "k1", "k2", "k3", "k4", "k5")
@@ -91,7 +103,7 @@ SYMBOLS = ["ecb_ctx_create", "ecb_ctx_destroy", "ecb_last_error", "ecb_launch_co
            "ecb_lm_state", "ecb_lm_trace", "ecb_calibrate", "ecb_lm_device_create", "ecb_lm_device_destroy",
            "ecb_lm_device_set_exchange", "ecb_lm_device_begin", "ecb_lm_device_iterate", "ecb_lm_device_running",
            "ecb_lm_device_result", "ecb_calibrate_device", "ecb_covariance", "ecb_pose_covariance",
-           "ecb_pose_covariance_device"]
+           "ecb_pose_covariance_device", "ecb_cost_residuals", "ecb_cost_residual_groups"]
 
 _lib = None
 
@@ -156,6 +168,8 @@ def load_library():
     lib.ecb_cost_set_residuals.argtypes = [vp, vp, vp, vp, vp, i64]
     lib.ecb_cost_eval.argtypes = [vp, vp, vp, vp, vp]
     lib.ecb_cost_normal_eq.argtypes = [vp, vp, vp, vp, vp, vp, vp]
+    lib.ecb_cost_residuals.argtypes = [vp, vp, vp, vp, vp, vp]
+    lib.ecb_cost_residual_groups.argtypes = [vp, vp, vp, vp, i32, vp, i32, i32, vp, i32, C.POINTER(C.c_int), vp]
     lib.ecb_lm_default_options.argtypes = [C.POINTER(LmOptions)]
     lib.ecb_lm_default_options.restype = None
     lib.ecb_lm_create.argtypes = [i32, vp, C.POINTER(LmOptions)]
@@ -522,6 +536,38 @@ class Context:
         ns = lay["total_spans"]
         blk = out[:ns * 1122].reshape(ns, 1122)
         return c.value, blk[:, :1089].reshape(ns, 33, 33).copy(), blk[:, 1089:].copy()
+
+    def cost_residuals(self, intr, rot, trans, d_out=None, host=True):
+        """Raw residuals r_k = ||X_w - L|| - radius of every record at the point (ecb_cost_residuals), in the order of
+        cost_association(): a distance on the board plane in the units of the board points, NOT pixels.  Returns an ndarray
+        (float64, n_residuals) when host=True; else leaves them in d_out (device pointer, or None for the context's own buffer),
+        enqueued on the context's stream, and returns None."""
+        a = [np.ascontiguousarray(v, np.float64) for v in (intr, rot, trans)]
+        d = C.c_void_p(d_out) if d_out else None
+        if not host:
+            self._chk(self.lib.ecb_cost_residuals(self.h, _ptr(a[0]), _ptr(a[1]), _ptr(a[2]), d, None))
+            return None
+        out = np.zeros(max(self.cost_layout()["n_residuals"], 1))
+        self._chk(self.lib.ecb_cost_residuals(self.h, _ptr(a[0]), _ptr(a[1]), _ptr(a[2]), d, _ptr(out)))
+        return out[:self.cost_layout()["n_residuals"]]
+
+    def residual_groups(self, intr, rot, trans, by, kf_t=None, cell_px=16):
+        """Statistics of the raw residuals (board units, not pixels) per group (ecb_cost_residual_groups).  by: "keyframe"
+        (kf_t: the stamps given to cost_associate), "circle" or "sensor_cell" (cells of cell_px pixels, row major).  Returns
+        (groups, total) as numpy structured arrays of RESIDUAL_GROUP_DTYPE (count, n_downweighted, sum, sum_sq, max_abs, cost);
+        total has shape () and covers every record."""
+        if by not in RESIDUALS_BY:
+            raise ValueError("by must be one of %s" % ", ".join(RESIDUALS_BY))
+        a = [np.ascontiguousarray(v, np.float64) for v in (intr, rot, trans)]
+        kf = np.ascontiguousarray(kf_t, np.float64) if kf_t is not None else None
+        nk = len(kf) if kf is not None else 0
+        args = (self.h, _ptr(a[0]), _ptr(a[1]), _ptr(a[2]), RESIDUALS_BY[by], _ptr(kf), nk, int(cell_px))
+        ng = C.c_int(0)
+        self._chk(self.lib.ecb_cost_residual_groups(*args, None, 0, C.byref(ng), None))
+        groups = np.zeros(max(ng.value, 1), RESIDUAL_GROUP_DTYPE)
+        total = np.zeros((), RESIDUAL_GROUP_DTYPE)
+        self._chk(self.lib.ecb_cost_residual_groups(*args, _ptr(groups), ng.value, C.byref(ng), _ptr(total)))
+        return groups[:ng.value], total
 
     def calibrate(self, n_cp, intr, rot, trans, options=None, trace_rows=256):
         """EventCalibSpline::optimize on one GPU: returns (intr, rot, trans, summary dict, trace[rows,4])."""

@@ -241,6 +241,7 @@ int64_t ecb_num_events(const ecb_ctx *ctx) { return ctx ? ctx->n_events : 0; }
 
 static int unpack_events(ecb_ctx *ctx, const void *d_raw, int64_t n) {
     int rc;
+    ++ctx->events_gen;
     if ((rc = ecb_reserve(ctx, ctx->ev_t, (size_t) n * 8))) return rc;
     if ((rc = ecb_reserve(ctx, ctx->ev_xyp, (size_t) n * 4))) return rc;
     if ((rc = ecb_reserve(ctx, ctx->ev_flag, 16))) return rc;

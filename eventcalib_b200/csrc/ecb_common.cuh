@@ -80,6 +80,8 @@ struct ecb_ctx {
     uint32_t const_intrinsics = 0;
     // staging of the host variant of ecb_pose_covariance (ecb_pose_cov.cu)
     DevBuf pose_io;
+    // incremented by every event load: the residual report by key frame needs the events its association read
+    uint64_t events_gen = 0;
 };
 
 // the splines of ecb_cost_setup on the device (ecb_cost.cu); ECB_ERR_STATE before the setup
@@ -112,6 +114,11 @@ inline
 double ecb_zero_constant(uint32_t mask, int ri, int ci, double v) {
     return ((ri >= 0 && ((mask >> ri) & 1u)) || (ci >= 0 && ((mask >> ci) & 1u))) ? 0.0 : v;
 }
+
+// Stable LSD radix sort (ecb_gridhash.cu) of (key, idx) pairs by the low `bits` bits of key, 8 bits per pass, n >= 1 and
+// n < 2^32; the result ends in key[*res] / idx[*res] (ping-pong buffers 0 / 1).  hist: gh_radix_hist_bytes(n) bytes.
+int gh_radix_sort(ecb_ctx *ctx, uint64_t *key[2], uint32_t *idx[2], int64_t n, int bits, uint32_t *hist, int *res);
+size_t gh_radix_hist_bytes(int64_t n);
 
 int ecb_fail(ecb_ctx *ctx, int code, const char *fmt, ...);
 int ecb_reserve(ecb_ctx *ctx, DevBuf &b, size_t bytes);

@@ -15,6 +15,7 @@
 //   k_reduce_*      fixed-order reduction of the per-work-item partials -> run-to-run identical J^T J / J^T r / cost
 //   k_cost          cost-only evaluation (LM step acceptance)
 #include <stdlib.h>
+#include <string.h>
 
 #include <algorithm>
 #include <vector>
@@ -48,6 +49,12 @@ struct CostState {
     DevBuf span_start, items, part, out, params, cost_part, flags;
     DevBuf ev_flag, ev_cnt, ev_tag, kf_t, kf_circ, kf_c32, lm_tab, sel_event, sel_circle;
     std::vector<int64_t> h_span_start;
+    // the records come from an association (event_index / circle_id exist) over K key frames, n_circ circles, and the events of
+    // ctx->events_gen == assoc_events_gen
+    bool assoc = false;
+    int assoc_K = 0, assoc_n_circ = 0;
+    uint64_t assoc_events_gen = 0;
+    DevBuf rep_r, rep_key[2], rep_idx[2], rep_hist, rep_start, rep_out, rep_kf;  // residual report (ecb_cost_residual_groups)
     uint64_t xch_last_epoch = 0;   // ecb_cost_normal_eq_exchange: last epoch sent / generation of the caller's sequence
     uint32_t xch_generation = 0;
 };
@@ -654,6 +661,128 @@ __global__ void __launch_bounds__(AS_THREADS) k_assoc_write(const AssocArgs a, c
     }
 }
 
+// ---------------------------------------------------------------------------- residual report ----
+// k_residuals   the loads and the residual call of k_cost, storing the raw residual r_k (board units) instead of the cost
+// k_group_keys  group of every record (key) and its index; a stable radix sort of (key, index) keeps record order per group
+// k_group_start lower bounds of every group in the sorted keys (as k_span_start)
+// k_group_reduce one block per group, fixed shape: thread-strided partials in record order, then a shared-memory tree
+constexpr int RG_THREADS = 256;
+
+template <bool SO3>
+__global__ void __launch_bounds__(256) k_residuals(const double *__restrict__ obs, const double *__restrict__ lm,
+                                                   const int *__restrict__ circ, const double *__restrict__ lm_tab,
+                                                   const double *__restrict__ basis, const int *__restrict__ cp0, int64_t n,
+                                                   const double *__restrict__ params, int total_cp, double radius, double huber,
+                                                   double *__restrict__ out) {
+    const double *intr = params, *rot = params + 9, *trans = params + 9 + 4 * (size_t) total_cp;
+    for (int64_t k = (int64_t) blockIdx.x * 256 + threadIdx.x; k < n; k += (int64_t) gridDim.x * 256) {
+        const int c0 = cp0[k];
+        const double4 b4 = reinterpret_cast<const double4 *>(basis)[k];
+        const double b[4] = {b4.x, b4.y, b4.z, b4.w};
+        const double2 o = reinterpret_cast<const double2 *>(obs)[k];
+        const double *L = circ ? lm_tab + 3 * circ[k] : lm + 3 * k;
+        const double Lx = L[0], Ly = L[1], Lz = L[2];
+        out[k] = SO3 ? ecb_residual_so3<false>(intr, rot + 4 * (size_t) c0, trans + 3 * (size_t) c0, b, o.x, o.y, Lx, Ly, Lz, radius,
+                                               huber, nullptr).raw
+                     : ecb_residual<false>(intr, rot + 4 * (size_t) c0, trans + 3 * (size_t) c0, b, o.x, o.y, Lx, Ly, Lz, radius, huber,
+                                           nullptr).raw;
+    }
+}
+
+struct GroupKeyArgs {
+    int by;                    // ECB_RESIDUALS_BY_*
+    const int64_t *sel_event;  // association: event of record k
+    const int *sel_circle;     // association: circle of record k
+    const double *ev_t, *kf_t;
+    int K;
+    const double *obs;
+    int width, height, cell, ncx;
+    uint32_t outside;          // key of the records that count in the total only (= number of groups)
+};
+
+__global__ void k_group_keys(const GroupKeyArgs a, int64_t n, uint64_t *__restrict__ key, uint32_t *__restrict__ idx) {
+    for (int64_t k = (int64_t) blockIdx.x * blockDim.x + threadIdx.x; k < n; k += (int64_t) gridDim.x * blockDim.x) {
+        uint32_t g;
+        if (a.by == ECB_RESIDUALS_BY_KEYFRAME) {
+            g = (uint32_t) nearest_kf(a.kf_t, a.K, a.ev_t[a.sel_event[k]]);
+        } else if (a.by == ECB_RESIDUALS_BY_CIRCLE) {
+            g = (uint32_t) a.sel_circle[k];
+        } else {
+            const double2 o = reinterpret_cast<const double2 *>(a.obs)[k];
+            if (o.x >= 0.0 && o.x < (double) a.width && o.y >= 0.0 && o.y < (double) a.height)
+                g = (uint32_t) floor(o.y / a.cell) * (uint32_t) a.ncx + (uint32_t) floor(o.x / a.cell);
+            else
+                g = a.outside;  // also NaN
+        }
+        key[k] = g;
+        idx[k] = (uint32_t) k;
+    }
+}
+
+// start[g] = first sorted position with key >= g, g = 0 .. n_keys (start[n_keys] = n)
+__global__ void k_group_start(const uint64_t *__restrict__ skey, int64_t n, int n_keys, int64_t *__restrict__ start) {
+    const int g = blockIdx.x * blockDim.x + threadIdx.x;
+    if (g > n_keys) return;
+    int64_t lo = 0, hi = n;
+    while (lo < hi) {
+        const int64_t m = (lo + hi) >> 1;
+        if (skey[m] < (uint64_t) g) lo = m + 1; else hi = m;
+    }
+    start[g] = lo;
+}
+
+__global__ void __launch_bounds__(RG_THREADS) k_group_reduce(const double *__restrict__ r, const uint32_t *__restrict__ sidx,
+                                                             const int64_t *__restrict__ start, double huber,
+                                                             ecb_residual_group *__restrict__ out) {
+    __shared__ double sh[4][RG_THREADS];
+    __shared__ long long shn[RG_THREADS];
+    const int g = blockIdx.x, t = threadIdx.x;
+    const int64_t b = start[g], e = start[g + 1];
+    const double a2 = huber * huber;
+    long long ndw = 0;
+    double sum = 0.0, ssq = 0.0, mx = 0.0, cost = 0.0;
+    for (int64_t i = b + t; i < e; i += RG_THREADS) {
+        const double v = r[sidx[i]];
+        // the Huber expressions of ecb_residual.h: rho = r^2 inside the band, 2 delta |r| - delta^2 outside
+        const double s2 = v * v;
+        double rho = s2;
+        if (s2 > a2) {
+            rho = 2.0 * huber * fabs(v) - a2;
+            ++ndw;
+        }
+        sum += v;
+        ssq += s2;
+        mx = fmax(mx, fabs(v));
+        cost += 0.5 * rho;
+    }
+    sh[0][t] = sum;
+    sh[1][t] = ssq;
+    sh[2][t] = mx;
+    sh[3][t] = cost;
+    shn[t] = ndw;
+    __syncthreads();
+    for (int o = RG_THREADS / 2; o > 0; o >>= 1) {
+        if (t < o) {
+            sh[0][t] += sh[0][t + o];
+            sh[1][t] += sh[1][t + o];
+            sh[2][t] = fmax(sh[2][t], sh[2][t + o]);
+            sh[3][t] += sh[3][t + o];
+            shn[t] += shn[t + o];
+        }
+        __syncthreads();
+    }
+    if (t == 0) {
+        ecb_residual_group q;
+        q.count = e - b;
+        q.n_downweighted = shn[0];
+        q.sum = sh[0][0];
+        q.sum_sq = sh[1][0];
+        q.max_abs = sh[2][0];
+        q.cost = sh[3][0];
+        out[g] = q;
+    }
+}
+
 int prepare_records(ecb_ctx *ctx, CostState *st, bool have_basis = false) {
     int rc;
     const int64_t n = st->n_res;
@@ -748,7 +877,8 @@ void ecb_cost_free(ecb_ctx *ctx) {
     DevBuf *bufs[] = {&st->d_knots, &st->d_knot_off, &st->d_ncp, &st->d_cp_off, &st->d_span_off, &st->obs, &st->lm, &st->tt,
                       &st->spl, &st->basis, &st->cp0, &st->span, &st->span_start, &st->items, &st->part, &st->out, &st->params,
                       &st->cost_part, &st->flags, &st->ev_flag, &st->ev_cnt, &st->ev_tag, &st->kf_t, &st->kf_circ, &st->kf_c32, &st->lm_tab,
-                      &st->sel_event, &st->sel_circle};
+                      &st->sel_event, &st->sel_circle, &st->rep_r, &st->rep_key[0], &st->rep_key[1], &st->rep_idx[0],
+                      &st->rep_idx[1], &st->rep_hist, &st->rep_start, &st->rep_out, &st->rep_kf};
     for (DevBuf *b : bufs)
         if (b->p) cudaFree(b->p);
     delete st;
@@ -783,6 +913,7 @@ int ecb_cost_setup(ecb_ctx *ctx, int n_splines, const int32_t *n_cp, const doubl
     st->huber = huber_delta;
     st->n_res = 0;
     st->n_items = 0;
+    st->assoc = false;
     int rc;
     if ((rc = ecb_reserve(ctx, st->d_knots, (size_t) ko * 8))) return rc;
     if ((rc = ecb_reserve(ctx, st->d_knot_off, (size_t) n_splines * 4))) return rc;
@@ -858,6 +989,7 @@ int ecb_cost_set_residuals(ecb_ctx *ctx, const double *obs_xy, const double *lm_
     }
     st->n_res = n;
     st->use_circ = false;
+    st->assoc = false;
     return prepare_records(ctx, st);
 }
 
@@ -991,6 +1123,10 @@ static int cost_associate(ecb_ctx *ctx, const double *kf_time, const double *kf_
     if ((rc = ecb_check(ctx, cudaGetLastError(), "association kernels"))) return rc;
     st->n_res = total;
     st->use_circ = fused;
+    st->assoc = true;
+    st->assoc_K = n_keyframes;
+    st->assoc_n_circ = n_circles;
+    st->assoc_events_gen = ctx->events_gen;
     if (n_residuals) *n_residuals = total;
     return prepare_records(ctx, st, fused);
 }
@@ -1225,6 +1361,139 @@ int ecb_cost_normal_eq(ecb_ctx *ctx, const double *intrinsics, const double *rot
         if (cost) *cost = h_out[(size_t) st->total_spans * OUT_STRIDE];
     } else if (cost) {
         return ecb_d2h(ctx, cost, out + (size_t) st->total_spans * OUT_STRIDE, 8);
+    }
+    return ECB_OK;
+}
+
+// ---- residual report ----
+// r_k at the point already uploaded to st->params -> out (device, n_res doubles); async
+static int launch_residuals(ecb_ctx *ctx, CostState *st, double *out) {
+    if (st->n_res == 0) return ECB_OK;
+    const int grid = (int) std::min<int64_t>((st->n_res + 255) / 256, (int64_t) ctx->sm_count * 8);
+    (st->so3 ? k_residuals<true> : k_residuals<false>)<<<grid, 256, 0, ctx->stream>>>(
+        (const double *) st->obs.p, (const double *) st->lm.p, st->use_circ ? (const int *) st->sel_circle.p : nullptr,
+        (const double *) st->lm_tab.p, (const double *) st->basis.p, (const int *) st->cp0.p, st->n_res,
+        (const double *) st->params.p, st->total_cp, st->radius, st->huber, out);
+    ECB_LAUNCHED(ctx);
+    return ecb_check(ctx, cudaGetLastError(), "k_residuals");
+}
+
+int ecb_cost_residuals(ecb_ctx *ctx, const double *intrinsics, const double *rot_cp, const double *trans_cp, double *d_out,
+                       double *h_out) {
+    if (!ctx || !intrinsics || !rot_cp || !trans_cp) return ECB_ERR_ARG;
+    if (!ctx->cost) return ecb_fail(ctx, ECB_ERR_STATE, "ecb_cost_setup first");
+    cudaSetDevice(ctx->device);
+    CostState *st = (CostState *) ctx->cost;
+    if (st->n_res > 0xFFFFFFFFll) return ecb_fail(ctx, ECB_ERR_UNSUPPORTED, "residual report over 2^32 or more records");
+    int rc;
+    if ((rc = upload_params(ctx, st, intrinsics, rot_cp, trans_cp))) return rc;
+    double *out = d_out;
+    if (!out) {
+        if ((rc = ecb_reserve(ctx, st->rep_r, (size_t) std::max<int64_t>(st->n_res, 1) * 8))) return rc;
+        out = (double *) st->rep_r.p;
+    }
+    if ((rc = launch_residuals(ctx, st, out))) return rc;
+    if (h_out) return ecb_d2h(ctx, h_out, out, (size_t) st->n_res * 8);
+    return ECB_OK;
+}
+
+int ecb_cost_residual_groups(ecb_ctx *ctx, const double *intrinsics, const double *rot_cp, const double *trans_cp, int by,
+                             const double *kf_time, int n_keyframes, int cell_px, ecb_residual_group *groups, int cap,
+                             int *n_groups, ecb_residual_group *total) {
+    if (!ctx || !intrinsics || !rot_cp || !trans_cp) return ECB_ERR_ARG;
+    if (by != ECB_RESIDUALS_BY_KEYFRAME && by != ECB_RESIDUALS_BY_CIRCLE && by != ECB_RESIDUALS_BY_SENSOR_CELL)
+        return ecb_fail(ctx, ECB_ERR_ARG, "unknown residual grouping %d", by);
+    if (cell_px < 1) return ecb_fail(ctx, ECB_ERR_ARG, "cell size %d px < 1", cell_px);
+    if (by == ECB_RESIDUALS_BY_KEYFRAME && !kf_time) return ecb_fail(ctx, ECB_ERR_ARG, "grouping by key frame needs the stamps");
+    if (!ctx->cost) return ecb_fail(ctx, ECB_ERR_STATE, "ecb_cost_setup first");
+    cudaSetDevice(ctx->device);
+    CostState *st = (CostState *) ctx->cost;
+    GroupKeyArgs a;
+    memset(&a, 0, sizeof a);
+    a.by = by;
+    int64_t G = 0;
+    if (by == ECB_RESIDUALS_BY_KEYFRAME || by == ECB_RESIDUALS_BY_CIRCLE) {
+        if (!st->assoc)
+            return ecb_fail(ctx, ECB_ERR_STATE, "residuals of ecb_cost_set_residuals have no key frame or circle: associate first");
+        if (by == ECB_RESIDUALS_BY_KEYFRAME) {
+            if (st->assoc_events_gen != ctx->events_gen)
+                return ecb_fail(ctx, ECB_ERR_STATE, "events were loaded after the association");
+            if (n_keyframes != st->assoc_K)
+                return ecb_fail(ctx, ECB_ERR_ARG, "%d key frames given, the association used %d", n_keyframes, st->assoc_K);
+            G = st->assoc_K;
+        } else {
+            G = st->assoc_n_circ;
+        }
+    } else {
+        if (ctx->width <= 0 || ctx->height <= 0) return ecb_fail(ctx, ECB_ERR_STATE, "grouping by sensor cell needs ecb_set_sensor");
+        a.width = ctx->width;
+        a.height = ctx->height;
+        a.cell = cell_px;
+        a.ncx = (ctx->width + cell_px - 1) / cell_px;
+        G = (int64_t) a.ncx * ((ctx->height + cell_px - 1) / cell_px);
+    }
+    if (n_groups) *n_groups = (int) G;
+    if (!groups && cap == 0) return ECB_OK;
+    if (cap < G || !groups) return ecb_fail(ctx, ECB_ERR_ARG, "%lld groups do not fit cap %d", (long long) G, cap);
+    const int64_t n = st->n_res;
+    if (n > 0xFFFFFFFFll) return ecb_fail(ctx, ECB_ERR_UNSUPPORTED, "residual report over 2^32 or more records");
+    std::vector<ecb_residual_group> h((size_t) G + 1);
+    memset(h.data(), 0, h.size() * sizeof(ecb_residual_group));
+    if (n > 0) {
+        int rc;
+        if ((rc = upload_params(ctx, st, intrinsics, rot_cp, trans_cp))) return rc;
+        const size_t un = (size_t) n;
+        if ((rc = ecb_reserve(ctx, st->rep_r, un * 8))) return rc;
+        for (int q = 0; q < 2; ++q) {
+            if ((rc = ecb_reserve(ctx, st->rep_key[q], un * 8))) return rc;
+            if ((rc = ecb_reserve(ctx, st->rep_idx[q], un * 4))) return rc;
+        }
+        if ((rc = ecb_reserve(ctx, st->rep_hist, gh_radix_hist_bytes(n)))) return rc;
+        if ((rc = ecb_reserve(ctx, st->rep_start, ((size_t) G + 2) * 8))) return rc;
+        if ((rc = ecb_reserve(ctx, st->rep_out, ((size_t) G + 1) * sizeof(ecb_residual_group)))) return rc;
+        if (by == ECB_RESIDUALS_BY_KEYFRAME) {
+            if ((rc = ecb_reserve(ctx, st->rep_kf, (size_t) G * 8))) return rc;
+            if ((rc = ecb_h2d(ctx, st->rep_kf.p, kf_time, (size_t) G * 8))) return rc;
+        }
+        a.sel_event = (const int64_t *) st->sel_event.p;
+        a.sel_circle = (const int *) st->sel_circle.p;
+        a.ev_t = (const double *) ctx->ev_t.p;
+        a.kf_t = (const double *) st->rep_kf.p;
+        a.K = (int) G;
+        a.obs = (const double *) st->obs.p;
+        a.outside = (uint32_t) G;
+        if ((rc = launch_residuals(ctx, st, (double *) st->rep_r.p))) return rc;
+        uint64_t *key[2] = {(uint64_t *) st->rep_key[0].p, (uint64_t *) st->rep_key[1].p};
+        uint32_t *idx[2] = {(uint32_t *) st->rep_idx[0].p, (uint32_t *) st->rep_idx[1].p};
+        const int grid = (int) std::min<int64_t>((n + 255) / 256, (int64_t) ctx->sm_count * 8);
+        k_group_keys<<<grid, 256, 0, ctx->stream>>>(a, n, key[0], idx[0]);
+        ECB_LAUNCHED(ctx);
+        int bits = 8;
+        while (bits < 64 && ((uint64_t) G >> bits)) bits += 8;  // keys 0 .. G
+        int res = 0;
+        if ((rc = gh_radix_sort(ctx, key, idx, n, bits, (uint32_t *) st->rep_hist.p, &res))) return rc;
+        k_group_start<<<(unsigned) ((G + 2 + 127) / 128), 128, 0, ctx->stream>>>(key[res], n, (int) G + 1, (int64_t *) st->rep_start.p);
+        ECB_LAUNCHED(ctx);
+        k_group_reduce<<<(unsigned) (G + 1), RG_THREADS, 0, ctx->stream>>>((const double *) st->rep_r.p, idx[res],
+                                                                         (const int64_t *) st->rep_start.p, st->huber,
+                                                                         (ecb_residual_group *) st->rep_out.p);
+        ECB_LAUNCHED(ctx);
+        if ((rc = ecb_check(ctx, cudaGetLastError(), "residual group kernels"))) return rc;
+        if ((rc = ecb_d2h(ctx, h.data(), st->rep_out.p, h.size() * sizeof(ecb_residual_group)))) return rc;
+    }
+    memcpy(groups, h.data(), (size_t) G * sizeof(ecb_residual_group));
+    if (total) {  // groups 0 .. G-1 and the records outside every group, in group order
+        ecb_residual_group s;
+        memset(&s, 0, sizeof s);
+        for (const ecb_residual_group &q : h) {
+            s.count += q.count;
+            s.n_downweighted += q.n_downweighted;
+            s.sum += q.sum;
+            s.sum_sq += q.sum_sq;
+            s.max_abs = std::max(s.max_abs, q.max_abs);
+            s.cost += q.cost;
+        }
+        *total = s;
     }
     return ECB_OK;
 }

@@ -542,7 +542,8 @@ static int gh_scan(ecb_ctx *ctx, uint32_t *a, int64_t n, uint32_t *sums) {
 }
 
 // Sorts (key, idx) by the low `bits` bits of key; the result ends in key[*res] / idx[*res] (ping-pong buffers 0 / 1).
-static int gh_radix_sort(ecb_ctx *ctx, uint64_t *key[2], uint32_t *idx[2], int64_t n, int bits, uint32_t *hist, int *res) {
+// Declared in ecb_common.cuh (the residual report of ecb_cost.cu sorts records by group with it).
+int gh_radix_sort(ecb_ctx *ctx, uint64_t *key[2], uint32_t *idx[2], int64_t n, int bits, uint32_t *hist, int *res) {
     const int nblk = (int) ((n + RS_TILE - 1) / RS_TILE);
     int cur = 0;
     for (int shift = 0; shift < bits; shift += 8) {
@@ -557,6 +558,8 @@ static int gh_radix_sort(ecb_ctx *ctx, uint64_t *key[2], uint32_t *idx[2], int64
     *res = cur;
     return ECB_OK;
 }
+
+size_t gh_radix_hist_bytes(int64_t n) { return (size_t) 256 * (size_t) ((n + RS_TILE - 1) / RS_TILE) * 4; }
 
 static int bits_for(uint64_t v) {  // bits needed to store values 0..v
     int b = 1;

@@ -27,6 +27,12 @@
 // spline optimisation, which the reference does not offer: it prints a "Constant intrinsics:" line before the optimisation, and
 // the covariance files (ECB_COVARIANCE, ECB_TRAJECTORY_COVARIANCE) are conditional on them.  An unknown name, or the variable
 // together with ECB_REFERENCE_SIGNATURES (the reference's constructor frees all nine), ends the program with exit code 1.
+//
+// ECB_RESIDUALS=1 reports how well the model fits after the optimisation, which the reference does not: a "Residuals:" line (count,
+// RMS, mean, max |r|, down-weighted share) and SavePath/ResidualsByKeyframe.txt, ResidualsByCircle.txt and ResidualMap.txt
+// (statistics per key frame, per board circle and per sensor cell of ECB_RESIDUAL_CELL pixels, default 16).  r is the raw
+// residual ||X_w - L|| - circleRadius, a distance on the board plane in the units of the board points, not pixels.  A cell size
+// that is not a positive integer ends the program with exit code 1 before any GPU work.
 #include <algorithm>
 #include <cstdio>
 #include <cstdlib>
@@ -92,6 +98,16 @@ int main(int argc, char **argv) {
             return 1;
         }
         constIntrinsics = (uint32_t) m;
+    }
+    int residualCell = 16;  // checked before any file or GPU work
+    if (const char *rc = getenv("ECB_RESIDUAL_CELL")) {
+        char *end = nullptr;
+        const long v = strtol(rc, &end, 10);
+        if (end == rc || *end != '\0' || v < 1 || v > 32767) {
+            std::cerr << "ecb: ECB_RESIDUAL_CELL must be a positive integer (pixels), got '" << rc << "'" << std::endl;
+            return 1;
+        }
+        residualCell = (int) v;
     }
     Settings fs;
     if (!fs.open(argv[1])) {
@@ -415,6 +431,58 @@ int main(int argc, char **argv) {
         std::cout << "Intrinsics after optimization:";
         printEigenLike(std::cout, spline.intrinsics().data(), 1, 9);
         std::cout << std::endl;
+        if (getenv("ECB_RESIDUALS") && atoi(getenv("ECB_RESIDUALS")) != 0) {  // how well the model fits (no reference output)
+            std::vector<ecb_residual_group> byKf, byCircle, byCell;
+            ecb_residual_group tot;
+            if (spline.residualGroups(ECB_RESIDUALS_BY_KEYFRAME, residualCell, byKf, &tot) != ECB_OK ||
+                spline.residualGroups(ECB_RESIDUALS_BY_CIRCLE, residualCell, byCircle, nullptr) != ECB_OK ||
+                spline.residualGroups(ECB_RESIDUALS_BY_SENSOR_CELL, residualCell, byCell, nullptr) != ECB_OK) {
+                std::cerr << "ecb: " << spline.lastError() << std::endl;
+                return 1;
+            }
+            const double nan = std::numeric_limits<double>::quiet_NaN();
+            auto mean = [&](const ecb_residual_group &g) { return g.count ? g.sum / (double) g.count : nan; };
+            auto rms = [&](const ecb_residual_group &g) { return g.count ? std::sqrt(g.sum_sq / (double) g.count) : nan; };
+            std::cout << "Residuals: " << tot.count << ", RMS " << rms(tot) << ", mean " << mean(tot) << ", max |r| " << tot.max_abs
+                      << ", down-weighted " << tot.n_downweighted << " ("
+                      << (tot.count ? 100.0 * (double) tot.n_downweighted / (double) tot.count : 0.0) << " %)" << std::endl;
+            auto stats = [&](std::ostream &f, const ecb_residual_group &g) {
+                f << std::defaultfloat << std::setprecision(17) << " " << g.count << " " << mean(g) << " " << rms(g) << " " << g.max_abs
+                  << " " << g.n_downweighted << " " << g.cost << "\n";
+            };
+            const char *units = "# r = ||X_w - L|| - circleRadius: distance on the board plane in the units of the board points (not "
+                                "pixels), before the Huber loss\n# down-weighted: r^2 > huber_delta^2; cost: sum rho(r^2) / 2\n";
+            const std::string dir = std::string(argv[3]) + "/";
+            {
+                std::ofstream f(dir + "ResidualsByKeyframe.txt");
+                f << units << "# stamp count mean RMS max_abs n_downweighted cost (one line per key frame)\n";
+                for (size_t k = 0; k < byKf.size(); ++k) {
+                    f << std::fixed << std::setprecision(10) << kfs[k].timeStamp;
+                    stats(f, byKf[k]);
+                }
+            }
+            {
+                std::ofstream f(dir + "ResidualsByCircle.txt");
+                f << units << "# id x y z count mean RMS max_abs n_downweighted cost (one line per board circle; x y z: board point)\n";
+                for (size_t c = 0; c < byCircle.size(); ++c) {
+                    f << c << std::defaultfloat << std::setprecision(17) << " " << landmarks[c][0] << " " << landmarks[c][1] << " "
+                      << landmarks[c][2];
+                    stats(f, byCircle[c]);
+                }
+            }
+            {
+                std::ofstream f(dir + "ResidualMap.txt");
+                const int ncx = (width + residualCell - 1) / residualCell;
+                f << units << "# cell " << residualCell << " px, " << ncx << " x " << (height + residualCell - 1) / residualCell
+                  << " cells of the " << width << " x " << height << " sensor\n"
+                  << "# u0 v0 count mean RMS max_abs n_downweighted cost (one line per non-empty cell; u0 v0: its top-left pixel)\n";
+                for (size_t c = 0; c < byCell.size(); ++c) {
+                    if (byCell[c].count == 0) continue;
+                    f << ((int) c % ncx) * residualCell << " " << ((int) c / ncx) * residualCell;
+                    stats(f, byCell[c]);
+                }
+            }
+        }
         const bool want_cov = getenv("ECB_COVARIANCE") && atoi(getenv("ECB_COVARIANCE")) != 0;
         const bool want_traj_cov = getenv("ECB_TRAJECTORY_COVARIANCE") && atoi(getenv("ECB_TRAJECTORY_COVARIANCE")) != 0;
         if (want_cov || want_traj_cov) {  // uncertainty of the result (no reference output)

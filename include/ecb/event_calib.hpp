@@ -987,6 +987,7 @@ public:
         int64_t n = 0;
         if (ecb_cost_associate(ev_->ctx, t.data(), c.data(), (int) kf.size(), nc, &landmarks[0][0], step_, &n) != ECB_OK)
             throw std::runtime_error(ecb_last_error(ev_->ctx));
+        kfTime_ = t;  // residualGroups(ECB_RESIDUALS_BY_KEYFRAME) groups by these stamps
         return n;
     }
     bool optimize(ecb_lm_summary *summary = nullptr) {  // EventCalibSpline.cpp:115-251
@@ -1054,6 +1055,48 @@ public:
         cov.assign(36 * times.size(), 0.0);
         return ecb_pose_covariance(ctx, times.data(), (int64_t) times.size(), pose.data(), cov.data(), n_valid);
     }
+    // How well the model fits (ecb_cost_residuals / ecb_cost_residual_groups) at the current point, where optimize() left it.
+    // r is the raw residual ||X_w - L|| - radius: a distance on the board plane in the units of the board points, NOT pixels.
+    // residuals: r of every record in the association's order.  residualGroups: statistics per key frame (the stamps of the last
+    // associate()), per circle or per sensor cell of cellPx pixels (by = ECB_RESIDUALS_BY_*); total (may be null) over every record.
+    int residuals(std::vector<double> &r) const { return residualsAt(ev_->ctx, intr_, seg_, r); }
+    int residualGroups(int by, int cellPx, std::vector<ecb_residual_group> &groups, ecb_residual_group *total) const {
+        return residualGroupsAt(ev_->ctx, intr_, seg_, kfTime_, by, cellPx, groups, total);
+    }
+    static int residualsAt(ecb_ctx *ctx, const std::array<double, 9> &intr, const std::vector<Segment> &seg, std::vector<double> &r) {
+        std::vector<double> rot, trans;
+        flatten(seg, rot, trans);
+        int64_t n = 0;
+        int rc = ecb_cost_layout(ctx, nullptr, nullptr, &n, nullptr);
+        if (rc != ECB_OK) return rc;
+        r.assign((size_t) n, 0.0);
+        return ecb_cost_residuals(ctx, intr.data(), rot.data(), trans.data(), nullptr, n > 0 ? r.data() : nullptr);
+    }
+    static int residualGroupsAt(ecb_ctx *ctx, const std::array<double, 9> &intr, const std::vector<Segment> &seg,
+                                const std::vector<double> &kfTime, int by, int cellPx, std::vector<ecb_residual_group> &groups,
+                                ecb_residual_group *total) {
+        std::vector<double> rot, trans;
+        flatten(seg, rot, trans);
+        const double *kf = kfTime.empty() ? nullptr : kfTime.data();
+        int ng = 0;
+        int rc = ecb_cost_residual_groups(ctx, intr.data(), rot.data(), trans.data(), by, kf, (int) kfTime.size(), cellPx, nullptr, 0,
+                                          &ng, nullptr);
+        if (rc != ECB_OK) return rc;
+        groups.assign((size_t) ng, ecb_residual_group{});
+        ecb_residual_group dummy;
+        return ecb_cost_residual_groups(ctx, intr.data(), rot.data(), trans.data(), by, kf, (int) kfTime.size(), cellPx,
+                                        ng > 0 ? groups.data() : &dummy, ng, &ng, total);
+    }
+    // adds group b into a: counts and sums added, max_abs the max (shards combine in rank order)
+    static void accumulateResidualGroup(ecb_residual_group &a, const ecb_residual_group &b) {
+        a.count += b.count;
+        a.n_downweighted += b.n_downweighted;
+        a.sum += b.sum;
+        a.sum_sq += b.sum_sq;
+        a.max_abs = std::max(a.max_abs, b.max_abs);
+        a.cost += b.cost;
+    }
+    const std::vector<double> &keyframeTimes() const { return kfTime_; }
     const std::array<double, 9> &intrinsics() const { return intr_; }
     const std::vector<Segment> &segments() const { return seg_; }
     // EventCalibSpline.hpp:286-303: index of the segment whose knot range holds t, else -1
@@ -1162,8 +1205,15 @@ private:
     std::vector<Segment> seg_;
     std::vector<int32_t> n_cp_;
     std::array<double, 9> intr_;
+    std::vector<double> kfTime_;  // key-frame stamps of the last associate()
     double step_, radius_;
     bool useSO3_ = false;
+    static void flatten(const std::vector<Segment> &seg, std::vector<double> &rot, std::vector<double> &trans) {
+        for (auto &s : seg) {
+            rot.insert(rot.end(), s.rot_cp.begin(), s.rot_cp.end());
+            trans.insert(trans.end(), s.trans_cp.begin(), s.trans_cp.end());
+        }
+    }
 };
 inline void EventCalibSpline::printEigenLikeRow(std::ostream &os, const double *v, int n) { printEigenLike(os, v, 1, n); }
 

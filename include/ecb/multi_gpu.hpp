@@ -332,6 +332,29 @@ public:
                        int64_t *n_valid = nullptr) const {
         return EventCalibSpline::poseCovarianceAt(ev_->shard[0]->ctx, times, pose, cov, n_valid);
     }
+    // Residual statistics at the current point (EventCalibSpline::residualGroups): every shard reports its own records (one host
+    // thread each), the groups are combined in rank order (counts and sums added, max_abs the max).
+    int residualGroups(int by, int cellPx, std::vector<ecb_residual_group> &groups, ecb_residual_group *total) const {
+        const int G = (int) sp_.size();
+        std::vector<std::vector<ecb_residual_group>> part((size_t) G);
+        std::vector<ecb_residual_group> tot((size_t) G);
+        std::vector<int> rc((size_t) G, ECB_OK);
+        forEachShard(G, [&](int g) {
+            rc[(size_t) g] = EventCalibSpline::residualGroupsAt(ev_->shard[(size_t) g]->ctx, intrinsics(), segments(),
+                                                                sp_[(size_t) g]->keyframeTimes(), by, cellPx, part[(size_t) g],
+                                                                &tot[(size_t) g]);
+        });
+        for (int g = 0; g < G; ++g)
+            if (rc[(size_t) g] != ECB_OK) return rc[(size_t) g];
+        groups = part[0];
+        ecb_residual_group t = tot[0];
+        for (int g = 1; g < G; ++g) {
+            for (size_t i = 0; i < groups.size(); ++i) EventCalibSpline::accumulateResidualGroup(groups[i], part[(size_t) g][i]);
+            EventCalibSpline::accumulateResidualGroup(t, tot[(size_t) g]);
+        }
+        if (total) *total = t;
+        return ECB_OK;
+    }
     const std::array<double, 9> &intrinsics() const { return solved_ ? result_intr_ : sp_[0]->intrinsics(); }
     const std::vector<Segment> &segments() const { return solved_ ? seg_ : sp_[0]->segments(); }
     int saveKeyFrameTrajectoryTUM(const std::string &filename, const std::vector<double> &keyframeStamps) const {

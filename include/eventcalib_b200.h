@@ -234,6 +234,44 @@ int ecb_cost_eval(ecb_ctx *ctx, const double *intrinsics, const double *rot_cp, 
 int ecb_cost_normal_eq(ecb_ctx *ctx, const double *intrinsics, const double *rot_cp, const double *trans_cp, void *d_out,
                        double *h_out, double *cost);
 
+/* ---- how well the model fits: the residuals of the calibration and their statistics --------------------------------------
+ * r_k is the raw residual of record k, ||X_w - L|| - circle_radius before the Huber loss (CalibReprojectionError; the rotation
+ * model of ecb_cost_set_rotation_model selects the quaternion or the SO(3) spline).  It is a DISTANCE ON THE BOARD PLANE, in the
+ * units of the board points and of circle_radius, NOT in pixels.  Records are in the order of ecb_cost_get_association (record k
+ * pairs with event_index[k] and circle_id[k]), or in the order given to ecb_cost_set_residuals.  The point (intrinsics, rot_cp,
+ * trans_cp) has the layout of ecb_cost_eval.  Record indices are 32-bit: n_residuals < 2^32 (ECB_ERR_UNSUPPORTED otherwise).
+ * Both calls read this context's records only: with several GPUs every shard reports its own share. */
+/* r_k of every record, FP64.  d_out: device buffer of n_residuals doubles, or NULL for a context-owned one; h_out: optional host
+ * copy.  Asynchronous on the context's stream unless h_out is given. */
+int ecb_cost_residuals(ecb_ctx *ctx, const double *intrinsics, const double *rot_cp, const double *trans_cp, double *d_out,
+                       double *h_out);
+/* Statistics of a group of residuals.  mean = sum / count and RMS = sqrt(sum_sq / count) are left to the caller.  A residual is
+ * down-weighted when r^2 > huber_delta^2 (the linear branch of the Huber loss).  cost = sum rho(r^2) / 2, the group's share of
+ * ecb_cost_eval.  Every field is a sum or a max, so the results of several shards combine by a fixed-order sum. */
+typedef struct {
+    int64_t count, n_downweighted;
+    double sum, sum_sq, max_abs;   /* of r (board units, not pixels); max_abs = 0 for an empty group */
+    double cost;
+} ecb_residual_group;
+#define ECB_RESIDUALS_BY_KEYFRAME 0     /* the key frame the association used: nearest stamp to the event, ties -> the earlier */
+#define ECB_RESIDUALS_BY_CIRCLE 1       /* circle_id: n_circles groups */
+#define ECB_RESIDUALS_BY_SENSOR_CELL 2  /* (floor(v / c)) * ceil(W / c) + floor(u / c) of the observation (u, v), row major */
+/* Statistics of the residuals at the point, grouped by `by`:
+ *   BY_KEYFRAME: kf_time[n_keyframes] are the host stamps given to the association (n_keyframes must equal its K, else
+ *                ECB_ERR_ARG); K groups.
+ *   BY_CIRCLE: n_circles groups, as given to the association.
+ *   BY_SENSOR_CELL: cells of cell_px x cell_px pixels of the sensor W x H of ecb_set_sensor, ceil(W/c) * ceil(H/c) groups;
+ *                an observation outside [0, W) x [0, H) (explicit residuals only) counts in `total` only.
+ * *n_groups (if non-NULL) is always set.  cap < *n_groups returns ECB_ERR_ARG and writes nothing else; groups = NULL with cap = 0
+ * is a pure size query (ECB_OK, nothing computed).  total (optional): all records.  Zero residuals give all-zero groups.
+ * Errors: unknown `by`, cell_px < 1, or kf_time == NULL for BY_KEYFRAME: ECB_ERR_ARG.  BY_KEYFRAME or BY_CIRCLE on residuals of
+ * ecb_cost_set_residuals, BY_KEYFRAME after events were loaded since the association, BY_SENSOR_CELL without ecb_set_sensor:
+ * ECB_ERR_STATE.  Deterministic: repeated calls are bit-identical (stable radix sort by group, fixed-order reductions, no
+ * floating-point atomics).  Synchronises the context's stream. */
+int ecb_cost_residual_groups(ecb_ctx *ctx, const double *intrinsics, const double *rot_cp, const double *trans_cp, int by,
+                             const double *kf_time, int n_keyframes, int cell_px, ecb_residual_group *groups, int cap,
+                             int *n_groups, ecb_residual_group *total);
+
 /* Multi-GPU (one process per GPU): the same evaluation with the inter-GPU sum fused in.  Every rank owns a receive
  * buffer of ecb_exchange_buffer_bytes() bytes, ZERO-FILLED once, in device memory its peers can write (same process:
  * any cudaMalloc pointer with peer access; other processes: ecb_device_alloc + ecb_ipc_export / ecb_ipc_open).
