@@ -65,6 +65,11 @@ RESIDUAL_GROUP_DTYPE = np.dtype([("count", "<i8"), ("n_downweighted", "<i8"), ("
 assert RESIDUAL_GROUP_DTYPE.itemsize == C.sizeof(ResidualGroup)
 RESIDUALS_BY = {"keyframe": 0, "circle": 1, "sensor_cell": 2}
 
+# ecb_reprojection_group: statistics of a group of reprojection errors e (pixels); count / sum / sum_sq / max_abs over the valid
+# records, n_invalid = the records that cannot be projected (NaN)
+REPROJECTION_GROUP_DTYPE = np.dtype([("count", "<i8"), ("n_invalid", "<i8"), ("sum", "<f8"), ("sum_sq", "<f8"),
+                                     ("max_abs", "<f8")])
+
 
 # the order of every intrinsics array (ecb_residual.h): bit i of a constant-intrinsics mask is INTRINSIC_NAMES[i].  In the spline
 # stage k1 .. k5 are the coefficients of the inverse radial polynomial, not OpenCV's distortion coefficients.
@@ -103,7 +108,8 @@ SYMBOLS = ["ecb_ctx_create", "ecb_ctx_destroy", "ecb_last_error", "ecb_launch_co
            "ecb_lm_state", "ecb_lm_trace", "ecb_calibrate", "ecb_lm_device_create", "ecb_lm_device_destroy",
            "ecb_lm_device_set_exchange", "ecb_lm_device_begin", "ecb_lm_device_iterate", "ecb_lm_device_running",
            "ecb_lm_device_result", "ecb_calibrate_device", "ecb_covariance", "ecb_pose_covariance",
-           "ecb_pose_covariance_device", "ecb_cost_residuals", "ecb_cost_residual_groups"]
+           "ecb_pose_covariance_device", "ecb_cost_residuals", "ecb_cost_residual_groups",
+           "ecb_inverse_radial_fold", "ecb_cost_reprojection_errors", "ecb_cost_reprojection_groups", "ecb_keyframe_reprojection"]
 
 _lib = None
 
@@ -170,6 +176,10 @@ def load_library():
     lib.ecb_cost_normal_eq.argtypes = [vp, vp, vp, vp, vp, vp, vp]
     lib.ecb_cost_residuals.argtypes = [vp, vp, vp, vp, vp, vp]
     lib.ecb_cost_residual_groups.argtypes = [vp, vp, vp, vp, i32, vp, i32, i32, vp, i32, C.POINTER(C.c_int), vp]
+    lib.ecb_inverse_radial_fold.argtypes = [vp, C.POINTER(dbl)]
+    lib.ecb_cost_reprojection_errors.argtypes = [vp, vp, vp, vp, vp, vp, C.POINTER(i64)]
+    lib.ecb_cost_reprojection_groups.argtypes = [vp, vp, vp, vp, i32, vp, i32, i32, vp, i32, C.POINTER(C.c_int), vp]
+    lib.ecb_keyframe_reprojection.argtypes = [vp, vp, vp, vp, vp, vp, i32, i32, vp, vp, vp, vp]
     lib.ecb_lm_default_options.argtypes = [C.POINTER(LmOptions)]
     lib.ecb_lm_default_options.restype = None
     lib.ecb_lm_create.argtypes = [i32, vp, C.POINTER(LmOptions)]
@@ -203,6 +213,20 @@ def load_library():
 
 def _ptr(a):
     return a.ctypes.data_as(C.c_void_p) if a is not None else None
+
+
+def inverse_radial_fold(k):
+    """rho_fold of the inverse radial polynomial k[5] = k1 .. k5 (ecb_inverse_radial_fold): g(rho) = rho s(rho^2) increases on
+    [0, rho_fold) only, so the forward model (projection) exists for distorted radii below it; inf when g increases everywhere.
+    Normalised units: rho_fold * fx is the radius in pixels."""
+    k = np.ascontiguousarray(k, np.float64)
+    if k.shape != (5,):
+        raise ValueError("k must hold the 5 coefficients k1 .. k5")
+    rho = C.c_double(0.0)
+    rc = load_library().ecb_inverse_radial_fold(_ptr(k), C.byref(rho))
+    if rc != OK:
+        raise EcbError(rc, "ecb_inverse_radial_fold")
+    return rho.value
 
 
 def default_params(eps=4.0, min_pts=2, cluster_min=5, knn_num=3, fit_circle=0, radius_threshold=15.511363636363637,
@@ -568,6 +592,57 @@ class Context:
         total = np.zeros((), RESIDUAL_GROUP_DTYPE)
         self._chk(self.lib.ecb_cost_residual_groups(*args, _ptr(groups), ng.value, C.byref(ng), _ptr(total)))
         return groups[:ng.value], total
+
+    def reprojection_errors(self, intr, rot, trans, d_out=None, host=True):
+        """Reprojection errors e_k of every record in pixels (ecb_cost_reprojection_errors), in the order of cost_residuals():
+        e_k = sign(|d| - radius) |q - o|, o the event pixel and q the projection of the residual's rim point, NaN where it cannot
+        be projected.  Returns (e as float64 ndarray, n_invalid) when host=True; else leaves e in d_out (device pointer, or None
+        for the context's own buffer), enqueued on the context's stream, and returns None."""
+        a = [np.ascontiguousarray(v, np.float64) for v in (intr, rot, trans)]
+        d = C.c_void_p(d_out) if d_out else None
+        if not host:
+            self._chk(self.lib.ecb_cost_reprojection_errors(self.h, _ptr(a[0]), _ptr(a[1]), _ptr(a[2]), d, None, None))
+            return None
+        n = self.cost_layout()["n_residuals"]
+        out = np.zeros(max(n, 1))
+        bad = C.c_int64(0)
+        self._chk(self.lib.ecb_cost_reprojection_errors(self.h, _ptr(a[0]), _ptr(a[1]), _ptr(a[2]), d, _ptr(out), C.byref(bad)))
+        return out[:n], bad.value
+
+    def reprojection_groups(self, intr, rot, trans, by, kf_t=None, cell_px=16):
+        """Statistics of the reprojection errors (pixels) per group (ecb_cost_reprojection_groups): the groups of residual_groups.
+        Returns (groups, total) as numpy structured arrays of REPROJECTION_GROUP_DTYPE (count, n_invalid, sum, sum_sq,
+        max_abs; count and the sums over the valid records only); total has shape () and covers every record."""
+        if by not in RESIDUALS_BY:
+            raise ValueError("by must be one of %s" % ", ".join(RESIDUALS_BY))
+        a = [np.ascontiguousarray(v, np.float64) for v in (intr, rot, trans)]
+        kf = np.ascontiguousarray(kf_t, np.float64) if kf_t is not None else None
+        nk = len(kf) if kf is not None else 0
+        args = (self.h, _ptr(a[0]), _ptr(a[1]), _ptr(a[2]), RESIDUALS_BY[by], _ptr(kf), nk, int(cell_px))
+        ng = C.c_int(0)
+        self._chk(self.lib.ecb_cost_reprojection_groups(*args, None, 0, C.byref(ng), None))
+        groups = np.zeros(max(ng.value, 1), REPROJECTION_GROUP_DTYPE)
+        total = np.zeros((), REPROJECTION_GROUP_DTYPE)
+        self._chk(self.lib.ecb_cost_reprojection_groups(*args, _ptr(groups), ng.value, C.byref(ng), _ptr(total)))
+        return groups[:ng.value], total
+
+    def keyframe_reprojection(self, intr, rot, trans, kf_t, circles, landmarks):
+        """Circle centres of the key frames reprojected at their stamps (ecb_keyframe_reprojection): kf_t[K], circles[K][n][3]
+        (cx, cy, r; r < 0 = absent) and landmarks[n][3] as for cost_associate.  Returns (proj[K, n, 2], err[K, n] = |proj -
+        (cx, cy)| in pixels, total of REPROJECTION_GROUP_DTYPE over the present features); NaN for an absent feature, a stamp
+        outside every segment, or a point that cannot be projected."""
+        a = [np.ascontiguousarray(v, np.float64) for v in (intr, rot, trans)]
+        kf = np.ascontiguousarray(kf_t, np.float64)
+        circ = np.ascontiguousarray(circles, np.float64)
+        lm = np.ascontiguousarray(landmarks, np.float64)
+        K, n = circ.shape[0], circ.shape[1]
+        if circ.shape != (K, n, 3) or kf.shape != (K,) or lm.shape != (n, 3):
+            raise ValueError("kf_t[K], circles[K][n][3] and landmarks[n][3] expected")
+        proj, err = np.zeros((K, n, 2)), np.zeros((K, n))
+        total = np.zeros((), REPROJECTION_GROUP_DTYPE)
+        self._chk(self.lib.ecb_keyframe_reprojection(self.h, _ptr(a[0]), _ptr(a[1]), _ptr(a[2]), _ptr(kf), _ptr(circ), K, n,
+                                                     _ptr(lm), _ptr(proj), _ptr(err), _ptr(total)))
+        return proj, err, total
 
     def calibrate(self, n_cp, intr, rot, trans, options=None, trace_rows=256):
         """EventCalibSpline::optimize on one GPU: returns (intr, rot, trans, summary dict, trace[rows,4])."""

@@ -14,13 +14,17 @@
 //                   CUDA-core register-tiled SYRK.  tcgen05 has no f64 kind.
 //   k_reduce_*      fixed-order reduction of the per-work-item partials -> run-to-run identical J^T J / J^T r / cost
 //   k_cost          cost-only evaluation (LM step acceptance)
+//   k_residuals, k_group_*            the residual report (board units)
+//   k_reprojection, k_reproj_reduce, k_keyframe_reproj   the same fit in pixels (forward model of ecb_camera.h)
 #include <stdlib.h>
 #include <string.h>
 
 #include <algorithm>
+#include <cmath>
 #include <vector>
 
 #include "ecb_bspline.cuh"
+#include "ecb_camera.h"
 #include "ecb_common.cuh"
 #include "ecb_residual_so3.h"
 
@@ -55,6 +59,7 @@ struct CostState {
     int assoc_K = 0, assoc_n_circ = 0;
     uint64_t assoc_events_gen = 0;
     DevBuf rep_r, rep_key[2], rep_idx[2], rep_hist, rep_start, rep_out, rep_kf;  // residual report (ecb_cost_residual_groups)
+    DevBuf rep_io;  // reprojection report: invalid count; staging of ecb_keyframe_reprojection
     uint64_t xch_last_epoch = 0;   // ecb_cost_normal_eq_exchange: last epoch sent / generation of the caller's sequence
     uint32_t xch_generation = 0;
 };
@@ -783,6 +788,139 @@ __global__ void __launch_bounds__(RG_THREADS) k_group_reduce(const double *__res
     }
 }
 
+// ------------------------------------------------------------------------ reprojection report ----
+// k_reprojection    the loads of k_residuals; the record's pose (ecb_pose_eval), then e_k in pixels (ecb_rim_reprojection), NaN
+//                   when not projectable; optional count of the NaN records (integer atomics, one per warp)
+// k_reproj_reduce   k_group_reduce for e: valid records counted and summed, NaN ones counted in n_invalid only.  e is signed
+//                   and its sums cancel (the mean error of a group is near 0 when the fit is good), so sum e is compensated
+//                   (Neumaier per thread, TwoSum in the tree): it keeps the relative accuracy of the sum itself instead of
+//                   n eps sum |e|
+// k_keyframe_reproj one thread per (key frame, circle): the board point at the key frame's pose, projected
+template <int SO3>
+__global__ void __launch_bounds__(256) k_reprojection(const double *__restrict__ obs, const double *__restrict__ lm,
+                                                      const int *__restrict__ circ, const double *__restrict__ lm_tab,
+                                                      const double *__restrict__ basis, const int *__restrict__ cp0, int64_t n,
+                                                      const double *__restrict__ params, int total_cp, double radius, EcbFold fold,
+                                                      double *__restrict__ out, unsigned long long *__restrict__ n_invalid) {
+    const double *intr = params, *rot = params + 9, *trans = params + 9 + 4 * (size_t) total_cp;
+    unsigned bad = 0;
+    for (int64_t k = (int64_t) blockIdx.x * 256 + threadIdx.x; k < n; k += (int64_t) gridDim.x * 256) {
+        const int c0 = cp0[k];
+        const double4 b4 = reinterpret_cast<const double4 *>(basis)[k];
+        const double b[4] = {b4.x, b4.y, b4.z, b4.w};
+        const double2 o = reinterpret_cast<const double2 *>(obs)[k];
+        const double *L = circ ? lm_tab + 3 * circ[k] : lm + 3 * k;
+        const double Lx = L[0], Ly = L[1], Lz = L[2];
+        double q[4], t[3];
+        ecb_pose_eval(rot + 4 * (size_t) c0, trans + 3 * (size_t) c0, b, SO3, q, t);
+        const double e = ecb_rim_reprojection(intr, fold, q, t, o.x, o.y, Lx, Ly, Lz, radius);
+        out[k] = e;
+        bad += isnan(e) ? 1u : 0u;
+    }
+    if (n_invalid) {
+        bad = __reduce_add_sync(0xffffffffu, bad);
+        if ((threadIdx.x & 31) == 0 && bad) atomicAdd(n_invalid, (unsigned long long) bad);
+    }
+}
+
+// (s, c) += v with the rounding error of s + v kept in c (Neumaier); Knuth's TwoSum, exact without branches
+ECB_HD void ecb_comp_add(double &s, double &c, double v) {
+    const double t = s + v, bp = t - s;
+    c += (s - (t - bp)) + (v - bp);
+    s = t;
+}
+
+__global__ void __launch_bounds__(RG_THREADS) k_reproj_reduce(const double *__restrict__ e, const uint32_t *__restrict__ sidx,
+                                                              const int64_t *__restrict__ start,
+                                                              ecb_reprojection_group *__restrict__ out) {
+    __shared__ double sh[4][RG_THREADS];
+    __shared__ long long shn[RG_THREADS];
+    const int g = blockIdx.x, t = threadIdx.x;
+    const int64_t b = start[g], en = start[g + 1];
+    long long nbad = 0;
+    double sum = 0.0, comp = 0.0, ssq = 0.0, mx = 0.0;
+    for (int64_t i = b + t; i < en; i += RG_THREADS) {
+        const double v = e[sidx[i]];
+        if (isnan(v)) {
+            ++nbad;
+            continue;
+        }
+        ecb_comp_add(sum, comp, v);
+        ssq += v * v;
+        mx = fmax(mx, fabs(v));
+    }
+    sh[0][t] = sum;
+    sh[1][t] = ssq;
+    sh[2][t] = mx;
+    sh[3][t] = comp;
+    shn[t] = nbad;
+    __syncthreads();
+    for (int o = RG_THREADS / 2; o > 0; o >>= 1) {
+        if (t < o) {
+            double s0 = sh[0][t], c0 = sh[3][t] + sh[3][t + o];
+            ecb_comp_add(s0, c0, sh[0][t + o]);
+            sh[0][t] = s0;
+            sh[3][t] = c0;
+            sh[1][t] += sh[1][t + o];
+            sh[2][t] = fmax(sh[2][t], sh[2][t + o]);
+            shn[t] += shn[t + o];
+        }
+        __syncthreads();
+    }
+    if (t == 0) {
+        ecb_reprojection_group q;
+        q.n_invalid = shn[0];
+        q.count = (en - b) - shn[0];
+        q.sum = sh[0][0] + sh[3][0];
+        q.sum_sq = sh[1][0];
+        q.max_abs = sh[2][0];
+        out[g] = q;
+    }
+}
+
+// kf_t[K], circ[K][nc][3] (cx cy r), lm[nc][3] -> proj[K][nc][2], err[K][nc]; the segment and span lookup of k_pose_cov
+template <int SO3>
+__global__ void __launch_bounds__(128) k_keyframe_reproj(const double *__restrict__ kf_t, const double *__restrict__ circ,
+                                                         const double *__restrict__ lm, int K, int nc, EcbSplineView sv,
+                                                         const double *__restrict__ params, EcbFold fold,
+                                                         double *__restrict__ proj, double *__restrict__ err) {
+    const int64_t i = (int64_t) blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (int64_t) K * nc) return;
+    const int kf = (int) (i / nc), c = (int) (i % nc);
+    const double *ci = circ + 3 * i;
+    double pu = NAN, pv = NAN, e = NAN;
+    const double u = kf_t[kf];
+    int s = 0;
+    const double *kn = nullptr;
+    int nk = 0;
+    for (; s < sv.n_splines; ++s) {  // EventCalibSpline::time2splineIdx; NaN holds in no range
+        kn = sv.knots + sv.knot_off[s];
+        nk = sv.ncp[s] + 4;
+        if (u >= kn[0] && u <= kn[nk - 1]) break;
+    }
+    if (ci[2] >= 0.0 && s < sv.n_splines) {
+        const int span = find_span_dev(kn, nk, u);
+        double N[4], q[4], t[3];
+        basis_dev(kn, span, u, N);
+        const int c0 = sv.cp_off[s] + span - 3;
+        ecb_pose_eval(params + 9 + 4 * (size_t) c0, params + 9 + 4 * (size_t) sv.total_cp + 3 * (size_t) c0, N, SO3, q, t);
+        const double P[3] = {lm[3 * c] - t[0], lm[3 * c + 1] - t[1], lm[3 * c + 2] - t[2]};
+        double pc[3], a, b;
+        ecb_quat_rotate(q, P, true, pc);
+        if (ecb_project(params, fold, pc, a, b)) {
+            const double d = sqrt((a - ci[0]) * (a - ci[0]) + (b - ci[1]) * (b - ci[1]));
+            if (d < INFINITY) {
+                pu = a;
+                pv = b;
+                e = d;
+            }
+        }
+    }
+    proj[2 * i] = pu;
+    proj[2 * i + 1] = pv;
+    err[i] = e;
+}
+
 int prepare_records(ecb_ctx *ctx, CostState *st, bool have_basis = false) {
     int rc;
     const int64_t n = st->n_res;
@@ -878,7 +1016,7 @@ void ecb_cost_free(ecb_ctx *ctx) {
                       &st->spl, &st->basis, &st->cp0, &st->span, &st->span_start, &st->items, &st->part, &st->out, &st->params,
                       &st->cost_part, &st->flags, &st->ev_flag, &st->ev_cnt, &st->ev_tag, &st->kf_t, &st->kf_circ, &st->kf_c32, &st->lm_tab,
                       &st->sel_event, &st->sel_circle, &st->rep_r, &st->rep_key[0], &st->rep_key[1], &st->rep_idx[0],
-                      &st->rep_idx[1], &st->rep_hist, &st->rep_start, &st->rep_out, &st->rep_kf};
+                      &st->rep_idx[1], &st->rep_hist, &st->rep_start, &st->rep_out, &st->rep_kf, &st->rep_io};
     for (DevBuf *b : bufs)
         if (b->p) cudaFree(b->p);
     delete st;
@@ -1397,21 +1535,17 @@ int ecb_cost_residuals(ecb_ctx *ctx, const double *intrinsics, const double *rot
     return ECB_OK;
 }
 
-int ecb_cost_residual_groups(ecb_ctx *ctx, const double *intrinsics, const double *rot_cp, const double *trans_cp, int by,
-                             const double *kf_time, int n_keyframes, int cell_px, ecb_residual_group *groups, int cap,
-                             int *n_groups, ecb_residual_group *total) {
-    if (!ctx || !intrinsics || !rot_cp || !trans_cp) return ECB_ERR_ARG;
+// The grouping shared by the residual and the reprojection report (ecb_cost_residual_groups): group_layout checks the
+// arguments, counts the groups (*G; *n_groups is always set) and fills the key arguments; *query is set for a pure size query.
+static int group_layout(ecb_ctx *ctx, CostState *st, int by, const double *kf_time, int n_keyframes, int cell_px, bool have_groups,
+                        int cap, int *n_groups, GroupKeyArgs &a, int64_t *G, bool *query) {
     if (by != ECB_RESIDUALS_BY_KEYFRAME && by != ECB_RESIDUALS_BY_CIRCLE && by != ECB_RESIDUALS_BY_SENSOR_CELL)
         return ecb_fail(ctx, ECB_ERR_ARG, "unknown residual grouping %d", by);
     if (cell_px < 1) return ecb_fail(ctx, ECB_ERR_ARG, "cell size %d px < 1", cell_px);
     if (by == ECB_RESIDUALS_BY_KEYFRAME && !kf_time) return ecb_fail(ctx, ECB_ERR_ARG, "grouping by key frame needs the stamps");
-    if (!ctx->cost) return ecb_fail(ctx, ECB_ERR_STATE, "ecb_cost_setup first");
-    cudaSetDevice(ctx->device);
-    CostState *st = (CostState *) ctx->cost;
-    GroupKeyArgs a;
+    if (!st) return ecb_fail(ctx, ECB_ERR_STATE, "ecb_cost_setup first");
     memset(&a, 0, sizeof a);
     a.by = by;
-    int64_t G = 0;
     if (by == ECB_RESIDUALS_BY_KEYFRAME || by == ECB_RESIDUALS_BY_CIRCLE) {
         if (!st->assoc)
             return ecb_fail(ctx, ECB_ERR_STATE, "residuals of ecb_cost_set_residuals have no key frame or circle: associate first");
@@ -1420,9 +1554,9 @@ int ecb_cost_residual_groups(ecb_ctx *ctx, const double *intrinsics, const doubl
                 return ecb_fail(ctx, ECB_ERR_STATE, "events were loaded after the association");
             if (n_keyframes != st->assoc_K)
                 return ecb_fail(ctx, ECB_ERR_ARG, "%d key frames given, the association used %d", n_keyframes, st->assoc_K);
-            G = st->assoc_K;
+            *G = st->assoc_K;
         } else {
-            G = st->assoc_n_circ;
+            *G = st->assoc_n_circ;
         }
     } else {
         if (ctx->width <= 0 || ctx->height <= 0) return ecb_fail(ctx, ECB_ERR_STATE, "grouping by sensor cell needs ecb_set_sensor");
@@ -1430,51 +1564,77 @@ int ecb_cost_residual_groups(ecb_ctx *ctx, const double *intrinsics, const doubl
         a.height = ctx->height;
         a.cell = cell_px;
         a.ncx = (ctx->width + cell_px - 1) / cell_px;
-        G = (int64_t) a.ncx * ((ctx->height + cell_px - 1) / cell_px);
+        *G = (int64_t) a.ncx * ((ctx->height + cell_px - 1) / cell_px);
     }
-    if (n_groups) *n_groups = (int) G;
-    if (!groups && cap == 0) return ECB_OK;
-    if (cap < G || !groups) return ecb_fail(ctx, ECB_ERR_ARG, "%lld groups do not fit cap %d", (long long) G, cap);
+    if (n_groups) *n_groups = (int) *G;
+    *query = !have_groups && cap == 0;
+    if (*query) return ECB_OK;
+    if (cap < *G || !have_groups) return ecb_fail(ctx, ECB_ERR_ARG, "%lld groups do not fit cap %d", (long long) *G, cap);
+    if (st->n_res > 0xFFFFFFFFll) return ecb_fail(ctx, ECB_ERR_UNSUPPORTED, "residual report over 2^32 or more records");
+    return ECB_OK;
+}
+
+// group_sort: the (group, record index) keys of the n_res >= 1 records, sorted with the stable radix sort, and the group bounds
+// st->rep_start[0 .. G + 1]; *sidx: the record indices in group order (record order inside a group).  Async.
+static int group_sort(ecb_ctx *ctx, CostState *st, GroupKeyArgs a, int64_t G, const double *kf_time, const uint32_t **sidx) {
+    int rc;
     const int64_t n = st->n_res;
-    if (n > 0xFFFFFFFFll) return ecb_fail(ctx, ECB_ERR_UNSUPPORTED, "residual report over 2^32 or more records");
+    const size_t un = (size_t) n;
+    for (int q = 0; q < 2; ++q) {
+        if ((rc = ecb_reserve(ctx, st->rep_key[q], un * 8))) return rc;
+        if ((rc = ecb_reserve(ctx, st->rep_idx[q], un * 4))) return rc;
+    }
+    if ((rc = ecb_reserve(ctx, st->rep_hist, gh_radix_hist_bytes(n)))) return rc;
+    if ((rc = ecb_reserve(ctx, st->rep_start, ((size_t) G + 2) * 8))) return rc;
+    if (a.by == ECB_RESIDUALS_BY_KEYFRAME) {
+        if ((rc = ecb_reserve(ctx, st->rep_kf, (size_t) G * 8))) return rc;
+        if ((rc = ecb_h2d(ctx, st->rep_kf.p, kf_time, (size_t) G * 8))) return rc;
+    }
+    a.sel_event = (const int64_t *) st->sel_event.p;
+    a.sel_circle = (const int *) st->sel_circle.p;
+    a.ev_t = (const double *) ctx->ev_t.p;
+    a.kf_t = (const double *) st->rep_kf.p;
+    a.K = (int) G;
+    a.obs = (const double *) st->obs.p;
+    a.outside = (uint32_t) G;
+    uint64_t *key[2] = {(uint64_t *) st->rep_key[0].p, (uint64_t *) st->rep_key[1].p};
+    uint32_t *idx[2] = {(uint32_t *) st->rep_idx[0].p, (uint32_t *) st->rep_idx[1].p};
+    const int grid = (int) std::min<int64_t>((n + 255) / 256, (int64_t) ctx->sm_count * 8);
+    k_group_keys<<<grid, 256, 0, ctx->stream>>>(a, n, key[0], idx[0]);
+    ECB_LAUNCHED(ctx);
+    int bits = 8;
+    while (bits < 64 && ((uint64_t) G >> bits)) bits += 8;  // keys 0 .. G
+    int res = 0;
+    if ((rc = gh_radix_sort(ctx, key, idx, n, bits, (uint32_t *) st->rep_hist.p, &res))) return rc;
+    k_group_start<<<(unsigned) ((G + 2 + 127) / 128), 128, 0, ctx->stream>>>(key[res], n, (int) G + 1, (int64_t *) st->rep_start.p);
+    ECB_LAUNCHED(ctx);
+    *sidx = idx[res];
+    return ecb_check(ctx, cudaGetLastError(), "group kernels");
+}
+
+int ecb_cost_residual_groups(ecb_ctx *ctx, const double *intrinsics, const double *rot_cp, const double *trans_cp, int by,
+                             const double *kf_time, int n_keyframes, int cell_px, ecb_residual_group *groups, int cap,
+                             int *n_groups, ecb_residual_group *total) {
+    if (!ctx || !intrinsics || !rot_cp || !trans_cp) return ECB_ERR_ARG;
+    cudaSetDevice(ctx->device);
+    CostState *st = (CostState *) ctx->cost;
+    GroupKeyArgs a;
+    int64_t G = 0;
+    bool query = false;
+    int rc;
+    if ((rc = group_layout(ctx, st, by, kf_time, n_keyframes, cell_px, groups != nullptr, cap, n_groups, a, &G, &query))) return rc;
+    if (query) return ECB_OK;
+    const int64_t n = st->n_res;
     std::vector<ecb_residual_group> h((size_t) G + 1);
     memset(h.data(), 0, h.size() * sizeof(ecb_residual_group));
     if (n > 0) {
-        int rc;
         if ((rc = upload_params(ctx, st, intrinsics, rot_cp, trans_cp))) return rc;
-        const size_t un = (size_t) n;
-        if ((rc = ecb_reserve(ctx, st->rep_r, un * 8))) return rc;
-        for (int q = 0; q < 2; ++q) {
-            if ((rc = ecb_reserve(ctx, st->rep_key[q], un * 8))) return rc;
-            if ((rc = ecb_reserve(ctx, st->rep_idx[q], un * 4))) return rc;
-        }
-        if ((rc = ecb_reserve(ctx, st->rep_hist, gh_radix_hist_bytes(n)))) return rc;
-        if ((rc = ecb_reserve(ctx, st->rep_start, ((size_t) G + 2) * 8))) return rc;
+        if ((rc = ecb_reserve(ctx, st->rep_r, (size_t) n * 8))) return rc;
         if ((rc = ecb_reserve(ctx, st->rep_out, ((size_t) G + 1) * sizeof(ecb_residual_group)))) return rc;
-        if (by == ECB_RESIDUALS_BY_KEYFRAME) {
-            if ((rc = ecb_reserve(ctx, st->rep_kf, (size_t) G * 8))) return rc;
-            if ((rc = ecb_h2d(ctx, st->rep_kf.p, kf_time, (size_t) G * 8))) return rc;
-        }
-        a.sel_event = (const int64_t *) st->sel_event.p;
-        a.sel_circle = (const int *) st->sel_circle.p;
-        a.ev_t = (const double *) ctx->ev_t.p;
-        a.kf_t = (const double *) st->rep_kf.p;
-        a.K = (int) G;
-        a.obs = (const double *) st->obs.p;
-        a.outside = (uint32_t) G;
         if ((rc = launch_residuals(ctx, st, (double *) st->rep_r.p))) return rc;
-        uint64_t *key[2] = {(uint64_t *) st->rep_key[0].p, (uint64_t *) st->rep_key[1].p};
-        uint32_t *idx[2] = {(uint32_t *) st->rep_idx[0].p, (uint32_t *) st->rep_idx[1].p};
-        const int grid = (int) std::min<int64_t>((n + 255) / 256, (int64_t) ctx->sm_count * 8);
-        k_group_keys<<<grid, 256, 0, ctx->stream>>>(a, n, key[0], idx[0]);
-        ECB_LAUNCHED(ctx);
-        int bits = 8;
-        while (bits < 64 && ((uint64_t) G >> bits)) bits += 8;  // keys 0 .. G
-        int res = 0;
-        if ((rc = gh_radix_sort(ctx, key, idx, n, bits, (uint32_t *) st->rep_hist.p, &res))) return rc;
-        k_group_start<<<(unsigned) ((G + 2 + 127) / 128), 128, 0, ctx->stream>>>(key[res], n, (int) G + 1, (int64_t *) st->rep_start.p);
-        ECB_LAUNCHED(ctx);
-        k_group_reduce<<<(unsigned) (G + 1), RG_THREADS, 0, ctx->stream>>>((const double *) st->rep_r.p, idx[res],
+        const uint32_t *sidx = nullptr;
+        if ((rc = group_sort(ctx, st, a, G, kf_time, &sidx))) return rc;
+        k_group_reduce<<<(unsigned) (G + 1), RG_THREADS, 0, ctx->stream>>>((const double *) st->rep_r.p, sidx,
                                                                          (const int64_t *) st->rep_start.p, st->huber,
                                                                          (ecb_residual_group *) st->rep_out.p);
         ECB_LAUNCHED(ctx);
@@ -1492,6 +1652,153 @@ int ecb_cost_residual_groups(ecb_ctx *ctx, const double *intrinsics, const doubl
             s.sum_sq += q.sum_sq;
             s.max_abs = std::max(s.max_abs, q.max_abs);
             s.cost += q.cost;
+        }
+        *total = s;
+    }
+    return ECB_OK;
+}
+
+// ---- reprojection report ----
+int ecb_inverse_radial_fold(const double *k, double *rho_fold) {
+    if (!k || !rho_fold) return ECB_ERR_ARG;
+    *rho_fold = ecb_inverse_radial_fold_host(k).rho;
+    return ECB_OK;
+}
+
+// e_k at the point already uploaded to st->params (intrinsics intr on the host, for the fold) -> out; d_invalid (optional,
+// zeroed here) counts the NaN records; async
+static int launch_reprojection(ecb_ctx *ctx, CostState *st, const double *intr, double *out, unsigned long long *d_invalid) {
+    if (d_invalid) ECB_CUDA(ctx, cudaMemsetAsync(d_invalid, 0, 8, ctx->stream));
+    if (st->n_res == 0) return ECB_OK;
+    const EcbFold fold = ecb_inverse_radial_fold_host(intr + 4);
+    const int grid = (int) std::min<int64_t>((st->n_res + 255) / 256, (int64_t) ctx->sm_count * 8);
+    (st->so3 ? k_reprojection<1> : k_reprojection<0>)<<<grid, 256, 0, ctx->stream>>>(
+        (const double *) st->obs.p, (const double *) st->lm.p, st->use_circ ? (const int *) st->sel_circle.p : nullptr,
+        (const double *) st->lm_tab.p, (const double *) st->basis.p, (const int *) st->cp0.p, st->n_res,
+        (const double *) st->params.p, st->total_cp, st->radius, fold, out, d_invalid);
+    ECB_LAUNCHED(ctx);
+    return ecb_check(ctx, cudaGetLastError(), "k_reprojection");
+}
+
+int ecb_cost_reprojection_errors(ecb_ctx *ctx, const double *intrinsics, const double *rot_cp, const double *trans_cp,
+                                 double *d_out, double *h_out, int64_t *n_invalid) {
+    if (!ctx || !intrinsics || !rot_cp || !trans_cp) return ECB_ERR_ARG;
+    if (!ctx->cost) return ecb_fail(ctx, ECB_ERR_STATE, "ecb_cost_setup first");
+    cudaSetDevice(ctx->device);
+    CostState *st = (CostState *) ctx->cost;
+    if (st->n_res > 0xFFFFFFFFll) return ecb_fail(ctx, ECB_ERR_UNSUPPORTED, "reprojection report over 2^32 or more records");
+    int rc;
+    if ((rc = upload_params(ctx, st, intrinsics, rot_cp, trans_cp))) return rc;
+    double *out = d_out;
+    if (!out) {
+        if ((rc = ecb_reserve(ctx, st->rep_r, (size_t) std::max<int64_t>(st->n_res, 1) * 8))) return rc;
+        out = (double *) st->rep_r.p;
+    }
+    unsigned long long *d_invalid = nullptr;
+    if (n_invalid) {
+        if ((rc = ecb_reserve(ctx, st->rep_io, 8))) return rc;
+        d_invalid = (unsigned long long *) st->rep_io.p;
+    }
+    if ((rc = launch_reprojection(ctx, st, intrinsics, out, d_invalid))) return rc;
+    if (h_out && (rc = ecb_d2h(ctx, h_out, out, (size_t) st->n_res * 8))) return rc;
+    if (n_invalid) {
+        unsigned long long c = 0;
+        if ((rc = ecb_d2h(ctx, &c, d_invalid, 8))) return rc;
+        *n_invalid = (int64_t) c;
+    }
+    return ECB_OK;
+}
+
+int ecb_cost_reprojection_groups(ecb_ctx *ctx, const double *intrinsics, const double *rot_cp, const double *trans_cp, int by,
+                                 const double *kf_time, int n_keyframes, int cell_px, ecb_reprojection_group *groups, int cap,
+                                 int *n_groups, ecb_reprojection_group *total) {
+    if (!ctx || !intrinsics || !rot_cp || !trans_cp) return ECB_ERR_ARG;
+    cudaSetDevice(ctx->device);
+    CostState *st = (CostState *) ctx->cost;
+    GroupKeyArgs a;
+    int64_t G = 0;
+    bool query = false;
+    int rc;
+    if ((rc = group_layout(ctx, st, by, kf_time, n_keyframes, cell_px, groups != nullptr, cap, n_groups, a, &G, &query))) return rc;
+    if (query) return ECB_OK;
+    const int64_t n = st->n_res;
+    std::vector<ecb_reprojection_group> h((size_t) G + 1);
+    memset(h.data(), 0, h.size() * sizeof(ecb_reprojection_group));
+    if (n > 0) {
+        if ((rc = upload_params(ctx, st, intrinsics, rot_cp, trans_cp))) return rc;
+        if ((rc = ecb_reserve(ctx, st->rep_r, (size_t) n * 8))) return rc;
+        if ((rc = ecb_reserve(ctx, st->rep_out, ((size_t) G + 1) * sizeof(ecb_reprojection_group)))) return rc;
+        if ((rc = launch_reprojection(ctx, st, intrinsics, (double *) st->rep_r.p, nullptr))) return rc;
+        const uint32_t *sidx = nullptr;
+        if ((rc = group_sort(ctx, st, a, G, kf_time, &sidx))) return rc;
+        k_reproj_reduce<<<(unsigned) (G + 1), RG_THREADS, 0, ctx->stream>>>((const double *) st->rep_r.p, sidx,
+                                                                          (const int64_t *) st->rep_start.p,
+                                                                          (ecb_reprojection_group *) st->rep_out.p);
+        ECB_LAUNCHED(ctx);
+        if ((rc = ecb_check(ctx, cudaGetLastError(), "k_reproj_reduce"))) return rc;
+        if ((rc = ecb_d2h(ctx, h.data(), st->rep_out.p, h.size() * sizeof(ecb_reprojection_group)))) return rc;
+    }
+    memcpy(groups, h.data(), (size_t) G * sizeof(ecb_reprojection_group));
+    if (total) {  // groups 0 .. G-1 and the records outside every group, in group order; sum compensated as in k_reproj_reduce
+        ecb_reprojection_group s;
+        memset(&s, 0, sizeof s);
+        double comp = 0.0;
+        for (const ecb_reprojection_group &q : h) {
+            s.count += q.count;
+            s.n_invalid += q.n_invalid;
+            ecb_comp_add(s.sum, comp, q.sum);
+            s.sum_sq += q.sum_sq;
+            s.max_abs = std::max(s.max_abs, q.max_abs);
+        }
+        s.sum += comp;
+        *total = s;
+    }
+    return ECB_OK;
+}
+
+int ecb_keyframe_reprojection(ecb_ctx *ctx, const double *intrinsics, const double *rot_cp, const double *trans_cp,
+                              const double *kf_time, const double *kf_circles, int n_keyframes, int n_circles,
+                              const double *landmarks_xyz, double *proj, double *err, ecb_reprojection_group *total) {
+    if (!ctx || !intrinsics || !rot_cp || !trans_cp || !kf_time || !kf_circles || !landmarks_xyz || n_keyframes < 1 ||
+        n_circles < 1)
+        return ECB_ERR_ARG;
+    if (!ctx->cost) return ecb_fail(ctx, ECB_ERR_STATE, "ecb_cost_setup first");
+    cudaSetDevice(ctx->device);
+    CostState *st = (CostState *) ctx->cost;
+    const size_t K = (size_t) n_keyframes, nc = (size_t) n_circles, m = K * nc;
+    int rc;
+    if ((rc = upload_params(ctx, st, intrinsics, rot_cp, trans_cp))) return rc;
+    // staging: kf_t K | circles 3 m | landmarks 3 nc | proj 2 m | err m
+    if ((rc = ecb_reserve(ctx, st->rep_io, (K + 6 * m + 3 * nc) * 8))) return rc;
+    double *d_t = (double *) st->rep_io.p, *d_c = d_t + K, *d_l = d_c + 3 * m, *d_p = d_l + 3 * nc, *d_e = d_p + 2 * m;
+    if ((rc = ecb_h2d(ctx, d_t, kf_time, K * 8))) return rc;
+    if ((rc = ecb_h2d(ctx, d_c, kf_circles, 3 * m * 8))) return rc;
+    if ((rc = ecb_h2d(ctx, d_l, landmarks_xyz, 3 * nc * 8))) return rc;
+    EcbSplineView sv;
+    ecb_cost_spline_view(ctx, &sv);
+    const EcbFold fold = ecb_inverse_radial_fold_host(intrinsics + 4);
+    (st->so3 ? k_keyframe_reproj<1> : k_keyframe_reproj<0>)<<<(unsigned) ((m + 127) / 128), 128, 0, ctx->stream>>>(
+        d_t, d_c, d_l, n_keyframes, n_circles, sv, (const double *) st->params.p, fold, d_p, d_e);
+    ECB_LAUNCHED(ctx);
+    if ((rc = ecb_check(ctx, cudaGetLastError(), "k_keyframe_reproj"))) return rc;
+    std::vector<double> h(3 * m);
+    if ((rc = ecb_d2h(ctx, h.data(), d_p, 3 * m * 8))) return rc;
+    if (proj) memcpy(proj, h.data(), 2 * m * 8);
+    if (err) memcpy(err, h.data() + 2 * m, m * 8);
+    if (total) {  // the present features in (key frame, circle) order
+        ecb_reprojection_group s;
+        memset(&s, 0, sizeof s);
+        for (size_t i = 0; i < m; ++i) {
+            if (!(kf_circles[3 * i + 2] >= 0.0)) continue;  // absent (as in k_keyframe_reproj)
+            const double e = h[2 * m + i];
+            if (std::isnan(e)) {
+                ++s.n_invalid;
+                continue;
+            }
+            ++s.count;
+            s.sum += e;
+            s.sum_sq += e * e;
+            s.max_abs = std::max(s.max_abs, e);
         }
         *total = s;
     }

@@ -32,6 +32,30 @@ ECB_HD void ecb_pose_dtheta(const double q[4], const double dq[4], double out[3]
     out[2] = 2.0 * (q[3] * dq[2] - dq[3] * q[2] - (q[0] * dq[1] - q[1] * dq[0]));
 }
 
+// The pose alone (rotation q = x y z w, translation t): the sums of ecb_pose_jacobian, without the Jacobian.
+ECB_HD void ecb_pose_eval(const double *Q, const double *T, const double N[4], int so3, double q[4], double t[3]) {
+    for (int c = 0; c < 3; ++c) {
+        double v = 0.0;
+        for (int j = 0; j < 4; ++j) v += N[j] * T[3 * j + c];
+        t[c] = v;
+    }
+    if (so3) {
+        double beta[3];
+        ecb_so3::cumulative_basis(N, beta);
+        ecb_so3::rotation_value(Q, beta, q);
+        return;
+    }
+    double n2 = 0.0;
+    for (int c = 0; c < 4; ++c) {
+        double v = 0.0;
+        for (int j = 0; j < 4; ++j) v += N[j] * Q[4 * j + c];
+        q[c] = v;
+        n2 += v * v;
+    }
+    const double nz = sqrt(n2);
+    for (int c = 0; c < 4; ++c) q[c] /= nz;
+}
+
 // Q: 4 rotation control points (x y z w each), T: 4 translation control points, N: the 4 basis values N_{i-3..i}(t);
 // so3: 0 normalised quaternion spline, 1 cumulative SO(3) spline.
 ECB_HD void ecb_pose_jacobian(const double *Q, const double *T, const double N[4], int so3, EcbPoseJac &o) {

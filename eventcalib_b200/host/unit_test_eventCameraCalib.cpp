@@ -33,6 +33,11 @@
 // (statistics per key frame, per board circle and per sensor cell of ECB_RESIDUAL_CELL pixels, default 16).  r is the raw
 // residual ||X_w - L|| - circleRadius, a distance on the board plane in the units of the board points, not pixels.  A cell size
 // that is not a positive integer ends the program with exit code 1 before any GPU work.
+//
+// ECB_REPROJECTION=1 reports the same fit in pixels after the optimisation, through the forward camera model: a "Reprojection:"
+// line (event-to-rim count, RMS, mean, max |e|, invalid count; key-frame-centre count and RMS; rho_fold * fx next to the farthest
+// sensor corner's distorted radius, in pixels) and SavePath/ReprojectionByKeyframe.txt, ReprojectionByCircle.txt and
+// ReprojectionMap.txt (cells of ECB_RESIDUAL_CELL pixels).
 #include <algorithm>
 #include <cstdio>
 #include <cstdlib>
@@ -480,6 +485,84 @@ int main(int argc, char **argv) {
                     if (byCell[c].count == 0) continue;
                     f << ((int) c % ncx) * residualCell << " " << ((int) c / ncx) * residualCell;
                     stats(f, byCell[c]);
+                }
+            }
+        }
+        if (getenv("ECB_REPROJECTION") && atoi(getenv("ECB_REPROJECTION")) != 0) {  // the same fit in pixels (no reference output)
+            std::vector<ecb_reprojection_group> byKf, byCircle, byCell;
+            ecb_reprojection_group tot, ctot;
+            std::vector<double> proj, cerr;
+            if (spline.reprojectionGroups(ECB_RESIDUALS_BY_KEYFRAME, residualCell, byKf, &tot) != ECB_OK ||
+                spline.reprojectionGroups(ECB_RESIDUALS_BY_CIRCLE, residualCell, byCircle, nullptr) != ECB_OK ||
+                spline.reprojectionGroups(ECB_RESIDUALS_BY_SENSOR_CELL, residualCell, byCell, nullptr) != ECB_OK ||
+                spline.keyframeReprojection(proj, cerr, &ctot) != ECB_OK) {
+                std::cerr << "ecb: " << spline.lastError() << std::endl;
+                return 1;
+            }
+            const std::array<double, 9> &in = spline.intrinsics();
+            double fold = 0.0, corner = 0.0;
+            ecb_inverse_radial_fold(in.data() + 4, &fold);
+            for (int c = 0; c < 4; ++c) {  // distorted radius of the sensor's corner pixels, in pixels of fx
+                const double x = ((c & 1) ? width - 1 : 0) - in[2], y = ((c & 2) ? height - 1 : 0) - in[3];
+                corner = std::max(corner, in[0] * std::sqrt((x / in[0]) * (x / in[0]) + (y / in[1]) * (y / in[1])));
+            }
+            const double nan = std::numeric_limits<double>::quiet_NaN();
+            auto mean = [&](const ecb_reprojection_group &g) { return g.count ? g.sum / (double) g.count : nan; };
+            auto rms = [&](const ecb_reprojection_group &g) { return g.count ? std::sqrt(g.sum_sq / (double) g.count) : nan; };
+            // key-frame centres per key frame / per circle: count and sum of squares over the projectable present features
+            const size_t K = byKf.size(), nc = byCircle.size();
+            std::vector<int64_t> ckN(K, 0), ccN(nc, 0);
+            std::vector<double> ckS(K, 0.0), ccS(nc, 0.0);
+            for (size_t k = 0; k < K; ++k)
+                for (size_t c = 0; c < nc; ++c) {
+                    const double e = cerr[k * nc + c];
+                    if (std::isnan(e)) continue;
+                    ++ckN[k], ++ccN[c];
+                    ckS[k] += e * e, ccS[c] += e * e;
+                }
+            auto crms = [&](int64_t n, double s) { return n ? std::sqrt(s / (double) n) : nan; };
+            std::cout << "Reprojection: " << tot.count << " events, RMS " << rms(tot) << " px, mean " << mean(tot) << " px, max |e| "
+                      << tot.max_abs << " px, invalid " << tot.n_invalid << "; " << ctot.count << " key-frame centres, RMS " << rms(ctot)
+                      << " px; fold at " << fold * in[0] << " px, farthest sensor corner at " << corner << " px" << std::endl;
+            auto stats = [&](std::ostream &f, const ecb_reprojection_group &g) {
+                f << std::defaultfloat << std::setprecision(17) << " " << g.count << " " << g.n_invalid << " " << mean(g) << " " << rms(g)
+                  << " " << g.max_abs;
+            };
+            const char *units = "# e = sign(|X_w - L| - circleRadius) |q - o| in pixels: o the event pixel, q the projection of the rim "
+                                "point L + circleRadius (X_w - L) / |X_w - L| (the residual's correspondence, not the distance to the "
+                                "projected ellipse); invalid: not projectable\n# centres: the board point at the key frame's stamp "
+                                "projected, against the detected circle centre (pixels)\n";
+            const std::string dir = std::string(argv[3]) + "/";
+            {
+                std::ofstream f(dir + "ReprojectionByKeyframe.txt");
+                f << units << "# stamp count n_invalid mean RMS max_abs centre_count centre_RMS (one line per key frame)\n";
+                for (size_t k = 0; k < K; ++k) {
+                    f << std::fixed << std::setprecision(10) << kfs[k].timeStamp;
+                    stats(f, byKf[k]);
+                    f << " " << ckN[k] << " " << crms(ckN[k], ckS[k]) << "\n";
+                }
+            }
+            {
+                std::ofstream f(dir + "ReprojectionByCircle.txt");
+                f << units << "# id x y z count n_invalid mean RMS max_abs centre_count centre_RMS (one line per board circle)\n";
+                for (size_t c = 0; c < nc; ++c) {
+                    f << c << std::defaultfloat << std::setprecision(17) << " " << landmarks[c][0] << " " << landmarks[c][1] << " "
+                      << landmarks[c][2];
+                    stats(f, byCircle[c]);
+                    f << " " << ccN[c] << " " << crms(ccN[c], ccS[c]) << "\n";
+                }
+            }
+            {
+                std::ofstream f(dir + "ReprojectionMap.txt");
+                const int ncx = (width + residualCell - 1) / residualCell;
+                f << units << "# cell " << residualCell << " px, " << ncx << " x " << (height + residualCell - 1) / residualCell
+                  << " cells of the " << width << " x " << height << " sensor\n"
+                  << "# u0 v0 count n_invalid mean RMS max_abs (one line per non-empty cell; u0 v0: its top-left pixel)\n";
+                for (size_t c = 0; c < byCell.size(); ++c) {
+                    if (byCell[c].count + byCell[c].n_invalid == 0) continue;
+                    f << ((int) c % ncx) * residualCell << " " << ((int) c / ncx) * residualCell;
+                    stats(f, byCell[c]);
+                    f << "\n";
                 }
             }
         }

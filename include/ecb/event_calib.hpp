@@ -988,6 +988,8 @@ public:
         if (ecb_cost_associate(ev_->ctx, t.data(), c.data(), (int) kf.size(), nc, &landmarks[0][0], step_, &n) != ECB_OK)
             throw std::runtime_error(ecb_last_error(ev_->ctx));
         kfTime_ = t;  // residualGroups(ECB_RESIDUALS_BY_KEYFRAME) groups by these stamps
+        kfCircles_ = c;  // keyframeReprojection reprojects these centres
+        landmarks_ = landmarks;
         return n;
     }
     bool optimize(ecb_lm_summary *summary = nullptr) {  // EventCalibSpline.cpp:115-251
@@ -1096,7 +1098,71 @@ public:
         a.max_abs = std::max(a.max_abs, b.max_abs);
         a.cost += b.cost;
     }
+    // The same fit in pixels, through the forward camera model (ecb_cost_reprojection_errors / ecb_cost_reprojection_groups /
+    // ecb_keyframe_reprojection), at the current point.  e_k = sign(|d| - radius) |q - o|: o the event pixel, q the projection of
+    // the rim point the residual measures; NaN where it cannot be projected.  reprojectionErrors: e of every record in the
+    // association's order; reprojectionGroups: the groups of residualGroups; keyframeReprojection: the board points at the stamps
+    // of the last associate() against the detected centres, proj[K][n][2] and err[K][n] (pixels, NaN for an absent feature).
+    int reprojectionErrors(std::vector<double> &e, int64_t *nInvalid = nullptr) const {
+        return reprojectionErrorsAt(ev_->ctx, intr_, seg_, e, nInvalid);
+    }
+    int reprojectionGroups(int by, int cellPx, std::vector<ecb_reprojection_group> &groups, ecb_reprojection_group *total) const {
+        return reprojectionGroupsAt(ev_->ctx, intr_, seg_, kfTime_, by, cellPx, groups, total);
+    }
+    int keyframeReprojection(std::vector<double> &proj, std::vector<double> &err, ecb_reprojection_group *total) const {
+        return keyframeReprojectionAt(ev_->ctx, intr_, seg_, kfTime_, kfCircles_, landmarks_, proj, err, total);
+    }
+    static int reprojectionErrorsAt(ecb_ctx *ctx, const std::array<double, 9> &intr, const std::vector<Segment> &seg,
+                                    std::vector<double> &e, int64_t *nInvalid) {
+        std::vector<double> rot, trans;
+        flatten(seg, rot, trans);
+        int64_t n = 0;
+        int rc = ecb_cost_layout(ctx, nullptr, nullptr, &n, nullptr);
+        if (rc != ECB_OK) return rc;
+        e.assign((size_t) n, 0.0);
+        return ecb_cost_reprojection_errors(ctx, intr.data(), rot.data(), trans.data(), nullptr, n > 0 ? e.data() : nullptr, nInvalid);
+    }
+    static int reprojectionGroupsAt(ecb_ctx *ctx, const std::array<double, 9> &intr, const std::vector<Segment> &seg,
+                                    const std::vector<double> &kfTime, int by, int cellPx, std::vector<ecb_reprojection_group> &groups,
+                                    ecb_reprojection_group *total) {
+        std::vector<double> rot, trans;
+        flatten(seg, rot, trans);
+        const double *kf = kfTime.empty() ? nullptr : kfTime.data();
+        int ng = 0;
+        int rc = ecb_cost_reprojection_groups(ctx, intr.data(), rot.data(), trans.data(), by, kf, (int) kfTime.size(), cellPx, nullptr,
+                                              0, &ng, nullptr);
+        if (rc != ECB_OK) return rc;
+        groups.assign((size_t) ng, ecb_reprojection_group{});
+        ecb_reprojection_group dummy;
+        return ecb_cost_reprojection_groups(ctx, intr.data(), rot.data(), trans.data(), by, kf, (int) kfTime.size(), cellPx,
+                                            ng > 0 ? groups.data() : &dummy, ng, &ng, total);
+    }
+    // kfCircles[K][n][3] (cx cy r, r < 0 absent) and landmarks[n] as given to ecb_cost_associate
+    static int keyframeReprojectionAt(ecb_ctx *ctx, const std::array<double, 9> &intr, const std::vector<Segment> &seg,
+                                      const std::vector<double> &kfTime, const std::vector<double> &kfCircles,
+                                      const std::vector<std::array<double, 3>> &landmarks, std::vector<double> &proj,
+                                      std::vector<double> &err, ecb_reprojection_group *total) {
+        std::vector<double> rot, trans;
+        flatten(seg, rot, trans);
+        const size_t m = kfTime.size() * landmarks.size();
+        if (m == 0 || kfCircles.size() != 3 * m) return ECB_ERR_STATE;  // no associate() yet
+        proj.assign(2 * m, 0.0);
+        err.assign(m, 0.0);
+        return ecb_keyframe_reprojection(ctx, intr.data(), rot.data(), trans.data(), kfTime.data(), kfCircles.data(),
+                                         (int) kfTime.size(), (int) landmarks.size(), &landmarks[0][0], proj.data(), err.data(),
+                                         total);
+    }
+    // adds group b into a: counts and sums added, max_abs the max (shards combine in rank order)
+    static void accumulateReprojectionGroup(ecb_reprojection_group &a, const ecb_reprojection_group &b) {
+        a.count += b.count;
+        a.n_invalid += b.n_invalid;
+        a.sum += b.sum;
+        a.sum_sq += b.sum_sq;
+        a.max_abs = std::max(a.max_abs, b.max_abs);
+    }
     const std::vector<double> &keyframeTimes() const { return kfTime_; }
+    const std::vector<double> &keyframeCircles() const { return kfCircles_; }
+    const std::vector<std::array<double, 3>> &landmarks() const { return landmarks_; }
     const std::array<double, 9> &intrinsics() const { return intr_; }
     const std::vector<Segment> &segments() const { return seg_; }
     // EventCalibSpline.hpp:286-303: index of the segment whose knot range holds t, else -1
@@ -1206,6 +1272,8 @@ private:
     std::vector<int32_t> n_cp_;
     std::array<double, 9> intr_;
     std::vector<double> kfTime_;  // key-frame stamps of the last associate()
+    std::vector<double> kfCircles_;  // ... its circles [K][n][3], r < 0 absent
+    std::vector<std::array<double, 3>> landmarks_;  // ... and its board points
     double step_, radius_;
     bool useSO3_ = false;
     static void flatten(const std::vector<Segment> &seg, std::vector<double> &rot, std::vector<double> &trans) {

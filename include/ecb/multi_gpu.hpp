@@ -355,6 +355,33 @@ public:
         if (total) *total = t;
         return ECB_OK;
     }
+    // Reprojection statistics in pixels (EventCalibSpline::reprojectionGroups), combined as residualGroups
+    int reprojectionGroups(int by, int cellPx, std::vector<ecb_reprojection_group> &groups, ecb_reprojection_group *total) const {
+        const int G = (int) sp_.size();
+        std::vector<std::vector<ecb_reprojection_group>> part((size_t) G);
+        std::vector<ecb_reprojection_group> tot((size_t) G);
+        std::vector<int> rc((size_t) G, ECB_OK);
+        forEachShard(G, [&](int g) {
+            rc[(size_t) g] = EventCalibSpline::reprojectionGroupsAt(ev_->shard[(size_t) g]->ctx, intrinsics(), segments(),
+                                                                    sp_[(size_t) g]->keyframeTimes(), by, cellPx, part[(size_t) g],
+                                                                    &tot[(size_t) g]);
+        });
+        for (int g = 0; g < G; ++g)
+            if (rc[(size_t) g] != ECB_OK) return rc[(size_t) g];
+        groups = part[0];
+        ecb_reprojection_group t = tot[0];
+        for (int g = 1; g < G; ++g) {
+            for (size_t i = 0; i < groups.size(); ++i) EventCalibSpline::accumulateReprojectionGroup(groups[i], part[(size_t) g][i]);
+            EventCalibSpline::accumulateReprojectionGroup(t, tot[(size_t) g]);
+        }
+        if (total) *total = t;
+        return ECB_OK;
+    }
+    // Key-frame centres reprojected (EventCalibSpline::keyframeReprojection): they read no records, rank 0's context answers
+    int keyframeReprojection(std::vector<double> &proj, std::vector<double> &err, ecb_reprojection_group *total) const {
+        return EventCalibSpline::keyframeReprojectionAt(ev_->shard[0]->ctx, intrinsics(), segments(), sp_[0]->keyframeTimes(),
+                                                        sp_[0]->keyframeCircles(), sp_[0]->landmarks(), proj, err, total);
+    }
     const std::array<double, 9> &intrinsics() const { return solved_ ? result_intr_ : sp_[0]->intrinsics(); }
     const std::vector<Segment> &segments() const { return solved_ ? seg_ : sp_[0]->segments(); }
     int saveKeyFrameTrajectoryTUM(const std::string &filename, const std::vector<double> &keyframeStamps) const {

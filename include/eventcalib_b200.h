@@ -272,6 +272,42 @@ int ecb_cost_residual_groups(ecb_ctx *ctx, const double *intrinsics, const doubl
                              const double *kf_time, int n_keyframes, int cell_px, ecb_residual_group *groups, int cap,
                              int *n_groups, ecb_residual_group *total);
 
+/* ---- the same fit in pixels: reprojection errors through the forward camera model --------------------------------------------
+ * The spline stage's distortion is the inverse radial polynomial (undistorted = distorted * s(rho_d^2), s = 1 + k1 rho^2 + ... +
+ * k5 rho^10, ecb_residual.h); projecting inverts g(rho) = rho s(rho^2) by safeguarded Newton (ecb_camera.h).  g is increasing
+ * on [0, rho_fold) only, rho_fold^2 = the smallest positive root of h(u) = 1 + 3 k1 u + 5 k2 u^2 + ... + 11 k5 u^5, so points
+ * whose undistorted radius reaches g(rho_fold) cannot be projected.
+ * e_k, the reprojection error of record k in pixels: X_w = the event pixel o back-projected onto the board plane at the record's
+ * pose (as in the residual), d = X_w - L, rim point P = L + radius d / |d| (the correspondence the residual measures), q = the
+ * pixel of P; e_k = sign(|d| - radius) |q - o|, positive when the event lies outside the projected rim.  It is the residual's
+ * correspondence seen in the image, NOT the distance to the projected ellipse of the circle.  e_k is NaN (not projectable)
+ * when |d| = 0, when the event's own distorted radius is >= rho_fold (the model folds inside the sensor there), when P lies
+ * behind the camera or past the fold, or when a value is not finite. */
+/* host only: rho_fold of the inverse radial polynomial k[5] (+INFINITY when g is increasing everywhere) */
+int ecb_inverse_radial_fold(const double *k, double *rho_fold);
+/* e_k of every record, in the order of ecb_cost_residuals; NaN = not projectable.  d_out / h_out as ecb_cost_residuals;
+ * n_invalid (optional) synchronises. */
+int ecb_cost_reprojection_errors(ecb_ctx *ctx, const double *intrinsics, const double *rot_cp, const double *trans_cp,
+                                 double *d_out, double *h_out, int64_t *n_invalid);
+/* Statistics of a group of reprojection errors, in pixels.  count, sum, sum_sq and max_abs cover the valid records only (RMS =
+ * sqrt(sum_sq / count)); an invalid record adds to n_invalid and to nothing else. */
+typedef struct { int64_t count, n_invalid; double sum, sum_sq, max_abs; } ecb_reprojection_group;  /* pixels */
+/* The groups of ecb_cost_residual_groups (by, kf_time, n_keyframes, cell_px, the size query, cap, every error code and the 2^32
+ * record limit are the same) over e_k.  Deterministic: repeated calls are bit-identical.  Synchronises. */
+int ecb_cost_reprojection_groups(ecb_ctx *ctx, const double *intrinsics, const double *rot_cp, const double *trans_cp, int by,
+                                 const double *kf_time, int n_keyframes, int cell_px, ecb_reprojection_group *groups, int cap,
+                                 int *n_groups, ecb_reprojection_group *total);
+/* circle centres of the key frames reprojected at their stamps: proj[K][n_circles][2], err[K][n_circles] = |proj - (cx,cy)|;
+ * NaN for an absent feature (r < 0), a stamp outside every segment, or a point that cannot be projected.
+ * kf_time / kf_circles / landmarks_xyz as ecb_cost_associate (host arrays); the pose is the spline of ecb_cost_setup at the
+ * point, in the rotation model of the context.  This is the quantity calibrateCamera reports, against the detected centre: the
+ * fitted ellipse centre is not the projected circle centre (OpenCV's circle-grid calibration has the same bias).  proj, err and
+ * total are optional; total covers the present features (absent ones count nowhere, unprojectable ones in n_invalid).  Needs
+ * ecb_cost_setup, reads no residual records.  Synchronises. */
+int ecb_keyframe_reprojection(ecb_ctx *ctx, const double *intrinsics, const double *rot_cp, const double *trans_cp,
+                              const double *kf_time, const double *kf_circles, int n_keyframes, int n_circles,
+                              const double *landmarks_xyz, double *proj, double *err, ecb_reprojection_group *total);
+
 /* Multi-GPU (one process per GPU): the same evaluation with the inter-GPU sum fused in.  Every rank owns a receive
  * buffer of ecb_exchange_buffer_bytes() bytes, ZERO-FILLED once, in device memory its peers can write (same process:
  * any cudaMalloc pointer with peer access; other processes: ecb_device_alloc + ecb_ipc_export / ecb_ipc_open).
