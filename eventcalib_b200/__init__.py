@@ -5,6 +5,7 @@ binds it with ctypes for the tests, ``bench.py`` and ``__graft_entry__``.  There
 library is missing or no CUDA device is present, every compute call raises.
 """
 import ctypes as C
+import math
 import os
 
 import numpy as np
@@ -108,7 +109,7 @@ SYMBOLS = ["ecb_ctx_create", "ecb_ctx_destroy", "ecb_last_error", "ecb_launch_co
            "ecb_lm_state", "ecb_lm_trace", "ecb_calibrate", "ecb_lm_device_create", "ecb_lm_device_destroy",
            "ecb_lm_device_set_exchange", "ecb_lm_device_begin", "ecb_lm_device_iterate", "ecb_lm_device_running",
            "ecb_lm_device_result", "ecb_calibrate_device", "ecb_covariance", "ecb_pose_covariance",
-           "ecb_pose_covariance_device", "ecb_cost_residuals", "ecb_cost_residual_groups",
+           "ecb_pose_covariance_device", "ecb_cost_residuals", "ecb_cost_residual_groups", "ecb_cost_reject",
            "ecb_inverse_radial_fold", "ecb_cost_reprojection_errors", "ecb_cost_reprojection_groups", "ecb_keyframe_reprojection"]
 
 _lib = None
@@ -176,6 +177,7 @@ def load_library():
     lib.ecb_cost_normal_eq.argtypes = [vp, vp, vp, vp, vp, vp, vp]
     lib.ecb_cost_residuals.argtypes = [vp, vp, vp, vp, vp, vp]
     lib.ecb_cost_residual_groups.argtypes = [vp, vp, vp, vp, i32, vp, i32, i32, vp, i32, C.POINTER(C.c_int), vp]
+    lib.ecb_cost_reject.argtypes = [vp, vp, vp, vp, dbl, vp, vp, i32, C.POINTER(i64), C.POINTER(i64)]
     lib.ecb_inverse_radial_fold.argtypes = [vp, C.POINTER(dbl)]
     lib.ecb_cost_reprojection_errors.argtypes = [vp, vp, vp, vp, vp, vp, C.POINTER(i64)]
     lib.ecb_cost_reprojection_groups.argtypes = [vp, vp, vp, vp, i32, vp, i32, i32, vp, i32, C.POINTER(C.c_int), vp]
@@ -592,6 +594,23 @@ class Context:
         total = np.zeros((), RESIDUAL_GROUP_DTYPE)
         self._chk(self.lib.ecb_cost_residual_groups(*args, _ptr(groups), ng.value, C.byref(ng), _ptr(total)))
         return groups[:ng.value], total
+
+    def reject_residuals(self, intr, rot, trans, max_abs_r=math.inf, drop_keyframes=None, kf_t=None):
+        """Removes outliers from this context's records (ecb_cost_reject): record k goes when not |r_k| <= max_abs_r (r_k as
+        cost_residuals returns it at the point; NaN always goes) or when drop_keyframes[j] is true for its key frame j (the
+        grouping of residual_groups(by="keyframe"); kf_t: the stamps given to cost_associate).  The kept records keep their
+        order, and every later call on the context sees only them until the next association or cost_set_residuals.
+        Returns (n_kept, n_removed)."""
+        a = [np.ascontiguousarray(v, np.float64) for v in (intr, rot, trans)]
+        kf = np.ascontiguousarray(kf_t, np.float64) if kf_t is not None else None
+        drop = np.ascontiguousarray(np.asarray(drop_keyframes) != 0, np.uint8) if drop_keyframes is not None else None
+        if drop is not None and kf is not None and len(kf) != len(drop):
+            raise ValueError("drop_keyframes and kf_t must have one entry per key frame")
+        nk = len(drop) if drop is not None else (len(kf) if kf is not None else 0)
+        kept, removed = C.c_int64(0), C.c_int64(0)
+        self._chk(self.lib.ecb_cost_reject(self.h, _ptr(a[0]), _ptr(a[1]), _ptr(a[2]), float(max_abs_r), _ptr(kf), _ptr(drop), nk,
+                                           C.byref(kept), C.byref(removed)))
+        return kept.value, removed.value
 
     def reprojection_errors(self, intr, rot, trans, d_out=None, host=True):
         """Reprojection errors e_k of every record in pixels (ecb_cost_reprojection_errors), in the order of cost_residuals():

@@ -16,6 +16,7 @@
 //   k_cost          cost-only evaluation (LM step acceptance)
 //   k_residuals, k_group_*            the residual report (board units)
 //   k_reprojection, k_reproj_reduce, k_keyframe_reproj   the same fit in pixels (forward model of ecb_camera.h)
+//   k_reject_count, k_reject_write    outlier rejection: ordered compaction of the records that are kept (ecb_cost_reject)
 #include <stdlib.h>
 #include <string.h>
 
@@ -60,6 +61,9 @@ struct CostState {
     uint64_t assoc_events_gen = 0;
     DevBuf rep_r, rep_key[2], rep_idx[2], rep_hist, rep_start, rep_out, rep_kf;  // residual report (ecb_cost_residual_groups)
     DevBuf rep_io;  // reprojection report: invalid count; staging of ecb_keyframe_reprojection
+    // ecb_cost_reject: the spare set of record buffers the kept records are compacted into, then swapped with the live ones
+    // (order of reject_bufs)
+    DevBuf rej[9];
     uint64_t xch_last_epoch = 0;   // ecb_cost_normal_eq_exchange: last epoch sent / generation of the caller's sequence
     uint32_t xch_generation = 0;
 };
@@ -788,6 +792,73 @@ __global__ void __launch_bounds__(RG_THREADS) k_group_reduce(const double *__res
     }
 }
 
+// ------------------------------------------------------------------------ outlier rejection ----
+// k_reject_count  keep flag of every record (|r_k| <= threshold, and its key frame not dropped) and the per-block count
+// k_reject_write  ordered compaction of the kept records into the spare buffers (k_assoc_write's scheme; blocks overlap, so
+//                 not in place)
+struct RejectArgs {
+    const double *r;           // r_k (k_residuals)
+    double max_abs;
+    const uint8_t *drop;       // per key frame, or null
+    const double *kf_t;        // the association's stamps (drop != null)
+    int K;
+    const int64_t *sel_event;  // association: event of record k
+    const double *ev_t;
+    int64_t n;
+};
+
+__global__ void __launch_bounds__(AS_THREADS) k_reject_count(const RejectArgs a, uint8_t *__restrict__ keep,
+                                                            uint32_t *__restrict__ block_cnt) {
+    __shared__ uint32_t ws[33];
+    const int64_t k = (int64_t) blockIdx.x * AS_THREADS + threadIdx.x;
+    uint32_t kp = 0;
+    if (k < a.n) {
+        kp = fabs(a.r[k]) <= a.max_abs ? 1u : 0u;  // NaN: removed
+        if (kp && a.drop && a.drop[nearest_kf(a.kf_t, a.K, a.ev_t[a.sel_event[k]])]) kp = 0;
+        keep[k] = (uint8_t) kp;
+    }
+    uint32_t tot;
+    block_excl_scan(kp, ws, &tot);
+    if (threadIdx.x == 0) block_cnt[blockIdx.x] = tot;
+}
+
+// the record arrays of one buffer set; a null pointer is an array the path does not hold
+struct RecordPtrs {
+    double2 *obs;
+    double4 *basis;
+    int *cp0, *span;
+    int64_t *sel_event;
+    int *sel_circle;
+    double *lm, *tt;
+    int *spl;
+};
+
+__global__ void __launch_bounds__(AS_THREADS) k_reject_write(const uint8_t *__restrict__ keep, const int64_t *__restrict__ block_off,
+                                                            int64_t n, const RecordPtrs s, const RecordPtrs d) {
+    __shared__ uint32_t ws[33];
+    const int64_t k = (int64_t) blockIdx.x * AS_THREADS + threadIdx.x;
+    const uint32_t kp = k < n ? keep[k] : 0u;
+    uint32_t tot;
+    const uint32_t ex = block_excl_scan(kp, ws, &tot);
+    if (!kp) return;
+    const int64_t o = block_off[blockIdx.x] + ex;
+    d.obs[o] = s.obs[k];
+    d.basis[o] = s.basis[k];
+    d.cp0[o] = s.cp0[k];
+    d.span[o] = s.span[k];
+    if (s.sel_event) {
+        d.sel_event[o] = s.sel_event[k];
+        d.sel_circle[o] = s.sel_circle[k];
+    }
+    if (s.lm) {
+        d.lm[3 * o] = s.lm[3 * k];
+        d.lm[3 * o + 1] = s.lm[3 * k + 1];
+        d.lm[3 * o + 2] = s.lm[3 * k + 2];
+        d.tt[o] = s.tt[k];
+        d.spl[o] = s.spl[k];
+    }
+}
+
 // ------------------------------------------------------------------------ reprojection report ----
 // k_reprojection    the loads of k_residuals; the record's pose (ecb_pose_eval), then e_k in pixels (ecb_rim_reprojection), NaN
 //                   when not projectable; optional count of the NaN records (integer atomics, one per warp)
@@ -1019,6 +1090,8 @@ void ecb_cost_free(ecb_ctx *ctx) {
                       &st->rep_idx[1], &st->rep_hist, &st->rep_start, &st->rep_out, &st->rep_kf, &st->rep_io};
     for (DevBuf *b : bufs)
         if (b->p) cudaFree(b->p);
+    for (DevBuf &b : st->rej)
+        if (b.p) cudaFree(b.p);
     delete st;
     ctx->cost = nullptr;
 }
@@ -1656,6 +1729,101 @@ int ecb_cost_residual_groups(ecb_ctx *ctx, const double *intrinsics, const doubl
         *total = s;
     }
     return ECB_OK;
+}
+
+// ---- outlier rejection ----
+int ecb_cost_reject(ecb_ctx *ctx, const double *intrinsics, const double *rot_cp, const double *trans_cp, double max_abs_residual,
+                    const double *kf_time, const uint8_t *drop_keyframe, int n_keyframes, int64_t *n_kept, int64_t *n_removed) {
+    if (!ctx || !intrinsics || !rot_cp || !trans_cp) return ECB_ERR_ARG;
+    if (!(max_abs_residual >= 0.0)) return ecb_fail(ctx, ECB_ERR_ARG, "max_abs_residual %g is NaN or negative", max_abs_residual);
+    if (drop_keyframe && !kf_time) return ecb_fail(ctx, ECB_ERR_ARG, "a key-frame mask needs the key-frame stamps");
+    if (!ctx->cost) return ecb_fail(ctx, ECB_ERR_STATE, "ecb_cost_setup first");
+    cudaSetDevice(ctx->device);
+    CostState *st = (CostState *) ctx->cost;
+    if (drop_keyframe) {
+        if (!st->assoc) return ecb_fail(ctx, ECB_ERR_STATE, "residuals of ecb_cost_set_residuals have no key frame: associate first");
+        if (st->assoc_events_gen != ctx->events_gen) return ecb_fail(ctx, ECB_ERR_STATE, "events were loaded after the association");
+        if (n_keyframes != st->assoc_K)
+            return ecb_fail(ctx, ECB_ERR_ARG, "%d key frames given, the association used %d", n_keyframes, st->assoc_K);
+    }
+    const int64_t n = st->n_res;
+    if (n > 0xFFFFFFFFll) return ecb_fail(ctx, ECB_ERR_UNSUPPORTED, "outlier rejection over 2^32 or more records");
+    if (n_kept) *n_kept = n;
+    if (n_removed) *n_removed = 0;
+    if (n == 0) return ECB_OK;
+    int rc;
+    const int nb = (int) ((n + AS_THREADS - 1) / AS_THREADS);
+    // r_k as ecb_cost_residuals returns it; the association's scratch holds the keep flags, block counts and offsets
+    if ((rc = upload_params(ctx, st, intrinsics, rot_cp, trans_cp))) return rc;
+    if ((rc = ecb_reserve(ctx, st->rep_r, (size_t) n * 8))) return rc;
+    if ((rc = ecb_reserve(ctx, st->ev_tag, (size_t) n + 16))) return rc;
+    if ((rc = ecb_reserve(ctx, st->ev_cnt, (size_t) nb * 4 + 16))) return rc;
+    if ((rc = ecb_reserve(ctx, st->ev_flag, (size_t) nb * 8 + 16))) return rc;
+    if ((rc = launch_residuals(ctx, st, (double *) st->rep_r.p))) return rc;
+    RejectArgs a;
+    memset(&a, 0, sizeof a);
+    a.r = (const double *) st->rep_r.p;
+    a.max_abs = max_abs_residual;
+    a.n = n;
+    if (drop_keyframe) {  // the mask and the stamps share one upload
+        const size_t K = (size_t) n_keyframes;
+        std::vector<uint8_t> up(K * 8 + K);
+        memcpy(up.data(), kf_time, K * 8);
+        memcpy(up.data() + K * 8, drop_keyframe, K);
+        if ((rc = ecb_reserve(ctx, st->rep_kf, up.size()))) return rc;
+        if ((rc = ecb_h2d(ctx, st->rep_kf.p, up.data(), up.size()))) return rc;
+        a.kf_t = (const double *) st->rep_kf.p;
+        a.drop = (const uint8_t *) st->rep_kf.p + K * 8;
+        a.K = n_keyframes;
+        a.sel_event = (const int64_t *) st->sel_event.p;
+        a.ev_t = (const double *) ctx->ev_t.p;
+    }
+    uint8_t *keep = (uint8_t *) st->ev_tag.p;
+    int64_t *off = (int64_t *) st->ev_flag.p, *d_total = off + nb;
+    k_reject_count<<<nb, AS_THREADS, 0, ctx->stream>>>(a, keep, (uint32_t *) st->ev_cnt.p);
+    ECB_LAUNCHED(ctx);
+    k_scan_blocks<<<1, 1024, 0, ctx->stream>>>((uint32_t *) st->ev_cnt.p, nb, off, d_total);
+    ECB_LAUNCHED(ctx);
+    int64_t kept = 0;
+    if ((rc = ecb_d2h(ctx, &kept, d_total, 8))) return rc;
+    if (n_kept) *n_kept = kept;
+    if (n_removed) *n_removed = n - kept;
+    if (kept == n) return ECB_OK;  // nothing removed: the records stay as they are, byte for byte
+    // every array the path holds: obs / basis / cp0 / span always, event and circle of an association, landmark / time /
+    // spline of explicit or unfused records
+    DevBuf *live[9] = {&st->obs, &st->basis, &st->cp0, &st->span, &st->sel_event, &st->sel_circle, &st->lm, &st->tt, &st->spl};
+    const size_t esz[9] = {16, 32, 4, 4, 8, 4, 24, 8, 4};
+    bool moved[9];
+    for (int i = 0; i < 9; ++i) moved[i] = i < 4 || (i < 6 ? st->assoc : !st->use_circ);
+    const size_t nk = (size_t) std::max<int64_t>(kept, 1);
+    void *src[9] = {}, *dst[9] = {};
+    for (int i = 0; i < 9; ++i) {
+        if (!moved[i]) continue;
+        if ((rc = ecb_reserve(ctx, st->rej[i], nk * esz[i]))) return rc;
+        src[i] = live[i]->p;
+        dst[i] = st->rej[i].p;
+    }
+    auto ptrs = [](void *const *p) {
+        RecordPtrs r;
+        r.obs = (double2 *) p[0];
+        r.basis = (double4 *) p[1];
+        r.cp0 = (int *) p[2];
+        r.span = (int *) p[3];
+        r.sel_event = (int64_t *) p[4];
+        r.sel_circle = (int *) p[5];
+        r.lm = (double *) p[6];
+        r.tt = (double *) p[7];
+        r.spl = (int *) p[8];
+        return r;
+    };
+    k_reject_write<<<nb, AS_THREADS, 0, ctx->stream>>>(keep, off, n, ptrs(src), ptrs(dst));
+    ECB_LAUNCHED(ctx);
+    if ((rc = ecb_check(ctx, cudaGetLastError(), "outlier rejection kernels"))) return rc;
+    for (int i = 0; i < 9; ++i)
+        if (moved[i]) std::swap(*live[i], st->rej[i]);
+    st->n_res = kept;
+    if ((rc = prepare_records(ctx, st, /*have_basis=*/true))) return rc;
+    return ecb_check(ctx, ecb_stream_sync(ctx), "outlier rejection");
 }
 
 // ---- reprojection report ----

@@ -34,6 +34,13 @@
 // residual ||X_w - L|| - circleRadius, a distance on the board plane in the units of the board points, not pixels.  A cell size
 // that is not a positive integer ends the program with exit code 1 before any GPU work.
 //
+// ECB_REJECT=k (a positive finite number) rejects outliers after the first optimisation, which the reference does not: the
+// statistics per key frame give s, the lower median of the key frames' RMS residuals; the key frames whose RMS exceeds k s and the
+// records with |r| > k s are removed (ecb::outlierRejection), an "Outlier rejection:" line is printed, and the optimisation runs
+// again from the first solution on the kept records ("Solver Summary (after rejection):").  The intrinsics, the trajectory and
+// every report and covariance file then describe the second solve.  An invalid value, or the variable together with
+// ECB_REFERENCE_SIGNATURES, ends the program with exit code 1 before any GPU work.
+//
 // ECB_REPROJECTION=1 reports the same fit in pixels after the optimisation, through the forward camera model: a "Reprojection:"
 // line (event-to-rim count, RMS, mean, max |e|, invalid count; key-frame-centre count and RMS; rho_fold * fx next to the farthest
 // sensor corner's distorted radius, in pixels) and SavePath/ReprojectionByKeyframe.txt, ReprojectionByCircle.txt and
@@ -103,6 +110,22 @@ int main(int argc, char **argv) {
             return 1;
         }
         constIntrinsics = (uint32_t) m;
+    }
+    double rejectK = 0.0;  // checked before any file or GPU work; 0: no outlier rejection
+    if (const char *rk = getenv("ECB_REJECT")) {
+        if (getenv("ECB_REFERENCE_SIGNATURES")) {
+            std::cerr << "ecb: ECB_REJECT cannot be combined with ECB_REFERENCE_SIGNATURES (the reference's EventCalibSpline "
+                         "optimises once on every residual)" << std::endl;
+            return 1;
+        }
+        char *end = nullptr;
+        const double v = strtod(rk, &end);
+        if (end == rk || *end != '\0' || !(v > 0.0) || !std::isfinite(v)) {
+            std::cerr << "ecb: ECB_REJECT must be a positive finite number (the factor k of the threshold k s), got '" << rk << "'"
+                      << std::endl;
+            return 1;
+        }
+        rejectK = v;
     }
     int residualCell = 16;  // checked before any file or GPU work
     if (const char *rc = getenv("ECB_RESIDUAL_CELL")) {
@@ -432,6 +455,33 @@ int main(int argc, char **argv) {
         std::cout << "Solver Summary: residuals " << n_res << ", splines " << segments.size() << ", iterations " << sum.iterations
                   << " (successful " << sum.successful_steps << "), cost " << sum.initial_cost << " -> " << sum.final_cost
                   << ", termination " << sum.termination << std::endl;
+        if (rejectK > 0.0) {  // outlier rejection, then the same optimisation again from the first solution (no reference output)
+            double s = 0.0, thr = 0.0;
+            std::vector<uint8_t> drop;
+            int64_t kept = 0, removed = 0;
+            if (spline.rejectOutliers(rejectK, &s, &thr, &drop, &kept, &removed) != ECB_OK) {
+                std::cerr << "ecb: " << spline.lastError() << std::endl;
+                return 1;
+            }
+            std::ostringstream line;
+            line.precision(8);
+            int nDrop = 0;
+            std::ostringstream dropped;
+            dropped << std::fixed << std::setprecision(10);
+            for (size_t k = 0; k < drop.size(); ++k)
+                if (drop[k]) dropped << (nDrop++ ? " " : "") << kfs[k].timeStamp;
+            line << "Outlier rejection: k " << rejectK << ", s " << s << ", threshold " << thr << ", key frames dropped " << nDrop
+                 << " [" << dropped.str() << "], records removed " << removed << " of " << kept + removed << " ("
+                 << (kept + removed ? 100.0 * (double) removed / (double) (kept + removed) : 0.0) << " %)";
+            std::cout << line.str() << std::endl;
+            if (!spline.optimize(&sum)) {
+                std::cerr << "ecb: " << spline.lastError() << std::endl;
+                return 1;
+            }
+            std::cout << "Solver Summary (after rejection): residuals " << kept << ", splines " << segments.size() << ", iterations "
+                      << sum.iterations << " (successful " << sum.successful_steps << "), cost " << sum.initial_cost << " -> "
+                      << sum.final_cost << ", termination " << sum.termination << std::endl;
+        }
         std::cout.precision(12);  // updateMap(), EventCalibSpline.cpp:263-264
         std::cout << "Intrinsics after optimization:";
         printEigenLike(std::cout, spline.intrinsics().data(), 1, 9);

@@ -65,6 +65,29 @@ inline int constantIntrinsicsMask(const std::string &names, std::string *unknown
     }
     return mask;
 }
+// Outlier policy over the residual statistics per key frame (ECB_RESIDUALS_BY_KEYFRAME, all shards combined): s = the lower median
+// (element floor((n - 1) / 2) after sorting) of the RMS sqrt(sum_sq / count) of the n key frames with count > 0; a key frame whose
+// RMS > k s is dropped, and a record is removed when |r| > k s.  The median over key frames keeps a minority of mislabelled
+// frames from inflating the scale, which a global RMS would not.  Empty key frames take no part and are never dropped.  Returns s
+// (0 without records); *threshold = k s, *drop = one flag per key frame (the arguments of ecb_cost_reject).
+inline double outlierRejection(const std::vector<ecb_residual_group> &byKeyframe, double k, double *threshold,
+                               std::vector<uint8_t> *drop) {
+    std::vector<double> rms(byKeyframe.size(), 0.0), sorted;
+    for (size_t j = 0; j < byKeyframe.size(); ++j)
+        if (byKeyframe[j].count > 0) {
+            rms[j] = std::sqrt(byKeyframe[j].sum_sq / (double) byKeyframe[j].count);
+            sorted.push_back(rms[j]);
+        }
+    std::sort(sorted.begin(), sorted.end());
+    const double s = sorted.empty() ? 0.0 : sorted[(sorted.size() - 1) / 2];
+    const double t = k * s;
+    if (threshold) *threshold = t;
+    if (drop) {
+        drop->assign(byKeyframe.size(), 0);
+        for (size_t j = 0; j < byKeyframe.size(); ++j) (*drop)[j] = byKeyframe[j].count > 0 && rms[j] > t ? 1 : 0;
+    }
+    return s;
+}
 }  // namespace ecb
 
 namespace opengv2 {
@@ -1088,6 +1111,22 @@ public:
         ecb_residual_group dummy;
         return ecb_cost_residual_groups(ctx, intr.data(), rot.data(), trans.data(), by, kf, (int) kfTime.size(), cellPx,
                                         ng > 0 ? groups.data() : &dummy, ng, &ng, total);
+    }
+    // Outlier rejection (ecb_cost_reject) at the current point: removes the records with !(|r| <= maxAbsR) and those of the key
+    // frames flagged in dropKeyframe (one flag per key frame of the last associate(); empty: no key-frame criterion).  A following
+    // optimize(), the reports and covariance() see only the kept records, until the next associate().  See ecb::outlierRejection.
+    int rejectResiduals(double maxAbsR, const std::vector<uint8_t> &dropKeyframe, int64_t *kept, int64_t *removed) {
+        return rejectResidualsAt(ev_->ctx, intr_, seg_, kfTime_, maxAbsR, dropKeyframe, kept, removed);
+    }
+    static int rejectResidualsAt(ecb_ctx *ctx, const std::array<double, 9> &intr, const std::vector<Segment> &seg,
+                                 const std::vector<double> &kfTime, double maxAbsR, const std::vector<uint8_t> &dropKeyframe,
+                                 int64_t *kept, int64_t *removed) {
+        std::vector<double> rot, trans;
+        flatten(seg, rot, trans);
+        const bool mask = !dropKeyframe.empty();
+        if (mask && dropKeyframe.size() != kfTime.size()) return ECB_ERR_ARG;
+        return ecb_cost_reject(ctx, intr.data(), rot.data(), trans.data(), maxAbsR, mask ? kfTime.data() : nullptr,
+                               mask ? dropKeyframe.data() : nullptr, (int) dropKeyframe.size(), kept, removed);
     }
     // adds group b into a: counts and sums added, max_abs the max (shards combine in rank order)
     static void accumulateResidualGroup(ecb_residual_group &a, const ecb_residual_group &b) {

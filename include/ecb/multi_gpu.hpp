@@ -210,12 +210,12 @@ public:
             for (int h = 0; h < g; ++h)
                 if (ev_->device[(size_t) g] == ev_->device[(size_t) h])
                     throw std::invalid_argument("ShardedCalibSpline::optimize: the shards must live on distinct devices");
-        std::vector<double> rot, trans;
-        for (auto &s : sp_[0]->segments()) {
+        std::vector<double> rot, trans;  // from the current point: a second optimize() continues from the first solution
+        for (auto &s : segments()) {
             rot.insert(rot.end(), s.rot_cp.begin(), s.rot_cp.end());
             trans.insert(trans.end(), s.trans_cp.begin(), s.trans_cp.end());
         }
-        std::array<double, 9> intr = sp_[0]->intrinsics();
+        std::array<double, 9> intr = intrinsics();
         ecb_lm_options opt;
         ecb_lm_default_options(&opt);
         opt.rotation_model = useSO3_ ? 1 : 0;
@@ -260,7 +260,7 @@ public:
         cleanup(lm, buf);
         if (summary) *summary = sum;
         // write the solution back into the segments
-        seg_ = sp_[0]->segments();
+        seg_ = segments();
         size_t ro = 0, to = 0;
         for (auto &s : seg_) {
             std::copy(result_rot_.begin() + ro, result_rot_.begin() + ro + s.rot_cp.size(), s.rot_cp.begin());
@@ -353,6 +353,36 @@ public:
             EventCalibSpline::accumulateResidualGroup(t, tot[(size_t) g]);
         }
         if (total) *total = t;
+        return ECB_OK;
+    }
+    // Outlier rejection at the current point: the shards' statistics per key frame combined in rank order (residualGroups), the
+    // policy applied once on the host (ecb::outlierRejection with factor k), then every shard removes its records with the same
+    // threshold and key-frame mask (EventCalibSpline::rejectResiduals, one host thread each), so the kept records do not depend
+    // on the sharding.  Outputs (each may be null): scale s, threshold k s, the mask, and the kept / removed records of all shards.
+    int rejectOutliers(double k, double *scale, double *threshold, std::vector<uint8_t> *drop, int64_t *kept, int64_t *removed) {
+        std::vector<ecb_residual_group> byKf;
+        int rc0 = residualGroups(ECB_RESIDUALS_BY_KEYFRAME, 16, byKf, nullptr);
+        if (rc0 != ECB_OK) return rc0;
+        double t = 0.0;
+        std::vector<uint8_t> mask;
+        const double s = ecb::outlierRejection(byKf, k, &t, &mask);
+        const int G = (int) sp_.size();
+        std::vector<int64_t> kp((size_t) G, 0), rm((size_t) G, 0);
+        std::vector<int> rc((size_t) G, ECB_OK);
+        forEachShard(G, [&](int g) {
+            rc[(size_t) g] = EventCalibSpline::rejectResidualsAt(ev_->shard[(size_t) g]->ctx, intrinsics(), segments(),
+                                                                 sp_[(size_t) g]->keyframeTimes(), t, mask, &kp[(size_t) g],
+                                                                 &rm[(size_t) g]);
+        });
+        for (int g = 0; g < G; ++g)
+            if (rc[(size_t) g] != ECB_OK) return rc[(size_t) g];
+        int64_t nk = 0, nr = 0;
+        for (int g = 0; g < G; ++g) nk += kp[(size_t) g], nr += rm[(size_t) g];
+        if (scale) *scale = s;
+        if (threshold) *threshold = t;
+        if (drop) *drop = mask;
+        if (kept) *kept = nk;
+        if (removed) *removed = nr;
         return ECB_OK;
     }
     // Reprojection statistics in pixels (EventCalibSpline::reprojectionGroups), combined as residualGroups

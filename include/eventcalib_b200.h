@@ -271,6 +271,22 @@ typedef struct {
 int ecb_cost_residual_groups(ecb_ctx *ctx, const double *intrinsics, const double *rot_cp, const double *trans_cp, int by,
                              const double *kf_time, int n_keyframes, int cell_px, ecb_residual_group *groups, int cap,
                              int *n_groups, ecb_residual_group *total);
+/* Outlier rejection: removes record k from this context when !(|r_k| <= max_abs_residual), r_k exactly as ecb_cost_residuals
+ * returns it at the point (so a non-finite r_k is always removed), or when drop_keyframe[j] != 0 for the key frame j the record
+ * counts under in ECB_RESIDUALS_BY_KEYFRAME (nearest stamp to the event, ties -> the earlier frame).  The kept records keep their
+ * order.  drop_keyframe = NULL: no key-frame criterion; max_abs_residual = INFINITY: no residual criterion.  kf_time /
+ * n_keyframes as in ecb_cost_residual_groups (the host stamps given to the association; only read with drop_keyframe).
+ * *n_kept / *n_removed (optional) count this context's records.  When nothing is removed the records are left untouched.
+ * The removal lasts until the next ecb_cost_associate[_device] or ecb_cost_set_residuals: ecb_cost_layout,
+ * ecb_cost_get_association, both reports, ecb_cost_eval, ecb_cost_normal_eq[_exchange], ecb_calibrate, the device LM (it reads
+ * the records at every evaluation, so one created before this call stays valid) and ecb_covariance see only the kept records.
+ * A covariance computed before the call still answers ecb_pose_covariance: call ecb_covariance again for the kept records.
+ * Errors: max_abs_residual NaN or negative, drop_keyframe without kf_time, or n_keyframes != the association's K: ECB_ERR_ARG.
+ * No ecb_cost_setup, drop_keyframe on records of ecb_cost_set_residuals, or drop_keyframe after events were loaded since the
+ * association: ECB_ERR_STATE.  n_residuals >= 2^32: ECB_ERR_UNSUPPORTED.  Zero records: ECB_OK, both counts 0.  No
+ * floating-point atomics: deterministic.  Synchronises. */
+int ecb_cost_reject(ecb_ctx *ctx, const double *intrinsics, const double *rot_cp, const double *trans_cp, double max_abs_residual,
+                    const double *kf_time, const uint8_t *drop_keyframe, int n_keyframes, int64_t *n_kept, int64_t *n_removed);
 
 /* ---- the same fit in pixels: reprojection errors through the forward camera model --------------------------------------------
  * The spline stage's distortion is the inverse radial polynomial (undistorted = distorted * s(rho_d^2), s = 1 + k1 rho^2 + ... +
