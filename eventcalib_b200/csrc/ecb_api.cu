@@ -403,7 +403,7 @@ int ecb_frontend_run(ecb_ctx *ctx, const double *windows, int n_win, const ecb_f
     ca.max_k = max_k;
     ca.W = ctx->width;
     ca.H = ctx->height;
-    ca.PW = ((ca.W + 2 * ca.E + 31) >> 5) + 1;
+    ca.PW = ecb_cluster_row_words(ca.W, ca.E);
     ca.PH = ca.H + 2 * ca.E;
     ca.min_pts = params->dbscan_min_pts;
     ca.cluster_min = params->cluster_min;
@@ -696,7 +696,7 @@ static int dbscan_batch(ecb_ctx *ctx, const double *xy, const int64_t *offsets, 
     ca.max_k = max_k;
     ca.W = Wmax;
     ca.H = Hmax;
-    ca.PW = ((ca.W + 2 * ca.E + 31) >> 5) + 1;
+    ca.PW = ecb_cluster_row_words(ca.W, ca.E);
     ca.PH = ca.H + 2 * ca.E;
     ca.min_pts = min_pts;
     ca.cluster_min = 0x7FFFFFFF;  // no kept-cluster tables on this path

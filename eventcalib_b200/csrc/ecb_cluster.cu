@@ -24,11 +24,15 @@
 
 namespace {
 
-template <typename RankT>
+// RankT: rank of the first pixel of every pair of bitmap words (u16 while every problem has fewer than 65535 points).
+// StT: r_st, per point the rank of a pid (steps 4 - 7), then the seed mask (8) and the member lists (9).  u16 (the narrow
+// layout) needs pid < 2^15 and n <= KD_PT * threads: the slow kd path keeps its node pid and tie flags in one 32-bit word.
+template <typename RankT, typename StT>
 struct Smem {
     uint32_t *U, *C;
     RankT *wrank;
-    uint32_t *r_pix, *r_lab, *r_kd, *r_st;
+    uint32_t *r_pix, *r_lab, *r_kd;
+    StT *r_st;
     uint8_t *r_flag;
 };
 
@@ -74,7 +78,7 @@ __device__ __forceinline__ void unite(uint32_t *parent, uint32_t a, uint32_t b) 
 
 // SM = true: bit planes AND per-point arrays live in shared memory — every pointer below is then derived from the
 // shared array alone, so the compiler emits LDS / STS / ATOMS with 32-bit addresses instead of generic accesses.
-template <typename RankT, bool SM>
+template <typename RankT, typename StT, bool SM>
 __global__ void __launch_bounds__(ECB_CL_THREADS, 2) k_cluster(const ClusterArgs a) {
     extern __shared__ __align__(16) uint32_t smem_raw[];
     __shared__ uint32_t ws[33];
@@ -83,8 +87,9 @@ __global__ void __launch_bounds__(ECB_CL_THREADS, 2) k_cluster(const ClusterArgs
 
     const int tid = threadIdx.x, nthr = blockDim.x, lane = tid & 31, wid = tid >> 5, nwarp = nthr >> 5;
     const int PW = a.PW, PH = a.PH, E = a.E, NW = PW * PH;
-    Smem<RankT> s;
-    const int plane_words = 2 * NW + (int) ((NW * sizeof(RankT) + 3) / 4);
+    const int NP = (NW + 1) >> 1;  // word pairs: one rank per pair (U is 8-byte aligned)
+    Smem<RankT, StT> s;
+    const int plane_words = 2 * NW + (int) ((NP * sizeof(RankT) + 3) / 4);
     uint32_t *arr;
     if constexpr (SM) {
         s.U = smem_raw;
@@ -100,10 +105,11 @@ __global__ void __launch_bounds__(ECB_CL_THREADS, 2) k_cluster(const ClusterArgs
     s.r_pix = arr;
     s.r_lab = arr + NC;
     s.r_kd = arr + 2 * NC;  // 2*NC words
-    s.r_st = arr + 4 * NC;
-    s.r_flag = reinterpret_cast<uint8_t *>(arr + 5 * NC);  // NC bytes, indexed by rank: kd tie flags (bit0 x, bit1 y)
+    const int st_words = sizeof(StT) == 4 ? NC : (NC + 1) >> 1;
+    s.r_st = reinterpret_cast<StT *>(arr + 4 * NC);
+    s.r_flag = reinterpret_cast<uint8_t *>(arr + (4 * NC + st_words));  // NC bytes, indexed by rank: kd tie flags (bit0 x, bit1 y)
     // kept-cluster scratch tables (raw id, size, member-list offset), max_k entries each (+1 for the end offset)
-    int32_t *k_raw = reinterpret_cast<int32_t *>(arr + 5 * NC + ((NC + 3) >> 2));
+    int32_t *k_raw = reinterpret_cast<int32_t *>(arr + (4 * NC + st_words + ((NC + 3) >> 2)));
     int32_t *k_size = k_raw + a.max_k, *k_off = k_size + a.max_k;
 
     // ---- 0. clear planes: once per CTA; every problem un-sets the words it touched when it is done with them (step 8) ----
@@ -148,29 +154,32 @@ __global__ void __launch_bounds__(ECB_CL_THREADS, 2) k_cluster(const ClusterArgs
             s.r_pix[pid] = loc;
         }
         __syncthreads();
-        // ---- 2. word-prefix popcounts: rank(x,y) = wrank[word] + popc(bits below) ---------------
+        // ---- 2. prefix popcounts per pair of words: rank(x,y) = wrank[pair] + popc(bits of the pair below) ----------
+        // bits of pair i; an odd NW leaves the last pair with one word of U (the other is C[0])
+        auto pair_bits = [&](int i) -> uint64_t { return 2 * i + 1 < NW ? reinterpret_cast<const uint64_t *>(s.U)[i] : (uint64_t) s.U[2 * i]; };
         uint32_t n_ranked;  // distinct in-range pixels = set bits of U (== n unless the input is flagged)
         {
-            const int per = (NW + nthr - 1) / nthr;
-            const int b = tid * per, e = min(NW, b + per);
+            const int per = (NP + nthr - 1) / nthr;
+            const int b = tid * per, e = min(NP, b + per);
             uint32_t c = 0;
 #if ECB_CL_ROLL
 #pragma unroll 1
 #endif
-            for (int i = b; i < e; ++i) c += __popc(s.U[i]);
+            for (int i = b; i < e; ++i) c += __popcll(pair_bits(i));
             uint32_t ex = block_excl_scan(c, ws, &n_ranked);
 #if ECB_CL_ROLL
 #pragma unroll 1
 #endif
             for (int i = b; i < e; ++i) {
                 s.wrank[i] = (RankT) ex;
-                ex += __popc(s.U[i]);
+                ex += __popcll(pair_bits(i));
             }
         }
         __syncthreads();
-        auto rank_of = [&](int x, int y) -> uint32_t {
+        auto rank_of = [&](int x, int y) -> uint32_t {  // (x,y) occupied: only bits below it are counted
             const int w = y * PW + (x >> 5);
-            return (uint32_t) s.wrank[w] + __popc(s.U[w] & ((1u << (x & 31)) - 1u));
+            const int b = ((w & 1) << 5) | (x & 31);
+            return (uint32_t) s.wrank[w >> 1] + __popcll(reinterpret_cast<const uint64_t *>(s.U)[w >> 1] & ((1ull << b) - 1ull));
         };
         // ---- 4. kd insertion-order emulation -> tie flags ---------------------------------------
         // NOTE: the root is pid 0 like kd_insert's first insertion.
@@ -219,9 +228,9 @@ __global__ void __launch_bounds__(ECB_CL_THREADS, 2) k_cluster(const ClusterArgs
                     const uint32_t rk = rank_of(mypix[k] & 0xFFFF, mypix[k] >> 16);
                     s.r_flag[rk] = (uint8_t) fl[k];
                     rloc[rk] = mypix[k];          // pixel of every rank: steps 5 - 6 walk the points in row-major order
-                    s.r_st[tid + k * nthr] = rk;  // rank of every pid: step 7
+                    s.r_st[tid + k * nthr] = (StT) rk;  // rank of every pid: step 7
                 }
-        } else {
+        } else if constexpr (sizeof(StT) == 4) {  // the launcher picks the narrow layout only where the fast path runs
             uint32_t *state = s.r_st;
             const uint32_t DONE = 0x3FFFFFFFu;
             for (int pid = tid; pid < n; pid += nthr) state[pid] = (pid == 0 || s.r_pix[pid] == ECB_NONE) ? DONE : 0u;
@@ -478,7 +487,7 @@ __global__ void __launch_bounds__(ECB_CL_THREADS, 2) k_cluster(const ClusterArgs
         }
         // ---- 8. seeds -> cluster ids ---------------------------------------------------------------------
         const int nw32 = (n + 31) >> 5;
-        uint32_t *seedmask = s.r_st, *seedpref = s.r_st + nw32;
+        uint32_t *seedmask = reinterpret_cast<uint32_t *>(s.r_st), *seedpref = seedmask + nw32;  // 8 * nw32 <= NC * sizeof(StT) bytes
         for (int i = tid; i < nw32; i += nthr) seedmask[i] = 0;
         __syncthreads();
         for (int pid = tid; pid < n; pid += nthr) {
@@ -580,7 +589,7 @@ __global__ void __launch_bounds__(ECB_CL_THREADS, 2) k_cluster(const ClusterArgs
             if (lane == 0) k_off[n_kept] = (int32_t) run;
         }
         __syncthreads();
-        uint32_t *members = s.r_st;  // seedmask/seedpref are dead
+        StT *members = s.r_st;  // seedmask/seedpref are dead
         uint32_t *gmem = a.kmem[d.pol] + d.off;
         KeptCluster *kt = a.ktab + (size_t) pb * a.max_k;
         if (n_kept > 0) {
@@ -631,7 +640,7 @@ __global__ void __launch_bounds__(ECB_CL_THREADS, 2) k_cluster(const ClusterArgs
                     uint32_t base = 0;
                     if (kidx >= 0) {
                         base = mycnt[kidx];
-                        members[k_off[kidx] + base + rk] = pid;
+                        members[k_off[kidx] + base + rk] = (StT) pid;
                     }
                     __syncwarp();
                     if (kidx >= 0 && rk == 0) mycnt[kidx] = base + __popc(peers);
@@ -647,7 +656,7 @@ __global__ void __launch_bounds__(ECB_CL_THREADS, 2) k_cluster(const ClusterArgs
                         const int pid = st + lane;
                         const bool m = pid < n && (int32_t) s.r_lab[pid] == cid;
                         const uint32_t ball = __ballot_sync(0xffffffffu, m);
-                        if (m) members[base + pos + __popc(ball & ((1u << lane) - 1u))] = pid;
+                        if (m) members[base + pos + __popc(ball & ((1u << lane) - 1u))] = (StT) pid;
                         pos += __popc(ball);
                     }
                 }
@@ -780,13 +789,16 @@ __global__ void __launch_bounds__(ECB_CL_THREADS, 2) k_cluster(const ClusterArgs
 
 }  // namespace
 
-// words of the per-point arrays + the kept-cluster scratch tables of one CTA
-static size_t cluster_array_words(int n_cap, int max_k) { return (size_t) 5 * n_cap + ((size_t) n_cap + 3) / 4 + (size_t) 3 * max_k + 1; }
+// words of the per-point arrays + the kept-cluster scratch tables of one CTA (st16: r_st as 16-bit words)
+static size_t cluster_array_words(int n_cap, int max_k, bool st16) {
+    return (size_t) 4 * n_cap + (st16 ? ((size_t) n_cap + 1) / 2 : (size_t) n_cap) + ((size_t) n_cap + 3) / 4 +
+           (size_t) 3 * max_k + 1;
+}
 
-size_t ecb_cluster_smem_bytes(int PW, int PH, int n_cap, int max_k, bool arrays_in_smem, bool rank32) {
-    size_t NW = (size_t) PW * PH;
-    size_t b = 2 * NW * 4 + ((NW * (rank32 ? 4 : 2) + 3) / 4) * 4;
-    if (arrays_in_smem) b += cluster_array_words(n_cap, max_k) * 4;
+size_t ecb_cluster_smem_bytes(int PW, int PH, int n_cap, int max_k, bool arrays_in_smem, bool rank32, bool st16) {
+    size_t NP = ((size_t) PW * PH + 1) / 2;
+    size_t b = (size_t) PW * PH * 8 + ((NP * (rank32 ? 4 : 2) + 3) / 4) * 4;
+    if (arrays_in_smem) b += cluster_array_words(n_cap, max_k, st16) * 4;
     return b;
 }
 
@@ -797,30 +809,40 @@ int ecb_launch_cluster(ecb_ctx *ctx, ClusterArgs &a, int max_n) {
     // static shared + reserve; also the (constant) dynamic-smem attribute value, so that concurrent launches from several
     // host threads with different sizes cannot race on cudaFuncSetAttribute
     const size_t limit = (size_t) ctx->smem_optin - 9 * 1024;
-    size_t planes = ecb_cluster_smem_bytes(a.PW, a.PH, a.n_cap, a.max_k, false, rank32);
-    size_t with_arrays = ecb_cluster_smem_bytes(a.PW, a.PH, a.n_cap, a.max_k, true, rank32);
+    const size_t planes = ecb_cluster_smem_bytes(a.PW, a.PH, a.n_cap, a.max_k, false, rank32, false);
     // sensors whose bit planes exceed one CTA's shared memory (e.g. 1280x720) run with the planes in per-CTA L2 scratch
     a.planes_in_smem = planes <= limit;
-    a.arrays_in_smem = with_arrays <= limit;  // else the per-point arrays live in per-CTA L2 scratch
-    size_t smem = a.arrays_in_smem ? with_arrays : (a.planes_in_smem ? planes : 0);
-    int per_sm = 1;
-    void (*kern)(const ClusterArgs) = rank32 ? (a.arrays_in_smem ? k_cluster<uint32_t, true> : k_cluster<uint32_t, false>)
-                                             : (a.arrays_in_smem ? k_cluster<uint16_t, true> : k_cluster<uint16_t, false>);
-    ECB_CUDA(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) limit));
     // CTA size: the kernel is barrier / latency bound, so more independent CTAs per SM beat bigger ones.  Shared memory
-    // decides how many CTAs fit (DAVIS346: 71 KB -> 3); at 64 registers an SM holds 1024 threads, so each CTA gets
-    // 1024 / CTAs threads (3 CTAs x 320 threads measured 16 % faster than 2 x 512).
-    int by_smem = 1;
-    ECB_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&by_smem, kern, 32, smem));
-    int threads = std::max(128, std::min(ECB_CL_THREADS, (1024 / std::max(by_smem, 1)) & ~31));
-    if (!a.arrays_in_smem) threads = ECB_CL_THREADS;  // large problems in L2 scratch: few CTAs, each wants all the threads it can get
-    if (const char *e = getenv("ECB_CL_THREADS")) threads = std::max(64, std::min(ECB_CL_THREADS, atoi(e) & ~31));
+    // decides how many CTAs fit (DAVIS346 at 1 235 points per problem: 54 KB -> 4); at 64 registers an SM holds 1024
+    // threads, so each CTA gets 1024 / CTAs threads (3 CTAs x 320 threads measured 16 % faster than 2 x 512).
+    // The narrow layout (16-bit r_st) is taken wherever it can run: pid < 2^15 and the fast kd path covers the batch.
+    void (*kern)(const ClusterArgs) = nullptr;
+    size_t smem = 0;
+    int threads = ECB_CL_THREADS;
+    for (int st16 = a.n_cap < 32768; st16 >= 0; --st16) {
+        const size_t with_arrays = ecb_cluster_smem_bytes(a.PW, a.PH, a.n_cap, a.max_k, true, rank32, st16);
+        a.arrays_in_smem = with_arrays <= limit;  // else the per-point arrays live in per-CTA L2 scratch
+        if (st16 && !a.arrays_in_smem) continue;
+        smem = a.arrays_in_smem ? with_arrays : (a.planes_in_smem ? planes : 0);
+        kern = st16 ? k_cluster<uint16_t, uint16_t, true>
+             : rank32 ? (a.arrays_in_smem ? k_cluster<uint32_t, uint32_t, true> : k_cluster<uint32_t, uint32_t, false>)
+                      : (a.arrays_in_smem ? k_cluster<uint16_t, uint32_t, true> : k_cluster<uint16_t, uint32_t, false>);
+        ECB_CUDA(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) limit));
+        int by_smem = 1;
+        ECB_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&by_smem, kern, 32, smem));
+        threads = std::max(128, std::min(ECB_CL_THREADS, (1024 / std::max(by_smem, 1)) & ~31));
+        if (!a.arrays_in_smem) threads = ECB_CL_THREADS;  // large problems in L2 scratch: few CTAs, each wants all the threads it can get
+        if (const char *e = getenv("ECB_CL_THREADS")) threads = std::max(64, std::min(ECB_CL_THREADS, atoi(e) & ~31));
+        if (!st16 || a.n_cap <= KD_PT * threads) break;
+    }
+    int per_sm = 1;
     ECB_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, threads, smem));
     if (per_sm < 1) per_sm = 1;
     int grid = ctx->sm_count * per_sm;
     if (grid > a.n_prob) grid = a.n_prob;
     if (!a.arrays_in_smem) {
-        a.gscratch_stride = cluster_array_words(a.n_cap, a.max_k) + (a.planes_in_smem ? 0 : (planes + 3) / 4);
+        // even: the bit planes at the start of a CTA's slice are read as 64-bit word pairs
+        a.gscratch_stride = (cluster_array_words(a.n_cap, a.max_k, false) + (a.planes_in_smem ? 0 : (planes + 3) / 4) + 1) & ~(size_t) 1;
         int rc = ecb_reserve(ctx, ctx->scratch, (size_t) grid * a.gscratch_stride * 4);
         if (rc) return rc;
         a.gscratch = (uint32_t *) ctx->scratch.p;

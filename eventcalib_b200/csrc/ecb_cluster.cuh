@@ -85,7 +85,10 @@ struct BfsArgs {
     double eps;
 };
 
-size_t ecb_cluster_smem_bytes(int PW, int PH, int n_cap, int max_k, bool arrays_in_smem, bool rank32);
+size_t ecb_cluster_smem_bytes(int PW, int PH, int n_cap, int max_k, bool arrays_in_smem, bool rank32, bool st16);
+// words per bitmap row: the padded sensor width W + 2E, rounded up to whole words (row_bits may read the word after a
+// row's last one, but for x0 + len <= W + 2E only for bits it masks off; the word after the last row of U and C exists)
+static inline int ecb_cluster_row_words(int W, int E) { return (W + 2 * E + 31) >> 5; }
 int ecb_launch_cluster(ecb_ctx *ctx, ClusterArgs &a, int max_n);
 int ecb_launch_bfs(ecb_ctx *ctx, BfsArgs &a);
 // general points: the tree is {left, right, parent, depth << 1 | side} and coordinates come from P[n][dim] (ecb_gridhash.cu)

@@ -171,7 +171,8 @@ __device__ __forceinline__ uint32_t block_excl_scan(uint32_t v, uint32_t *ws, ui
     return ws[wid] + inc - v;
 }
 
-// bits [x0, x0+len) of a bitmap row (len <= 32), row has at least one spare word after the last used one
+// bits [x0, x0+len) of a bitmap row (len <= 32); reads the word after x0's, which must be readable (it only supplies bits
+// when x0 + len crosses into it)
 __device__ __forceinline__ uint32_t row_bits(const uint32_t *row, int x0, int len) {
     const int wi = x0 >> 5, sh = x0 & 31;
     uint64_t v = (uint64_t) row[wi] | ((uint64_t) row[wi + 1] << 32);
