@@ -110,7 +110,7 @@ SYMBOLS = ["ecb_ctx_create", "ecb_ctx_destroy", "ecb_last_error", "ecb_launch_co
            "ecb_lm_device_set_exchange", "ecb_lm_device_begin", "ecb_lm_device_iterate", "ecb_lm_device_running",
            "ecb_lm_device_result", "ecb_calibrate_device", "ecb_covariance", "ecb_pose_covariance",
            "ecb_pose_covariance_device", "ecb_cost_residuals", "ecb_cost_residual_groups", "ecb_cost_reject",
-           "ecb_inverse_radial_fold", "ecb_cost_reprojection_errors", "ecb_cost_reprojection_groups", "ecb_keyframe_reprojection"]
+           "ecb_cost_reassociate", "ecb_inverse_radial_fold", "ecb_cost_reprojection_errors", "ecb_cost_reprojection_groups", "ecb_keyframe_reprojection"]
 
 _lib = None
 
@@ -178,6 +178,7 @@ def load_library():
     lib.ecb_cost_residuals.argtypes = [vp, vp, vp, vp, vp, vp]
     lib.ecb_cost_residual_groups.argtypes = [vp, vp, vp, vp, i32, vp, i32, i32, vp, i32, C.POINTER(C.c_int), vp]
     lib.ecb_cost_reject.argtypes = [vp, vp, vp, vp, dbl, vp, vp, i32, C.POINTER(i64), C.POINTER(i64)]
+    lib.ecb_cost_reassociate.argtypes = [vp, vp, vp, vp, dbl, dbl] + [C.POINTER(i64)] * 5
     lib.ecb_inverse_radial_fold.argtypes = [vp, C.POINTER(dbl)]
     lib.ecb_cost_reprojection_errors.argtypes = [vp, vp, vp, vp, vp, vp, C.POINTER(i64)]
     lib.ecb_cost_reprojection_groups.argtypes = [vp, vp, vp, vp, i32, vp, i32, i32, vp, i32, C.POINTER(C.c_int), vp]
@@ -611,6 +612,18 @@ class Context:
         self._chk(self.lib.ecb_cost_reject(self.h, _ptr(a[0]), _ptr(a[1]), _ptr(a[2]), float(max_abs_r), _ptr(kf), _ptr(drop), nk,
                                            C.byref(kept), C.byref(removed)))
         return kept.value, removed.value
+
+    def reassociate(self, intr, rot, trans, gate_px=5.0, max_dt=0.0):
+        """Re-associates the loaded events with the board circles at a calibrated point (ecb_cost_reassociate): every candidate
+        event of the association (max_dt = 0: its window; > 0: |t - t_kf| <= max_dt) is matched to the landmark nearest to its
+        back-projection at its own pose on the spline and kept when its event-to-rim error is below gate_px pixels.  The kept
+        events replace the records (event order, the layout of cost_associate); key frames and landmarks stay the association's.
+        Returns (n_residuals, n_same, n_changed, n_new, n_lost), the last four against the records held before the call."""
+        a = [np.ascontiguousarray(v, np.float64) for v in (intr, rot, trans)]
+        out = [C.c_int64(0) for _ in range(5)]
+        self._chk(self.lib.ecb_cost_reassociate(self.h, _ptr(a[0]), _ptr(a[1]), _ptr(a[2]), float(gate_px), float(max_dt),
+                                                *[C.byref(v) for v in out]))
+        return tuple(v.value for v in out)
 
     def reprojection_errors(self, intr, rot, trans, d_out=None, host=True):
         """Reprojection errors e_k of every record in pixels (ecb_cost_reprojection_errors), in the order of cost_residuals():

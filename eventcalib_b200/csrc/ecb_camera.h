@@ -170,6 +170,24 @@ ECB_HD void ecb_quat_rotate(const double q[4], const double v[3], bool conj, dou
     o[2] = v[2] + w * u2 + (x * u1 - y * u0);
 }
 
+// X_w: the event pixel (ou, ov) back-projected onto the board plane z = 0 at the pose (q, t), with the operations of the residual
+// (ecb_residual.h: unDistort, the third row of R(q), the ray-plane depth, q * v + t), so that X_w - L is the residual's d.
+// Not finite when the ray is parallel to the plane.
+ECB_HD void ecb_board_point(const double *intr, const double q[4], const double t[3], double ou, double ov, double Xw[3]) {
+    const double q0 = q[0], q1 = q[1], q2 = q[2], q3 = q[3];
+    const double x = (ou - intr[2]) * (1.0 / intr[0]), y = (ov - intr[3]) * (1.0 / intr[1]);
+    const double r2 = x * x + y * y, r4 = r2 * r2, r6 = r4 * r2, r8 = r6 * r2, r10 = r8 * r2;
+    const double s = 1.0 + intr[4] * r2 + intr[5] * r4 + intr[6] * r6 + intr[7] * r8 + intr[8] * r10;
+    const double X0 = x * s, X1 = y * s;
+    const double R30 = 2.0 * (q0 * q2 - q3 * q1), R31 = 2.0 * (q1 * q2 + q3 * q0), R32 = 1.0 - 2.0 * (q0 * q0 + q1 * q1);
+    const double lam = -t[2] * (1.0 / (R30 * X0 + R31 * X1 + R32));
+    const double v0 = lam * X0, v1 = lam * X1, v2 = lam;
+    const double uv0 = 2.0 * (q1 * v2 - q2 * v1), uv1 = 2.0 * (q2 * v0 - q0 * v2), uv2 = 2.0 * (q0 * v1 - q1 * v0);
+    Xw[0] = v0 + q3 * uv0 + (q1 * uv2 - q2 * uv1) + t[0];
+    Xw[1] = v1 + q3 * uv1 + (q2 * uv0 - q0 * uv2) + t[1];
+    Xw[2] = v2 + q3 * uv2 + (q0 * uv1 - q1 * uv0) + t[2];
+}
+
 // Reprojection error of one residual record, in pixels (the residual's correspondence seen in the image):
 //   X_w = back-projection of the event pixel o onto the board plane z = 0 at the pose (q, t) (as in ecb_residual.h),
 //   d = X_w - L, rim point P = L + radius d / |d|, p_c = R^T (P - t), q_px = its projection,

@@ -17,6 +17,7 @@
 //   k_residuals, k_group_*            the residual report (board units)
 //   k_reprojection, k_reproj_reduce, k_keyframe_reproj   the same fit in pixels (forward model of ecb_camera.h)
 //   k_reject_count, k_reject_write    outlier rejection: ordered compaction of the records that are kept (ecb_cost_reject)
+//   k_reassoc_count the association's pass 1 through the calibrated model (ecb_cost_reassociate); pass 2 is k_assoc_write
 #include <stdlib.h>
 #include <string.h>
 
@@ -59,6 +60,9 @@ struct CostState {
     bool assoc = false;
     int assoc_K = 0, assoc_n_circ = 0;
     uint64_t assoc_events_gen = 0;
+    // what ecb_cost_reassociate reuses of the association: its stamps (st->kf_t, or the caller's device table) and window
+    const double *assoc_kf_t = nullptr;
+    double assoc_gate2 = 0.0;
     DevBuf rep_r, rep_key[2], rep_idx[2], rep_hist, rep_start, rep_out, rep_kf;  // residual report (ecb_cost_residual_groups)
     DevBuf rep_io;  // reprojection report: invalid count; staging of ecb_keyframe_reprojection
     // ecb_cost_reject: the spare set of record buffers the kept records are compacted into, then swapped with the live ones
@@ -505,17 +509,19 @@ struct AssocArgs {
     int *cp0, *span;
 };
 
+// the first spline segment whose knot range holds u, or -1
+__device__ __forceinline__ int segment_of(const AssocArgs &a, double u) {
+    for (int q = 0; q < a.n_splines; ++q) {
+        const double *kn = a.knots + a.knot_off[q];
+        if (u >= kn[0] && u <= kn[a.ncp[q] + 3]) return q;
+    }
+    return -1;
+}
+
 // returns the spline index and the circle id (or -1) of one raw event
 __device__ __forceinline__ int assoc_one(const AssocArgs &a, int64_t i, int *spline_out) {
     const double u = a.ev_t[i];
-    int s = -1;
-    for (int q = 0; q < a.n_splines; ++q) {
-        const double *kn = a.knots + a.knot_off[q];
-        if (u >= kn[0] && u <= kn[a.ncp[q] + 3]) {
-            s = q;
-            break;
-        }
-    }
+    const int s = segment_of(a, u);
     if (s < 0) return -1;
     *spline_out = s;
     int lo = 0, hi = a.K;  // lower_bound over keyframe times
@@ -667,6 +673,135 @@ __global__ void __launch_bounds__(AS_THREADS) k_assoc_write(const AssocArgs a, c
             a.cp0[k] = a.cp_off[s] + sp - 3;
             a.span[k] = a.span_off[s] + sp - 3;
         }
+    }
+}
+
+// ------------------------------------------------------------------------------ re-association ----
+// k_reassoc_count  pass 1 of the association through the calibrated model: a candidate event (segment, valid pixel, near its
+//                  key frame) gets its pose on the spline, its board point X_w, the landmark nearest to X_w and the event-to-rim
+//                  error e of that pair; the 16-bit tag of k_assoc_count records the kept ones, so k_scan_blocks and k_assoc_write
+//                  write the records as for an association.  A kept event is looked up in the previous records (ordered by
+//                  event) for the counts against them, summed with integer atomics.
+struct ReassocArgs {
+    AssocArgs as;                // events, segments, the association's stamps / window / landmarks
+    double max_dt;               // > 0: |t - t_kf| <= max_dt instead of the association's window
+    const double *params;        // intr 9 | rot 4C | trans 3C
+    int total_cp;
+    EcbFold fold;
+    double radius, gate_px;
+    const int64_t *prev_event;   // the records before the call
+    const int *prev_circle;
+    int64_t n_prev;
+    unsigned long long *counts;  // same, changed, new
+};
+
+constexpr int RA_MAX_CIRC = 256;  // > the association's limit of 254 circles
+
+// circle of one candidate event (or -1); L32: FP32 landmarks, lmax: their largest |coordinate|
+template <int SO3>
+__device__ __forceinline__ int reassoc_one(const ReassocArgs &r, const float4 *L32, float lmax, int64_t i, int *spline_out) {
+    const AssocArgs &a = r.as;
+    const double u = a.ev_t[i];
+    const int s = segment_of(a, u);
+    if (s < 0) return -1;
+    *spline_out = s;
+    const double dt = u - a.kf_t[nearest_kf(a.kf_t, a.K, u)];
+    if (r.max_dt > 0.0 ? !(fabs(dt) <= r.max_dt) : !(__dmul_rn(dt, dt) < a.gate2)) return -1;
+    const uint32_t e = a.ev_xyp[i];
+    if (e & ECB_PIX_INVALID) return -1;
+    const double ou = (double) ECB_PIX_X(e), ov = (double) ECB_PIX_Y(e);
+    // the pose as the record's evaluation sees it: the basis of k_assoc_write, ecb_pose_eval as in k_reprojection
+    const double *kn = a.knots + a.knot_off[s];
+    const int sp = find_span_guess(kn, a.ncp[s] + 4, u);
+    double N[4], q[4], t[3], X[3];
+    basis_dev(kn, sp, u, N);
+    const int c0 = a.cp_off[s] + sp - 3;
+    const double *intr = r.params;
+    ecb_pose_eval(intr + 9 + 4 * (size_t) c0, intr + 9 + 4 * (size_t) r.total_cp + 3 * (size_t) c0, N, SO3, q, t);
+    ecb_board_point(intr, q, t, ou, ov, X);
+    if (!(fabs(X[0]) < INFINITY && fabs(X[1]) < INFINITY && fabs(X[2]) < INFINITY)) return -1;
+    // Nearest landmark, assoc_one's scheme: FP32 preselection with sortable keys (distance bits | index), the two smallest kept.
+    // The FP32 distance of any landmark is within 1e-6 S of the exact one (S: the largest |coordinate| of X_w and the landmarks),
+    // so when the runner-up's lower bound clears the winner's upper bound by 1e-5 S the winner is the exact FP64 arg-min; else
+    // the exact FP64 loop decides (ties -> the smaller index).
+    int bi = -1;
+    {
+        const float xf = (float) X[0], yf = (float) X[1], zf = (float) X[2];
+        uint32_t k1 = 0xFFFFFFFFu, k2 = 0xFFFFFFFFu;
+#pragma unroll 1  // unrolled by 4, the quaternion variant spills 8 bytes
+        for (int c = 0; c < a.n_circ; ++c) {
+            const float4 L = L32[c];
+            const float dx = xf - L.x, dy = yf - L.y, dz = zf - L.z;
+            const uint32_t k = (__float_as_uint(fmaf(dx, dx, fmaf(dy, dy, dz * dz))) & 0xFFFFFF00u) | (uint32_t) c;
+            k2 = min(k2, max(k, k1));
+            k1 = min(k1, k);
+        }
+        const float d1 = sqrtf(__uint_as_float(k1 | 0xFFu)), d2 = sqrtf(__uint_as_float(k2 & 0xFFFFFF00u));
+        const float S = fmaxf(lmax, fmaxf(fabsf(xf), fmaxf(fabsf(yf), fabsf(zf))));
+        if (d2 > d1 * 1.0001f + 1e-5f * S) {  // NaN (one circle, overflow): the FP64 loop
+            bi = (int) (k1 & 0xFFu);
+        } else {
+            double bd = 0.0;
+            for (int c = 0; c < a.n_circ; ++c) {
+                const double *L = a.lm_tab + 3 * c;
+                const double dx = X[0] - L[0], dy = X[1] - L[1], dz = X[2] - L[2];
+                const double dd = __dadd_rn(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)), __dmul_rn(dz, dz));
+                if (bi < 0 || dd < bd) {
+                    bi = c;
+                    bd = dd;
+                }
+            }
+        }
+    }
+    const double *L = a.lm_tab + 3 * bi;
+    const double err = ecb_rim_reprojection(intr, r.fold, q, t, ou, ov, L[0], L[1], L[2], r.radius);
+    return fabs(err) < r.gate_px ? bi : -1;  // NaN: not kept
+}
+
+template <int SO3>
+__global__ void __launch_bounds__(AS_THREADS) k_reassoc_count(const ReassocArgs r, uint16_t *__restrict__ tag,
+                                                             uint32_t *__restrict__ block_cnt) {
+    __shared__ uint32_t ws[33];
+    __shared__ float4 L32[RA_MAX_CIRC];
+    __shared__ uint32_t lmax_bits;  // a non-negative float: its bits order as the values (integer max: deterministic)
+    const AssocArgs &a = r.as;
+    if (threadIdx.x == 0) lmax_bits = 0;
+    __syncthreads();
+    for (int c = threadIdx.x; c < a.n_circ; c += AS_THREADS) {
+        const double *L = a.lm_tab + 3 * c;
+        const float4 v = make_float4((float) L[0], (float) L[1], (float) L[2], 0.f);
+        L32[c] = v;
+        atomicMax(&lmax_bits, __float_as_uint(fmaxf(fabsf(v.x), fmaxf(fabsf(v.y), fabsf(v.z)))));
+    }
+    __syncthreads();
+    const int64_t i = (int64_t) blockIdx.x * AS_THREADS + threadIdx.x;
+    int s = 0;
+    const int bi = i < a.n_ev ? reassoc_one<SO3>(r, L32, __uint_as_float(lmax_bits), i, &s) : -1;
+    if (i < a.n_ev) tag[i] = bi >= 0 ? (uint16_t) ((s << 8) | (bi + 1)) : (uint16_t) 0;
+    uint32_t tot;
+    block_excl_scan(bi >= 0 ? 1u : 0u, ws, &tot);
+    if (threadIdx.x == 0) block_cnt[blockIdx.x] = tot;
+    uint32_t same = 0, changed = 0, fresh = 0;
+    if (bi >= 0) {
+        int64_t lo = 0, hi = r.n_prev;  // lower_bound of i in the previous records' events
+        while (lo < hi) {
+            const int64_t m = (lo + hi) >> 1;
+            if (r.prev_event[m] < i) lo = m + 1; else hi = m;
+        }
+        if (lo < r.n_prev && r.prev_event[lo] == i) {
+            same = r.prev_circle[lo] == bi;
+            changed = !same;
+        } else {
+            fresh = 1;
+        }
+    }
+    same = __reduce_add_sync(0xffffffffu, same);
+    changed = __reduce_add_sync(0xffffffffu, changed);
+    fresh = __reduce_add_sync(0xffffffffu, fresh);
+    if ((threadIdx.x & 31) == 0) {
+        if (same) atomicAdd(&r.counts[0], (unsigned long long) same);
+        if (changed) atomicAdd(&r.counts[1], (unsigned long long) changed);
+        if (fresh) atomicAdd(&r.counts[2], (unsigned long long) fresh);
     }
 }
 
@@ -1204,6 +1339,50 @@ int ecb_cost_set_residuals(ecb_ctx *ctx, const double *obs_xy, const double *lm_
     return prepare_records(ctx, st);
 }
 
+// pass 2 of an association from the tags in st->ev_tag and the block offsets in st->ev_flag: the record buffers sized for
+// `total`, then k_assoc_write (fused: the basis pass folded in); async
+static int write_assoc_records(ecb_ctx *ctx, CostState *st, AssocArgs a, int nb, int64_t total, bool fused) {
+    int rc;
+    const size_t nn = (size_t) std::max<int64_t>(total, 1);
+    if ((rc = ecb_reserve(ctx, st->obs, nn * 16))) return rc;
+    if ((rc = ecb_reserve(ctx, st->lm, nn * 24))) return rc;
+    if ((rc = ecb_reserve(ctx, st->tt, nn * 8))) return rc;
+    if ((rc = ecb_reserve(ctx, st->spl, nn * 4))) return rc;
+    if ((rc = ecb_reserve(ctx, st->sel_event, nn * 8))) return rc;
+    if ((rc = ecb_reserve(ctx, st->sel_circle, nn * 4))) return rc;
+    a.cp_off = (const int *) st->d_cp_off.p;
+    a.span_off = (const int *) st->d_span_off.p;
+    a.basis = nullptr;
+    a.cp0 = a.span = nullptr;
+    if (fused) {
+        if ((rc = ecb_reserve(ctx, st->basis, nn * 32))) return rc;
+        if ((rc = ecb_reserve(ctx, st->cp0, nn * 4))) return rc;
+        if ((rc = ecb_reserve(ctx, st->span, nn * 4))) return rc;
+        a.basis = (double *) st->basis.p;
+        a.cp0 = (int *) st->cp0.p;
+        a.span = (int *) st->span.p;
+    }
+    k_assoc_write<<<nb, AS_THREADS, 0, ctx->stream>>>(a, (const uint16_t *) st->ev_tag.p, (const int64_t *) st->ev_flag.p, (double *) st->obs.p, (double *) st->lm.p,
+                                                      (double *) st->tt.p, (int *) st->spl.p, (int64_t *) st->sel_event.p,
+                                                      (int *) st->sel_circle.p);
+    ECB_LAUNCHED(ctx);
+    return ECB_OK;
+}
+
+// the association's arguments for the current events and splines (pass 1 reads cp_off for the fused basis of its records)
+static void assoc_args(ecb_ctx *ctx, CostState *st, AssocArgs &a) {
+    memset(&a, 0, sizeof a);
+    a.ev_t = (const double *) ctx->ev_t.p;
+    a.ev_xyp = (const uint32_t *) ctx->ev_xyp.p;
+    a.n_ev = ctx->n_events;
+    a.knots = (const double *) st->d_knots.p;
+    a.knot_off = (const int *) st->d_knot_off.p;
+    a.ncp = (const int *) st->d_ncp.p;
+    a.n_splines = st->n_splines;
+    a.lm_tab = (const double *) st->lm_tab.p;
+    a.cp_off = (const int *) st->d_cp_off.p;
+}
+
 static int cost_associate(ecb_ctx *ctx, const double *kf_time, const double *kf_circles, int n_keyframes, int n_circles,
                           const double *landmarks_xyz, double motion_time_step, int64_t *n_residuals, bool on_device);
 
@@ -1252,16 +1431,9 @@ static int cost_associate(ecb_ctx *ctx, const double *kf_time, const double *kf_
         ECB_CUDA(ctx, cudaMemcpyAsync(st->lm_tab.p, landmarks_xyz, (size_t) n_circles * 24, cudaMemcpyDeviceToDevice, ctx->stream));
     }
     AssocArgs a;
-    a.ev_t = (const double *) ctx->ev_t.p;
-    a.ev_xyp = (const uint32_t *) ctx->ev_xyp.p;
-    a.n_ev = n;
-    a.knots = (const double *) st->d_knots.p;
-    a.knot_off = (const int *) st->d_knot_off.p;
-    a.ncp = (const int *) st->d_ncp.p;
-    a.n_splines = st->n_splines;
+    assoc_args(ctx, st, a);
     a.kf_t = d_kf_t;
     a.kf_circ = d_kf_circ;
-    a.lm_tab = (const double *) st->lm_tab.p;
     a.kf_c32 = (const float2 *) st->kf_c32.p;
     a.K = n_keyframes;
     a.n_circ = n_circles;
@@ -1278,13 +1450,6 @@ static int cost_associate(ecb_ctx *ctx, const double *kf_time, const double *kf_
     ECB_LAUNCHED(ctx);
     int64_t total = 0;
     if ((rc = ecb_d2h(ctx, &total, d_total, 8))) return rc;
-    const size_t nn = (size_t) std::max<int64_t>(total, 1);
-    if ((rc = ecb_reserve(ctx, st->obs, nn * 16))) return rc;
-    if ((rc = ecb_reserve(ctx, st->lm, nn * 24))) return rc;
-    if ((rc = ecb_reserve(ctx, st->tt, nn * 8))) return rc;
-    if ((rc = ecb_reserve(ctx, st->spl, nn * 4))) return rc;
-    if ((rc = ecb_reserve(ctx, st->sel_event, nn * 8))) return rc;
-    if ((rc = ecb_reserve(ctx, st->sel_circle, nn * 4))) return rc;
     // time-sorted events + spline ranges in ascending, disjoint order => records come out ordered by (spline, time): the
     // basis pass (k_prepare) is folded into the record write; otherwise k_prepare runs and checks the order
     bool fused = true;
@@ -1314,22 +1479,7 @@ static int cost_associate(ecb_ctx *ctx, const double *kf_time, const double *kf_
             ko += (size_t) st->n_cp[(size_t) q] + 4;
         }
     }
-    a.cp_off = (const int *) st->d_cp_off.p;
-    a.span_off = (const int *) st->d_span_off.p;
-    a.basis = nullptr;
-    a.cp0 = a.span = nullptr;
-    if (fused) {
-        if ((rc = ecb_reserve(ctx, st->basis, nn * 32))) return rc;
-        if ((rc = ecb_reserve(ctx, st->cp0, nn * 4))) return rc;
-        if ((rc = ecb_reserve(ctx, st->span, nn * 4))) return rc;
-        a.basis = (double *) st->basis.p;
-        a.cp0 = (int *) st->cp0.p;
-        a.span = (int *) st->span.p;
-    }
-    k_assoc_write<<<nb, AS_THREADS, 0, ctx->stream>>>(a, (const uint16_t *) st->ev_tag.p, (const int64_t *) st->ev_flag.p, (double *) st->obs.p, (double *) st->lm.p,
-                                                      (double *) st->tt.p, (int *) st->spl.p, (int64_t *) st->sel_event.p,
-                                                      (int *) st->sel_circle.p);
-    ECB_LAUNCHED(ctx);
+    if ((rc = write_assoc_records(ctx, st, a, nb, total, fused))) return rc;
     ECB_PROF_END(ctx, ECB_STAGE_ASSOC);
     if ((rc = ecb_check(ctx, cudaGetLastError(), "association kernels"))) return rc;
     st->n_res = total;
@@ -1338,6 +1488,8 @@ static int cost_associate(ecb_ctx *ctx, const double *kf_time, const double *kf_
     st->assoc_K = n_keyframes;
     st->assoc_n_circ = n_circles;
     st->assoc_events_gen = ctx->events_gen;
+    st->assoc_kf_t = d_kf_t;
+    st->assoc_gate2 = a.gate2;
     if (n_residuals) *n_residuals = total;
     return prepare_records(ctx, st, fused);
 }
@@ -1824,6 +1976,67 @@ int ecb_cost_reject(ecb_ctx *ctx, const double *intrinsics, const double *rot_cp
     st->n_res = kept;
     if ((rc = prepare_records(ctx, st, /*have_basis=*/true))) return rc;
     return ecb_check(ctx, ecb_stream_sync(ctx), "outlier rejection");
+}
+
+// ---- re-association ----
+int ecb_cost_reassociate(ecb_ctx *ctx, const double *intrinsics, const double *rot_cp, const double *trans_cp, double gate_px,
+                         double max_dt, int64_t *n_residuals, int64_t *n_same, int64_t *n_changed, int64_t *n_new,
+                         int64_t *n_lost) {
+    if (!ctx || !intrinsics || !rot_cp || !trans_cp) return ECB_ERR_ARG;
+    if (!(gate_px > 0.0)) return ecb_fail(ctx, ECB_ERR_ARG, "gate_px %g is NaN or not positive", gate_px);
+    if (!(max_dt >= 0.0)) return ecb_fail(ctx, ECB_ERR_ARG, "max_dt %g is NaN or negative", max_dt);
+    if (!ctx->cost) return ecb_fail(ctx, ECB_ERR_STATE, "ecb_cost_setup first");
+    cudaSetDevice(ctx->device);
+    CostState *st = (CostState *) ctx->cost;
+    if (!st->assoc) return ecb_fail(ctx, ECB_ERR_STATE, "the records do not come from an association: associate first");
+    if (st->assoc_events_gen != ctx->events_gen) return ecb_fail(ctx, ECB_ERR_STATE, "events were loaded after the association");
+    if (st->n_res > 0xFFFFFFFFll) return ecb_fail(ctx, ECB_ERR_UNSUPPORTED, "re-association of 2^32 or more records");
+    int rc;
+    const int64_t n = ctx->n_events, n_prev = st->n_res;  // n < 2^32: the association checked it for these events
+    const int nb = (int) ((n + AS_THREADS - 1) / AS_THREADS);
+    if ((rc = upload_params(ctx, st, intrinsics, rot_cp, trans_cp))) return rc;
+    if ((rc = ecb_reserve(ctx, st->ev_cnt, (size_t) nb * 4 + 16))) return rc;
+    if ((rc = ecb_reserve(ctx, st->ev_tag, (size_t) n * 2 + 16))) return rc;
+    if ((rc = ecb_reserve(ctx, st->ev_flag, (size_t) nb * 8 + 48))) return rc;
+    // block offsets | total | same, changed, new: one read-back
+    int64_t *off = (int64_t *) st->ev_flag.p, *d_total = off + nb;
+    ECB_CUDA(ctx, cudaMemsetAsync(d_total + 1, 0, 24, ctx->stream));
+    ReassocArgs r;
+    memset(&r, 0, sizeof r);
+    assoc_args(ctx, st, r.as);
+    r.as.kf_t = st->assoc_kf_t;
+    r.as.K = st->assoc_K;
+    r.as.n_circ = st->assoc_n_circ;
+    r.as.gate2 = st->assoc_gate2;
+    r.max_dt = max_dt;
+    r.params = (const double *) st->params.p;
+    r.total_cp = st->total_cp;
+    r.fold = ecb_inverse_radial_fold_host(intrinsics + 4);
+    r.radius = st->radius;
+    r.gate_px = gate_px;
+    r.prev_event = (const int64_t *) st->sel_event.p;
+    r.prev_circle = (const int *) st->sel_circle.p;
+    r.n_prev = n_prev;
+    r.counts = (unsigned long long *) (d_total + 1);
+    (st->so3 ? k_reassoc_count<1> : k_reassoc_count<0>)<<<nb, AS_THREADS, 0, ctx->stream>>>(r, (uint16_t *) st->ev_tag.p,
+                                                                                           (uint32_t *) st->ev_cnt.p);
+    ECB_LAUNCHED(ctx);
+    k_scan_blocks<<<1, 1024, 0, ctx->stream>>>((uint32_t *) st->ev_cnt.p, nb, off, d_total);
+    ECB_LAUNCHED(ctx);
+    int64_t h[4] = {0, 0, 0, 0};  // total, same, changed, new
+    if ((rc = ecb_d2h(ctx, h, d_total, sizeof h))) return rc;
+    // the previous records have been read: the new ones may take their buffers
+    if ((rc = write_assoc_records(ctx, st, r.as, nb, h[0], st->use_circ))) return rc;
+    if ((rc = ecb_check(ctx, cudaGetLastError(), "re-association kernels"))) return rc;
+    st->n_res = h[0];
+    if ((rc = prepare_records(ctx, st, st->use_circ))) return rc;
+    if ((rc = ecb_check(ctx, ecb_stream_sync(ctx), "re-association"))) return rc;
+    if (n_residuals) *n_residuals = h[0];
+    if (n_same) *n_same = h[1];
+    if (n_changed) *n_changed = h[2];
+    if (n_new) *n_new = h[3];
+    if (n_lost) *n_lost = n_prev - h[1] - h[2];
+    return ECB_OK;
 }
 
 // ---- reprojection report ----

@@ -41,6 +41,14 @@
 // every report and covariance file then describe the second solve.  An invalid value, or the variable together with
 // ECB_REFERENCE_SIGNATURES, ends the program with exit code 1 before any GPU work.
 //
+// ECB_REASSOCIATE=n (a positive integer, at most 1000) refines the association after the first optimisation, which the
+// reference does not: n rounds, each re-associating every event near a key frame with the board circle nearest to its
+// back-projection at its own pose on the current spline (kept when its event-to-rim error is below 5 px, the association's
+// tolerance), printing a "Re-association r:" line with the record counts against the previous records, and optimising again from the current solution
+// ("Solver Summary (after re-association r):").  ECB_REJECT then applies after the last round; the intrinsics, the trajectory and
+// every report and covariance file describe the final solve.  An invalid value, or the variable together with
+// ECB_REFERENCE_SIGNATURES, ends the program with exit code 1 before any GPU work.
+//
 // ECB_REPROJECTION=1 reports the same fit in pixels after the optimisation, through the forward camera model: a "Reprojection:"
 // line (event-to-rim count, RMS, mean, max |e|, invalid count; key-frame-centre count and RMS; rho_fold * fx next to the farthest
 // sensor corner's distorted radius, in pixels) and SavePath/ReprojectionByKeyframe.txt, ReprojectionByCircle.txt and
@@ -126,6 +134,21 @@ int main(int argc, char **argv) {
             return 1;
         }
         rejectK = v;
+    }
+    int reassociateRounds = 0;  // checked before any file or GPU work; 0: no re-association
+    if (const char *ra = getenv("ECB_REASSOCIATE")) {
+        if (getenv("ECB_REFERENCE_SIGNATURES")) {
+            std::cerr << "ecb: ECB_REASSOCIATE cannot be combined with ECB_REFERENCE_SIGNATURES (the reference's EventCalibSpline "
+                         "associates once, from the detected circles)" << std::endl;
+            return 1;
+        }
+        char *end = nullptr;
+        const long v = strtol(ra, &end, 10);
+        if (end == ra || *end != '\0' || v < 1 || v > 1000) {
+            std::cerr << "ecb: ECB_REASSOCIATE must be a positive integer (rounds, at most 1000), got '" << ra << "'" << std::endl;
+            return 1;
+        }
+        reassociateRounds = (int) v;
     }
     int residualCell = 16;  // checked before any file or GPU work
     if (const char *rc = getenv("ECB_RESIDUAL_CELL")) {
@@ -455,6 +478,22 @@ int main(int argc, char **argv) {
         std::cout << "Solver Summary: residuals " << n_res << ", splines " << segments.size() << ", iterations " << sum.iterations
                   << " (successful " << sum.successful_steps << "), cost " << sum.initial_cost << " -> " << sum.final_cost
                   << ", termination " << sum.termination << std::endl;
+        for (int round = 1; round <= reassociateRounds; ++round) {  // re-association, then the optimisation again (no reference output)
+            EventCalibSpline::ReassociationCounts rc;
+            if (spline.reassociate(5.0, 0.0, &rc) != ECB_OK) {
+                std::cerr << "ecb: " << spline.lastError() << std::endl;
+                return 1;
+            }
+            std::cout << "Re-association " << round << ": residuals " << rc.residuals << " (same " << rc.same << ", changed "
+                      << rc.changed << ", new " << rc.added << ", lost " << rc.lost << ")" << std::endl;
+            if (!spline.optimize(&sum)) {
+                std::cerr << "ecb: " << spline.lastError() << std::endl;
+                return 1;
+            }
+            std::cout << "Solver Summary (after re-association " << round << "): residuals " << rc.residuals << ", splines "
+                      << segments.size() << ", iterations " << sum.iterations << " (successful " << sum.successful_steps << "), cost "
+                      << sum.initial_cost << " -> " << sum.final_cost << ", termination " << sum.termination << std::endl;
+        }
         if (rejectK > 0.0) {  // outlier rejection, then the same optimisation again from the first solution (no reference output)
             double s = 0.0, thr = 0.0;
             std::vector<uint8_t> drop;

@@ -1128,6 +1128,27 @@ public:
         return ecb_cost_reject(ctx, intr.data(), rot.data(), trans.data(), maxAbsR, mask ? kfTime.data() : nullptr,
                                mask ? dropKeyframe.data() : nullptr, (int) dropKeyframe.size(), kept, removed);
     }
+    // Re-association (ecb_cost_reassociate) at the current point: every event near a key frame of the last associate() (maxDt = 0:
+    // the association's window) is matched to the board circle nearest to its back-projection at its own pose and kept when its
+    // event-to-rim error is below gatePx pixels (5: the association's tolerance).  The kept events replace the records; a following
+    // optimize() solves again on them.  Counts (each may be null): the new records, and against the records before the call the
+    // events with the same circle, another circle, newly recorded, and records lost.
+    struct ReassociationCounts {
+        int64_t residuals = 0, same = 0, changed = 0, added = 0, lost = 0;
+    };
+    int reassociate(double gatePx, double maxDt, ReassociationCounts *counts) {
+        return reassociateAt(ev_->ctx, intr_, seg_, gatePx, maxDt, counts);
+    }
+    static int reassociateAt(ecb_ctx *ctx, const std::array<double, 9> &intr, const std::vector<Segment> &seg, double gatePx,
+                             double maxDt, ReassociationCounts *counts) {
+        std::vector<double> rot, trans;
+        flatten(seg, rot, trans);
+        ReassociationCounts c;
+        const int rc = ecb_cost_reassociate(ctx, intr.data(), rot.data(), trans.data(), gatePx, maxDt, &c.residuals, &c.same,
+                                            &c.changed, &c.added, &c.lost);
+        if (rc == ECB_OK && counts) *counts = c;
+        return rc;
+    }
     // adds group b into a: counts and sums added, max_abs the max (shards combine in rank order)
     static void accumulateResidualGroup(ecb_residual_group &a, const ecb_residual_group &b) {
         a.count += b.count;

@@ -385,6 +385,29 @@ public:
         if (removed) *removed = nr;
         return ECB_OK;
     }
+    // Re-association at the current point (EventCalibSpline::reassociate): every shard re-associates its own events (one host
+    // thread each); the counts are summed in rank order.
+    int reassociate(double gatePx, double maxDt, EventCalibSpline::ReassociationCounts *counts) {
+        const int G = (int) sp_.size();
+        std::vector<EventCalibSpline::ReassociationCounts> part((size_t) G);
+        std::vector<int> rc((size_t) G, ECB_OK);
+        forEachShard(G, [&](int g) {
+            rc[(size_t) g] = EventCalibSpline::reassociateAt(ev_->shard[(size_t) g]->ctx, intrinsics(), segments(), gatePx, maxDt,
+                                                             &part[(size_t) g]);
+        });
+        for (int g = 0; g < G; ++g)
+            if (rc[(size_t) g] != ECB_OK) return rc[(size_t) g];
+        EventCalibSpline::ReassociationCounts t;
+        for (const auto &p : part) {
+            t.residuals += p.residuals;
+            t.same += p.same;
+            t.changed += p.changed;
+            t.added += p.added;
+            t.lost += p.lost;
+        }
+        if (counts) *counts = t;
+        return ECB_OK;
+    }
     // Reprojection statistics in pixels (EventCalibSpline::reprojectionGroups), combined as residualGroups
     int reprojectionGroups(int by, int cellPx, std::vector<ecb_reprojection_group> &groups, ecb_reprojection_group *total) const {
         const int G = (int) sp_.size();

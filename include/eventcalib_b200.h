@@ -287,6 +287,28 @@ int ecb_cost_residual_groups(ecb_ctx *ctx, const double *intrinsics, const doubl
  * floating-point atomics: deterministic.  Synchronises. */
 int ecb_cost_reject(ecb_ctx *ctx, const double *intrinsics, const double *rot_cp, const double *trans_cp, double max_abs_residual,
                     const double *kf_time, const uint8_t *drop_keyframe, int n_keyframes, int64_t *n_kept, int64_t *n_removed);
+/* Re-association at a calibrated point (intrinsics / rot_cp / trans_cp as ecb_cost_eval): every loaded event i is matched again to
+ * a board circle through the model instead of the detected ellipses of its key frame.  Candidates are the events that lie in a
+ * spline segment, have a valid pixel and lie near their key frame (the nearest stamp of the association, ties -> the earlier one):
+ * max_dt = 0 applies the association's own test (dt^2 < (5 motion_time_step)^2, so the candidates are exactly the association's),
+ * max_dt > 0 keeps |t_i - t_kf| <= max_dt.  For a candidate: the pose at t_i on the spline (rotation model of the context), X_w =
+ * the back-projection of the event pixel onto the board plane (the arithmetic of the residual), c* = the landmark of the
+ * association nearest to X_w in FP64 over ALL n_circles (detected in that key frame or not; ties -> the smaller index; no circle
+ * when X_w is not finite), e = ecb_rim_reprojection of (i, c*), the value ecb_cost_reprojection_errors returns for that record.
+ * The event is kept iff |e| < gate_px (NaN never; 5 is the association's pixel tolerance).  The kept events replace the
+ * records, in event order and in the layout of ecb_cost_associate; key frames, landmarks and K stay those of the association,
+ * so the groupings, ecb_cost_reject with a mask and ecb_cost_get_association keep working.  Like an association, it undoes an
+ * earlier rejection.  After ecb_cost_associate_device the stamps are read at the association's d_kf_time, which must still
+ * hold them.  *n_residuals: the new record count; *n_same / *n_changed (same event, same / another circle), *n_new (event not
+ * recorded before) and *n_lost (record whose event is not kept) compare with the records held just before the call (after any
+ * rejection); all optional.  A device LM created before the call stays valid: it reads the records at every evaluation.  A
+ * covariance computed before still answers ecb_pose_covariance: call ecb_covariance again for the new records.
+ * Errors: gate_px NaN or <= 0, max_dt NaN or < 0: ECB_ERR_ARG.  No ecb_cost_setup, records of ecb_cost_set_residuals or of no
+ * association, events loaded since the association: ECB_ERR_STATE.  A record count >= 2^32: ECB_ERR_UNSUPPORTED.  Zero kept
+ * events: ECB_OK.  No floating-point atomics: repeated calls give bit-identical records.  Synchronises. */
+int ecb_cost_reassociate(ecb_ctx *ctx, const double *intrinsics, const double *rot_cp, const double *trans_cp, double gate_px,
+                         double max_dt, int64_t *n_residuals, int64_t *n_same, int64_t *n_changed, int64_t *n_new,
+                         int64_t *n_lost);
 
 /* ---- the same fit in pixels: reprojection errors through the forward camera model --------------------------------------------
  * The spline stage's distortion is the inverse radial polynomial (undistorted = distorted * s(rho_d^2), s = 1 + k1 rho^2 + ... +
