@@ -569,32 +569,14 @@ class Context:
         cost_association(): a distance on the board plane in the units of the board points, NOT pixels.  Returns an ndarray
         (float64, n_residuals) when host=True; else leaves them in d_out (device pointer, or None for the context's own buffer),
         enqueued on the context's stream, and returns None."""
-        a = [np.ascontiguousarray(v, np.float64) for v in (intr, rot, trans)]
-        d = C.c_void_p(d_out) if d_out else None
-        if not host:
-            self._chk(self.lib.ecb_cost_residuals(self.h, _ptr(a[0]), _ptr(a[1]), _ptr(a[2]), d, None))
-            return None
-        out = np.zeros(max(self.cost_layout()["n_residuals"], 1))
-        self._chk(self.lib.ecb_cost_residuals(self.h, _ptr(a[0]), _ptr(a[1]), _ptr(a[2]), d, _ptr(out)))
-        return out[:self.cost_layout()["n_residuals"]]
+        return self._record_report(self.lib.ecb_cost_residuals, intr, rot, trans, d_out, host)
 
     def residual_groups(self, intr, rot, trans, by, kf_t=None, cell_px=16):
         """Statistics of the raw residuals (board units, not pixels) per group (ecb_cost_residual_groups).  by: "keyframe"
         (kf_t: the stamps given to cost_associate), "circle" or "sensor_cell" (cells of cell_px pixels, row major).  Returns
         (groups, total) as numpy structured arrays of RESIDUAL_GROUP_DTYPE (count, n_downweighted, sum, sum_sq, max_abs, cost);
         total has shape () and covers every record."""
-        if by not in RESIDUALS_BY:
-            raise ValueError("by must be one of %s" % ", ".join(RESIDUALS_BY))
-        a = [np.ascontiguousarray(v, np.float64) for v in (intr, rot, trans)]
-        kf = np.ascontiguousarray(kf_t, np.float64) if kf_t is not None else None
-        nk = len(kf) if kf is not None else 0
-        args = (self.h, _ptr(a[0]), _ptr(a[1]), _ptr(a[2]), RESIDUALS_BY[by], _ptr(kf), nk, int(cell_px))
-        ng = C.c_int(0)
-        self._chk(self.lib.ecb_cost_residual_groups(*args, None, 0, C.byref(ng), None))
-        groups = np.zeros(max(ng.value, 1), RESIDUAL_GROUP_DTYPE)
-        total = np.zeros((), RESIDUAL_GROUP_DTYPE)
-        self._chk(self.lib.ecb_cost_residual_groups(*args, _ptr(groups), ng.value, C.byref(ng), _ptr(total)))
-        return groups[:ng.value], total
+        return self._group_report(self.lib.ecb_cost_residual_groups, RESIDUAL_GROUP_DTYPE, intr, rot, trans, by, kf_t, cell_px)
 
     def reject_residuals(self, intr, rot, trans, max_abs_r=math.inf, drop_keyframes=None, kf_t=None):
         """Removes outliers from this context's records (ecb_cost_reject): record k goes when not |r_k| <= max_abs_r (r_k as
@@ -630,21 +612,33 @@ class Context:
         e_k = sign(|d| - radius) |q - o|, o the event pixel and q the projection of the residual's rim point, NaN where it cannot
         be projected.  Returns (e as float64 ndarray, n_invalid) when host=True; else leaves e in d_out (device pointer, or None
         for the context's own buffer), enqueued on the context's stream, and returns None."""
-        a = [np.ascontiguousarray(v, np.float64) for v in (intr, rot, trans)]
-        d = C.c_void_p(d_out) if d_out else None
-        if not host:
-            self._chk(self.lib.ecb_cost_reprojection_errors(self.h, _ptr(a[0]), _ptr(a[1]), _ptr(a[2]), d, None, None))
-            return None
-        n = self.cost_layout()["n_residuals"]
-        out = np.zeros(max(n, 1))
         bad = C.c_int64(0)
-        self._chk(self.lib.ecb_cost_reprojection_errors(self.h, _ptr(a[0]), _ptr(a[1]), _ptr(a[2]), d, _ptr(out), C.byref(bad)))
-        return out[:n], bad.value
+        e = self._record_report(self.lib.ecb_cost_reprojection_errors, intr, rot, trans, d_out, host, C.byref(bad) if host else None)
+        return (e, bad.value) if host else None
 
     def reprojection_groups(self, intr, rot, trans, by, kf_t=None, cell_px=16):
         """Statistics of the reprojection errors (pixels) per group (ecb_cost_reprojection_groups): the groups of residual_groups.
         Returns (groups, total) as numpy structured arrays of REPROJECTION_GROUP_DTYPE (count, n_invalid, sum, sum_sq,
         max_abs; count and the sums over the valid records only); total has shape () and covers every record."""
+        return self._group_report(self.lib.ecb_cost_reprojection_groups, REPROJECTION_GROUP_DTYPE, intr, rot, trans, by, kf_t,
+                                  cell_px)
+
+    def _record_report(self, fn, intr, rot, trans, d_out, host, *extra):
+        """one value per record (fn: ecb_cost_residuals or ecb_cost_reprojection_errors; extra: its arguments after h_out): an
+        ndarray when host, else None with the values left in d_out"""
+        a = [np.ascontiguousarray(v, np.float64) for v in (intr, rot, trans)]
+        d = C.c_void_p(d_out) if d_out else None
+        if not host:
+            self._chk(fn(self.h, _ptr(a[0]), _ptr(a[1]), _ptr(a[2]), d, None, *extra))
+            return None
+        n = self.cost_layout()["n_residuals"]
+        out = np.zeros(max(n, 1))
+        self._chk(fn(self.h, _ptr(a[0]), _ptr(a[1]), _ptr(a[2]), d, _ptr(out), *extra))
+        return out[:n]
+
+    def _group_report(self, fn, dtype, intr, rot, trans, by, kf_t, cell_px):
+        """the groups of one report (fn: ecb_cost_residual_groups or ecb_cost_reprojection_groups, dtype: its group record): the
+        size query, then the filled call"""
         if by not in RESIDUALS_BY:
             raise ValueError("by must be one of %s" % ", ".join(RESIDUALS_BY))
         a = [np.ascontiguousarray(v, np.float64) for v in (intr, rot, trans)]
@@ -652,10 +646,10 @@ class Context:
         nk = len(kf) if kf is not None else 0
         args = (self.h, _ptr(a[0]), _ptr(a[1]), _ptr(a[2]), RESIDUALS_BY[by], _ptr(kf), nk, int(cell_px))
         ng = C.c_int(0)
-        self._chk(self.lib.ecb_cost_reprojection_groups(*args, None, 0, C.byref(ng), None))
-        groups = np.zeros(max(ng.value, 1), REPROJECTION_GROUP_DTYPE)
-        total = np.zeros((), REPROJECTION_GROUP_DTYPE)
-        self._chk(self.lib.ecb_cost_reprojection_groups(*args, _ptr(groups), ng.value, C.byref(ng), _ptr(total)))
+        self._chk(fn(*args, None, 0, C.byref(ng), None))
+        groups = np.zeros(max(ng.value, 1), dtype)
+        total = np.zeros((), dtype)
+        self._chk(fn(*args, _ptr(groups), ng.value, C.byref(ng), _ptr(total)))
         return groups[:ng.value], total
 
     def keyframe_reprojection(self, intr, rot, trans, kf_t, circles, landmarks):

@@ -89,6 +89,16 @@ struct EcbSplineView {
     const double *knots;
     const int *knot_off, *ncp, *cp_off;
     int n_splines, total_cp, so3;
+    // the first segment whose knot range holds u (EventCalibSpline::time2splineIdx; NaN holds in no range), with *kn its knots
+    // and *nk their count; -1 when there is none
+    __device__ __forceinline__ int segment(double u, const double **kn, int *nk) const {
+        for (int s = 0; s < n_splines; ++s) {
+            *kn = knots + knot_off[s];
+            *nk = ncp[s] + 4;
+            if (u >= (*kn)[0] && u <= (*kn)[*nk - 1]) return s;
+        }
+        return -1;
+    }
 };
 extern "C" int ecb_cost_spline_view(ecb_ctx *ctx, EcbSplineView *v);
 // the result of the last successful ecb_covariance (ecb_lmdev.cu): the band of Z (layout of cov_band), the point x

@@ -14,8 +14,9 @@
 //                   CUDA-core register-tiled SYRK.  tcgen05 has no f64 kind.
 //   k_reduce_*      fixed-order reduction of the per-work-item partials -> run-to-run identical J^T J / J^T r / cost
 //   k_cost          cost-only evaluation (LM step acceptance)
-//   k_residuals, k_group_*            the residual report (board units)
-//   k_reprojection, k_reproj_reduce, k_keyframe_reproj   the same fit in pixels (forward model of ecb_camera.h)
+//   k_record_report, k_group_*        the residual report (board units) and the same fit in pixels (forward model of
+//                                     ecb_camera.h): one value per record, then statistics per group
+//   k_keyframe_reproj                 the key frames' circle centres reprojected at their stamps
 //   k_reject_count, k_reject_write    outlier rejection: ordered compaction of the records that are kept (ecb_cost_reject)
 //   k_reassoc_count the association's pass 1 through the calibrated model (ecb_cost_reassociate); pass 2 is k_assoc_write
 #include <stdlib.h>
@@ -138,6 +139,23 @@ struct NeArgs {
     const int *go;         // device flag (may be null): 0 = the launch is a no-op (device-side LM loop: step rejected / finished)
 };
 
+// the residual records (SoA) as the evaluation kernels read them: record k's first control point c0, basis b, observation o
+// and landmark L (lm_tab[circ[k]] on the association path, else the explicit lm[3k])
+struct RecordView {
+    const double *obs, *lm;
+    const int *circ;
+    const double *lm_tab, *basis;
+    const int *cp0;
+    __device__ __forceinline__ void load(int64_t k, int &c0, double b[4], double2 &o, double L[3]) const {
+        c0 = cp0[k];
+        const double4 b4 = reinterpret_cast<const double4 *>(basis)[k];
+        b[0] = b4.x, b[1] = b4.y, b[2] = b4.z, b[3] = b4.w;
+        o = reinterpret_cast<const double2 *>(obs)[k];
+        const double *p = circ ? lm_tab + 3 * circ[k] : lm + 3 * k;
+        L[0] = p[0], L[1] = p[1], L[2] = p[2];
+    }
+};
+
 __device__ __forceinline__ void dmma(double &c0, double &c1, double a, double b) {
     asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};\n"
                  : "+d"(c0), "+d"(c1)
@@ -167,19 +185,17 @@ __global__ void __launch_bounds__(NE_THREADS, MINB) k_normal_eq(const NeArgs a) 
             double res = 0.0;
             __syncwarp();  // the previous group's fragment loads are done
             if (k < item.end) {
-                const int c0 = a.cp0[k];
-                const double4 b4 = reinterpret_cast<const double4 *>(a.basis)[k];
-                const double b[4] = {b4.x, b4.y, b4.z, b4.w};
-                const double2 o = reinterpret_cast<const double2 *>(a.obs)[k];
-                const double *L = a.circ ? a.lm_tab + 3 * a.circ[k] : a.lm + 3 * k;
-                const double Lx = L[0], Ly = L[1], Lz = L[2];
+                int c0;
+                double b[4], L[3];
+                double2 o;
+                RecordView{a.obs, a.lm, a.circ, a.lm_tab, a.basis, a.cp0}.load(k, c0, b, o, L);
                 // the Jacobian is scattered straight into column `lane` of the shared tile (no register array)
                 const EcbResidualOut r =
                     SO3 ? ecb_residual_so3<true, TILE_LD>(intr, rot + 4 * (size_t) c0, trans + 3 * (size_t) c0, b, o.x, o.y,
-                                                          Lx, Ly, Lz, a.radius, a.huber,
+                                                          L[0], L[1], L[2], a.radius, a.huber,
                                                           tile + lane)
                         : ecb_residual<true, TILE_LD>(intr, rot + 4 * (size_t) c0, trans + 3 * (size_t) c0, b, o.x, o.y,
-                                                      Lx, Ly, Lz, a.radius, a.huber,
+                                                      L[0], L[1], L[2], a.radius, a.huber,
                                                       tile + lane);
                 res = r.res;
                 cost += r.cost;
@@ -470,17 +486,16 @@ __global__ void __launch_bounds__(256, MINB) k_cost(const double *__restrict__ o
     if (go && *go == 0) return;
     const double *intr = params, *rot = params + 9, *trans = params + 9 + 4 * (size_t) total_cp;
     double c = 0.0;
+    const RecordView rv{obs, lm, circ, lm_tab, basis, cp0};
     for (int64_t k = (int64_t) blockIdx.x * 256 + threadIdx.x; k < n; k += (int64_t) gridDim.x * 256) {
-        const int c0 = cp0[k];
-        const double4 b4 = reinterpret_cast<const double4 *>(basis)[k];
-        const double b[4] = {b4.x, b4.y, b4.z, b4.w};
-        const double2 o = reinterpret_cast<const double2 *>(obs)[k];
-        const double *L = circ ? lm_tab + 3 * circ[k] : lm + 3 * k;
-        const double Lx = L[0], Ly = L[1], Lz = L[2];
-        c += SO3 ? ecb_residual_so3<false>(intr, rot + 4 * (size_t) c0, trans + 3 * (size_t) c0, b, o.x, o.y, Lx, Ly, Lz, radius,
-                                           huber, nullptr).cost
-                 : ecb_residual<false>(intr, rot + 4 * (size_t) c0, trans + 3 * (size_t) c0, b, o.x, o.y, Lx, Ly, Lz, radius, huber,
-                                       nullptr).cost;
+        int c0;
+        double b[4], L[3];
+        double2 o;
+        rv.load(k, c0, b, o, L);
+        c += SO3 ? ecb_residual_so3<false>(intr, rot + 4 * (size_t) c0, trans + 3 * (size_t) c0, b, o.x, o.y, L[0], L[1], L[2],
+                                           radius, huber, nullptr).cost
+                 : ecb_residual<false>(intr, rot + 4 * (size_t) c0, trans + 3 * (size_t) c0, b, o.x, o.y, L[0], L[1], L[2], radius,
+                                       huber, nullptr).cost;
     }
     sh[threadIdx.x] = c;
     __syncthreads();
@@ -710,7 +725,7 @@ __device__ __forceinline__ int reassoc_one(const ReassocArgs &r, const float4 *L
     const uint32_t e = a.ev_xyp[i];
     if (e & ECB_PIX_INVALID) return -1;
     const double ou = (double) ECB_PIX_X(e), ov = (double) ECB_PIX_Y(e);
-    // the pose as the record's evaluation sees it: the basis of k_assoc_write, ecb_pose_eval as in k_reprojection
+    // the pose as the record's evaluation sees it: the basis of k_assoc_write, ecb_pose_eval as in the reprojection metric
     const double *kn = a.knots + a.knot_off[s];
     const int sp = find_span_guess(kn, a.ncp[s] + 4, u);
     double N[4], q[4], t[3], X[3];
@@ -805,31 +820,137 @@ __global__ void __launch_bounds__(AS_THREADS) k_reassoc_count(const ReassocArgs 
     }
 }
 
-// ---------------------------------------------------------------------------- residual report ----
-// k_residuals   the loads and the residual call of k_cost, storing the raw residual r_k (board units) instead of the cost
-// k_group_keys  group of every record (key) and its index; a stable radix sort of (key, index) keeps record order per group
-// k_group_start lower bounds of every group in the sorted keys (as k_span_start)
-// k_group_reduce one block per group, fixed shape: thread-strided partials in record order, then a shared-memory tree
+// ------------------------------------------------------------------- residual and reprojection reports ----
+// Both reports evaluate one value per record (a metric) and the same statistics per group:
+// k_record_report  the loads of k_cost and the metric of record k -> out[k]; optional count of the NaN values (integer atomics,
+//                  one per warp)
+// k_group_keys     group of every record (key) and its index; a stable radix sort of (key, index) keeps record order per group
+// k_group_start    lower bounds of every group in the sorted keys (as k_span_start)
+// k_group_stats    one block per group, fixed shape: thread-strided partials in record order, then a shared-memory tree
 constexpr int RG_THREADS = 256;
 
-template <bool SO3>
-__global__ void __launch_bounds__(256) k_residuals(const double *__restrict__ obs, const double *__restrict__ lm,
-                                                   const int *__restrict__ circ, const double *__restrict__ lm_tab,
-                                                   const double *__restrict__ basis, const int *__restrict__ cp0, int64_t n,
-                                                   const double *__restrict__ params, int total_cp, double radius, double huber,
-                                                   double *__restrict__ out) {
+// (s, c) += v with the rounding error of s + v kept in c (Neumaier); Knuth's TwoSum, exact without branches
+ECB_HD void ecb_comp_add(double &s, double &c, double v) {
+    const double t = s + v, bp = t - s;
+    c += (s - (t - bp)) + (v - bp);
+    s = t;
+}
+
+// The statistics of one group: add() one record's value, merge() another partial, result() the group.  Host and device: the
+// total over the groups is the tree's merge.
+struct ResidualStats {  // raw residuals r (board units)
+    using Group = ecb_residual_group;
+    Group q;
+    double huber;
+    ECB_HD void add(double v) {
+        // the Huber expressions of ecb_residual.h: rho = r^2 inside the band, 2 delta |r| - delta^2 outside
+        const double a2 = huber * huber, s2 = v * v;
+        double rho = s2;
+        if (s2 > a2) {
+            rho = 2.0 * huber * fabs(v) - a2;
+            ++q.n_downweighted;
+        }
+        ++q.count;
+        q.sum += v;
+        q.sum_sq += s2;
+        q.max_abs = fmax(q.max_abs, fabs(v));
+        q.cost += 0.5 * rho;
+    }
+    ECB_HD void merge(const ResidualStats &o) {
+        q.count += o.q.count;
+        q.n_downweighted += o.q.n_downweighted;
+        q.sum += o.q.sum;
+        q.sum_sq += o.q.sum_sq;
+        q.max_abs = fmax(q.max_abs, o.q.max_abs);
+        q.cost += o.q.cost;
+    }
+    ECB_HD Group result() const { return q; }
+};
+
+// Reprojection errors e (pixels): valid records counted and summed, NaN ones counted in n_invalid only.  e is signed and its
+// sums cancel (the mean error of a group is near 0 when the fit is good), so sum e is compensated (Neumaier per thread, TwoSum
+// in the tree): it keeps the relative accuracy of the sum itself instead of n eps sum |e|.
+struct ReprojectionStats {
+    using Group = ecb_reprojection_group;
+    Group q;
+    double comp;  // rounding error of q.sum
+    ECB_HD void add(double v) {
+        if (isnan(v)) {
+            ++q.n_invalid;
+            return;
+        }
+        ++q.count;
+        ecb_comp_add(q.sum, comp, v);
+        q.sum_sq += v * v;
+        q.max_abs = fmax(q.max_abs, fabs(v));
+    }
+    ECB_HD void merge(const ReprojectionStats &o) {
+        q.count += o.q.count;
+        q.n_invalid += o.q.n_invalid;
+        comp += o.comp;
+        ecb_comp_add(q.sum, comp, o.q.sum);
+        q.sum_sq += o.q.sum_sq;
+        q.max_abs = fmax(q.max_abs, o.q.max_abs);
+    }
+    ECB_HD Group result() const {
+        Group g = q;
+        g.sum = q.sum + comp;
+        return g;
+    }
+};
+
+// The metrics: at() takes them from the context and the host intrinsics, stats() starts a group of their statistics.
+struct ResidualMetric {  // r_k = ||X_w - L|| - radius, the raw residual of ecb_residual (board units)
+    using Stats = ResidualStats;
+    static constexpr const char *report = "residual";
+    double radius, huber;
+    static ResidualMetric at(const CostState *st, const double *) { return {st->radius, st->huber}; }
+    Stats stats() const { return Stats{{}, huber}; }
+    template <int SO3>
+    __device__ __forceinline__ double operator()(const double *intr, const double *rot, const double *trans, const double b[4],
+                                                 double2 o, const double L[3]) const {
+        return SO3 ? ecb_residual_so3<false>(intr, rot, trans, b, o.x, o.y, L[0], L[1], L[2], radius, huber, nullptr).raw
+                   : ecb_residual<false>(intr, rot, trans, b, o.x, o.y, L[0], L[1], L[2], radius, huber, nullptr).raw;
+    }
+};
+
+struct RimReprojectionMetric {  // e_k in pixels: the record's pose (ecb_pose_eval), then ecb_rim_reprojection; NaN when not projectable
+    using Stats = ReprojectionStats;
+    static constexpr const char *report = "reprojection";
+    double radius;
+    EcbFold fold;
+    static RimReprojectionMetric at(const CostState *st, const double *intr) { return {st->radius, ecb_inverse_radial_fold_host(intr + 4)}; }
+    Stats stats() const { return Stats{{}, 0.0}; }
+    template <int SO3>
+    __device__ __forceinline__ double operator()(const double *intr, const double *rot, const double *trans, const double b[4],
+                                                 double2 o, const double L[3]) const {
+        double q[4], t[3];
+        ecb_pose_eval(rot, trans, b, SO3, q, t);
+        return ecb_rim_reprojection(intr, fold, q, t, o.x, o.y, L[0], L[1], L[2], radius);
+    }
+};
+
+template <int SO3, class Metric>
+__global__ void __launch_bounds__(256) k_record_report(const double *__restrict__ obs, const double *__restrict__ lm,
+                                                       const int *__restrict__ circ, const double *__restrict__ lm_tab,
+                                                       const double *__restrict__ basis, const int *__restrict__ cp0, int64_t n,
+                                                       const double *__restrict__ params, int total_cp, const Metric m,
+                                                       double *__restrict__ out, unsigned long long *__restrict__ n_invalid) {
     const double *intr = params, *rot = params + 9, *trans = params + 9 + 4 * (size_t) total_cp;
+    const RecordView rv{obs, lm, circ, lm_tab, basis, cp0};
+    unsigned bad = 0;
     for (int64_t k = (int64_t) blockIdx.x * 256 + threadIdx.x; k < n; k += (int64_t) gridDim.x * 256) {
-        const int c0 = cp0[k];
-        const double4 b4 = reinterpret_cast<const double4 *>(basis)[k];
-        const double b[4] = {b4.x, b4.y, b4.z, b4.w};
-        const double2 o = reinterpret_cast<const double2 *>(obs)[k];
-        const double *L = circ ? lm_tab + 3 * circ[k] : lm + 3 * k;
-        const double Lx = L[0], Ly = L[1], Lz = L[2];
-        out[k] = SO3 ? ecb_residual_so3<false>(intr, rot + 4 * (size_t) c0, trans + 3 * (size_t) c0, b, o.x, o.y, Lx, Ly, Lz, radius,
-                                               huber, nullptr).raw
-                     : ecb_residual<false>(intr, rot + 4 * (size_t) c0, trans + 3 * (size_t) c0, b, o.x, o.y, Lx, Ly, Lz, radius, huber,
-                                           nullptr).raw;
+        int c0;
+        double b[4], L[3];
+        double2 o;
+        rv.load(k, c0, b, o, L);
+        const double v = m.template operator()<SO3>(intr, rot + 4 * (size_t) c0, trans + 3 * (size_t) c0, b, o, L);
+        out[k] = v;
+        bad += isnan(v) ? 1u : 0u;
+    }
+    if (n_invalid) {
+        bad = __reduce_add_sync(0xffffffffu, bad);
+        if ((threadIdx.x & 31) == 0 && bad) atomicAdd(n_invalid, (unsigned long long) bad);
     }
 }
 
@@ -875,56 +996,22 @@ __global__ void k_group_start(const uint64_t *__restrict__ skey, int64_t n, int 
     start[g] = lo;
 }
 
-__global__ void __launch_bounds__(RG_THREADS) k_group_reduce(const double *__restrict__ r, const uint32_t *__restrict__ sidx,
-                                                             const int64_t *__restrict__ start, double huber,
-                                                             ecb_residual_group *__restrict__ out) {
-    __shared__ double sh[4][RG_THREADS];
-    __shared__ long long shn[RG_THREADS];
+// s: an empty group of the statistics (carrying their parameters)
+template <class Stats>
+__global__ void __launch_bounds__(RG_THREADS) k_group_stats(const double *__restrict__ v, const uint32_t *__restrict__ sidx,
+                                                            const int64_t *__restrict__ start, Stats s,
+                                                            typename Stats::Group *__restrict__ out) {
+    __shared__ Stats sh[RG_THREADS];
     const int g = blockIdx.x, t = threadIdx.x;
     const int64_t b = start[g], e = start[g + 1];
-    const double a2 = huber * huber;
-    long long ndw = 0;
-    double sum = 0.0, ssq = 0.0, mx = 0.0, cost = 0.0;
-    for (int64_t i = b + t; i < e; i += RG_THREADS) {
-        const double v = r[sidx[i]];
-        // the Huber expressions of ecb_residual.h: rho = r^2 inside the band, 2 delta |r| - delta^2 outside
-        const double s2 = v * v;
-        double rho = s2;
-        if (s2 > a2) {
-            rho = 2.0 * huber * fabs(v) - a2;
-            ++ndw;
-        }
-        sum += v;
-        ssq += s2;
-        mx = fmax(mx, fabs(v));
-        cost += 0.5 * rho;
-    }
-    sh[0][t] = sum;
-    sh[1][t] = ssq;
-    sh[2][t] = mx;
-    sh[3][t] = cost;
-    shn[t] = ndw;
+    for (int64_t i = b + t; i < e; i += RG_THREADS) s.add(v[sidx[i]]);
+    sh[t] = s;
     __syncthreads();
     for (int o = RG_THREADS / 2; o > 0; o >>= 1) {
-        if (t < o) {
-            sh[0][t] += sh[0][t + o];
-            sh[1][t] += sh[1][t + o];
-            sh[2][t] = fmax(sh[2][t], sh[2][t + o]);
-            sh[3][t] += sh[3][t + o];
-            shn[t] += shn[t + o];
-        }
+        if (t < o) sh[t].merge(sh[t + o]);
         __syncthreads();
     }
-    if (t == 0) {
-        ecb_residual_group q;
-        q.count = e - b;
-        q.n_downweighted = shn[0];
-        q.sum = sh[0][0];
-        q.sum_sq = sh[1][0];
-        q.max_abs = sh[2][0];
-        q.cost = sh[3][0];
-        out[g] = q;
-    }
+    if (t == 0) out[g] = sh[0].result();
 }
 
 // ------------------------------------------------------------------------ outlier rejection ----
@@ -932,7 +1019,7 @@ __global__ void __launch_bounds__(RG_THREADS) k_group_reduce(const double *__res
 // k_reject_write  ordered compaction of the kept records into the spare buffers (k_assoc_write's scheme; blocks overlap, so
 //                 not in place)
 struct RejectArgs {
-    const double *r;           // r_k (k_residuals)
+    const double *r;           // r_k (k_record_report)
     double max_abs;
     const uint8_t *drop;       // per key frame, or null
     const double *kf_t;        // the association's stamps (drop != null)
@@ -994,96 +1081,8 @@ __global__ void __launch_bounds__(AS_THREADS) k_reject_write(const uint8_t *__re
     }
 }
 
-// ------------------------------------------------------------------------ reprojection report ----
-// k_reprojection    the loads of k_residuals; the record's pose (ecb_pose_eval), then e_k in pixels (ecb_rim_reprojection), NaN
-//                   when not projectable; optional count of the NaN records (integer atomics, one per warp)
-// k_reproj_reduce   k_group_reduce for e: valid records counted and summed, NaN ones counted in n_invalid only.  e is signed
-//                   and its sums cancel (the mean error of a group is near 0 when the fit is good), so sum e is compensated
-//                   (Neumaier per thread, TwoSum in the tree): it keeps the relative accuracy of the sum itself instead of
-//                   n eps sum |e|
+// ------------------------------------------------------------------------ key-frame reprojection ----
 // k_keyframe_reproj one thread per (key frame, circle): the board point at the key frame's pose, projected
-template <int SO3>
-__global__ void __launch_bounds__(256) k_reprojection(const double *__restrict__ obs, const double *__restrict__ lm,
-                                                      const int *__restrict__ circ, const double *__restrict__ lm_tab,
-                                                      const double *__restrict__ basis, const int *__restrict__ cp0, int64_t n,
-                                                      const double *__restrict__ params, int total_cp, double radius, EcbFold fold,
-                                                      double *__restrict__ out, unsigned long long *__restrict__ n_invalid) {
-    const double *intr = params, *rot = params + 9, *trans = params + 9 + 4 * (size_t) total_cp;
-    unsigned bad = 0;
-    for (int64_t k = (int64_t) blockIdx.x * 256 + threadIdx.x; k < n; k += (int64_t) gridDim.x * 256) {
-        const int c0 = cp0[k];
-        const double4 b4 = reinterpret_cast<const double4 *>(basis)[k];
-        const double b[4] = {b4.x, b4.y, b4.z, b4.w};
-        const double2 o = reinterpret_cast<const double2 *>(obs)[k];
-        const double *L = circ ? lm_tab + 3 * circ[k] : lm + 3 * k;
-        const double Lx = L[0], Ly = L[1], Lz = L[2];
-        double q[4], t[3];
-        ecb_pose_eval(rot + 4 * (size_t) c0, trans + 3 * (size_t) c0, b, SO3, q, t);
-        const double e = ecb_rim_reprojection(intr, fold, q, t, o.x, o.y, Lx, Ly, Lz, radius);
-        out[k] = e;
-        bad += isnan(e) ? 1u : 0u;
-    }
-    if (n_invalid) {
-        bad = __reduce_add_sync(0xffffffffu, bad);
-        if ((threadIdx.x & 31) == 0 && bad) atomicAdd(n_invalid, (unsigned long long) bad);
-    }
-}
-
-// (s, c) += v with the rounding error of s + v kept in c (Neumaier); Knuth's TwoSum, exact without branches
-ECB_HD void ecb_comp_add(double &s, double &c, double v) {
-    const double t = s + v, bp = t - s;
-    c += (s - (t - bp)) + (v - bp);
-    s = t;
-}
-
-__global__ void __launch_bounds__(RG_THREADS) k_reproj_reduce(const double *__restrict__ e, const uint32_t *__restrict__ sidx,
-                                                              const int64_t *__restrict__ start,
-                                                              ecb_reprojection_group *__restrict__ out) {
-    __shared__ double sh[4][RG_THREADS];
-    __shared__ long long shn[RG_THREADS];
-    const int g = blockIdx.x, t = threadIdx.x;
-    const int64_t b = start[g], en = start[g + 1];
-    long long nbad = 0;
-    double sum = 0.0, comp = 0.0, ssq = 0.0, mx = 0.0;
-    for (int64_t i = b + t; i < en; i += RG_THREADS) {
-        const double v = e[sidx[i]];
-        if (isnan(v)) {
-            ++nbad;
-            continue;
-        }
-        ecb_comp_add(sum, comp, v);
-        ssq += v * v;
-        mx = fmax(mx, fabs(v));
-    }
-    sh[0][t] = sum;
-    sh[1][t] = ssq;
-    sh[2][t] = mx;
-    sh[3][t] = comp;
-    shn[t] = nbad;
-    __syncthreads();
-    for (int o = RG_THREADS / 2; o > 0; o >>= 1) {
-        if (t < o) {
-            double s0 = sh[0][t], c0 = sh[3][t] + sh[3][t + o];
-            ecb_comp_add(s0, c0, sh[0][t + o]);
-            sh[0][t] = s0;
-            sh[3][t] = c0;
-            sh[1][t] += sh[1][t + o];
-            sh[2][t] = fmax(sh[2][t], sh[2][t + o]);
-            shn[t] += shn[t + o];
-        }
-        __syncthreads();
-    }
-    if (t == 0) {
-        ecb_reprojection_group q;
-        q.n_invalid = shn[0];
-        q.count = (en - b) - shn[0];
-        q.sum = sh[0][0] + sh[3][0];
-        q.sum_sq = sh[1][0];
-        q.max_abs = sh[2][0];
-        out[g] = q;
-    }
-}
-
 // kf_t[K], circ[K][nc][3] (cx cy r), lm[nc][3] -> proj[K][nc][2], err[K][nc]; the segment and span lookup of k_pose_cov
 template <int SO3>
 __global__ void __launch_bounds__(128) k_keyframe_reproj(const double *__restrict__ kf_t, const double *__restrict__ circ,
@@ -1096,15 +1095,10 @@ __global__ void __launch_bounds__(128) k_keyframe_reproj(const double *__restric
     const double *ci = circ + 3 * i;
     double pu = NAN, pv = NAN, e = NAN;
     const double u = kf_t[kf];
-    int s = 0;
     const double *kn = nullptr;
     int nk = 0;
-    for (; s < sv.n_splines; ++s) {  // EventCalibSpline::time2splineIdx; NaN holds in no range
-        kn = sv.knots + sv.knot_off[s];
-        nk = sv.ncp[s] + 4;
-        if (u >= kn[0] && u <= kn[nk - 1]) break;
-    }
-    if (ci[2] >= 0.0 && s < sv.n_splines) {
+    const int s = sv.segment(u, &kn, &nk);
+    if (ci[2] >= 0.0 && s >= 0) {
         const int span = find_span_dev(kn, nk, u);
         double N[4], q[4], t[3];
         basis_dev(kn, span, u, N);
@@ -1728,26 +1722,33 @@ int ecb_cost_normal_eq(ecb_ctx *ctx, const double *intrinsics, const double *rot
     return ECB_OK;
 }
 
-// ---- residual report ----
-// r_k at the point already uploaded to st->params -> out (device, n_res doubles); async
-static int launch_residuals(ecb_ctx *ctx, CostState *st, double *out) {
+}  // extern "C"
+
+// ---- residual and reprojection reports ----
+// the metric m of every record at the point already uploaded to st->params -> out (device, n_res doubles); d_invalid (optional,
+// zeroed here) counts the NaN values; async
+template <class Metric>
+static int launch_record_report(ecb_ctx *ctx, CostState *st, const Metric &m, double *out, unsigned long long *d_invalid) {
+    if (d_invalid) ECB_CUDA(ctx, cudaMemsetAsync(d_invalid, 0, 8, ctx->stream));
     if (st->n_res == 0) return ECB_OK;
     const int grid = (int) std::min<int64_t>((st->n_res + 255) / 256, (int64_t) ctx->sm_count * 8);
-    (st->so3 ? k_residuals<true> : k_residuals<false>)<<<grid, 256, 0, ctx->stream>>>(
+    (st->so3 ? k_record_report<1, Metric> : k_record_report<0, Metric>)<<<grid, 256, 0, ctx->stream>>>(
         (const double *) st->obs.p, (const double *) st->lm.p, st->use_circ ? (const int *) st->sel_circle.p : nullptr,
         (const double *) st->lm_tab.p, (const double *) st->basis.p, (const int *) st->cp0.p, st->n_res,
-        (const double *) st->params.p, st->total_cp, st->radius, st->huber, out);
+        (const double *) st->params.p, st->total_cp, m, out, d_invalid);
     ECB_LAUNCHED(ctx);
-    return ecb_check(ctx, cudaGetLastError(), "k_residuals");
+    return ecb_check(ctx, cudaGetLastError(), "k_record_report");
 }
 
-int ecb_cost_residuals(ecb_ctx *ctx, const double *intrinsics, const double *rot_cp, const double *trans_cp, double *d_out,
-                       double *h_out) {
+// ecb_cost_residuals and ecb_cost_reprojection_errors
+template <class Metric>
+static int record_report(ecb_ctx *ctx, const double *intrinsics, const double *rot_cp, const double *trans_cp, double *d_out,
+                         double *h_out, int64_t *n_invalid) {
     if (!ctx || !intrinsics || !rot_cp || !trans_cp) return ECB_ERR_ARG;
     if (!ctx->cost) return ecb_fail(ctx, ECB_ERR_STATE, "ecb_cost_setup first");
     cudaSetDevice(ctx->device);
     CostState *st = (CostState *) ctx->cost;
-    if (st->n_res > 0xFFFFFFFFll) return ecb_fail(ctx, ECB_ERR_UNSUPPORTED, "residual report over 2^32 or more records");
+    if (st->n_res > 0xFFFFFFFFll) return ecb_fail(ctx, ECB_ERR_UNSUPPORTED, "%s report over 2^32 or more records", Metric::report);
     int rc;
     if ((rc = upload_params(ctx, st, intrinsics, rot_cp, trans_cp))) return rc;
     double *out = d_out;
@@ -1755,8 +1756,28 @@ int ecb_cost_residuals(ecb_ctx *ctx, const double *intrinsics, const double *rot
         if ((rc = ecb_reserve(ctx, st->rep_r, (size_t) std::max<int64_t>(st->n_res, 1) * 8))) return rc;
         out = (double *) st->rep_r.p;
     }
-    if ((rc = launch_residuals(ctx, st, out))) return rc;
-    if (h_out) return ecb_d2h(ctx, h_out, out, (size_t) st->n_res * 8);
+    unsigned long long *d_invalid = nullptr;
+    if (n_invalid) {
+        if ((rc = ecb_reserve(ctx, st->rep_io, 8))) return rc;
+        d_invalid = (unsigned long long *) st->rep_io.p;
+    }
+    if ((rc = launch_record_report(ctx, st, Metric::at(st, intrinsics), out, d_invalid))) return rc;
+    if (h_out && (rc = ecb_d2h(ctx, h_out, out, (size_t) st->n_res * 8))) return rc;
+    if (n_invalid) {
+        unsigned long long c = 0;
+        if ((rc = ecb_d2h(ctx, &c, d_invalid, 8))) return rc;
+        *n_invalid = (int64_t) c;
+    }
+    return ECB_OK;
+}
+
+// The records come from an association (else ECB_ERR_STATE with the message `none`); with `events`, of the events loaded now;
+// with n_keyframes, over that many key frames (else ECB_ERR_ARG).
+static int check_association(ecb_ctx *ctx, const CostState *st, const char *none, bool events, const int *n_keyframes) {
+    if (!st->assoc) return ecb_fail(ctx, ECB_ERR_STATE, "%s", none);
+    if (events && st->assoc_events_gen != ctx->events_gen) return ecb_fail(ctx, ECB_ERR_STATE, "events were loaded after the association");
+    if (n_keyframes && *n_keyframes != st->assoc_K)
+        return ecb_fail(ctx, ECB_ERR_ARG, "%d key frames given, the association used %d", *n_keyframes, st->assoc_K);
     return ECB_OK;
 }
 
@@ -1772,17 +1793,12 @@ static int group_layout(ecb_ctx *ctx, CostState *st, int by, const double *kf_ti
     memset(&a, 0, sizeof a);
     a.by = by;
     if (by == ECB_RESIDUALS_BY_KEYFRAME || by == ECB_RESIDUALS_BY_CIRCLE) {
-        if (!st->assoc)
-            return ecb_fail(ctx, ECB_ERR_STATE, "residuals of ecb_cost_set_residuals have no key frame or circle: associate first");
-        if (by == ECB_RESIDUALS_BY_KEYFRAME) {
-            if (st->assoc_events_gen != ctx->events_gen)
-                return ecb_fail(ctx, ECB_ERR_STATE, "events were loaded after the association");
-            if (n_keyframes != st->assoc_K)
-                return ecb_fail(ctx, ECB_ERR_ARG, "%d key frames given, the association used %d", n_keyframes, st->assoc_K);
-            *G = st->assoc_K;
-        } else {
-            *G = st->assoc_n_circ;
-        }
+        const bool kf = by == ECB_RESIDUALS_BY_KEYFRAME;
+        int rc;
+        if ((rc = check_association(ctx, st, "residuals of ecb_cost_set_residuals have no key frame or circle: associate first", kf,
+                                    kf ? &n_keyframes : nullptr)))
+            return rc;
+        *G = kf ? st->assoc_K : st->assoc_n_circ;
     } else {
         if (ctx->width <= 0 || ctx->height <= 0) return ecb_fail(ctx, ECB_ERR_STATE, "grouping by sensor cell needs ecb_set_sensor");
         a.width = ctx->width;
@@ -1837,9 +1853,10 @@ static int group_sort(ecb_ctx *ctx, CostState *st, GroupKeyArgs a, int64_t G, co
     return ecb_check(ctx, cudaGetLastError(), "group kernels");
 }
 
-int ecb_cost_residual_groups(ecb_ctx *ctx, const double *intrinsics, const double *rot_cp, const double *trans_cp, int by,
-                             const double *kf_time, int n_keyframes, int cell_px, ecb_residual_group *groups, int cap,
-                             int *n_groups, ecb_residual_group *total) {
+// ecb_cost_residual_groups and ecb_cost_reprojection_groups
+template <class Metric, class Stats = typename Metric::Stats, class Group = typename Stats::Group>
+static int group_report(ecb_ctx *ctx, const double *intrinsics, const double *rot_cp, const double *trans_cp, int by,
+                        const double *kf_time, int n_keyframes, int cell_px, Group *groups, int cap, int *n_groups, Group *total) {
     if (!ctx || !intrinsics || !rot_cp || !trans_cp) return ECB_ERR_ARG;
     cudaSetDevice(ctx->device);
     CostState *st = (CostState *) ctx->cost;
@@ -1850,37 +1867,56 @@ int ecb_cost_residual_groups(ecb_ctx *ctx, const double *intrinsics, const doubl
     if ((rc = group_layout(ctx, st, by, kf_time, n_keyframes, cell_px, groups != nullptr, cap, n_groups, a, &G, &query))) return rc;
     if (query) return ECB_OK;
     const int64_t n = st->n_res;
-    std::vector<ecb_residual_group> h((size_t) G + 1);
-    memset(h.data(), 0, h.size() * sizeof(ecb_residual_group));
+    const Metric m = Metric::at(st, intrinsics);
+    std::vector<Group> h((size_t) G + 1);
+    memset(h.data(), 0, h.size() * sizeof(Group));
     if (n > 0) {
         if ((rc = upload_params(ctx, st, intrinsics, rot_cp, trans_cp))) return rc;
         if ((rc = ecb_reserve(ctx, st->rep_r, (size_t) n * 8))) return rc;
-        if ((rc = ecb_reserve(ctx, st->rep_out, ((size_t) G + 1) * sizeof(ecb_residual_group)))) return rc;
-        if ((rc = launch_residuals(ctx, st, (double *) st->rep_r.p))) return rc;
+        if ((rc = ecb_reserve(ctx, st->rep_out, ((size_t) G + 1) * sizeof(Group)))) return rc;
+        if ((rc = launch_record_report(ctx, st, m, (double *) st->rep_r.p, nullptr))) return rc;
         const uint32_t *sidx = nullptr;
         if ((rc = group_sort(ctx, st, a, G, kf_time, &sidx))) return rc;
-        k_group_reduce<<<(unsigned) (G + 1), RG_THREADS, 0, ctx->stream>>>((const double *) st->rep_r.p, sidx,
-                                                                         (const int64_t *) st->rep_start.p, st->huber,
-                                                                         (ecb_residual_group *) st->rep_out.p);
+        k_group_stats<Stats><<<(unsigned) (G + 1), RG_THREADS, 0, ctx->stream>>>((const double *) st->rep_r.p, sidx,
+                                                                               (const int64_t *) st->rep_start.p, m.stats(),
+                                                                               (Group *) st->rep_out.p);
         ECB_LAUNCHED(ctx);
-        if ((rc = ecb_check(ctx, cudaGetLastError(), "residual group kernels"))) return rc;
-        if ((rc = ecb_d2h(ctx, h.data(), st->rep_out.p, h.size() * sizeof(ecb_residual_group)))) return rc;
+        if ((rc = ecb_check(ctx, cudaGetLastError(), "k_group_stats"))) return rc;
+        if ((rc = ecb_d2h(ctx, h.data(), st->rep_out.p, h.size() * sizeof(Group)))) return rc;
     }
-    memcpy(groups, h.data(), (size_t) G * sizeof(ecb_residual_group));
+    memcpy(groups, h.data(), (size_t) G * sizeof(Group));
     if (total) {  // groups 0 .. G-1 and the records outside every group, in group order
-        ecb_residual_group s;
-        memset(&s, 0, sizeof s);
-        for (const ecb_residual_group &q : h) {
-            s.count += q.count;
-            s.n_downweighted += q.n_downweighted;
-            s.sum += q.sum;
-            s.sum_sq += q.sum_sq;
-            s.max_abs = std::max(s.max_abs, q.max_abs);
-            s.cost += q.cost;
-        }
-        *total = s;
+        Stats s = m.stats();
+        for (const Group &q : h) s.merge(Stats{q});
+        *total = s.result();
     }
     return ECB_OK;
+}
+
+extern "C" {
+
+int ecb_cost_residuals(ecb_ctx *ctx, const double *intrinsics, const double *rot_cp, const double *trans_cp, double *d_out,
+                       double *h_out) {
+    return record_report<ResidualMetric>(ctx, intrinsics, rot_cp, trans_cp, d_out, h_out, nullptr);
+}
+
+int ecb_cost_reprojection_errors(ecb_ctx *ctx, const double *intrinsics, const double *rot_cp, const double *trans_cp,
+                                 double *d_out, double *h_out, int64_t *n_invalid) {
+    return record_report<RimReprojectionMetric>(ctx, intrinsics, rot_cp, trans_cp, d_out, h_out, n_invalid);
+}
+
+int ecb_cost_residual_groups(ecb_ctx *ctx, const double *intrinsics, const double *rot_cp, const double *trans_cp, int by,
+                             const double *kf_time, int n_keyframes, int cell_px, ecb_residual_group *groups, int cap,
+                             int *n_groups, ecb_residual_group *total) {
+    return group_report<ResidualMetric>(ctx, intrinsics, rot_cp, trans_cp, by, kf_time, n_keyframes, cell_px, groups, cap,
+                                         n_groups, total);
+}
+
+int ecb_cost_reprojection_groups(ecb_ctx *ctx, const double *intrinsics, const double *rot_cp, const double *trans_cp, int by,
+                                 const double *kf_time, int n_keyframes, int cell_px, ecb_reprojection_group *groups, int cap,
+                                 int *n_groups, ecb_reprojection_group *total) {
+    return group_report<RimReprojectionMetric>(ctx, intrinsics, rot_cp, trans_cp, by, kf_time, n_keyframes, cell_px, groups, cap,
+                                               n_groups, total);
 }
 
 // ---- outlier rejection ----
@@ -1892,18 +1928,15 @@ int ecb_cost_reject(ecb_ctx *ctx, const double *intrinsics, const double *rot_cp
     if (!ctx->cost) return ecb_fail(ctx, ECB_ERR_STATE, "ecb_cost_setup first");
     cudaSetDevice(ctx->device);
     CostState *st = (CostState *) ctx->cost;
-    if (drop_keyframe) {
-        if (!st->assoc) return ecb_fail(ctx, ECB_ERR_STATE, "residuals of ecb_cost_set_residuals have no key frame: associate first");
-        if (st->assoc_events_gen != ctx->events_gen) return ecb_fail(ctx, ECB_ERR_STATE, "events were loaded after the association");
-        if (n_keyframes != st->assoc_K)
-            return ecb_fail(ctx, ECB_ERR_ARG, "%d key frames given, the association used %d", n_keyframes, st->assoc_K);
-    }
+    int rc;
+    if (drop_keyframe &&
+        (rc = check_association(ctx, st, "residuals of ecb_cost_set_residuals have no key frame: associate first", true, &n_keyframes)))
+        return rc;
     const int64_t n = st->n_res;
     if (n > 0xFFFFFFFFll) return ecb_fail(ctx, ECB_ERR_UNSUPPORTED, "outlier rejection over 2^32 or more records");
     if (n_kept) *n_kept = n;
     if (n_removed) *n_removed = 0;
     if (n == 0) return ECB_OK;
-    int rc;
     const int nb = (int) ((n + AS_THREADS - 1) / AS_THREADS);
     // r_k as ecb_cost_residuals returns it; the association's scratch holds the keep flags, block counts and offsets
     if ((rc = upload_params(ctx, st, intrinsics, rot_cp, trans_cp))) return rc;
@@ -1911,7 +1944,7 @@ int ecb_cost_reject(ecb_ctx *ctx, const double *intrinsics, const double *rot_cp
     if ((rc = ecb_reserve(ctx, st->ev_tag, (size_t) n + 16))) return rc;
     if ((rc = ecb_reserve(ctx, st->ev_cnt, (size_t) nb * 4 + 16))) return rc;
     if ((rc = ecb_reserve(ctx, st->ev_flag, (size_t) nb * 8 + 16))) return rc;
-    if ((rc = launch_residuals(ctx, st, (double *) st->rep_r.p))) return rc;
+    if ((rc = launch_record_report(ctx, st, ResidualMetric::at(st, intrinsics), (double *) st->rep_r.p, nullptr))) return rc;
     RejectArgs a;
     memset(&a, 0, sizeof a);
     a.r = (const double *) st->rep_r.p;
@@ -1988,10 +2021,9 @@ int ecb_cost_reassociate(ecb_ctx *ctx, const double *intrinsics, const double *r
     if (!ctx->cost) return ecb_fail(ctx, ECB_ERR_STATE, "ecb_cost_setup first");
     cudaSetDevice(ctx->device);
     CostState *st = (CostState *) ctx->cost;
-    if (!st->assoc) return ecb_fail(ctx, ECB_ERR_STATE, "the records do not come from an association: associate first");
-    if (st->assoc_events_gen != ctx->events_gen) return ecb_fail(ctx, ECB_ERR_STATE, "events were loaded after the association");
-    if (st->n_res > 0xFFFFFFFFll) return ecb_fail(ctx, ECB_ERR_UNSUPPORTED, "re-association of 2^32 or more records");
     int rc;
+    if ((rc = check_association(ctx, st, "the records do not come from an association: associate first", true, nullptr))) return rc;
+    if (st->n_res > 0xFFFFFFFFll) return ecb_fail(ctx, ECB_ERR_UNSUPPORTED, "re-association of 2^32 or more records");
     const int64_t n = ctx->n_events, n_prev = st->n_res;  // n < 2^32: the association checked it for these events
     const int nb = (int) ((n + AS_THREADS - 1) / AS_THREADS);
     if ((rc = upload_params(ctx, st, intrinsics, rot_cp, trans_cp))) return rc;
@@ -2043,97 +2075,6 @@ int ecb_cost_reassociate(ecb_ctx *ctx, const double *intrinsics, const double *r
 int ecb_inverse_radial_fold(const double *k, double *rho_fold) {
     if (!k || !rho_fold) return ECB_ERR_ARG;
     *rho_fold = ecb_inverse_radial_fold_host(k).rho;
-    return ECB_OK;
-}
-
-// e_k at the point already uploaded to st->params (intrinsics intr on the host, for the fold) -> out; d_invalid (optional,
-// zeroed here) counts the NaN records; async
-static int launch_reprojection(ecb_ctx *ctx, CostState *st, const double *intr, double *out, unsigned long long *d_invalid) {
-    if (d_invalid) ECB_CUDA(ctx, cudaMemsetAsync(d_invalid, 0, 8, ctx->stream));
-    if (st->n_res == 0) return ECB_OK;
-    const EcbFold fold = ecb_inverse_radial_fold_host(intr + 4);
-    const int grid = (int) std::min<int64_t>((st->n_res + 255) / 256, (int64_t) ctx->sm_count * 8);
-    (st->so3 ? k_reprojection<1> : k_reprojection<0>)<<<grid, 256, 0, ctx->stream>>>(
-        (const double *) st->obs.p, (const double *) st->lm.p, st->use_circ ? (const int *) st->sel_circle.p : nullptr,
-        (const double *) st->lm_tab.p, (const double *) st->basis.p, (const int *) st->cp0.p, st->n_res,
-        (const double *) st->params.p, st->total_cp, st->radius, fold, out, d_invalid);
-    ECB_LAUNCHED(ctx);
-    return ecb_check(ctx, cudaGetLastError(), "k_reprojection");
-}
-
-int ecb_cost_reprojection_errors(ecb_ctx *ctx, const double *intrinsics, const double *rot_cp, const double *trans_cp,
-                                 double *d_out, double *h_out, int64_t *n_invalid) {
-    if (!ctx || !intrinsics || !rot_cp || !trans_cp) return ECB_ERR_ARG;
-    if (!ctx->cost) return ecb_fail(ctx, ECB_ERR_STATE, "ecb_cost_setup first");
-    cudaSetDevice(ctx->device);
-    CostState *st = (CostState *) ctx->cost;
-    if (st->n_res > 0xFFFFFFFFll) return ecb_fail(ctx, ECB_ERR_UNSUPPORTED, "reprojection report over 2^32 or more records");
-    int rc;
-    if ((rc = upload_params(ctx, st, intrinsics, rot_cp, trans_cp))) return rc;
-    double *out = d_out;
-    if (!out) {
-        if ((rc = ecb_reserve(ctx, st->rep_r, (size_t) std::max<int64_t>(st->n_res, 1) * 8))) return rc;
-        out = (double *) st->rep_r.p;
-    }
-    unsigned long long *d_invalid = nullptr;
-    if (n_invalid) {
-        if ((rc = ecb_reserve(ctx, st->rep_io, 8))) return rc;
-        d_invalid = (unsigned long long *) st->rep_io.p;
-    }
-    if ((rc = launch_reprojection(ctx, st, intrinsics, out, d_invalid))) return rc;
-    if (h_out && (rc = ecb_d2h(ctx, h_out, out, (size_t) st->n_res * 8))) return rc;
-    if (n_invalid) {
-        unsigned long long c = 0;
-        if ((rc = ecb_d2h(ctx, &c, d_invalid, 8))) return rc;
-        *n_invalid = (int64_t) c;
-    }
-    return ECB_OK;
-}
-
-int ecb_cost_reprojection_groups(ecb_ctx *ctx, const double *intrinsics, const double *rot_cp, const double *trans_cp, int by,
-                                 const double *kf_time, int n_keyframes, int cell_px, ecb_reprojection_group *groups, int cap,
-                                 int *n_groups, ecb_reprojection_group *total) {
-    if (!ctx || !intrinsics || !rot_cp || !trans_cp) return ECB_ERR_ARG;
-    cudaSetDevice(ctx->device);
-    CostState *st = (CostState *) ctx->cost;
-    GroupKeyArgs a;
-    int64_t G = 0;
-    bool query = false;
-    int rc;
-    if ((rc = group_layout(ctx, st, by, kf_time, n_keyframes, cell_px, groups != nullptr, cap, n_groups, a, &G, &query))) return rc;
-    if (query) return ECB_OK;
-    const int64_t n = st->n_res;
-    std::vector<ecb_reprojection_group> h((size_t) G + 1);
-    memset(h.data(), 0, h.size() * sizeof(ecb_reprojection_group));
-    if (n > 0) {
-        if ((rc = upload_params(ctx, st, intrinsics, rot_cp, trans_cp))) return rc;
-        if ((rc = ecb_reserve(ctx, st->rep_r, (size_t) n * 8))) return rc;
-        if ((rc = ecb_reserve(ctx, st->rep_out, ((size_t) G + 1) * sizeof(ecb_reprojection_group)))) return rc;
-        if ((rc = launch_reprojection(ctx, st, intrinsics, (double *) st->rep_r.p, nullptr))) return rc;
-        const uint32_t *sidx = nullptr;
-        if ((rc = group_sort(ctx, st, a, G, kf_time, &sidx))) return rc;
-        k_reproj_reduce<<<(unsigned) (G + 1), RG_THREADS, 0, ctx->stream>>>((const double *) st->rep_r.p, sidx,
-                                                                          (const int64_t *) st->rep_start.p,
-                                                                          (ecb_reprojection_group *) st->rep_out.p);
-        ECB_LAUNCHED(ctx);
-        if ((rc = ecb_check(ctx, cudaGetLastError(), "k_reproj_reduce"))) return rc;
-        if ((rc = ecb_d2h(ctx, h.data(), st->rep_out.p, h.size() * sizeof(ecb_reprojection_group)))) return rc;
-    }
-    memcpy(groups, h.data(), (size_t) G * sizeof(ecb_reprojection_group));
-    if (total) {  // groups 0 .. G-1 and the records outside every group, in group order; sum compensated as in k_reproj_reduce
-        ecb_reprojection_group s;
-        memset(&s, 0, sizeof s);
-        double comp = 0.0;
-        for (const ecb_reprojection_group &q : h) {
-            s.count += q.count;
-            s.n_invalid += q.n_invalid;
-            ecb_comp_add(s.sum, comp, q.sum);
-            s.sum_sq += q.sum_sq;
-            s.max_abs = std::max(s.max_abs, q.max_abs);
-        }
-        s.sum += comp;
-        *total = s;
-    }
     return ECB_OK;
 }
 

@@ -72,15 +72,10 @@ __global__ void __launch_bounds__(POSE_THREADS) k_pose_cov(const double *__restr
     bool valid = false;
     if (k < n) {
         const double u = times[k];
-        int s = 0;
         const double *kn = nullptr;
         int nk = 0;
-        for (; s < sv.n_splines; ++s) {  // EventCalibSpline::time2splineIdx; NaN holds in no range
-            kn = sv.knots + sv.knot_off[s];
-            nk = sv.ncp[s] + 4;
-            if (u >= kn[0] && u <= kn[nk - 1]) break;
-        }
-        valid = s < sv.n_splines;
+        const int s = sv.segment(u, &kn, &nk);
+        valid = s >= 0;
         double out[7], S[6][6];
         if (valid) {
             const int span = find_span_dev(kn, nk, u);

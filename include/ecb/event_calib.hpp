@@ -1017,10 +1017,7 @@ public:
     }
     bool optimize(ecb_lm_summary *summary = nullptr) {  // EventCalibSpline.cpp:115-251
         std::vector<double> rot, trans;
-        for (auto &s : seg_) {
-            rot.insert(rot.end(), s.rot_cp.begin(), s.rot_cp.end());
-            trans.insert(trans.end(), s.trans_cp.begin(), s.trans_cp.end());
-        }
+        flatten(seg_, rot, trans);
         ecb_lm_options opt;
         ecb_lm_default_options(&opt);
         opt.rotation_model = useSO3_ ? 1 : 0;
@@ -1057,10 +1054,7 @@ public:
     static int covarianceAt(ecb_ctx *ctx, const std::vector<int32_t> &n_cp, const std::array<double, 9> &intr,
                             const std::vector<Segment> &seg, const void *d_packed, int64_t n_residuals_total, Covariance &out) {
         std::vector<double> rot, trans;
-        for (auto &s : seg) {
-            rot.insert(rot.end(), s.rot_cp.begin(), s.rot_cp.end());
-            trans.insert(trans.end(), s.trans_cp.begin(), s.trans_cp.end());
-        }
+        flatten(seg, rot, trans);
         const size_t n = trans.size() * 2;  // 6 C
         out.band.assign(n * 24, 0.0);
         out.cross.assign(9 * n, 0.0);
@@ -1089,28 +1083,12 @@ public:
         return residualGroupsAt(ev_->ctx, intr_, seg_, kfTime_, by, cellPx, groups, total);
     }
     static int residualsAt(ecb_ctx *ctx, const std::array<double, 9> &intr, const std::vector<Segment> &seg, std::vector<double> &r) {
-        std::vector<double> rot, trans;
-        flatten(seg, rot, trans);
-        int64_t n = 0;
-        int rc = ecb_cost_layout(ctx, nullptr, nullptr, &n, nullptr);
-        if (rc != ECB_OK) return rc;
-        r.assign((size_t) n, 0.0);
-        return ecb_cost_residuals(ctx, intr.data(), rot.data(), trans.data(), nullptr, n > 0 ? r.data() : nullptr);
+        return recordReportAt(ctx, intr, seg, false, r, nullptr);
     }
     static int residualGroupsAt(ecb_ctx *ctx, const std::array<double, 9> &intr, const std::vector<Segment> &seg,
                                 const std::vector<double> &kfTime, int by, int cellPx, std::vector<ecb_residual_group> &groups,
                                 ecb_residual_group *total) {
-        std::vector<double> rot, trans;
-        flatten(seg, rot, trans);
-        const double *kf = kfTime.empty() ? nullptr : kfTime.data();
-        int ng = 0;
-        int rc = ecb_cost_residual_groups(ctx, intr.data(), rot.data(), trans.data(), by, kf, (int) kfTime.size(), cellPx, nullptr, 0,
-                                          &ng, nullptr);
-        if (rc != ECB_OK) return rc;
-        groups.assign((size_t) ng, ecb_residual_group{});
-        ecb_residual_group dummy;
-        return ecb_cost_residual_groups(ctx, intr.data(), rot.data(), trans.data(), by, kf, (int) kfTime.size(), cellPx,
-                                        ng > 0 ? groups.data() : &dummy, ng, &ng, total);
+        return groupReportAt(ecb_cost_residual_groups, ctx, intr, seg, kfTime, by, cellPx, groups, total);
     }
     // Outlier rejection (ecb_cost_reject) at the current point: removes the records with !(|r| <= maxAbsR) and those of the key
     // frames flagged in dropKeyframe (one flag per key frame of the last associate(); empty: no key-frame criterion).  A following
@@ -1174,28 +1152,12 @@ public:
     }
     static int reprojectionErrorsAt(ecb_ctx *ctx, const std::array<double, 9> &intr, const std::vector<Segment> &seg,
                                     std::vector<double> &e, int64_t *nInvalid) {
-        std::vector<double> rot, trans;
-        flatten(seg, rot, trans);
-        int64_t n = 0;
-        int rc = ecb_cost_layout(ctx, nullptr, nullptr, &n, nullptr);
-        if (rc != ECB_OK) return rc;
-        e.assign((size_t) n, 0.0);
-        return ecb_cost_reprojection_errors(ctx, intr.data(), rot.data(), trans.data(), nullptr, n > 0 ? e.data() : nullptr, nInvalid);
+        return recordReportAt(ctx, intr, seg, true, e, nInvalid);
     }
     static int reprojectionGroupsAt(ecb_ctx *ctx, const std::array<double, 9> &intr, const std::vector<Segment> &seg,
                                     const std::vector<double> &kfTime, int by, int cellPx, std::vector<ecb_reprojection_group> &groups,
                                     ecb_reprojection_group *total) {
-        std::vector<double> rot, trans;
-        flatten(seg, rot, trans);
-        const double *kf = kfTime.empty() ? nullptr : kfTime.data();
-        int ng = 0;
-        int rc = ecb_cost_reprojection_groups(ctx, intr.data(), rot.data(), trans.data(), by, kf, (int) kfTime.size(), cellPx, nullptr,
-                                              0, &ng, nullptr);
-        if (rc != ECB_OK) return rc;
-        groups.assign((size_t) ng, ecb_reprojection_group{});
-        ecb_reprojection_group dummy;
-        return ecb_cost_reprojection_groups(ctx, intr.data(), rot.data(), trans.data(), by, kf, (int) kfTime.size(), cellPx,
-                                            ng > 0 ? groups.data() : &dummy, ng, &ng, total);
+        return groupReportAt(ecb_cost_reprojection_groups, ctx, intr, seg, kfTime, by, cellPx, groups, total);
     }
     // kfCircles[K][n][3] (cx cy r, r < 0 absent) and landmarks[n] as given to ecb_cost_associate
     static int keyframeReprojectionAt(ecb_ctx *ctx, const std::array<double, 9> &intr, const std::vector<Segment> &seg,
@@ -1225,6 +1187,13 @@ public:
     const std::vector<std::array<double, 3>> &landmarks() const { return landmarks_; }
     const std::array<double, 9> &intrinsics() const { return intr_; }
     const std::vector<Segment> &segments() const { return seg_; }
+    // the control points of all segments in order: rotation (4 per point) and translation (3 per point), as the C ABI takes them
+    static void flatten(const std::vector<Segment> &seg, std::vector<double> &rot, std::vector<double> &trans) {
+        for (auto &s : seg) {
+            rot.insert(rot.end(), s.rot_cp.begin(), s.rot_cp.end());
+            trans.insert(trans.end(), s.trans_cp.begin(), s.trans_cp.end());
+        }
+    }
     // EventCalibSpline.hpp:286-303: index of the segment whose knot range holds t, else -1
     int time2splineIdx(double t) const { return time2splineIdx(seg_, t); }
     static int time2splineIdx(const std::vector<Segment> &seg, double t) {
@@ -1336,11 +1305,35 @@ private:
     std::vector<std::array<double, 3>> landmarks_;  // ... and its board points
     double step_, radius_;
     bool useSO3_ = false;
-    static void flatten(const std::vector<Segment> &seg, std::vector<double> &rot, std::vector<double> &trans) {
-        for (auto &s : seg) {
-            rot.insert(rot.end(), s.rot_cp.begin(), s.rot_cp.end());
-            trans.insert(trans.end(), s.trans_cp.begin(), s.trans_cp.end());
-        }
+    // one value per record (ecb_cost_reprojection_errors when pixels, else ecb_cost_residuals) -> out, sized from ecb_cost_layout
+    static int recordReportAt(ecb_ctx *ctx, const std::array<double, 9> &intr, const std::vector<Segment> &seg, bool pixels,
+                              std::vector<double> &out, int64_t *nInvalid) {
+        std::vector<double> rot, trans;
+        flatten(seg, rot, trans);
+        int64_t n = 0;
+        int rc = ecb_cost_layout(ctx, nullptr, nullptr, &n, nullptr);
+        if (rc != ECB_OK) return rc;
+        out.assign((size_t) n, 0.0);
+        double *h = n > 0 ? out.data() : nullptr;
+        return pixels ? ecb_cost_reprojection_errors(ctx, intr.data(), rot.data(), trans.data(), nullptr, h, nInvalid)
+                      : ecb_cost_residuals(ctx, intr.data(), rot.data(), trans.data(), nullptr, h);
+    }
+    // the groups of one report (fn: ecb_cost_residual_groups or ecb_cost_reprojection_groups): the size query, then the filled call
+    template <class Group>
+    static int groupReportAt(int (*fn)(ecb_ctx *, const double *, const double *, const double *, int, const double *, int, int, Group *,
+                                       int, int *, Group *),
+                             ecb_ctx *ctx, const std::array<double, 9> &intr, const std::vector<Segment> &seg,
+                             const std::vector<double> &kfTime, int by, int cellPx, std::vector<Group> &groups, Group *total) {
+        std::vector<double> rot, trans;
+        flatten(seg, rot, trans);
+        const double *kf = kfTime.empty() ? nullptr : kfTime.data();
+        int ng = 0;
+        int rc = fn(ctx, intr.data(), rot.data(), trans.data(), by, kf, (int) kfTime.size(), cellPx, nullptr, 0, &ng, nullptr);
+        if (rc != ECB_OK) return rc;
+        groups.assign((size_t) ng, Group{});
+        Group dummy;
+        return fn(ctx, intr.data(), rot.data(), trans.data(), by, kf, (int) kfTime.size(), cellPx, ng > 0 ? groups.data() : &dummy, ng, &ng,
+                  total);
     }
 };
 inline void EventCalibSpline::printEigenLikeRow(std::ostream &os, const double *v, int n) { printEigenLike(os, v, 1, n); }

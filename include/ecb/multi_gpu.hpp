@@ -211,10 +211,7 @@ public:
                 if (ev_->device[(size_t) g] == ev_->device[(size_t) h])
                     throw std::invalid_argument("ShardedCalibSpline::optimize: the shards must live on distinct devices");
         std::vector<double> rot, trans;  // from the current point: a second optimize() continues from the first solution
-        for (auto &s : segments()) {
-            rot.insert(rot.end(), s.rot_cp.begin(), s.rot_cp.end());
-            trans.insert(trans.end(), s.trans_cp.begin(), s.trans_cp.end());
-        }
+        EventCalibSpline::flatten(segments(), rot, trans);
         std::array<double, 9> intr = intrinsics();
         ecb_lm_options opt;
         ecb_lm_default_options(&opt);
@@ -279,10 +276,7 @@ public:
         if (G == 1) return EventCalibSpline::covarianceAt(ev_->shard[0]->ctx, n_cp_, intrinsics(), segments(), nullptr, 0, out);
         auto ctx = [&](int g) { return ev_->shard[(size_t) g]->ctx; };
         std::vector<double> rot, trans;
-        for (auto &s : segments()) {
-            rot.insert(rot.end(), s.rot_cp.begin(), s.rot_cp.end());
-            trans.insert(trans.end(), s.trans_cp.begin(), s.trans_cp.end());
-        }
+        EventCalibSpline::flatten(segments(), rot, trans);
         const std::array<double, 9> intr = intrinsics();
         std::vector<void *> buf((size_t) G, nullptr), packed((size_t) G, nullptr);
         std::vector<EventCalibSpline::Covariance> cov((size_t) G);
@@ -335,25 +329,7 @@ public:
     // Residual statistics at the current point (EventCalibSpline::residualGroups): every shard reports its own records (one host
     // thread each), the groups are combined in rank order (counts and sums added, max_abs the max).
     int residualGroups(int by, int cellPx, std::vector<ecb_residual_group> &groups, ecb_residual_group *total) const {
-        const int G = (int) sp_.size();
-        std::vector<std::vector<ecb_residual_group>> part((size_t) G);
-        std::vector<ecb_residual_group> tot((size_t) G);
-        std::vector<int> rc((size_t) G, ECB_OK);
-        forEachShard(G, [&](int g) {
-            rc[(size_t) g] = EventCalibSpline::residualGroupsAt(ev_->shard[(size_t) g]->ctx, intrinsics(), segments(),
-                                                                sp_[(size_t) g]->keyframeTimes(), by, cellPx, part[(size_t) g],
-                                                                &tot[(size_t) g]);
-        });
-        for (int g = 0; g < G; ++g)
-            if (rc[(size_t) g] != ECB_OK) return rc[(size_t) g];
-        groups = part[0];
-        ecb_residual_group t = tot[0];
-        for (int g = 1; g < G; ++g) {
-            for (size_t i = 0; i < groups.size(); ++i) EventCalibSpline::accumulateResidualGroup(groups[i], part[(size_t) g][i]);
-            EventCalibSpline::accumulateResidualGroup(t, tot[(size_t) g]);
-        }
-        if (total) *total = t;
-        return ECB_OK;
+        return combineGroups(EventCalibSpline::residualGroupsAt, EventCalibSpline::accumulateResidualGroup, by, cellPx, groups, total);
     }
     // Outlier rejection at the current point: the shards' statistics per key frame combined in rank order (residualGroups), the
     // policy applied once on the host (ecb::outlierRejection with factor k), then every shard removes its records with the same
@@ -410,25 +386,8 @@ public:
     }
     // Reprojection statistics in pixels (EventCalibSpline::reprojectionGroups), combined as residualGroups
     int reprojectionGroups(int by, int cellPx, std::vector<ecb_reprojection_group> &groups, ecb_reprojection_group *total) const {
-        const int G = (int) sp_.size();
-        std::vector<std::vector<ecb_reprojection_group>> part((size_t) G);
-        std::vector<ecb_reprojection_group> tot((size_t) G);
-        std::vector<int> rc((size_t) G, ECB_OK);
-        forEachShard(G, [&](int g) {
-            rc[(size_t) g] = EventCalibSpline::reprojectionGroupsAt(ev_->shard[(size_t) g]->ctx, intrinsics(), segments(),
-                                                                    sp_[(size_t) g]->keyframeTimes(), by, cellPx, part[(size_t) g],
-                                                                    &tot[(size_t) g]);
-        });
-        for (int g = 0; g < G; ++g)
-            if (rc[(size_t) g] != ECB_OK) return rc[(size_t) g];
-        groups = part[0];
-        ecb_reprojection_group t = tot[0];
-        for (int g = 1; g < G; ++g) {
-            for (size_t i = 0; i < groups.size(); ++i) EventCalibSpline::accumulateReprojectionGroup(groups[i], part[(size_t) g][i]);
-            EventCalibSpline::accumulateReprojectionGroup(t, tot[(size_t) g]);
-        }
-        if (total) *total = t;
-        return ECB_OK;
+        return combineGroups(EventCalibSpline::reprojectionGroupsAt, EventCalibSpline::accumulateReprojectionGroup, by, cellPx, groups,
+                             total);
     }
     // Key-frame centres reprojected (EventCalibSpline::keyframeReprojection): they read no records, rank 0's context answers
     int keyframeReprojection(std::vector<double> &proj, std::vector<double> &err, ecb_reprojection_group *total) const {
@@ -443,6 +402,29 @@ public:
     const char *lastError() const { return ecb_last_error(ev_->shard[0]->ctx); }
 
 private:
+    // the groups of one report, every shard its own records (at: EventCalibSpline::residualGroupsAt or reprojectionGroupsAt, one
+    // host thread each), combined in rank order by add
+    template <class Group, class At, class Add>
+    int combineGroups(At at, Add add, int by, int cellPx, std::vector<Group> &groups, Group *total) const {
+        const int G = (int) sp_.size();
+        std::vector<std::vector<Group>> part((size_t) G);
+        std::vector<Group> tot((size_t) G);
+        std::vector<int> rc((size_t) G, ECB_OK);
+        forEachShard(G, [&](int g) {
+            rc[(size_t) g] = at(ev_->shard[(size_t) g]->ctx, intrinsics(), segments(), sp_[(size_t) g]->keyframeTimes(), by, cellPx,
+                                part[(size_t) g], &tot[(size_t) g]);
+        });
+        for (int g = 0; g < G; ++g)
+            if (rc[(size_t) g] != ECB_OK) return rc[(size_t) g];
+        groups = part[0];
+        Group t = tot[0];
+        for (int g = 1; g < G; ++g) {
+            for (size_t i = 0; i < groups.size(); ++i) add(groups[i], part[(size_t) g][i]);
+            add(t, tot[(size_t) g]);
+        }
+        if (total) *total = t;
+        return ECB_OK;
+    }
     void cleanup(std::vector<ecb_lm_device *> &lm, std::vector<void *> &buf) {
         for (size_t g = 0; g < lm.size(); ++g) {
             if (lm[g]) ecb_lm_device_destroy(lm[g]);
