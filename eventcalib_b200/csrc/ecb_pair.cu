@@ -1,8 +1,11 @@
 // k_pair — candidate circles of one window from the kept clusters of both polarities
 // (CirclesEventFrame::extractFeatures, CirclesEventFrame.cpp:137-312) and the batched Kasa circle fit
-// (CirclesEventFrame::fitCircle, CirclesEventFrame.cpp:361-415).  One CTA per window, one warp per
-// positive cluster ("warp-per-cluster batched fit"); k-NN over <= max_k medians by warp arg-min
-// (replaces the nanoflann trees, :160-168; ties -> lowest index).
+// (CirclesEventFrame::fitCircle, CirclesEventFrame.cpp:361-415).  One CTA per window at a time.  Small windows (member
+// pixels staged in shared memory, <= PAIR_LANE_MAX_POINTS points per polarity) run one LANE per positive cluster in
+// 64-thread CTAs: each lane does its cluster's k-NN over the medians (one pass keeping the k smallest keys), Kasa fits and
+// fit errors (one sequential sum, like the reference's fitErr) alone.  Larger windows and kept-cluster tables in global
+// scratch run one WARP per positive cluster in 256-thread CTAs: k-NN by warp arg-min, fit errors summed warp-wide.  The
+// k-NN replaces the nanoflann trees (:160-168); ties -> lowest index.
 //
 // This translation unit is compiled with -fmad=false: the reference is built without FMA contraction
 // (CMakeLists.txt:6-19, x86-64 baseline), and the 3x3 LU / fit-error arithmetic below follows it operation
@@ -26,6 +29,12 @@ constexpr int KNN_MAX = 8;
 #ifndef ECB_PAIR_KM4
 #define ECB_PAIR_KM4 1  // knn_num <= ECB_PAIR_KM: small candidate arrays, a fraction of the unrolled code
 #endif
+// lane per cluster: 64-thread CTAs (~40 positive clusters per DAVIS346 window), 8 of them resident per SM (<= 128 registers)
+constexpr int PAIR_LANE_THREADS = 64, PAIR_LANE_CTAS = 8;
+// one lane sums a cluster's members alone: that pays while clusters are a few dozen members wide (DAVIS346 1.5 ms windows,
+// ~1 200 points and ~30-member clusters per polarity).  Larger problems (VGA 10 ms windows: ~8 800 points, ~180-member
+// clusters) keep a warp per cluster
+constexpr int PAIR_LANE_MAX_POINTS = 4096;
 
 // Eigen PartialPivLU<Matrix3d>::solve, unblocked, first-max pivot [external: Eigen, not in /root/reference]
 // (kept out of line, like warp_abs_dev / warp_knn: k_pair inlined was 180 KB of SASS and stalled on instruction fetch)
@@ -100,6 +109,61 @@ __device__ __noinline__ double warp_abs_dev(const uint32_t *pts, const uint32_t 
     return warp_sum(s);
 }
 
+// sum over the members of |‖p-c‖ - r|, positive members then negative members into one accumulator, then one division
+// (CirclesEventFrame.cpp:209-214,300-305): one lane, one member at a time, over the staged pixels in member-list order
+__device__ __noinline__ double lane_fit_err(const uint32_t *pixP, int szP, const uint32_t *pixN, int szN, double cx, double cy,
+                                            double r) {
+    double e = 0;
+    const int tot = szP + szN;
+#pragma unroll 1  // unrolled by 4 it needs more than the 128 registers of 8 resident CTAs (0.60 -> 0.58 ms at 7 CTAs)
+    for (int i = 0; i < tot; ++i) {
+        const uint32_t p = i < szP ? pixP[i] : pixN[i - szP];
+        const double dx = (double) ECB_PIX_X(p) - cx, dy = (double) ECB_PIX_Y(p) - cy;
+        e += fabs(sqrt(dx * dx + dy * dy) - r);
+    }
+    return e / ((double) tot * r);
+}
+
+// the KM nearest medians of (qx, qy) for one lane, in one pass: keys (squared distance << 32 | index), ascending; unused
+// slots stay ~0.  Every lane walks the same table in the same order, so the median reads are broadcasts.
+template <int KM>
+__device__ __forceinline__ void lane_knn(const int *mx, const int *my, int n, int qx, int qy, unsigned long long (&key)[KM]) {
+#pragma unroll
+    for (int q = 0; q < KM; ++q) key[q] = ~0ull;
+#pragma unroll 1
+    for (int i = 0; i < n; ++i) {
+        const long long dx = qx - mx[i], dy = qy - my[i];
+        const unsigned long long k = ((unsigned long long) (dx * dx + dy * dy) << 32) | (unsigned) i;
+        if (k < key[KM - 1]) {  // keys are unique (they carry the index): ties go to the lower index
+#pragma unroll
+            for (int q = KM - 1; q > 0; --q) key[q] = k < key[q - 1] ? key[q - 1] : (k < key[q] ? k : key[q]);
+            key[0] = k < key[0] ? k : key[0];
+        }
+    }
+}
+
+template <int KM>
+__device__ __forceinline__ unsigned long long pick(const unsigned long long (&key)[KM], int j) {
+    unsigned long long v = key[0];
+#pragma unroll
+    for (int q = 1; q < KM; ++q)
+        if (j == q) v = key[q];
+    return v;
+}
+
+// the reference's `real` cut over the first K neighbours: the first one farther than 4x the nearest or than the gate
+template <int KM>
+__device__ __forceinline__ int knn_real(const unsigned long long (&key)[KM], int K, double gate) {
+    int real = K;
+    const double d0 = (double) (key[0] >> 32);
+#pragma unroll
+    for (int q = KM - 1; q >= 0; --q) {
+        const double d = (double) (key[q] >> 32);
+        if (q < K && (d > d0 * 4 || d > gate)) real = q;
+    }
+    return real;
+}
+
 // k nearest medians (ascending squared distance, ties by index), warp cooperative
 __device__ __noinline__ void warp_knn(const int *mx, const int *my, int n, int qx, int qy, int k, int *idx, unsigned long long *d2) {
     // key = (squared distance, index); the k smallest keys in ascending order.  n <= 64 (the usual case: ~40 kept clusters):
@@ -158,8 +222,10 @@ __device__ __noinline__ void warp_knn(const int *mx, const int *my, int n, int q
 // `no_instruction` the second largest stall at 4.8 per issue): the reference's default is 3 neighbours, and KM = 3 instead of 8
 // together with the un-unrolled member / staging / candidate loops takes the code to 47 KB and the kernel from 1.25 to 0.91 ms
 // (profiles/r2t_pair_code_size.md; folding the two candidate passes into one loop body — 50 KB — was slower again: 1.04 ms)
-template <bool DIRECT, bool FIT, bool GT, int KM = KNN_MAX>
-__global__ void __launch_bounds__(PAIR_THREADS, 4) k_pair(const PairArgs a) {
+template <bool DIRECT, bool FIT, bool GT, int KM, bool LANE>
+__global__ void __launch_bounds__(LANE ? PAIR_LANE_THREADS : PAIR_THREADS, LANE ? PAIR_LANE_CTAS : 4) k_pair(const PairArgs a) {
+    constexpr int NT = LANE ? PAIR_LANE_THREADS : PAIR_THREADS;
+    static_assert(!LANE || (DIRECT && !GT), "lane per cluster reads the staged member pixels");
     extern __shared__ __align__(16) uint32_t sm_dyn[];
     double (*acc_c)[3];
     if constexpr (GT) acc_c = reinterpret_cast<double (*)[3]>(a.gtab + (size_t) blockIdx.x * a.gtab_stride);
@@ -187,12 +253,12 @@ __global__ void __launch_bounds__(PAIR_THREADS, 4) k_pair(const PairArgs a) {
         const int nkn = hn.n_kept, nkp = hp.n_kept;
         __syncthreads();
 #pragma unroll 1
-        for (int i = tid; i < nkn; i += PAIR_THREADS) {
+        for (int i = tid; i < nkn; i += NT) {
             mx[0][i] = kn[i].med_x;
             my[0][i] = kn[i].med_y;
         }
 #pragma unroll 1
-        for (int i = tid; i < nkp; i += PAIR_THREADS) {
+        for (int i = tid; i < nkp; i += NT) {
             mx[1][i] = kp[i].med_x;
             my[1][i] = kp[i].med_y;
             acc_ni[i] = -1;
@@ -207,16 +273,87 @@ __global__ void __launch_bounds__(PAIR_THREADS, 4) k_pair(const PairArgs a) {
             // stage the kept clusters' member pixels once (coalesced list read, gathered pixel read), then every
             // fit-error loop runs out of shared memory
             const int totP = nkp ? kp[nkp - 1].mem_off + kp[nkp - 1].size : 0, totN = nkn ? kn[nkn - 1].mem_off + kn[nkn - 1].size : 0;
-#pragma unroll 1
-            for (int i = tid; i < totN; i += PAIR_THREADS) sm_pix[i] = ptsN[memN[i]];
-#pragma unroll 1
-            for (int i = tid; i < totP; i += PAIR_THREADS) sm_pix[a.smem_cap + i] = ptsP[memP[i]];
+#pragma unroll LANE ? 4 : 1  // a small CTA needs several gathers in flight per thread
+            for (int i = tid; i < totN; i += NT) sm_pix[i] = ptsN[memN[i]];
+#pragma unroll LANE ? 4 : 1
+            for (int i = tid; i < totP; i += NT) sm_pix[a.smem_cap + i] = ptsP[memP[i]];
             memN = sm_pix;
             memP = sm_pix + a.smem_cap;
             __syncthreads();
         }
         const double gate = 4 * a.rthr * a.rthr;
-        if (enough) {
+        if (LANE && enough) {
+            // one lane carries one positive cluster through the whole pipeline: acc_ni[pi] depends on pi alone
+#pragma unroll 1
+            for (int pi = tid; pi < nkp; pi += NT) {
+                if (!FIT) {  // CirclesEventFrame.cpp:282-312
+                    unsigned long long key[1];
+                    lane_knn<1>(mx[0], my[0], nkn, mx[1][pi], my[1][pi], key);
+                    if ((double) (key[0] >> 32) > gate) continue;
+                    const int n0 = (int) (unsigned) key[0];
+                    lane_knn<1>(mx[1], my[1], nkp, mx[0][n0], my[0][n0], key);
+                    if ((int) (unsigned) key[0] != pi) continue;
+                    const double px = mx[1][pi], py = my[1][pi], qx = mx[0][n0], qy = my[0][n0];
+                    const double cx = (px + qx) / 2, cy = (py + qy) / 2;
+                    const double ddx = px - qx, ddy = py - qy;
+                    const double r = sqrt(ddx * ddx + ddy * ddy) / 2;
+                    const double e = lane_fit_err(memP + kp[pi].mem_off, kp[pi].size, memN + kn[n0].mem_off, kn[n0].size, cx, cy, r);
+                    if (e < 10 / r) {
+                        acc_ni[pi] = n0;
+                        acc_c[pi][0] = cx;
+                        acc_c[pi][1] = cy;
+                        acc_c[pi][2] = r;
+                    }
+                } else {  // CirclesEventFrame.cpp:180-281
+                    const int K = min(min(a.knn_num, KM), min(nkn, nkp));
+                    // the best of the first `real` candidate pairs, (pi, key[j]) or (key[j], nsel), as the reference's
+                    // min_element over fitErrs; the (pi, nsel) fit of the first pass is memoised like the reference's fit
+                    // cache (CirclesEventFrame.cpp:199-225)
+                    double b_err = 0, b_cx = 0, b_cy = 0, b_r = 0, m_err = 0, m_cx = 0, m_cy = 0, m_r = 0;
+                    int b_c = 0;
+                    auto best_pair = [&](const unsigned long long (&key)[KM], int real, bool rev, int fixed) {
+#pragma unroll 1
+                        for (int j = 0; j < real; ++j) {
+                            const int c = (int) (unsigned) pick(key, j);
+                            const int p = rev ? c : fixed, n = rev ? fixed : c;
+                            double e, cx, cy, r;
+                            if (rev && p == pi) {  // same pair, same numbers
+                                e = m_err, cx = m_cx, cy = m_cy, r = m_r;
+                            } else {
+                                double m[9];
+#pragma unroll
+                                for (int q = 0; q < 9; ++q) m[q] = kp[p].m[q] + kn[n].m[q];
+                                fit_from_moments(m, (double) (kp[p].size + kn[n].size), cx, cy, r);
+                                const double ddx = (double) mx[1][p] - (double) mx[0][n], ddy = (double) my[1][p] - (double) my[0][n];
+                                const double approx = sqrt(ddx * ddx + ddy * ddy) / 2;
+                                e = r > a.rthr || r > 2 * approx
+                                        ? DBL_MAX
+                                        : lane_fit_err(memP + kp[p].mem_off, kp[p].size, memN + kn[n].mem_off, kn[n].size, cx, cy, r);
+                            }
+                            if (j == 0 || e < b_err) b_err = e, b_cx = cx, b_cy = cy, b_r = r, b_c = c;
+                        }
+                    };
+                    unsigned long long key[KM];
+                    lane_knn<KM>(mx[0], my[0], nkn, mx[1][pi], my[1][pi], key);
+                    int real = knn_real(key, K, gate);
+                    if (real == 0) continue;
+                    best_pair(key, real, false, pi);
+                    if (!(b_err < 2 / b_r)) continue;
+                    const int nsel = b_c;
+                    m_err = b_err, m_cx = b_cx, m_cy = b_cy, m_r = b_r;
+                    lane_knn<KM>(mx[1], my[1], nkp, mx[0][nsel], my[0][nsel], key);
+                    real = knn_real(key, K, gate);
+                    if (real == 0) continue;
+                    best_pair(key, real, true, nsel);
+                    if (b_c == pi) {
+                        acc_ni[pi] = nsel;
+                        acc_c[pi][0] = b_cx;
+                        acc_c[pi][1] = b_cy;
+                        acc_c[pi][2] = b_r;
+                    }
+                }
+            }
+        } else if (!LANE && enough) {
             for (;;) {
                 int pi = 0;
                 if (lane == 0) pi = atomicAdd(&s_next, 1);
@@ -336,7 +473,7 @@ __global__ void __launch_bounds__(PAIR_THREADS, 4) k_pair(const PairArgs a) {
         // ordered compaction (candidates are pushed in ascending pi, CirclesEventFrame.cpp:274-278,306-310)
         uint32_t run = 0;
         double *out = a.cand + (size_t) w * a.cand_stride * 5;
-        for (int c0 = 0; c0 < nkp; c0 += PAIR_THREADS) {
+        for (int c0 = 0; c0 < nkp; c0 += NT) {
             const int pi = c0 + tid;
             const bool ok = enough && pi < nkp && acc_ni[pi] >= 0;
             uint32_t tot;
@@ -508,10 +645,14 @@ __global__ void k_fit(const double *__restrict__ xy, const int64_t *__restrict__
 
 }  // namespace
 
+template <bool LANE>
+static void (*direct_pair_kernel(bool fit, bool small_km))(const PairArgs) {
+    return fit ? (small_km ? k_pair<true, true, false, ECB_PAIR_KM, LANE> : k_pair<true, true, false, KNN_MAX, LANE>)
+               : k_pair<true, false, false, KNN_MAX, LANE>;
+}
+
 int ecb_launch_pair(ecb_ctx *ctx, PairArgs &a) {
     if (a.n_win <= 0) return ECB_OK;
-    int grid = a.n_win < ctx->sm_count * 8 ? a.n_win : ctx->sm_count * 8;
-    if (a.win_counter) grid = std::min(a.n_win, ctx->sm_count * 4);  // the resident CTAs (__launch_bounds__(256, 4))
     // kept-cluster tables: 44 bytes per entry, in shared memory unless there are very many kept clusters; member pixels are
     // staged in shared memory as well when both polarities of the largest window fit next to the tables
     const size_t tab = (((size_t) a.max_k * 44) + 15) & ~(size_t) 15;
@@ -520,6 +661,20 @@ int ecb_launch_pair(ecb_ctx *ctx, PairArgs &a) {
     const bool gt = tab > cap;
     const bool direct = !gt && a.smem_cap > 0 && tab + pix <= cap;
     const size_t smem = gt ? 0 : tab + (direct ? pix : 0);
+    const bool lane = direct && a.smem_cap <= PAIR_LANE_MAX_POINTS;
+    const bool small_km = ECB_PAIR_KM4 && a.knn_num <= ECB_PAIR_KM;
+    void (*kern)(const PairArgs) =
+        gt ? (a.fit_circle ? k_pair<false, true, true, KNN_MAX, false> : k_pair<false, false, true, KNN_MAX, false>)
+           : direct ? (lane ? direct_pair_kernel<true>(a.fit_circle, small_km) : direct_pair_kernel<false>(a.fit_circle, small_km))
+                    : (a.fit_circle ? k_pair<false, true, false, KNN_MAX, false> : k_pair<false, false, false, KNN_MAX, false>);
+    const int nt = lane ? PAIR_LANE_THREADS : PAIR_THREADS;
+    ECB_CUDA(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) cap)  /* constant: race-free */);
+    int grid = a.n_win < ctx->sm_count * 8 ? a.n_win : ctx->sm_count * 8;
+    if (a.win_counter) {  // dynamic hand-out: the resident CTAs
+        int per_sm = 0;
+        ECB_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, nt, smem));
+        grid = std::min(a.n_win, ctx->sm_count * std::max(per_sm, 1));
+    }
     a.gtab = nullptr;
     a.gtab_stride = 0;
     if (gt) {
@@ -529,12 +684,7 @@ int ecb_launch_pair(ecb_ctx *ctx, PairArgs &a) {
         a.gtab = (double *) ctx->pair_tab.p;
     }
     ECB_PROF_BEGIN(ctx, ECB_STAGE_PAIR);
-    void (*kern)(const PairArgs) = gt ? (a.fit_circle ? k_pair<false, true, true> : k_pair<false, false, true>)
-                                   : direct ? (a.fit_circle ? (ECB_PAIR_KM4 && a.knn_num <= ECB_PAIR_KM ? k_pair<true, true, false, ECB_PAIR_KM> : k_pair<true, true, false>)
-                                                            : k_pair<true, false, false>)
-                                            : (a.fit_circle ? k_pair<false, true, false> : k_pair<false, false, false>);
-    ECB_CUDA(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) cap)  /* constant: race-free */);
-    kern<<<grid, PAIR_THREADS, smem, ctx->stream>>>(a);
+    kern<<<grid, nt, smem, ctx->stream>>>(a);
     ECB_PROF_END(ctx, ECB_STAGE_PAIR);
     ECB_LAUNCHED(ctx);
     return ecb_check(ctx, cudaGetLastError(), "k_pair launch");
