@@ -110,7 +110,8 @@ SYMBOLS = ["ecb_ctx_create", "ecb_ctx_destroy", "ecb_last_error", "ecb_launch_co
            "ecb_lm_device_set_exchange", "ecb_lm_device_begin", "ecb_lm_device_iterate", "ecb_lm_device_running",
            "ecb_lm_device_result", "ecb_calibrate_device", "ecb_covariance", "ecb_pose_covariance",
            "ecb_pose_covariance_device", "ecb_cost_residuals", "ecb_cost_residual_groups", "ecb_cost_reject",
-           "ecb_cost_reassociate", "ecb_inverse_radial_fold", "ecb_cost_reprojection_errors", "ecb_cost_reprojection_groups", "ecb_keyframe_reprojection"]
+           "ecb_cost_reassociate", "ecb_inverse_radial_fold", "ecb_cost_reprojection_errors", "ecb_cost_reprojection_groups", "ecb_keyframe_reprojection",
+           "ecb_trajectory_motion", "ecb_trajectory_motion_device", "ecb_motion_covariance", "ecb_motion_covariance_device"]
 
 _lib = None
 
@@ -210,6 +211,10 @@ def load_library():
     lib.ecb_covariance.argtypes = [vp, i32, vp, vp, vp, vp, vp, i64, vp, vp, vp, C.POINTER(CovarianceSummary)]
     lib.ecb_pose_covariance.argtypes = [vp, vp, i64, vp, vp, C.POINTER(C.c_int64)]
     lib.ecb_pose_covariance_device.argtypes = [vp, vp, i64, vp, vp, C.POINTER(C.c_int64)]
+    lib.ecb_trajectory_motion.argtypes = [vp, vp, vp, vp, i64, vp, C.POINTER(C.c_int64)]
+    lib.ecb_trajectory_motion_device.argtypes = [vp, vp, vp, vp, i64, vp, C.POINTER(C.c_int64)]
+    lib.ecb_motion_covariance.argtypes = [vp, vp, i64, vp, vp, C.POINTER(C.c_int64)]
+    lib.ecb_motion_covariance_device.argtypes = [vp, vp, i64, vp, vp, C.POINTER(C.c_int64)]
     _lib = lib
     return lib
 
@@ -727,6 +732,60 @@ class Context:
                                                       C.c_void_p(d_pose) if d_pose else None,
                                                       C.c_void_p(d_cov) if d_cov else None, C.byref(nv) if count else None))
         return nv.value if count else None
+
+    def trajectory_motion(self, rot, trans, times):
+        """Motion of the trajectory at the given times (ecb_trajectory_motion) at the control points rot (4 per point, x y z w)
+        and trans (3 per point), in the layout of cost_eval and the rotation model of this context; needs cost_setup only.
+        Returns a dict: pose (n, 7) = tx ty tz qx qy qz qw, omega (n, 3) body-frame angular velocity in radians per time unit,
+        velocity (n, 3) and acceleration (n, 3) in the world frame, n_valid.  Times outside every segment, and NaN, give NaN
+        rows."""
+        r, tr = (np.ascontiguousarray(v, np.float64) for v in (rot, trans))
+        t = np.ascontiguousarray(np.atleast_1d(times), np.float64)
+        n = len(t)
+        motion = np.empty((n, 16))
+        nv = C.c_int64()
+        self._chk(self.lib.ecb_trajectory_motion(self.h, _ptr(r), _ptr(tr), _ptr(t), n, _ptr(motion), C.byref(nv)))
+        return _motion_dict(motion, nv.value)
+
+    def trajectory_motion_device(self, rot, trans, d_times, n, d_motion, count=True):
+        """ecb_trajectory_motion_device: control points as host arrays, raw device pointers (e.g. torch CUDA tensors'
+        data_ptr()) for n float64 times in and n x 16 motion rows out (the pointer may be 0).  Enqueued on the context's stream;
+        with count=True it waits and returns the number of valid queries, else returns None at once."""
+        r, tr = (np.ascontiguousarray(v, np.float64) for v in (rot, trans))
+        nv = C.c_int64()
+        self._chk(self.lib.ecb_trajectory_motion_device(self.h, _ptr(r), _ptr(tr), C.c_void_p(d_times) if d_times else None,
+                                                        int(n), C.c_void_p(d_motion) if d_motion else None,
+                                                        C.byref(nv) if count else None))
+        return nv.value if count else None
+
+    def motion_covariance(self, times):
+        """Motion of the trajectory and its 9 x 9 covariance over (omega, velocity, acceleration) at the given times
+        (ecb_motion_covariance), at the point and with the Z of the last successful covariance() on this context.  Returns the
+        dict of trajectory_motion plus cov (n, 9, 9).  Not scaled by sigma2."""
+        t = np.ascontiguousarray(np.atleast_1d(times), np.float64)
+        n = len(t)
+        motion, cov = np.empty((n, 16)), np.empty((n, 9, 9))
+        nv = C.c_int64()
+        self._chk(self.lib.ecb_motion_covariance(self.h, _ptr(t), n, _ptr(motion), _ptr(cov), C.byref(nv)))
+        out = _motion_dict(motion, nv.value)
+        out["cov"] = cov
+        return out
+
+    def motion_covariance_device(self, d_times, n, d_motion, d_cov, count=True):
+        """ecb_motion_covariance_device on raw device pointers: n float64 times in, n x 16 motion rows and n x 81 covariances
+        out (either pointer may be 0).  Enqueued on the context's stream; with count=True it waits and returns the number of
+        valid queries, else returns None at once."""
+        nv = C.c_int64()
+        self._chk(self.lib.ecb_motion_covariance_device(self.h, C.c_void_p(d_times) if d_times else None, int(n),
+                                                        C.c_void_p(d_motion) if d_motion else None,
+                                                        C.c_void_p(d_cov) if d_cov else None, C.byref(nv) if count else None))
+        return nv.value if count else None
+
+
+def _motion_dict(motion, n_valid):
+    """the columns of a motion row (ecb_trajectory_motion): pose 7, omega 3, velocity 3, acceleration 3"""
+    return {"pose": motion[:, :7], "omega": motion[:, 7:10], "velocity": motion[:, 10:13], "acceleration": motion[:, 13:16],
+            "n_valid": n_valid}
 
 
 def control_point_covariance(cov, c):

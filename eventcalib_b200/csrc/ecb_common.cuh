@@ -80,6 +80,8 @@ struct ecb_ctx {
     uint32_t const_intrinsics = 0;
     // staging of the host variant of ecb_pose_covariance (ecb_pose_cov.cu)
     DevBuf pose_io;
+    // control points, count and host staging of ecb_trajectory_motion / ecb_motion_covariance (ecb_pose_cov.cu)
+    DevBuf motion_io;
     // incremented by every event load: the residual report by key frame needs the events its association read
     uint64_t events_gen = 0;
 };

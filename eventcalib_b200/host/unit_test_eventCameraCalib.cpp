@@ -53,6 +53,13 @@
 // line (event-to-rim count, RMS, mean, max |e|, invalid count; key-frame-centre count and RMS; rho_fold * fx next to the farthest
 // sensor corner's distorted radius, in pixels) and SavePath/ReprojectionByKeyframe.txt, ReprojectionByCircle.txt and
 // ReprojectionMap.txt (cells of ECB_RESIDUAL_CELL pixels).
+//
+// ECB_TRAJECTORY_MOTION=rate (Hz, a positive finite number) samples the motion of the final trajectory, which the reference does
+// not: SavePath/TrajectoryMotion.txt has one line per stamp t0 + k / rate from the first knot of the first segment to the last
+// knot of the last (stamps in the gaps between segments are skipped): the stamp, the body-frame angular velocity, the world-frame
+// velocity and acceleration, then their 9 standard deviations sqrt(sigma2 Sigma_m,ii) (NaN when the covariance is rank
+// deficient).  A "Trajectory motion:" line gives the sample count, the rate, max |omega| and max |v|.  An invalid value ends the
+// program with exit code 1 before any file or GPU work.
 #include <algorithm>
 #include <cstdio>
 #include <cstdlib>
@@ -159,6 +166,17 @@ int main(int argc, char **argv) {
             return 1;
         }
         residualCell = (int) v;
+    }
+    double motionRate = 0.0;  // checked before any file or GPU work; 0: no motion file
+    if (const char *mr = getenv("ECB_TRAJECTORY_MOTION")) {
+        char *end = nullptr;
+        const double v = strtod(mr, &end);
+        if (end == mr || *end != '\0' || !(v > 0.0) || !std::isfinite(v)) {
+            std::cerr << "ecb: ECB_TRAJECTORY_MOTION must be a positive finite number (samples per second), got '" << mr << "'"
+                      << std::endl;
+            return 1;
+        }
+        motionRate = v;
     }
     Settings fs;
     if (!fs.open(argv[1])) {
@@ -657,7 +675,7 @@ int main(int argc, char **argv) {
         }
         const bool want_cov = getenv("ECB_COVARIANCE") && atoi(getenv("ECB_COVARIANCE")) != 0;
         const bool want_traj_cov = getenv("ECB_TRAJECTORY_COVARIANCE") && atoi(getenv("ECB_TRAJECTORY_COVARIANCE")) != 0;
-        if (want_cov || want_traj_cov) {  // uncertainty of the result (no reference output)
+        if (want_cov || want_traj_cov || motionRate > 0) {  // uncertainty of the result (no reference output)
             EventCalibSpline::Covariance cov;
             const int rc = spline.covariance(cov);
             if (rc == ECB_OK && want_cov) {
@@ -696,6 +714,43 @@ int main(int argc, char **argv) {
                     for (int e = 0; e < 36; ++e) f << " " << cov.summary.sigma2 * pc[36 * k + (size_t) e];
                     f << "\n";
                 }
+            }
+            if (motionRate > 0) {  // the motion of the final trajectory at t0 + k / rate, with its deviations when rc == ECB_OK
+                const auto &seg = spline.segments();
+                const double t0 = seg.front().knots.front(), t1 = seg.back().knots.back();
+                std::ofstream f(std::string(argv[3]) + "/TrajectoryMotion.txt");
+                f << "# motion of the trajectory at t0 + k / rate, rate = " << std::setprecision(17) << motionRate
+                  << " Hz, t0 = the first knot; stamps between segments are skipped\n"
+                  << "# stamp [s], omega_x omega_y omega_z (body frame, rad/s), v_x v_y v_z (world frame, board units/s), a_x a_y a_z "
+                     "(world frame, board units/s^2), then the standard deviations sqrt(sigma2 Sigma_m,ii) of those 9 (NaN without a "
+                     "covariance)\n";
+                const int64_t total = (int64_t) std::floor((t1 - t0) * motionRate) + 1;
+                int64_t samples = 0;
+                double maxW = 0.0, maxV = 0.0;
+                std::vector<double> times, motion, mc;
+                for (int64_t lo = 0; lo < total; lo += (int64_t) 1 << 20) {
+                    times.clear();
+                    for (int64_t k = lo; k < std::min(total, lo + ((int64_t) 1 << 20)); ++k) times.push_back(t0 + (double) k / motionRate);
+                    const int mrc = rc == ECB_OK ? spline.motionCovariance(times, motion, mc) : spline.trajectoryMotion(times, motion);
+                    if (mrc != ECB_OK) {
+                        std::cerr << "ecb: " << spline.lastError() << std::endl;
+                        return 1;
+                    }
+                    for (size_t k = 0; k < times.size(); ++k) {
+                        const double *m = &motion[16 * k];
+                        if (std::isnan(m[0])) continue;  // in a gap between segments
+                        ++samples;
+                        maxW = std::max(maxW, std::sqrt(m[7] * m[7] + m[8] * m[8] + m[9] * m[9]));
+                        maxV = std::max(maxV, std::sqrt(m[10] * m[10] + m[11] * m[11] + m[12] * m[12]));
+                        f << std::fixed << std::setprecision(10) << times[k] << std::defaultfloat << std::setprecision(17);
+                        for (int e = 7; e < 16; ++e) f << " " << m[e];
+                        for (int e = 0; e < 9; ++e)
+                            f << " " << (rc == ECB_OK ? std::sqrt(cov.summary.sigma2 * mc[81 * k + 10 * (size_t) e]) : NAN);
+                        f << "\n";
+                    }
+                }
+                std::cout << "Trajectory motion: " << samples << " samples at " << motionRate << " Hz, max |omega| " << maxW
+                          << " rad/s, max |v| " << maxV << " board units/s" << std::endl;
             }
         }
         spline.saveKeyFrameTrajectoryTUM(std::string(argv[3]) + "/TrajectoryByEvent.txt", stamps);  // eventCameraCalib.cpp:212

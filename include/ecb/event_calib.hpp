@@ -1074,6 +1074,32 @@ public:
         cov.assign(36 * times.size(), 0.0);
         return ecb_pose_covariance(ctx, times.data(), (int64_t) times.size(), pose.data(), cov.data(), n_valid);
     }
+    // Motion of the trajectory (ecb_trajectory_motion) at the current control points: motion[16 n] = tx ty tz qx qy qz qw, body
+    // angular velocity wx wy wz (rad per time unit), world velocity vx vy vz and acceleration ax ay az at each time; NaN rows for
+    // times outside every segment.  ECB_OK, or < 0.
+    int trajectoryMotion(const std::vector<double> &times, std::vector<double> &motion, int64_t *n_valid = nullptr) const {
+        return trajectoryMotionAt(ev_->ctx, seg_, times, motion, n_valid);
+    }
+    static int trajectoryMotionAt(ecb_ctx *ctx, const std::vector<Segment> &seg, const std::vector<double> &times,
+                                  std::vector<double> &motion, int64_t *n_valid) {
+        std::vector<double> rot, trans;
+        flatten(seg, rot, trans);
+        motion.assign(16 * times.size(), 0.0);
+        return ecb_trajectory_motion(ctx, rot.data(), trans.data(), times.data(), (int64_t) times.size(), motion.data(), n_valid);
+    }
+    // The same motion with its covariance (ecb_motion_covariance), after covariance(): cov[81 n] = Sigma_m(t) row major over
+    // (w body frame, v, a world frame).  The covariance is cov.summary.sigma2 Sigma_m.  ECB_OK, or < 0 (ECB_ERR_STATE without a
+    // successful covariance()).
+    int motionCovariance(const std::vector<double> &times, std::vector<double> &motion, std::vector<double> &cov,
+                         int64_t *n_valid = nullptr) const {
+        return motionCovarianceAt(ev_->ctx, times, motion, cov, n_valid);
+    }
+    static int motionCovarianceAt(ecb_ctx *ctx, const std::vector<double> &times, std::vector<double> &motion,
+                                  std::vector<double> &cov, int64_t *n_valid) {
+        motion.assign(16 * times.size(), 0.0);
+        cov.assign(81 * times.size(), 0.0);
+        return ecb_motion_covariance(ctx, times.data(), (int64_t) times.size(), motion.data(), cov.data(), n_valid);
+    }
     // How well the model fits (ecb_cost_residuals / ecb_cost_residual_groups) at the current point, where optimize() left it.
     // r is the raw residual ||X_w - L|| - radius: a distance on the board plane in the units of the board points, NOT pixels.
     // residuals: r of every record in the association's order.  residualGroups: statistics per key frame (the stamps of the last

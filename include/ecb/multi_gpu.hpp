@@ -326,6 +326,15 @@ public:
                        int64_t *n_valid = nullptr) const {
         return EventCalibSpline::poseCovarianceAt(ev_->shard[0]->ctx, times, pose, cov, n_valid);
     }
+    // Motion of the trajectory at the current control points (EventCalibSpline::trajectoryMotion) and, after covariance(), with
+    // its covariance (EventCalibSpline::motionCovariance): rank 0's context answers.
+    int trajectoryMotion(const std::vector<double> &times, std::vector<double> &motion, int64_t *n_valid = nullptr) const {
+        return EventCalibSpline::trajectoryMotionAt(ev_->shard[0]->ctx, segments(), times, motion, n_valid);
+    }
+    int motionCovariance(const std::vector<double> &times, std::vector<double> &motion, std::vector<double> &cov,
+                         int64_t *n_valid = nullptr) const {
+        return EventCalibSpline::motionCovarianceAt(ev_->shard[0]->ctx, times, motion, cov, n_valid);
+    }
     // Residual statistics at the current point (EventCalibSpline::residualGroups): every shard reports its own records (one host
     // thread each), the groups are combined in rank order (counts and sums added, max_abs the max).
     int residualGroups(int by, int cellPx, std::vector<ecb_residual_group> &groups, ecb_residual_group *total) const {

@@ -494,6 +494,33 @@ int ecb_covariance(ecb_ctx *ctx, int n_splines, const int32_t *n_cp, const doubl
 int ecb_pose_covariance(ecb_ctx *ctx, const double *times, int64_t n, double *pose, double *cov, int64_t *n_valid);
 int ecb_pose_covariance_device(ecb_ctx *ctx, const double *d_times, int64_t n, double *d_pose, double *d_cov, int64_t *n_valid);
 
+/* ---- motion of the trajectory: angular velocity, velocity and acceleration at any time on the spline ------------------------
+ * For a time t, s, i and the pose (R^, t^) are those of ecb_pose_covariance.  Nd_j and Ndd_j are the first and second time
+ * derivatives of the cubic basis functions N_{i-3..i} on the same clamped knots (NURBS-book A2.3, BsplineReal::dersBasisFuns).
+ *   w_b  body-frame angular velocity, R^T dR/dt = [w_b]x, radians per time unit: quaternion model 2 vec(q~^* (x) q~') / |q~|^2
+ *        with q~ = sum N_j Q_j, q~' = sum Nd_j Q_j; SO(3) model sum_k b'_k (E_{k+1} .. E_3)^T d_k with E_k = Exp(b_k d_k), d_k =
+ *        Log(R_{k-1}^-1 R_k) and b' the cumulative sum of Nd.
+ *   v_w  = sum Nd_j T_j (world frame, translation units per time unit); a_w = sum Ndd_j T_j (per time unit squared).
+ *   motion[n][16] = tx ty tz qx qy qz qw (the pose of ecb_pose_covariance, bit for bit), wx wy wz, vx vy vz, ax ay az.
+ *   cov[n][81] = Sigma_m(t) = J Z_blk J^T over (w_b, v_w, a_w), row major, exactly symmetric.  J (9 x 24) is the derivative with
+ *   respect to the tangent parameters of control points i-3 .. i in the order and rotation model of ecb_covariance: per control
+ *   point j a block d w_b / d delta_j, Nd_j I3 and Ndd_j I3.  No sigma^2 scaling, as for ecb_pose_covariance.
+ * Every output pointer may be NULL.  A time outside every segment, or NaN, gives a NaN row and is not counted in *n_valid.
+ * n == 0 is valid, n < 0 returns ECB_ERR_ARG.  A query's output does not depend on the batch it is in.  FP64.
+ * The host variants take host arrays (staged through device buffers); the _device variants take device arrays and are
+ * asynchronous on the context's stream unless n_valid (a host pointer, may be NULL) is asked for.
+ * ecb_trajectory_motion[_device]: the motion at the control points rot_cp / trans_cp (host arrays, layout of ecb_cost_eval),
+ * in the rotation model of the context; needs ecb_cost_setup only (ECB_ERR_STATE before it), no covariance. */
+int ecb_trajectory_motion(ecb_ctx *ctx, const double *rot_cp, const double *trans_cp, const double *times, int64_t n,
+                          double *motion, int64_t *n_valid);
+int ecb_trajectory_motion_device(ecb_ctx *ctx, const double *rot_cp, const double *trans_cp, const double *d_times, int64_t n,
+                                 double *d_motion, int64_t *n_valid);
+/* ecb_motion_covariance[_device]: the motion and Sigma_m at the x of the last successful ecb_covariance on ctx, with its Z; the
+ * ECB_ERR_STATE rules of ecb_pose_covariance. */
+int ecb_motion_covariance(ecb_ctx *ctx, const double *times, int64_t n, double *motion, double *cov, int64_t *n_valid);
+int ecb_motion_covariance_device(ecb_ctx *ctx, const double *d_times, int64_t n, double *d_motion, double *d_cov,
+                                 int64_t *n_valid);
+
 #ifdef __cplusplus
 }
 #endif
