@@ -55,6 +55,17 @@ class CovarianceSummary(C.Structure):
                 ("dimension", C.c_int32), ("deficient_index", C.c_int32)]
 
 
+class GyroCalibration(C.Structure):
+    """ecb_gyro_calibration: camera-gyroscope rotation, time offset and bias with their covariance"""
+    _fields_ = [("q_gc", C.c_double * 4), ("offset", C.c_double), ("bias", C.c_double * 3), ("cov", C.c_double * 49),
+                ("std", C.c_double * 7), ("sigma2", C.c_double), ("cost", C.c_double), ("rms", C.c_double),
+                ("scan_offset", C.c_double), ("n_used", C.c_int64), ("n_unused", C.c_int64), ("iterations", C.c_int32),
+                ("termination", C.c_int32), ("n_params", C.c_int32), ("status", C.c_int32)]
+
+
+GYRO_OK, GYRO_TOO_FEW_SAMPLES, GYRO_OFFSET_AT_EDGE, GYRO_RANK_DEFICIENT = 0, 1, 2, 3
+
+
 class ResidualGroup(C.Structure):
     """ecb_residual_group: statistics of a group of raw residuals r (board units, not pixels)"""
     _fields_ = [("count", C.c_int64), ("n_downweighted", C.c_int64), ("sum", C.c_double), ("sum_sq", C.c_double),
@@ -111,7 +122,8 @@ SYMBOLS = ["ecb_ctx_create", "ecb_ctx_destroy", "ecb_last_error", "ecb_launch_co
            "ecb_lm_device_result", "ecb_calibrate_device", "ecb_covariance", "ecb_pose_covariance",
            "ecb_pose_covariance_device", "ecb_cost_residuals", "ecb_cost_residual_groups", "ecb_cost_reject",
            "ecb_cost_reassociate", "ecb_inverse_radial_fold", "ecb_cost_reprojection_errors", "ecb_cost_reprojection_groups", "ecb_keyframe_reprojection",
-           "ecb_trajectory_motion", "ecb_trajectory_motion_device", "ecb_motion_covariance", "ecb_motion_covariance_device"]
+           "ecb_trajectory_motion", "ecb_trajectory_motion_device", "ecb_motion_covariance", "ecb_motion_covariance_device",
+           "ecb_gyro_calibrate"]
 
 _lib = None
 
@@ -215,6 +227,7 @@ def load_library():
     lib.ecb_trajectory_motion_device.argtypes = [vp, vp, vp, vp, i64, vp, C.POINTER(C.c_int64)]
     lib.ecb_motion_covariance.argtypes = [vp, vp, i64, vp, vp, C.POINTER(C.c_int64)]
     lib.ecb_motion_covariance_device.argtypes = [vp, vp, i64, vp, vp, C.POINTER(C.c_int64)]
+    lib.ecb_gyro_calibrate.argtypes = [vp, vp, vp, i64, C.c_double, i32, C.POINTER(GyroCalibration), vp, vp]
     _lib = lib
     return lib
 
@@ -780,6 +793,40 @@ class Context:
                                                         C.c_void_p(d_motion) if d_motion else None,
                                                         C.c_void_p(d_cov) if d_cov else None, C.byref(nv) if count else None))
         return nv.value if count else None
+
+    def gyro_calibrate(self, rot, gyro, max_offset, n_offsets):
+        """Camera-gyroscope calibration (ecb_gyro_calibrate) at the rotation control points rot (4 per point, x y z w, layout of
+        cost_eval, rotation model of this context); needs cost_setup only.  gyro (n, 4) = t wx wy wz: gyroscope stamps (time
+        units of the knots) and readings (rad per time unit, gyroscope frame).  Model w_g = R_gc w_c(t + offset) + bias; the
+        offset is searched on n_offsets (odd) points over [-max_offset, max_offset] (max_offset 0 with n_offsets 1: held at 0),
+        then refined with the rotation and the bias by least squares.  Returns a dict: ok, status (GYRO_*), message (when not
+        ok), q_gc (x y z w), R_gc (3, 3), offset, bias, cov (7, 7) over (rotation tangent, offset, bias), not scaled by sigma2,
+        std, sigma2, cost, rms, scan_offset, offset_grid and offset_cost (the scan), residuals (n, 3) (NaN rows for unused
+        samples), n_used, n_unused, iterations, termination (ECB_LM_* code), n_params.  A failed calibration (too few samples,
+        the scan's minimum at the edge of the grid, a rank-deficient system) gives ok=False with what was computed; other
+        errors raise."""
+        r = np.ascontiguousarray(rot, np.float64)
+        g = np.ascontiguousarray(np.asarray(gyro, np.float64).reshape(-1, 4))
+        n, M = len(g), int(n_offsets)
+        res = np.full((n, 3), np.nan)
+        cost = np.full(max(M, 0), np.nan)
+        s = GyroCalibration()
+        rc = self.lib.ecb_gyro_calibrate(self.h, _ptr(r), _ptr(g), n, float(max_offset), M, C.byref(s), _ptr(cost), _ptr(res))
+        if rc != FAILED:
+            self._chk(rc)
+        q = np.array(s.q_gc)
+        out = {"ok": rc == OK, "status": s.status, "q_gc": q, "offset": s.offset, "bias": np.array(s.bias),
+               "cov": np.array(s.cov).reshape(7, 7), "std": np.array(s.std), "sigma2": s.sigma2, "cost": s.cost, "rms": s.rms,
+               "scan_offset": s.scan_offset, "offset_cost": cost, "residuals": res, "n_used": s.n_used, "n_unused": s.n_unused,
+               "iterations": s.iterations, "termination": s.termination, "n_params": s.n_params,
+               "offset_grid": (max_offset * (2.0 * np.arange(M) - (M - 1)) / (M - 1)) if M > 1 else np.zeros(M)}
+        x, y, z, w = q
+        out["R_gc"] = np.array([[1 - 2 * (y * y + z * z), 2 * (x * y - z * w), 2 * (x * z + y * w)],
+                                [2 * (x * y + z * w), 1 - 2 * (x * x + z * z), 2 * (y * z - x * w)],
+                                [2 * (x * z - y * w), 2 * (y * z + x * w), 1 - 2 * (x * x + y * y)]])
+        if rc == FAILED:
+            out["message"] = self.lib.ecb_last_error(self.h).decode()
+        return out
 
 
 def _motion_dict(motion, n_valid):

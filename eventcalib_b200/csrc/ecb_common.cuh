@@ -82,6 +82,8 @@ struct ecb_ctx {
     DevBuf pose_io;
     // control points, count and host staging of ecb_trajectory_motion / ecb_motion_covariance (ecb_pose_cov.cu)
     DevBuf motion_io;
+    // control points, samples, partial sums and residuals of ecb_gyro_calibrate (ecb_gyro.cu)
+    DevBuf gyro_io;
     // incremented by every event load: the residual report by key frame needs the events its association read
     uint64_t events_gen = 0;
 };

@@ -13,6 +13,7 @@
 //          q q^T part of the normalisation drops out, vec(q^* (x) q) = 0);
 //          SO(3) model (R = R0 E1 E2 E3, E_k = Exp(b_k d_k), d_k = Log(R_{k-1}^-1 R_k), ecb_so3::spline_rotation):
 //          w_b = sum_k b'_k (E_{k+1} .. E3)^T d_k, b' the cumulative sum of Nd as b is of N.
+//   dw_b/dt body angular acceleration (ecb_angular_velocity<true>, for the gyroscope calibration), from N, Nd and Ndd.
 // The covariance of (w_b, v_w, a_w) is Sigma_m(t) = J Z_blk J^T (9 x 9).  J (9 x 24) is the derivative with respect to the tangent
 // parameters of control points i-3 .. i in the order and rotation model of ecb_covariance (per control point: rotation tangent
 // 3, translation 3).  J is sparse: the w_b rows of control point j are a 3 x 3 block B_j = d w_b / d delta_j (zero in the
@@ -109,13 +110,15 @@ ECB_HD void rotate_inv(const Quat<S> &q, S w[3]) {
     w[2] = w[2] - 2.0 * (q.w * c2) + 2.0 * e2;
 }
 
-// quaternion model: w = 2 vec(q~^* (x) q~') / |q~|^2; vec(a (x) b) = a_w b_v + b_w a_v + a_v x b_v with a = q~^* = (-q~_v, q~_w)
-template <class S>
-ECB_HD void omega_quat(const Quat<S> R[4], const double N[4], const double Nd[4], S w[3]) {
-    S p[4], d[4];
+// quaternion model: w = 2 vec(q~^* (x) q~') / |q~|^2; vec(a (x) b) = a_w b_v + b_w a_v + a_v x b_v with a = q~^* = (-q~_v, q~_w).
+// DOT: also wd = dw/dt = 2 vec(q~^* (x) q~'') / |q~|^2 - 2 (q~ . q~') / |q~|^2 w (vec(q~'^* (x) q~') = 0), q~'' = sum Ndd_j Q_j.
+template <class S, bool DOT = false>
+ECB_HD void omega_quat(const Quat<S> R[4], const double N[4], const double Nd[4], S w[3], const double *Ndd = nullptr,
+                       S *wd = nullptr) {
+    S p[4], d[4], e[4];
     const S zero = ecb_so3::Lift<S>::of(0.0);
 #pragma unroll
-    for (int c = 0; c < 4; ++c) p[c] = d[c] = zero;
+    for (int c = 0; c < 4; ++c) p[c] = d[c] = e[c] = zero;
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
         const S Rc[4] = {R[j].x, R[j].y, R[j].z, R[j].w};
@@ -123,6 +126,7 @@ ECB_HD void omega_quat(const Quat<S> R[4], const double N[4], const double Nd[4]
         for (int c = 0; c < 4; ++c) {
             p[c] = p[c] + N[j] * Rc[c];
             d[c] = d[c] + Nd[j] * Rc[c];
+            if constexpr (DOT) e[c] = e[c] + Ndd[j] * Rc[c];
         }
     }
     const S n2 = p[0] * p[0] + p[1] * p[1] + p[2] * p[2] + p[3] * p[3];
@@ -130,23 +134,43 @@ ECB_HD void omega_quat(const Quat<S> R[4], const double N[4], const double Nd[4]
     w[0] = s * (p[3] * d[0] - d[3] * p[0] - (p[1] * d[2] - p[2] * d[1]));
     w[1] = s * (p[3] * d[1] - d[3] * p[1] - (p[2] * d[0] - p[0] * d[2]));
     w[2] = s * (p[3] * d[2] - d[3] * p[2] - (p[0] * d[1] - p[1] * d[0]));
+    if constexpr (DOT) {
+        const S f = (p[0] * d[0] + p[1] * d[1] + p[2] * d[2] + p[3] * d[3]) * s;
+        wd[0] = s * (p[3] * e[0] - e[3] * p[0] - (p[1] * e[2] - p[2] * e[1])) - f * w[0];
+        wd[1] = s * (p[3] * e[1] - e[3] * p[1] - (p[2] * e[0] - p[0] * e[2])) - f * w[1];
+        wd[2] = s * (p[3] * e[2] - e[3] * p[2] - (p[0] * e[1] - p[1] * e[0])) - f * w[2];
+    }
 }
 
-// SO(3) model: w_1 = b'_1 d_1, w_k = E_k^T w_{k-1} + b'_k d_k, w_b = w_3 (= sum_k b'_k (E_{k+1} .. E3)^T d_k)
-template <class S>
-ECB_HD void omega_so3(const Quat<S> R[4], const double beta[3], const double dbeta[3], S w[3]) {
+// SO(3) model: w_1 = b'_1 d_1, w_k = E_k^T w_{k-1} + b'_k d_k, w_b = w_3 (= sum_k b'_k (E_{k+1} .. E3)^T d_k).
+// DOT: also wd = dw/dt from d(E_k^T)/dt = -[b'_k d_k]x E_k^T: wd_1 = b''_1 d_1, wd_k = E_k^T wd_{k-1} + (E_k^T w_{k-1}) x (b'_k d_k)
+// + b''_k d_k, b'' the cumulative sum of Ndd (Sommer et al., CVPR 2020).
+template <class S, bool DOT = false>
+ECB_HD void omega_so3(const Quat<S> R[4], const double beta[3], const double dbeta[3], S w[3], const double *ddbeta = nullptr,
+                      S *wd = nullptr) {
 #pragma unroll
     for (int k = 1; k <= 3; ++k) {
         S d[3];
         ecb_so3::so3_log(ecb_so3::qmul(ecb_so3::qinv(R[k - 1]), R[k]), d);
         if (k > 1) {
             const S bd[3] = {beta[k - 1] * d[0], beta[k - 1] * d[1], beta[k - 1] * d[2]};
-            rotate_inv(ecb_so3::so3_exp(bd), w);
+            const Quat<S> E = ecb_so3::so3_exp(bd);
+            rotate_inv(E, w);
+            if constexpr (DOT) {
+                const S v[3] = {dbeta[k - 1] * d[0], dbeta[k - 1] * d[1], dbeta[k - 1] * d[2]};
+                rotate_inv(E, wd);
+                wd[0] = wd[0] + (w[1] * v[2] - w[2] * v[1]) + ddbeta[k - 1] * d[0];
+                wd[1] = wd[1] + (w[2] * v[0] - w[0] * v[2]) + ddbeta[k - 1] * d[1];
+                wd[2] = wd[2] + (w[0] * v[1] - w[1] * v[0]) + ddbeta[k - 1] * d[2];
+            }
 #pragma unroll
             for (int c = 0; c < 3; ++c) w[c] = w[c] + dbeta[k - 1] * d[c];
         } else {
 #pragma unroll
             for (int c = 0; c < 3; ++c) w[c] = dbeta[0] * d[c];
+            if constexpr (DOT)
+#pragma unroll
+                for (int c = 0; c < 3; ++c) wd[c] = ddbeta[0] * d[c];
         }
     }
 }
@@ -224,4 +248,24 @@ ECB_HD void ecb_motion_jacobian(const double *Q, const double N[4], const double
     for (int r = 0; r < 3; ++r)
 #pragma unroll
         for (int k = 0; k < 3; ++k) B[r][k] = om[r].d[k];
+}
+
+// Body angular velocity w (bit for bit ecb_motion_eval's: the same omega_quat / omega_so3) and, with DOT, its time derivative wd
+// (body angular acceleration, radians per time unit squared) from the rotation control points Q and N / Nd / Ndd of
+// ecb_ders_basis; so3 as for ecb_motion_eval.  Without DOT, Ndd and wd are not read.
+template <bool DOT>
+ECB_HD void ecb_angular_velocity(const double *Q, const double N[4], const double Nd[4], const double Ndd[4], int so3, double w[3],
+                                 double wd[3]) {
+    ecb_so3::Quat<double> R[4];
+#pragma unroll
+    for (int j = 0; j < 4; ++j) R[j] = ecb_so3::Quat<double>{Q[4 * j], Q[4 * j + 1], Q[4 * j + 2], Q[4 * j + 3]};
+    if (so3) {
+        double beta[3], dbeta[3], ddbeta[3];
+        ecb_so3::cumulative_basis(N, beta);
+        ecb_so3::cumulative_basis(Nd, dbeta);
+        if constexpr (DOT) ecb_so3::cumulative_basis(Ndd, ddbeta);
+        ecb_motion::omega_so3<double, DOT>(R, beta, dbeta, w, ddbeta, wd);
+    } else {
+        ecb_motion::omega_quat<double, DOT>(R, N, Nd, w, Ndd, wd);
+    }
 }

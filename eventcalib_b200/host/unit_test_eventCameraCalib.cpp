@@ -60,6 +60,14 @@
 // velocity and acceleration, then their 9 standard deviations sqrt(sigma2 Sigma_m,ii) (NaN when the covariance is rank
 // deficient).  A "Trajectory motion:" line gives the sample count, the rate, max |omega| and max |v|.  An invalid value ends the
 // program with exit code 1 before any file or GPU work.
+//
+// ECB_GYRO=path calibrates a gyroscope against the final trajectory, which the reference does not.  The file has one sample per
+// line, "t wx wy wz" (s, rad/s; further columns, e.g. an accelerometer, are ignored; lines starting with '#' and blank lines are
+// skipped).  ECB_GYRO_MAX_OFFSET=seconds (finite, >= 0, default 0.05) bounds the time offset, scanned on 1001 points (held at 0
+// when it is 0).  The model is w_g = R_gc w_c(t + offset) + bias (ecb_gyro_calibrate).  SavePath/CameraGyroscope.txt gets the
+// estimate, its standard deviations and the scan curve, and a "Camera-gyroscope:" line is printed.  A failed calibration (too
+// few samples, the offset at the edge of the search window, rotation about one axis only) is reported on stderr and writes no
+// file.  A missing or malformed file, or an invalid offset, ends the program with exit code 1 before any file or GPU work.
 #include <algorithm>
 #include <cstdio>
 #include <cstdlib>
@@ -177,6 +185,36 @@ int main(int argc, char **argv) {
             return 1;
         }
         motionRate = v;
+    }
+    std::vector<double> gyro;  // t wx wy wz per sample; read and checked before any file or GPU work
+    double gyroMaxOffset = 0.05;
+    if (const char *gp = getenv("ECB_GYRO")) {
+        if (const char *mo = getenv("ECB_GYRO_MAX_OFFSET")) {
+            char *end = nullptr;
+            const double v = strtod(mo, &end);
+            if (end == mo || *end != '\0' || !(v >= 0.0) || !std::isfinite(v)) {
+                std::cerr << "ecb: ECB_GYRO_MAX_OFFSET must be a finite number >= 0 (seconds), got '" << mo << "'" << std::endl;
+                return 1;
+            }
+            gyroMaxOffset = v;
+        }
+        std::ifstream gf(gp);
+        if (!gf.is_open()) {
+            std::cerr << "ecb: ECB_GYRO: cannot open '" << gp << "'" << std::endl;
+            return 1;
+        }
+        std::string line;
+        for (long no = 1; std::getline(gf, line); ++no) {
+            const size_t b = line.find_first_not_of(" \t\r");
+            if (b == std::string::npos || line[b] == '#') continue;
+            std::istringstream ls(line);
+            double v[4];
+            if (!(ls >> v[0] >> v[1] >> v[2] >> v[3])) {
+                std::cerr << "ecb: ECB_GYRO: line " << no << " of '" << gp << "' is not \"t wx wy wz\" (4 numbers)" << std::endl;
+                return 1;
+            }
+            gyro.insert(gyro.end(), v, v + 4);
+        }
     }
     Settings fs;
     if (!fs.open(argv[1])) {
@@ -751,6 +789,44 @@ int main(int argc, char **argv) {
                 }
                 std::cout << "Trajectory motion: " << samples << " samples at " << motionRate << " Hz, max |omega| " << maxW
                           << " rad/s, max |v| " << maxV << " board units/s" << std::endl;
+            }
+        }
+        if (getenv("ECB_GYRO")) {  // camera-gyroscope calibration at the final control points (no reference output)
+            const int nOff = gyroMaxOffset > 0.0 ? 1001 : 1;
+            ecb_gyro_calibration g;
+            std::vector<double> offCost;
+            const int grc = spline.calibrateGyroscope(gyro, gyroMaxOffset, nOff, g, &offCost);
+            if (grc == ECB_FAILED) {
+                std::cerr << "ecb: no camera-gyroscope calibration: " << spline.lastError() << std::endl;
+            } else if (grc != ECB_OK) {
+                std::cerr << "ecb: " << spline.lastError() << std::endl;
+                return 1;
+            } else {
+                const double x = g.q_gc[0], y = g.q_gc[1], z = g.q_gc[2], w = g.q_gc[3];
+                const double R[9] = {1 - 2 * (y * y + z * z), 2 * (x * y - z * w), 2 * (x * z + y * w),
+                                     2 * (x * y + z * w), 1 - 2 * (x * x + z * z), 2 * (y * z - x * w),
+                                     2 * (x * z - y * w), 2 * (y * z + x * w), 1 - 2 * (x * x + y * y)};
+                const double angle = 2.0 * std::atan2(std::sqrt(x * x + y * y + z * z), std::fabs(w)) * 180.0 / M_PI;
+                std::ofstream f(std::string(argv[3]) + "/CameraGyroscope.txt");
+                f << std::setprecision(17)
+                  << "# camera-gyroscope calibration: w_g(t) = R_gc w_c(t + offset) + bias + noise\n"
+                  << "# w_c: body-frame angular velocity of the calibrated trajectory (camera frame, rad/s); w_g: gyroscope reading "
+                     "(gyroscope frame, rad/s); R_gc rotates camera-frame vectors into the gyroscope frame (q_gc x y z w, R_gc row "
+                     "major); gyroscope stamp t is event time t + offset; offset, scan_offset in s; bias, rms in rad/s; rotation_std "
+                     "in rad (gyroscope frame); sigma2 in (rad/s)^2\n"
+                  << "q_gc " << x << " " << y << " " << z << " " << w << "\nR_gc";
+                for (double v : R) f << " " << v;
+                f << "\nrotation_std " << g.std[0] << " " << g.std[1] << " " << g.std[2] << "\noffset " << g.offset
+                  << "\noffset_std " << g.std[3] << "\nbias " << g.bias[0] << " " << g.bias[1] << " " << g.bias[2] << "\nbias_std "
+                  << g.std[4] << " " << g.std[5] << " " << g.std[6] << "\nrms " << g.rms << "\nsigma2 " << g.sigma2 << "\nn_used "
+                  << g.n_used << "\nn_unused " << g.n_unused << "\nscan_offset " << g.scan_offset << "\niterations " << g.iterations
+                  << "\ntermination " << g.termination << "\n# scan: offset d_m (s), mean (|w_c(t + d_m)| - |w_g|)^2 ((rad/s)^2)\n";
+                for (int m = 0; m < nOff; ++m)
+                    f << (nOff > 1 ? gyroMaxOffset * (double) (2 * m - (nOff - 1)) / (double) (nOff - 1) : 0.0) << " " << offCost[m]
+                      << "\n";
+                std::cout << "Camera-gyroscope: offset " << 1e3 * g.offset << " ms (+- " << 1e3 * g.std[3] << "), rotation " << angle
+                          << " deg, bias " << g.bias[0] << " " << g.bias[1] << " " << g.bias[2] << " rad/s, RMS " << g.rms
+                          << " rad/s, " << g.n_used << " samples" << std::endl;
             }
         }
         spline.saveKeyFrameTrajectoryTUM(std::string(argv[3]) + "/TrajectoryByEvent.txt", stamps);  // eventCameraCalib.cpp:212

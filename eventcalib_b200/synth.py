@@ -118,6 +118,18 @@ class Trajectory:
                   + R[:, :, 0] * (self.amp_t[0] * self._sig(t, 0))[:, None] + R[:, :, 1] * (self.amp_t[1] * self._sig(t, 1))[:, None])
         return R, tw
 
+    def _dsig(self, t, k):
+        return (self.w[k][None, :] * np.cos(self.w[k][None, :] * t[:, None] + self.ph[k][None, :])).sum(axis=1)
+
+    def angular_velocity(self, t):
+        """body-frame angular velocity w_b of pose()'s rotation (R_wb^T dR_wb/dt = [w_b]x), rad/s, analytic: for
+        R = Rz(c) Rx(a) Ry(b), w_b = Ry^T Rx^T (c' e_z) + Ry^T (a' e_x) + b' e_y"""
+        t = np.atleast_1d(np.asarray(t, np.float64))
+        a, b = self.amp_r[0] * self._sig(t, 3), self.amp_r[1] * self._sig(t, 4)
+        da, db, dc = self.amp_r[0] * self._dsig(t, 3), self.amp_r[1] * self._dsig(t, 4), self.amp_r[2] * self._dsig(t, 5)
+        ca, sa, cb, sb = np.cos(a), np.sin(a), np.cos(b), np.sin(b)
+        return np.stack([cb * da - sb * ca * dc, sa * dc + db, sb * da + cb * ca * dc], axis=1)
+
     def quat_xyzw(self, t):
         R, tw = self.pose(t)
         q = np.zeros((len(R), 4))
@@ -241,3 +253,13 @@ def tiling_windows(t_begin, t_end, length):
     a = t_begin + np.arange(n) * length
     b = np.nextafter(t_begin + (np.arange(n) + 1) * length, -np.inf)
     return np.stack([a, b], axis=1)
+
+
+def gyro_samples(traj, t0, t1, rate, R_gc=np.eye(3), offset=0.0, bias=(0.0, 0.0, 0.0), noise=0.0, seed=0):
+    """A gyroscope rigidly mounted with the camera of traj: stamps t = t0 + k / rate <= t1 on the gyroscope clock, readings
+    w_g = R_gc w_b(t + offset) + bias + N(0, noise^2) (rad/s, gyroscope frame; R_gc rotates camera-frame vectors into the
+    gyroscope frame, gyroscope stamp t is event time t + offset).  Returns (n, 4) = t wx wy wz."""
+    t = t0 + np.arange(int(np.floor((t1 - t0) * rate)) + 1) / rate
+    w = traj.angular_velocity(t + offset) @ np.asarray(R_gc, np.float64).T + np.asarray(bias, np.float64)
+    w += np.random.default_rng(seed).normal(0.0, noise, w.shape)
+    return np.column_stack([t, w])

@@ -1087,6 +1087,24 @@ public:
         motion.assign(16 * times.size(), 0.0);
         return ecb_trajectory_motion(ctx, rot.data(), trans.data(), times.data(), (int64_t) times.size(), motion.data(), n_valid);
     }
+    // Camera-gyroscope calibration (ecb_gyro_calibrate) at the current control points: gyro[4 n] = t wx wy wz (gyroscope stamps
+    // and readings, rad per time unit), the offset scanned on nOffsets points over [-maxOffset, maxOffset] (nOffsets 1 with
+    // maxOffset 0: held at 0).  offsetCost (nOffsets) and residuals (3 n) are filled when non-null.  ECB_OK, ECB_FAILED with
+    // result.status (too few samples, the scan's minimum at the grid's edge, a rank-deficient system), or < 0.
+    int calibrateGyroscope(const std::vector<double> &gyro, double maxOffset, int nOffsets, ecb_gyro_calibration &result,
+                           std::vector<double> *offsetCost = nullptr, std::vector<double> *residuals = nullptr) const {
+        return calibrateGyroscopeAt(ev_->ctx, seg_, gyro, maxOffset, nOffsets, result, offsetCost, residuals);
+    }
+    static int calibrateGyroscopeAt(ecb_ctx *ctx, const std::vector<Segment> &seg, const std::vector<double> &gyro, double maxOffset,
+                                    int nOffsets, ecb_gyro_calibration &result, std::vector<double> *offsetCost,
+                                    std::vector<double> *residuals) {
+        std::vector<double> rot, trans;
+        flatten(seg, rot, trans);
+        if (offsetCost) offsetCost->assign((size_t) std::max(nOffsets, 0), 0.0);
+        if (residuals) residuals->assign(3 * (gyro.size() / 4), 0.0);
+        return ecb_gyro_calibrate(ctx, rot.data(), gyro.data(), (int64_t) (gyro.size() / 4), maxOffset, nOffsets, &result,
+                                  offsetCost ? offsetCost->data() : nullptr, residuals ? residuals->data() : nullptr);
+    }
     // The same motion with its covariance (ecb_motion_covariance), after covariance(): cov[81 n] = Sigma_m(t) row major over
     // (w body frame, v, a world frame).  The covariance is cov.summary.sigma2 Sigma_m.  ECB_OK, or < 0 (ECB_ERR_STATE without a
     // successful covariance()).

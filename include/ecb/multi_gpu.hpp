@@ -335,6 +335,12 @@ public:
                          int64_t *n_valid = nullptr) const {
         return EventCalibSpline::motionCovarianceAt(ev_->shard[0]->ctx, times, motion, cov, n_valid);
     }
+    // Camera-gyroscope calibration at the current control points (EventCalibSpline::calibrateGyroscope): rank 0's context answers.
+    int calibrateGyroscope(const std::vector<double> &gyro, double maxOffset, int nOffsets, ecb_gyro_calibration &result,
+                           std::vector<double> *offsetCost = nullptr, std::vector<double> *residuals = nullptr) const {
+        return EventCalibSpline::calibrateGyroscopeAt(ev_->shard[0]->ctx, segments(), gyro, maxOffset, nOffsets, result, offsetCost,
+                                                      residuals);
+    }
     // Residual statistics at the current point (EventCalibSpline::residualGroups): every shard reports its own records (one host
     // thread each), the groups are combined in rank order (counts and sums added, max_abs the max).
     int residualGroups(int by, int cellPx, std::vector<ecb_residual_group> &groups, ecb_residual_group *total) const {

@@ -521,6 +521,57 @@ int ecb_motion_covariance(ecb_ctx *ctx, const double *times, int64_t n, double *
 int ecb_motion_covariance_device(ecb_ctx *ctx, const double *d_times, int64_t n, double *d_motion, double *d_cov,
                                  int64_t *n_valid);
 
+/* ---- camera-gyroscope calibration: rotation, time offset and bias from the trajectory's angular velocity ---------------------
+ * Gyroscope sample i: stamp t_i (gyroscope clock, time units of the knots) and reading w_g,i (radians per time unit, gyroscope
+ * frame).  Model, with w_c the body-frame (camera) angular velocity of ecb_trajectory_motion in the context's rotation model:
+ *   w_g,i = R_gc w_c(t_i + d) + b + noise
+ *   R_gc rotates camera-frame vectors into the gyroscope frame; d is the time offset (gyroscope stamp t is event time t + d); b the
+ *   bias (radians per time unit).  Residual r_i = R_gc w_c(t_i + d) + b - w_g,i, cost = 1/2 sum |r_i|^2 (no robust loss).
+ *   Parameters (delta, d, b) with R_gc = Exp(delta) R^_gc (left perturbation, gyroscope frame); Jacobian of r_i
+ *   [ -[R^ w_c]x, R^ dw_c/dt, I3 ].  The trajectory is held fixed: the result is conditional on the spline, whose own
+ *   covariance is not propagated.
+ * Used samples: t_i and w_g,i finite, and t_i - D and t_i + D (D = max_offset) in the same segment (the first whose knot range
+ * holds the time).  The set is fixed for the whole call.  Unsorted stamps are allowed.
+ * 1. Scan: offsets d_m = D (2m - (M-1)) / (M-1), m = 0 .. M-1 (M = n_offsets, odd, d = 0 on the grid; M = 1: d_0 = 0) and
+ *    cost_m = sum_used (|w_c(t_i + d_m)| - |w_g,i|)^2 / n_used (norms: no rotation needed).  scan_offset = d_m of the least cost
+ *    (ties: the lowest m).
+ * 2. Horn's closed-form rotation from the centred cross-covariance of (w_c(t_i + scan_offset), w_g,i), then b = mean w_g -
+ *    R mean w_c.
+ * 3. Levenberg-Marquardt on (delta, d, b), 7 parameters, or 6 when D = 0 (d held at exactly 0): the trust-region rules of
+ *    ecb_lm on a dense Cholesky, with the tolerances and iteration limit of ecb_lm_default_options; the parameter and function
+ *    tolerances are tested after a step is accepted (the last successful step is kept); a candidate with |d| > D is rejected
+ *    like a cost increase.
+ * 4. cov = Z = (J^T J)^-1 at the solution, 7 x 7 row major over (delta, d, b), not scaled (the covariance is sigma2 Z); with 6
+ *    parameters the offset's row and column are 0.  sigma2 = 2 cost / (3 n_used - n_params), std = sqrt(sigma2 diag Z),
+ *    rms = sqrt(sum |r_i|^2 / (3 n_used)).
+ * Sums are deterministic (fixed-order reductions, no floating-point atomics): repeated calls are bit-identical.  FP64.
+ * ECB_FAILED (out->status says why; out is filled as far as it was computed): fewer used samples than parameters
+ * (ECB_GYRO_TOO_FEW_SAMPLES); the scan's least cost at m = 0 or M-1 with M > 1 (ECB_GYRO_OFFSET_AT_EDGE: widen max_offset);
+ * J^T J rank deficient, least relative Cholesky pivot < 1e-12, e.g. motion about one axis only (ECB_GYRO_RANK_DEFICIENT: cov and
+ * std NaN).
+ * rot_cp: rotation control points (layout of ecb_cost_eval); gyro[n][4] = t wx wy wz.  offset_cost[n_offsets] (cost_m) and
+ * residuals[n][3] (r_i at the solution, NaN rows for unused samples) may be NULL.  Needs ecb_cost_setup (ECB_ERR_STATE before it).
+ * ECB_ERR_ARG: ctx, out or rot_cp NULL, n < 0, gyro NULL with n > 0, max_offset NaN, negative or infinite, n_offsets even, < 1 or
+ * > 65535, n_offsets > 1 with max_offset 0, or n_offsets 1 with max_offset > 0. */
+#define ECB_GYRO_OK 0
+#define ECB_GYRO_TOO_FEW_SAMPLES 1
+#define ECB_GYRO_OFFSET_AT_EDGE 2
+#define ECB_GYRO_RANK_DEFICIENT 3
+typedef struct {
+    double q_gc[4];      /* R_gc as x y z w */
+    double offset;       /* d */
+    double bias[3];
+    double cov[49];      /* Z over (delta, d, b), not scaled by sigma2 */
+    double std[7];       /* sqrt(sigma2 diag Z) */
+    double sigma2, cost, rms;
+    double scan_offset;  /* the offset of the scan's least cost */
+    int64_t n_used, n_unused;
+    int32_t iterations, termination;  /* LM iterations and ECB_LM_* code */
+    int32_t n_params, status;         /* 7, or 6 with max_offset = 0; ECB_GYRO_* */
+} ecb_gyro_calibration;
+int ecb_gyro_calibrate(ecb_ctx *ctx, const double *rot_cp, const double *gyro, int64_t n, double max_offset, int32_t n_offsets,
+                       ecb_gyro_calibration *out, double *offset_cost, double *residuals);
+
 #ifdef __cplusplus
 }
 #endif
